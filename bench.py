@@ -19,6 +19,12 @@ The same line carries the second half of BASELINE.json's metric in "topn": top-1
 configs[4] (1 048 576 users x 1 048 576 items, k=128, sharded by user block over the N ranks, no
 collective), measured through lrk_topn with pinned host result buffers (D2H inside the timed region),
 with the tensor-pipe roofline of topn_tc_kernel from CUDA events on its stream.
+--dump-outputs DIR (N=1) writes what the last timed step computed as DIR/<name>.npy, so that two builds can be compared output
+for output on identical seeded inputs: the factors a trainModel() caller reads back after the last timed epoch (P, Q, bu, bi,
+fp32 like the device state), that epoch's loss, and the top-10 lists of the last timed top-N call for a fixed seeded sample of
+users (topn_users / topn_items / topn_scores / topn_counts).  The epochs update the factors with float atomics whose order varies,
+so two runs of one build agree on the factors and the loss only to a tolerance (13 epochs on a B200: factors within 5e-5 of
+each other, biases within 1.2e-2, loss within 1e-5 relative); the top-N lists are bit-identical.
 """
 import argparse
 import csv
@@ -35,6 +41,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True                # the benchmark writes nothing into the tree (it may be read-only)
 
 METRIC = "MF SGD rating-updates/s"
 UNIT = "updates/s"
@@ -45,6 +52,8 @@ E2E_EPOCHS = 10                               # epochs per trainModel() call in 
 # config C4 (BASELINE configs[3]): PMF k=128 on the Netflix shape, pmf-test.properties, DSGD at 2/4/8 GPUs (strong scaling)
 C4_K, C4_LR, C4_REG = 128, 0.01, 0.08
 C4_BYTES_PER_UPDATE = 12 + 4 * C4_K * 4      # SURVEY.md 8(d): 2060 B for k=128 fp32
+DUMP_LIMIT = 64 << 20                         # bytes of --dump-outputs in all
+DUMP_TOPN_USERS, DUMP_SEED = 1 << 15, 0x4C52D0  # the full top-N lists (1M users) exceed DUMP_LIMIT: a fixed sample of users
 
 
 def log(*a):
@@ -320,14 +329,17 @@ def run_ours(args):
     if not os.path.exists(_build.LIB_PATH):
         _build.build()
     capi.load()
+    outputs = {} if args.dump_outputs else None
     if world > 1:
         line = run_c4_dsgd(args, torch, dist, capi, synth, rank, world, local, dev)
     else:
-        line = run_c2_single(args, torch, capi, synth, local, dev)
+        line = run_c2_single(args, torch, capi, synth, local, dev, outputs)
     if not args.no_topn:
-        tn = topn_leg(args, capi, torch, dist, rank, world, local, dev)
+        tn = topn_leg(args, capi, torch, dist, rank, world, local, dev, outputs)
         if rank == 0:
             line["topn"] = tn
+    if outputs is not None:
+        write_outputs(args.dump_outputs, outputs)
     if rank == 0:
         print(json.dumps(line), flush=True)
     if world > 1:
@@ -363,7 +375,19 @@ def timed_epochs(torch, dist, h, world, stream, flush, steps, warmup, hyper, fir
     return total_ms, float(np.mean(kernel_ms)), losses
 
 
-def run_c2_single(args, torch, capi, synth, local, dev):
+def write_outputs(out_dir, outputs):
+    """--dump-outputs: one DIR/<name>.npy per array (float32 or float64)"""
+    total = sum(a.nbytes for a in outputs.values())
+    if total > DUMP_LIMIT:
+        raise RuntimeError("--dump-outputs: %d bytes exceed the %d-byte limit" % (total, DUMP_LIMIT))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in outputs.items():
+        assert a.dtype in (np.float32, np.float64), (name, a.dtype)
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+    log("--dump-outputs: %d arrays, %d bytes in %s" % (len(outputs), total, out_dir))
+
+
+def run_c2_single(args, torch, capi, synth, local, dev, outputs=None):
     d = synth.make_ratings("ml-20m")
     U, I, nnz = d["U"], d["I"], int(d["rowptr"][-1])
     P0, _, bu0, _ = synth.init_factors(U, I, K_FACTORS, 100, True)
@@ -383,6 +407,10 @@ def run_c2_single(args, torch, capi, synth, local, dev):
     total_ms, kms, losses = timed_epochs(torch, None, h, 1, stream, flush, args.steps, 0, (LR, REG, REG, REG_B), args.warmup + 1)
     clocks = sampler.stop()
     launches = h.launch_count() - launches0
+    if outputs is not None:                     # the device state is fp32, so float32 holds the factors exactly
+        gP, gQ, gbu, gbi = h.get_factors()
+        outputs.update(P=gP.astype(np.float32), Q=gQ.astype(np.float32), bu=gbu.astype(np.float32), bi=gbi.astype(np.float32),
+                       loss=np.array([losses[-1]], np.float64))
     value = nnz * args.steps / (total_ms * 1e-3)
     peaks, which = measured_peaks()
     traffic, traffic_how = (None, "skipped (--no-traffic)") if args.no_traffic else ncu_dram_bytes("sgd", "sgd_rating_epoch_kernel", 4)
@@ -715,7 +743,7 @@ def topn_inputs(rank, world):
     return nu, rowptr, col, val, P, Q
 
 
-def topn_leg(args, capi, torch, dist, rank, world, local, dev):
+def topn_leg(args, capi, torch, dist, rank, world, local, dev, outputs=None):
     """top-10 users scored/s on configs[4]; users are sharded by contiguous block over the ranks (strong scaling,
     no collective: every rank holds the full item matrix).  Returns the "topn" object (rank 0) or None."""
     U, I, k, N = TOPN_USERS, TOPN_ITEMS, TOPN_K, TOPN_N
@@ -739,6 +767,10 @@ def topn_leg(args, capi, torch, dist, rank, world, local, dev):
         wall.append(time.perf_counter() - t0)
         stats = h.topn_stats()
         sweep.append(stats["phase_ms"]["sweep"]); dev_ms.append(stats["ms"])
+    if outputs is not None:                     # user and item ids are < 2^24: exact in float32
+        users = np.sort(np.random.default_rng(DUMP_SEED).choice(nu, min(nu, DUMP_TOPN_USERS), replace=False))
+        outputs.update(topn_users=users.astype(np.float32), topn_items=items[users].astype(np.float32),
+                       topn_scores=scores[users].astype(np.float64), topn_counts=counts[users].astype(np.float32))
     t = torch.tensor([float(np.sum(wall))], dtype=torch.float64, device=dev)
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -800,7 +832,13 @@ def main():
     ap.add_argument("--no-base", action="store_true", help="skip the 1-GPU base of the strong-scaling workload (N>1)")
     ap.add_argument("--no-weak", action="store_true", help="skip the weak-scaling ML-20M extra line (N>1)")
     ap.add_argument("--traffic-probe", default="", help="internal: child mode of the ncu traffic probe (sgd | topn)")
+    ap.add_argument("--dump-outputs", default="", metavar="DIR",
+                    help="write what the last timed step computed to DIR/<name>.npy (N=1; see the module docstring)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be >= 1")
+    if args.dump_outputs and (args.impl != "ours" or args.gpus != 1 or dist_env()[1] != 1):
+        ap.error("--dump-outputs covers the one-GPU run of --impl ours")
     if args.traffic_probe:
         traffic_probe(args.traffic_probe)
         return

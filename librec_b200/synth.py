@@ -4,9 +4,11 @@ ML-20M shape: 138 493 users x 26 744 items, 20 000 263 ratings; Netflix shape: 4
 100 480 507 ratings.  User activity is log-normal, item popularity Zipf(1.0), ratings come from a
 planted rank-16 model + biases + noise rounded to half stars, rows are sorted by item (CSR, like
 SequentialAccessSparseMatrix).  Everything is numpy on the host; results are cached under
-$LRK_CACHE (default /tmp/lrk_synth) because generation takes tens of seconds.
+$LRK_CACHE (default lrk_synth-<uid> in the system's temporary directory) because generation takes tens of seconds.
+The default is per user: a machine's other users can neither block the cache nor hand this one their files.
 """
 import os
+import tempfile
 
 import numpy as np
 
@@ -24,7 +26,7 @@ SHAPES = {
 
 
 def _cache_dir():
-    d = os.environ.get("LRK_CACHE", "/tmp/lrk_synth")
+    d = os.environ.get("LRK_CACHE") or os.path.join(tempfile.gettempdir(), "lrk_synth-%d" % os.getuid())
     os.makedirs(d, exist_ok=True)
     return d
 
