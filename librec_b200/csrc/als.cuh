@@ -21,6 +21,7 @@
 #pragma once
 #include "lrk_common.cuh"
 #include "staging.cuh"
+#include "lrk_epoch.cuh"
 
 struct AlsState {
     double* d_val = nullptr;        // weighted train values, CSR order (fp64: the weights are log / affine functions of the rating)
@@ -518,42 +519,40 @@ static int als_epoch(lrk_handle_s* h, float reg_u, float reg_i, double* loss_out
     const bool eals = h->cfg.model == LRK_MODEL_EALS;
     LRK_REQUIRE(h, !eals || a->has_conf, "eALS needs the item confidences: lrk_set_matrix(h, \"eals.confidences\", c)");
     LRK_REQUIRE(h, h->f64_valid, "internal: fp64 masters out of date");
-    cudaStream_t st = h->stream;
-    const int k = h->k;
-    int rc;
-    LRK_CUDA(h, cudaEventRecord(h->ev0, st));
-    if (!eals) {
-        AlsSolveParams p;
-        memset(&p, 0, sizeof p);
-        p.k = k; p.G = a->d_gram;
-        if ((rc = als_gram(h, h->Q64, h->I, nullptr, a->d_gram))) return rc;
-        p.ptr = h->d_rowptr; p.idx = h->d_col; p.w = a->d_val; p.F = h->Q64; p.OUT = h->P64; p.reg = (double)reg_u; p.n_rows = h->U;
-        if ((rc = als_wrmf_side(h, p))) return rc;
-        if ((rc = als_gram(h, h->P64, h->U, nullptr, a->d_gram))) return rc;
-        p.ptr = a->d_colptr; p.idx = a->d_cusers; p.w = a->d_cval; p.F = h->P64; p.OUT = h->Q64; p.reg = (double)reg_i; p.n_rows = h->I;
-        if ((rc = als_wrmf_side(h, p))) return rc;
-    } else {
-        AlsEalsParams p;
-        memset(&p, 0, sizeof p);
-        p.k = k; p.S = a->d_gram; p.conf = a->d_conf; p.pred = a->d_pred; p.tn = a->d_tn; p.td = a->d_td; p.counter = a->d_counter;
-        {
-            const char* env = getenv("LRK_EALS_HEAVY");          // test hook: a small value sends the rows of small matrices down the CTA-per-row path
-            p.heavy = env && atoi(env) > 0 ? atoi(env) : 512;
+    LrkEpoch e;
+    e.enqueue = [&](int) -> int {
+        cudaStream_t st = h->stream;
+        const int k = h->k;
+        int rc;
+        if (!eals) {
+            AlsSolveParams p;
+            memset(&p, 0, sizeof p);
+            p.k = k; p.G = a->d_gram;
+            if ((rc = als_gram(h, h->Q64, h->I, nullptr, a->d_gram))) return rc;
+            p.ptr = h->d_rowptr; p.idx = h->d_col; p.w = a->d_val; p.F = h->Q64; p.OUT = h->P64; p.reg = (double)reg_u; p.n_rows = h->U;
+            if ((rc = als_wrmf_side(h, p))) return rc;
+            if ((rc = als_gram(h, h->P64, h->U, nullptr, a->d_gram))) return rc;
+            p.ptr = a->d_colptr; p.idx = a->d_cusers; p.w = a->d_cval; p.F = h->P64; p.OUT = h->Q64; p.reg = (double)reg_i; p.n_rows = h->I;
+            if ((rc = als_wrmf_side(h, p))) return rc;
+        } else {
+            AlsEalsParams p;
+            memset(&p, 0, sizeof p);
+            p.k = k; p.S = a->d_gram; p.conf = a->d_conf; p.pred = a->d_pred; p.tn = a->d_tn; p.td = a->d_td; p.counter = a->d_counter;
+            {
+                const char* env = getenv("LRK_EALS_HEAVY");          // test hook: a small value sends the rows of small matrices down the CTA-per-row path
+                p.heavy = env && atoi(env) > 0 ? atoi(env) : 512;
+            }
+            if ((rc = als_gram(h, h->Q64, h->I, a->d_conf, a->d_gram))) return rc;
+            p.ptr = h->d_rowptr; p.idx = h->d_col; p.w = a->d_val; p.Fself = h->P64; p.Fother = h->Q64; p.reg = (double)reg_u; p.n_rows = h->U;
+            if ((rc = als_eals_side<false>(h, p))) return rc;
+            if ((rc = als_gram(h, h->P64, h->U, nullptr, a->d_gram))) return rc;
+            p.ptr = a->d_colptr; p.idx = a->d_cusers; p.w = a->d_cval; p.Fself = h->Q64; p.Fother = h->P64; p.reg = (double)reg_i; p.n_rows = h->I;
+            if ((rc = als_eals_side<true>(h, p))) return rc;
         }
-        if ((rc = als_gram(h, h->Q64, h->I, a->d_conf, a->d_gram))) return rc;
-        p.ptr = h->d_rowptr; p.idx = h->d_col; p.w = a->d_val; p.Fself = h->P64; p.Fother = h->Q64; p.reg = (double)reg_u; p.n_rows = h->U;
-        if ((rc = als_eals_side<false>(h, p))) return rc;
-        if ((rc = als_gram(h, h->P64, h->U, nullptr, a->d_gram))) return rc;
-        p.ptr = a->d_colptr; p.idx = a->d_cusers; p.w = a->d_cval; p.Fself = h->Q64; p.Fother = h->P64; p.reg = (double)reg_i; p.n_rows = h->I;
-        if ((rc = als_eals_side<true>(h, p))) return rc;
-    }
-    // keep the fp32 working copies in step (nothing on this path reads them, the scoring entry points use the masters)
-    f64_to_f32_rows_kernel<<<lrk_ceil_div((int64_t)h->U * h->ld, 256), 256, 0, st>>>(h->P64, h->P32, h->U, k, h->ld); LRK_LAUNCH_CHECK(h);
-    f64_to_f32_rows_kernel<<<lrk_ceil_div((int64_t)h->I * h->ld, 256), 256, 0, st>>>(h->Q64, h->Q32, h->I, k, h->ld); LRK_LAUNCH_CHECK(h);
-    LRK_CUDA(h, cudaEventRecord(h->ev1, st));
-    LRK_CUDA(h, cudaStreamSynchronize(st));
-    LRK_CUDA(h, cudaEventElapsedTime(&h->last_epoch_ms, h->ev0, h->ev1));
-    if (loss_out) *loss_out = 0.0;                 // trainModel never assigns `loss` in either class
-    h->epochs_done++;
-    return LRK_OK;
+        // keep the fp32 working copies in step (nothing on this path reads them, the scoring entry points use the masters)
+        f64_to_f32_rows_kernel<<<lrk_ceil_div((int64_t)h->U * h->ld, 256), 256, 0, st>>>(h->P64, h->P32, h->U, k, h->ld); LRK_LAUNCH_CHECK(h);
+        f64_to_f32_rows_kernel<<<lrk_ceil_div((int64_t)h->I * h->ld, 256), 256, 0, st>>>(h->Q64, h->Q32, h->I, k, h->ld); LRK_LAUNCH_CHECK(h);
+        return LRK_OK;
+    };
+    return lrk_epoch(h, e, loss_out);             // loss 0: trainModel never assigns `loss` in either class
 }

@@ -17,6 +17,7 @@
 #include "sgd.cuh"
 #include "sgd_group.cuh"
 #include "dsgd_fused.cuh"
+#include "lrk_epoch.cuh"
 #include <nccl.h>
 #include <dlfcn.h>
 #include <vector>
@@ -83,7 +84,6 @@ struct DsgdState {
     std::vector<int32_t> bounds;        // world+1 item block bounds
     std::vector<int64_t> seg_off;       // world+1 offsets of the COO segments
     std::vector<double> seg_hot_share;  // per segment: largest share one item has of its ratings
-    std::vector<int64_t> bpr_qualify;   // per block: local users with 0 < |row in block| < width (population of bpr_draw_block)
     int32_t max_blk = 0;                // rows of the largest item block
     size_t buf_floats = 0;              // floats per rotating buffer: max_blk*ld + max_blk
     float* qbuf[2] = {nullptr, nullptr};
@@ -174,19 +174,6 @@ static int dsgd_comm_init(lrk_handle_s* h, int rank, int world, const uint8_t* u
     return LRK_OK;
 }
 
-// per (user, block): does the user have at least one and not all items of the block in the train row?  -> qualify[b] = number of
-// such users (the population bpr_draw_block samples from; 0 means the stratum has nobody to draw and must be skipped)
-__global__ void dsgd_bpr_qualify_kernel(const int64_t* __restrict__ rowptr, const int32_t* __restrict__ col, int32_t U,
-                                        const int32_t* __restrict__ bounds, int world, unsigned long long* __restrict__ qualify) {
-    const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (t >= (int64_t)U * world) return;
-    const int32_t u = (int32_t)(t / world);
-    const int b = (int)(t - (int64_t)u * world);
-    const int64_t rb = rowptr[u], re = rowptr[u + 1];
-    const int64_t lo = row_lower_bound(col, rb, re, bounds[b]), hi = row_lower_bound(col, lo, re, bounds[b + 1]);
-    const int64_t len = hi - lo;
-    if (len > 0 && len < (int64_t)(bounds[b + 1] - bounds[b])) atomicAdd(qualify + b, 1ULL);
-}
 // local ratings per item block from the local item degrees (one thread per item)
 __global__ void dsgd_block_counts_kernel(const uint32_t* __restrict__ deg, int32_t I, const int32_t* __restrict__ bounds, int world,
                                          unsigned long long* __restrict__ cnt) {
@@ -241,16 +228,16 @@ static int dsgd_set_train_csr(lrk_handle_s* h, int32_t U, int32_t I, const int64
     w.max_deg = sc.take<uint32_t>(64);
     w.tmp = sc.take<char>(tmp_bytes); w.tmp_bytes = tmp_bytes;
     unsigned long long* d_cnt = sc.take<unsigned long long>((size_t)I);
-    unsigned long long* d_small = sc.take<unsigned long long>(192);        // [0,64) block counts, [64,128) BPR qualify counts, [128] flags
+    unsigned long long* d_small = sc.take<unsigned long long>(128);        // [0,64) block counts, [64] flags
     if (!d_val || !row_of || !keys || !keys2 || !idx || !perm || !w.k32 || !w.v32 || !w.k32_out || !w.sorted_e || !w.deg || !w.item_start ||
         !w.runs || !w.run_base || !w.max_deg || !w.tmp || !d_cnt || !d_small)
         return lrk_fail(h, LRK_ERR_NOMEM, "dsgd_set_train_csr", "scratch arena too small", __FILE__, __LINE__);
-    int* d_flags = reinterpret_cast<int*>(d_small + 128);
+    int* d_flags = reinterpret_cast<int*>(d_small + 64);
     const int nb = lrk_ceil_div(nn, 256), ib = lrk_ceil_div(I, 256);
 
     // validate the shard BEFORE anything indexes by column (same checks and messages as the single-GPU path); the flag is
     // all-reduced so that every rank fails together and nobody is left waiting in a collective
-    LRK_CUDA(h, cudaMemsetAsync(d_small, 0, sizeof(unsigned long long) * 192, st));
+    LRK_CUDA(h, cudaMemsetAsync(d_small, 0, sizeof(unsigned long long) * 128, st));
     if (nnz > 0) {
         LRK_CUDA(h, cudaMemcpyAsync(d_val, val, sizeof(double) * (size_t)nnz, cudaMemcpyHostToDevice, st));
         coo_rows_kernel<<<nb, 256, 0, st>>>(h->d_rowptr, U, nnz, row_of); LRK_LAUNCH_CHECK(h);
@@ -288,12 +275,7 @@ static int dsgd_set_train_csr(lrk_handle_s* h, int32_t U, int32_t I, const int64
     // bucket by item block; inside a block: item-run tiles, then the shuffled rest (staging.cuh, stage_tile_keys)
     s->seg_off.assign((size_t)world + 1, 0);
     s->seg_hot_share.assign((size_t)world, 0.0);
-    s->bpr_qualify.assign((size_t)world, 0);
     dsgd_block_counts_kernel<<<ib, 256, 0, st>>>(h->d_item_deg, I, s->d_bounds, world, d_small); LRK_LAUNCH_CHECK(h);
-    if (h->cfg.model == LRK_MODEL_BPR && U > 0) {
-        dsgd_bpr_qualify_kernel<<<lrk_ceil_div((int64_t)U * world, 256), 256, 0, st>>>(h->d_rowptr, h->d_col, U, s->d_bounds, world, d_small + 64);
-        LRK_LAUNCH_CHECK(h);
-    }
     group_units_release((GroupUnits*)h->group);
     h->group = nullptr;
     const bool want_group = lrk_use_group_kernel(h) && group_order_supported(U, I, nnz, world);
@@ -310,7 +292,7 @@ static int dsgd_set_train_csr(lrk_handle_s* h, int32_t U, int32_t I, const int64
         dsgd_gather_kernel<<<nb, 256, 0, st>>>(perm, keys2, row_of, h->d_col, d_val, s->d_bounds, nnz, h->d_su, h->d_si, h->d_sr);
         LRK_LAUNCH_CHECK(h);
     }
-    unsigned long long small[128];
+    unsigned long long small[64];
     uint32_t md[64] = {0}, last_base = 0, last_runs = 0;
     if (nnz > 0 && !h->group) {
         LRK_CUDA(h, cudaMemcpyAsync(&last_base, w.run_base + (I - 1), sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
@@ -325,7 +307,6 @@ static int dsgd_set_train_csr(lrk_handle_s* h, int32_t U, int32_t I, const int64
     for (int b = 0; b < world; ++b) {
         s->seg_off[(size_t)b + 1] = s->seg_off[(size_t)b] + (int64_t)small[b];
         if (small[b] > 0) s->seg_hot_share[(size_t)b] = (double)md[b] / (double)small[b];
-        s->bpr_qualify[(size_t)b] = (int64_t)small[64 + b];
     }
     if (h->cfg.model == LRK_MODEL_BPR) {
         // BPRRecommender.java:48-58 draws numRates samples per iteration, the user uniformly over ALL users: this rank's share is
@@ -385,7 +366,7 @@ static int dsgd_set_factors(lrk_handle_s* h, const double* P, const double* Q, c
     }
     s->cur = 0; s->cur_block = b;
     s->fused.needs_reset = s->fused.mapped;
-    if (h->cfg.model != LRK_MODEL_BPR) { int rc_n = refresh_user_norm2(h, false); if (rc_n) return rc_n; }
+    if (k_lrk_models[h->cfg.model].damped) { int rc_n = refresh_user_norm2(h, false); if (rc_n) return rc_n; }
     LRK_CUDA(h, cudaStreamSynchronize(st));
     h->prev_loss = -1.0; h->conc_div = 1; h->good_epochs = 0; h->epochs_done = 0;
     h->mu = mu; h->has_factors = true; h->f64_valid = false;
@@ -678,113 +659,87 @@ static int dsgd_epoch(lrk_handle_s* h, float lr, float reg_u, float reg_i, doubl
     DsgdState* s = (DsgdState*)h->dsgd;
     cudaStream_t st = h->stream;
     const int world = h->world, rank = h->rank;
-    // safeguard (lrk_common.cuh): snapshot of what this rank owns at the epoch boundary -- its user block and the
-    // item block it holds; the loss is all-reduced, so every rank takes the same rollback decision
-    const bool biased_ = h->cfg.model == LRK_MODEL_BIASEDMF;
     const bool bpr_ = h->cfg.model == LRK_MODEL_BPR;
-    const size_t np_ = (size_t)h->U * h->ld;
-    {
-        int rc_a;
-        if ((rc_a = lrk_dev_alloc(h, &h->bk_P, np_))) return rc_a;
-        if ((rc_a = lrk_dev_alloc(h, &h->bk_Q, bpr_ ? (size_t)h->I * h->ld : s->buf_floats))) return rc_a;
-        if (biased_ && (rc_a = lrk_dev_alloc(h, &h->bk_bu, (size_t)h->U))) return rc_a;
-    }
-    LRK_CUDA(h, cudaMemcpyAsync(h->bk_P, h->P32, sizeof(float) * np_, cudaMemcpyDeviceToDevice, st));
-    if (bpr_) LRK_CUDA(h, cudaMemcpyAsync(h->bk_Q, h->Q32, sizeof(float) * (size_t)h->I * h->ld, cudaMemcpyDeviceToDevice, st));
-    else LRK_CUDA(h, cudaMemcpyAsync(h->bk_Q, s->qbuf[s->cur], sizeof(float) * s->buf_floats, cudaMemcpyDeviceToDevice, st));
-    if (biased_) LRK_CUDA(h, cudaMemcpyAsync(h->bk_bu, h->bu32, sizeof(float) * (size_t)h->U, cudaMemcpyDeviceToDevice, st));
+    LrkEpoch e;
+    // safeguard: what this rank owns at the epoch boundary -- its user block and the item block it holds (BPR: the full item
+    // matrix); the loss is all-reduced, so every rank takes the same rollback decision
+    e.saved = [&] {
+        std::vector<LrkSaved> v{{h->P32, &h->bk_P, (size_t)h->U * h->ld}};
+        if (bpr_) v.push_back({h->Q32, &h->bk_Q, (size_t)h->I * h->ld});
+        else v.push_back({s->qbuf[s->cur], &h->bk_Q, s->buf_floats});
+        if (lrk_has_bias(h)) v.push_back({h->bu32, &h->bk_bu, (size_t)h->U});
+        return v;
+    };
     if (h->h_pnorm2) { h->pnorm2_prev = h->pnorm2_host; h->pnorm2_host = *h->h_pnorm2; }
-    bool fused_done_last = false;
-    for (int attempt = 0;; ++attempt) {
-    LRK_CUDA(h, cudaMemsetAsync(h->d_loss, 0, sizeof(double), st));
-    if (h->group) LRK_CUDA(h, cudaMemsetAsync(((GroupUnits*)h->group)->d_counter, 0, sizeof(unsigned int) * 64, st));
-    LRK_CUDA(h, cudaEventRecord(h->ev0, st));
-    if (s->trace < 0) { const char* t = getenv("LRK_DSGD_TRACE"); s->trace = t && atoi(t) ? 1 : 0; }
-    if (s->trace && s->trace_ev.empty()) {
-        s->trace_ev.resize((size_t)2 * world + 1);
-        for (auto& ev : s->trace_ev) LRK_CUDA(h, cudaEventCreate(&ev));
-    }
-    if (s->trace) LRK_CUDA(h, cudaEventRecord(s->trace_ev[0], st));
     bool fused_done = false;
-    fused_done_last = false;
-    if (bpr_) { int rc_b = dsgd_bpr_epoch(h, s, lr, reg_u, reg_i, epoch_idx); if (rc_b) return rc_b; }
-    else { int rc_f = dsgd_fused_epoch(h, s, lr, reg_u, reg_i, reg_b, epoch_idx, &fused_done); if (rc_f) return rc_f; }
-    for (int sub = 0; !bpr_ && !fused_done && sub < world; ++sub) {
-        const int b = dsgd_block_at(rank, world, sub);
-        float* buf = s->qbuf[s->cur];
-        const int64_t off = s->seg_off[(size_t)b], cnt = s->seg_off[(size_t)b + 1] - off;
-        const bool nobody = h->cfg.model == LRK_MODEL_BPR && (size_t)b < s->bpr_qualify.size() && s->bpr_qualify[(size_t)b] == 0;
-        if (cnt > 0 && !nobody) {
-            SgdParams sp;
-            memset(&sp, 0, sizeof sp);
-            sp.su = h->d_su + off; sp.si = h->d_si + off; sp.sr = h->d_sr + off; sp.n = cnt;
-            sp.P = h->P32; sp.Q = buf; sp.bu = h->bu32; sp.bi = buf + (size_t)s->max_blk * h->ld;
-            sp.mu = (float)h->mu; sp.lr = lr; sp.reg_u = reg_u; sp.reg_i = reg_i; sp.reg_b = (float)reg_b;
-            sp.loss = h->d_loss; sp.ld = h->ld; sp.epoch = (uint32_t)epoch_idx;
-            if (h->cfg.model == LRK_MODEL_BPR) {
-                // stratified sampling inside the held block; as many samples as the rank has ratings in it
-                sp.rowptr = h->d_rowptr; sp.col = h->d_col; sp.U = h->U; sp.I = h->I;
-                sp.seed_lo = (uint32_t)(h->cfg.seed + 977u * (uint64_t)rank); sp.seed_hi = (uint32_t)((h->cfg.seed + 977u * (uint64_t)rank) >> 32);
-                sp.blk_lo = s->bounds[(size_t)b]; sp.blk_hi = s->bounds[(size_t)b + 1];
-                sp.sample_base = off;
+    e.enqueue = [&](int) -> int {
+        if (h->group) LRK_CUDA(h, cudaMemsetAsync(((GroupUnits*)h->group)->d_counter, 0, sizeof(unsigned int) * 64, st));
+        if (s->trace < 0) { const char* t = getenv("LRK_DSGD_TRACE"); s->trace = t && atoi(t) ? 1 : 0; }
+        if (s->trace && s->trace_ev.empty()) {
+            s->trace_ev.resize((size_t)2 * world + 1);
+            for (auto& ev : s->trace_ev) LRK_CUDA(h, cudaEventCreate(&ev));
+        }
+        if (s->trace) LRK_CUDA(h, cudaEventRecord(s->trace_ev[0], st));
+        fused_done = false;
+        int rc;
+        if (bpr_) { if ((rc = dsgd_bpr_epoch(h, s, lr, reg_u, reg_i, epoch_idx))) return rc; }
+        else if ((rc = dsgd_fused_epoch(h, s, lr, reg_u, reg_i, reg_b, epoch_idx, &fused_done))) return rc;
+        for (int sub = 0; !bpr_ && !fused_done && sub < world; ++sub) {
+            const int b = dsgd_block_at(rank, world, sub);
+            float* buf = s->qbuf[s->cur];
+            const int64_t off = s->seg_off[(size_t)b], cnt = s->seg_off[(size_t)b + 1] - off;
+            if (cnt > 0) {
+                SgdParams sp;
+                memset(&sp, 0, sizeof sp);
+                sp.su = h->d_su + off; sp.si = h->d_si + off; sp.sr = h->d_sr + off; sp.n = cnt;
+                sp.P = h->P32; sp.Q = buf; sp.bu = h->bu32; sp.bi = buf + (size_t)s->max_blk * h->ld;
+                sp.mu = (float)h->mu; sp.lr = lr; sp.reg_u = reg_u; sp.reg_i = reg_i; sp.reg_b = (float)reg_b;
+                sp.loss = h->d_loss; sp.ld = h->ld; sp.epoch = (uint32_t)epoch_idx;
+                sp.hot_share = (size_t)b < s->seg_hot_share.size() ? s->seg_hot_share[(size_t)b] : 0.0;
+                sp.conc_div = h->conc_div;
+                sp.item_deg = h->d_item_deg ? h->d_item_deg + s->bounds[(size_t)b] : nullptr;   // block-local item ids
+                sp.pnorm2 = sp.item_deg ? h->d_pnorm2 : nullptr;
+                GroupUnits* gu = (GroupUnits*)h->group;
+                if (gu) {
+                    SgdGroupParams gp;
+                    memset(&gp, 0, sizeof gp);
+                    gp.su = h->d_su; gp.si = h->d_si; gp.sr = h->d_sr;                      // unit starts index the whole stream
+                    gp.units = gu->d_units + gu->unit_base[(size_t)b];
+                    gp.n_units = (int32_t)(gu->unit_base[(size_t)b + 1] - gu->unit_base[(size_t)b]);
+                    gp.counter = gu->d_counter + b;
+                    gp.P = sp.P; gp.Q = sp.Q; gp.bu = sp.bu; gp.bi = sp.bi; gp.mu = sp.mu; gp.lr = sp.lr; gp.reg_u = sp.reg_u; gp.reg_i = sp.reg_i;
+                    gp.reg_b = sp.reg_b; gp.loss = sp.loss; gp.ld = sp.ld; gp.item_deg = sp.item_deg;
+                    rc = sgd_group_launch(h, gp, cnt, h->conc_div);
+                } else rc = sgd_launch(h, sp);
+                if (rc) return rc;
             }
-            sp.hot_share = (h->cfg.model != LRK_MODEL_BPR && (size_t)b < s->seg_hot_share.size()) ? s->seg_hot_share[(size_t)b] : 0.0;
-            sp.conc_div = h->conc_div;
-            sp.item_deg = (h->cfg.model != LRK_MODEL_BPR && h->d_item_deg) ? h->d_item_deg + s->bounds[(size_t)b] : nullptr;   // block-local item ids
-            sp.pnorm2 = sp.item_deg ? h->d_pnorm2 : nullptr;
-            int rc;
-            GroupUnits* gu = (GroupUnits*)h->group;
-            if (gu && h->cfg.model != LRK_MODEL_BPR) {
-                SgdGroupParams gp;
-                memset(&gp, 0, sizeof gp);
-                gp.su = h->d_su; gp.si = h->d_si; gp.sr = h->d_sr;                      // unit starts index the whole stream
-                gp.units = gu->d_units + gu->unit_base[(size_t)b];
-                gp.n_units = (int32_t)(gu->unit_base[(size_t)b + 1] - gu->unit_base[(size_t)b]);
-                gp.counter = gu->d_counter + b;
-                gp.P = sp.P; gp.Q = sp.Q; gp.bu = sp.bu; gp.bi = sp.bi; gp.mu = sp.mu; gp.lr = sp.lr; gp.reg_u = sp.reg_u; gp.reg_i = sp.reg_i;
-                gp.reg_b = sp.reg_b; gp.loss = sp.loss; gp.ld = sp.ld; gp.item_deg = sp.item_deg;
-                rc = sgd_group_launch(h, gp, cnt, h->conc_div);
-            } else rc = sgd_launch(h, sp);
-            if (rc) return rc;
+            if (s->trace) LRK_CUDA(h, cudaEventRecord(s->trace_ev[(size_t)2 * sub + 1], st));
+            if (world > 1) {
+                float* nxt = s->qbuf[s->cur ^ 1];
+                LRK_NCCL(h, n->GroupStart());
+                LRK_NCCL(h, n->Send(buf, s->buf_floats, ncclFloat32, dsgd_send_peer(rank, world), (ncclComm_t)h->comm, st));
+                LRK_NCCL(h, n->Recv(nxt, s->buf_floats, ncclFloat32, dsgd_recv_peer(rank, world), (ncclComm_t)h->comm, st));
+                LRK_NCCL(h, n->GroupEnd());
+                s->cur ^= 1;
+            }
+            if (s->trace) LRK_CUDA(h, cudaEventRecord(s->trace_ev[(size_t)2 * sub + 2], st));
+            s->cur_block = dsgd_block_at(rank, world, sub + 1);
         }
-        if (s->trace) LRK_CUDA(h, cudaEventRecord(s->trace_ev[(size_t)2 * sub + 1], st));
-        if (world > 1) {
-            float* nxt = s->qbuf[s->cur ^ 1];
-            LRK_NCCL(h, n->GroupStart());
-            LRK_NCCL(h, n->Send(buf, s->buf_floats, ncclFloat32, dsgd_send_peer(rank, world), (ncclComm_t)h->comm, st));
-            LRK_NCCL(h, n->Recv(nxt, s->buf_floats, ncclFloat32, dsgd_recv_peer(rank, world), (ncclComm_t)h->comm, st));
-            LRK_NCCL(h, n->GroupEnd());
-            s->cur ^= 1;
-        }
-        if (s->trace) LRK_CUDA(h, cudaEventRecord(s->trace_ev[(size_t)2 * sub + 2], st));
-        s->cur_block = dsgd_block_at(rank, world, sub + 1);
-    }
-    LRK_NCCL(h, n->AllReduce(h->d_loss, h->d_loss, 1, ncclFloat64, ncclSum, (ncclComm_t)h->comm, st));
-    LRK_CUDA(h, cudaEventRecord(h->ev1, st));
-    if (h->cfg.model != LRK_MODEL_BPR && h->d_item_deg && !h->group) { int rc_n = refresh_user_norm2(h, false); if (rc_n) return rc_n; }
-    h->f64_valid = false;
-    LRK_CUDA(h, cudaMemcpyAsync(h->h_loss, h->d_loss, sizeof(double), cudaMemcpyDeviceToHost, st));
-    LRK_CUDA(h, cudaStreamSynchronize(st));
-    fused_done_last = fused_done;
-    if (fused_done) {
+        LRK_NCCL(h, n->AllReduce(h->d_loss, h->d_loss, 1, ncclFloat64, ncclSum, (ncclComm_t)h->comm, st));
+        return LRK_OK;
+    };
+    e.refresh_norm = k_lrk_models[h->cfg.model].damped && h->d_item_deg && !h->group;
+    e.after_sync = [&]() -> int {
+        if (!fused_done) return LRK_OK;
         int aborted = 0;
         LRK_CUDA(h, cudaMemcpy(&aborted, s->fused.d_abort, sizeof(int), cudaMemcpyDeviceToHost));
         if (aborted) return lrk_fail(h, LRK_ERR_NCCL, "lrk_sgd_epoch", "fused DSGD epoch: a ring neighbour did not answer within the spin limit", __FILE__, __LINE__);
-    }
-    LRK_CUDA(h, cudaEventElapsedTime(&h->last_epoch_ms, h->ev0, h->ev1));
-    {
-        const double l_ = (h->cfg.model == LRK_MODEL_BPR ? 1.0 : 0.5) * h->h_loss[0];
-        const bool bad = !std::isfinite(l_) || (h->prev_loss > 0.0 && l_ > 10.0 * h->prev_loss);
-        if (!bad || attempt >= 6 || h->conc_div >= 4096) break;
-        LRK_CUDA(h, cudaMemcpyAsync(h->P32, h->bk_P, sizeof(float) * np_, cudaMemcpyDeviceToDevice, st));
-        if (bpr_) LRK_CUDA(h, cudaMemcpyAsync(h->Q32, h->bk_Q, sizeof(float) * (size_t)h->I * h->ld, cudaMemcpyDeviceToDevice, st));
-        else LRK_CUDA(h, cudaMemcpyAsync(s->qbuf[s->cur], h->bk_Q, sizeof(float) * s->buf_floats, cudaMemcpyDeviceToDevice, st));
-        if (biased_) LRK_CUDA(h, cudaMemcpyAsync(h->bu32, h->bk_bu, sizeof(float) * (size_t)h->U, cudaMemcpyDeviceToDevice, st));
-        h->conc_div *= 4; h->good_epochs = 0; h->rollbacks++;
-        if (h->cfg.model != LRK_MODEL_BPR && h->d_item_deg && !h->group) { int rc_n = refresh_user_norm2(h, false); if (rc_n) return rc_n; }
-    }
-    }
-    if (s->trace && !fused_done_last && !bpr_) {
+        return LRK_OK;
+    };
+    // unlike the single-device path, the restored norm is not read back: the retry keeps the epoch's kernel variant
+    e.rolled_back = [&]() { return e.refresh_norm ? refresh_user_norm2(h, false) : (int)LRK_OK; };
+    const int rc = lrk_epoch(h, e, loss_out);
+    if (s->trace && !fused_done && !bpr_ && (rc == LRK_OK || rc == LRK_ERR_DIVERGED)) {
         std::string line = "[dsgd rank " + std::to_string(rank) + " epoch " + std::to_string(epoch_idx) + "]";
         for (int sub = 0; sub < world; ++sub) {
             float k_ms = 0.f, x_ms = 0.f;
@@ -797,14 +752,7 @@ static int dsgd_epoch(lrk_handle_s* h, float lr, float reg_u, float reg_i, doubl
         }
         fprintf(stderr, "%s total %.3f ms\n", line.c_str(), h->last_epoch_ms);
     }
-    const double loss = (h->cfg.model == LRK_MODEL_BPR ? 1.0 : 0.5) * h->h_loss[0];   // BPR has no 0.5 (BPRRecommender.java:77-92)
-    if (loss_out) *loss_out = loss;
-    if (std::isnan(loss) || std::isinf(loss))
-        return lrk_fail(h, LRK_ERR_DIVERGED, "lrk_sgd_epoch", "Loss = NaN or Infinity: current settings does not fit the recommender!", __FILE__, __LINE__);
-    h->prev_loss = loss;
-    h->epochs_done++;
-    if (h->conc_div > 1 && ++h->good_epochs >= 8) { h->conc_div /= 2; h->good_epochs = 0; }
-    return LRK_OK;
+    return rc;
 }
 
 // P/bu: the rank's user block; Q/bi: the full item factors, gathered from the ring

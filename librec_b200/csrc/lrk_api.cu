@@ -10,6 +10,7 @@
 #include "sgd_svdpp.cuh"
 #include "sgd_aobpr.cuh"
 #include "als.cuh"
+#include "lrk_epoch.cuh"
 #include <chrono>
 #include "topn_exact.cuh"
 #include "topn_tc.cuh"
@@ -106,37 +107,18 @@ static int gbpr_epoch(lrk_handle_s* h, float lr, float reg_u, float reg_i, doubl
     if ((rc = lrk_dev_alloc(h, &g->tQ, nq_))) return rc;
     LRK_CUDA(h, cudaMemsetAsync(g->tP, 0, sizeof(float) * np_, st));
     LRK_CUDA(h, cudaMemsetAsync(g->tQ, 0, sizeof(float) * nq_, st));
-    LRK_CUDA(h, cudaMemsetAsync(h->d_loss, 0, sizeof(double), st));
     GbprParams p;
     gbpr_fill(h, p, lr, reg_u, reg_i, reg_b, epoch_idx);
-    LRK_CUDA(h, cudaEventRecord(h->ev0, st));
-    if (h->nnz > 0) {
-        switch (h->G * 100 + h->V) {
-            case 101: rc = gbpr_launch_gv<1, 1>(h, p); break;
-            case 201: rc = gbpr_launch_gv<2, 1>(h, p); break;
-            case 401: rc = gbpr_launch_gv<4, 1>(h, p); break;
-            case 801: rc = gbpr_launch_gv<8, 1>(h, p); break;
-            case 1601: rc = gbpr_launch_gv<16, 1>(h, p); break;
-            case 3201: rc = gbpr_launch_gv<32, 1>(h, p); break;
-            case 3202: rc = gbpr_launch_gv<32, 2>(h, p); break;
-            default: rc = lrk_fail(h, LRK_ERR_INVALID, "gbpr_epoch", "unsupported factor layout", __FILE__, __LINE__);
-        }
-        if (rc) return rc;
+    LrkEpoch e;
+    e.enqueue = [&](int) -> int {
+        if (h->nnz == 0) return LRK_OK;
+        const int rc_l = lrk_with_layout(h, [&](auto G, auto V) { return gbpr_launch_gv<decltype(G)::value, decltype(V)::value>(h, p); });
+        if (rc_l) return rc_l;
         gbpr_apply_kernel<<<lrk_ceil_div((int64_t)np_, 256), 256, 0, st>>>(h->P32, g->tP, (int64_t)np_); LRK_LAUNCH_CHECK(h);
         gbpr_apply_kernel<<<lrk_ceil_div((int64_t)nq_, 256), 256, 0, st>>>(h->Q32, g->tQ, (int64_t)nq_); LRK_LAUNCH_CHECK(h);
-    }
-    LRK_CUDA(h, cudaEventRecord(h->ev1, st));
-    LRK_CUDA(h, cudaMemcpyAsync(h->h_loss, h->d_loss, sizeof(double), cudaMemcpyDeviceToHost, st));
-    LRK_CUDA(h, cudaStreamSynchronize(st));
-    LRK_CUDA(h, cudaEventElapsedTime(&h->last_epoch_ms, h->ev0, h->ev1));
-    h->f64_valid = false;
-    topn_tc_invalidate(h);
-    const double loss = h->h_loss[0];                 // no 0.5 (GBPRRecommender.java:130-165)
-    if (loss_out) *loss_out = loss;
-    if (std::isnan(loss) || std::isinf(loss))
-        return lrk_fail(h, LRK_ERR_DIVERGED, "lrk_sgd_epoch", "Loss = NaN or Infinity: current settings does not fit the recommender!", __FILE__, __LINE__);
-    h->epochs_done++;
-    return LRK_OK;
+        return LRK_OK;
+    };
+    return lrk_epoch(h, e, loss_out);                 // no 0.5 (GBPRRecommender.java:130-165)
 }
 
 // SVD++: train values in CSR order + users by descending degree
@@ -196,34 +178,13 @@ static int svdpp_epoch(lrk_handle_s* h, float lr, float reg_u, float reg_i, doub
     p.P = h->P32; p.Q = h->Q32; p.Y = g->Y32; p.bu = h->bu32; p.bi = h->bi32;
     p.mu = (float)h->mu; p.lr = lr; p.reg_u = reg_u; p.reg_i = reg_i; p.reg_b = (float)reg_b; p.reg_imp = (float)g->reg_imp;
     p.loss = h->d_loss; p.ld = h->ld;
-    LRK_CUDA(h, cudaMemsetAsync(h->d_loss, 0, sizeof(double), st));
     LRK_CUDA(h, cudaMemsetAsync(g->d_counter, 0, sizeof(unsigned int), st));
-    LRK_CUDA(h, cudaEventRecord(h->ev0, st));
-    int rc = LRK_OK;
-    if (h->nnz > 0) {
-        switch (h->G * 100 + h->V) {
-            case 101: rc = svdpp_launch_gv<1, 1>(h, p); break;
-            case 201: rc = svdpp_launch_gv<2, 1>(h, p); break;
-            case 401: rc = svdpp_launch_gv<4, 1>(h, p); break;
-            case 801: rc = svdpp_launch_gv<8, 1>(h, p); break;
-            case 1601: rc = svdpp_launch_gv<16, 1>(h, p); break;
-            case 3201: rc = svdpp_launch_gv<32, 1>(h, p); break;
-            case 3202: rc = svdpp_launch_gv<32, 2>(h, p); break;
-            default: rc = lrk_fail(h, LRK_ERR_INVALID, "svdpp_epoch", "unsupported factor layout", __FILE__, __LINE__);
-        }
-        if (rc) return rc;
-    }
-    LRK_CUDA(h, cudaEventRecord(h->ev1, st));
-    LRK_CUDA(h, cudaMemcpyAsync(h->h_loss, h->d_loss, sizeof(double), cudaMemcpyDeviceToHost, st));
-    LRK_CUDA(h, cudaStreamSynchronize(st));
-    LRK_CUDA(h, cudaEventElapsedTime(&h->last_epoch_ms, h->ev0, h->ev1));
-    h->f64_valid = false;
-    const double loss = 0.5 * h->h_loss[0];            // SVDPlusPlusRecommender.java:109
-    if (loss_out) *loss_out = loss;
-    if (std::isnan(loss) || std::isinf(loss))
-        return lrk_fail(h, LRK_ERR_DIVERGED, "lrk_sgd_epoch", "Loss = NaN or Infinity: current settings does not fit the recommender!", __FILE__, __LINE__);
-    h->epochs_done++;
-    return LRK_OK;
+    LrkEpoch e;
+    e.enqueue = [&](int) -> int {
+        if (h->nnz == 0) return LRK_OK;
+        return lrk_with_layout(h, [&](auto G, auto V) { return svdpp_launch_gv<decltype(G)::value, decltype(V)::value>(h, p); });
+    };
+    return lrk_epoch(h, e, loss_out);                 // 0.5 * sum: SVDPlusPlusRecommender.java:109
 }
 
 __global__ void pairs_validate_kernel(const int32_t* __restrict__ u, const int32_t* __restrict__ i, int64_t n, int32_t U, int32_t I, int* __restrict__ flag) {
@@ -267,13 +228,13 @@ int lrk_create(const lrk_config_t* cfg, lrk_handle_t* out) {
     *out = nullptr;
     if (cfg->num_factors < 1 || cfg->num_factors > LRK_MAX_FACTORS)
         return lrk_fail(nullptr, LRK_ERR_INVALID, "lrk_create", "num_factors must be in 1..256", __FILE__, __LINE__);
-    if (cfg->model < LRK_MODEL_BIASEDMF || cfg->model > LRK_MODEL_EALS)
+    if (!lrk_model_known(cfg->model))
         return lrk_fail(nullptr, LRK_ERR_INVALID, "lrk_create", "unknown model", __FILE__, __LINE__);
     if (cfg->model == LRK_MODEL_WRMF && cfg->num_factors > ALS_MAX_K)
         return lrk_fail(nullptr, LRK_ERR_INVALID, "lrk_create", "WRMF on the device needs rec.factor.number <= 112 (the Gauss-Jordan step lives in shared memory)", __FILE__, __LINE__);
     if (cfg->update_mode < LRK_UPDATE_ATOMIC || cfg->update_mode > LRK_UPDATE_REFERENCE_ORDER)
         return lrk_fail(nullptr, LRK_ERR_INVALID, "lrk_create", "unknown update_mode", __FILE__, __LINE__);
-    if (cfg->update_mode == LRK_UPDATE_REFERENCE_ORDER && !(cfg->model == LRK_MODEL_BIASEDMF || cfg->model == LRK_MODEL_PMF))
+    if (cfg->update_mode == LRK_UPDATE_REFERENCE_ORDER && !k_lrk_models[cfg->model].rating)
         return lrk_fail(nullptr, LRK_ERR_INVALID, "lrk_create", "reference-order mode covers BiasedMF and PMF", __FILE__, __LINE__);
     int ndev = 0;
     LRK_CUDA(nullptr, cudaGetDeviceCount(&ndev));
@@ -290,7 +251,7 @@ int lrk_create(const lrk_config_t* cfg, lrk_handle_t* out) {
     layout_for_k(h->k, &h->ld, &h->G, &h->V);
     {   // the user-group kernel (LRK_SGD_GROUP=1, sgd_group.cuh) needs at least 8 lanes per rating: small k are padded to 32 columns
         const char* env = getenv("LRK_SGD_GROUP");
-        if (env && atoi(env) != 0 && lrk_is_rating_model(h) && cfg->update_mode == LRK_UPDATE_ATOMIC && h->ld < 32) { h->ld = 32; h->G = 8; h->V = 1; }
+        if (env && atoi(env) != 0 && k_lrk_models[cfg->model].rating && cfg->update_mode == LRK_UPDATE_ATOMIC && h->ld < 32) { h->ld = 32; h->G = 8; h->V = 1; }
     }
     h->sm_count = prop.multiProcessorCount;
     int rc = LRK_OK;
@@ -421,7 +382,7 @@ int lrk_set_train_csr(lrk_handle_t h, int32_t U, int32_t I, const int64_t* rowpt
     }
     if (h->cfg.model == LRK_MODEL_GBPR && (rc = gbpr_stage(h))) return rc;
     if (h->cfg.model == LRK_MODEL_SVDPP && (rc = svdpp_stage(h, val))) return rc;
-    if (lrk_is_als(h) && (rc = als_stage(h, val))) return rc;
+    if (k_lrk_models[h->cfg.model].als && (rc = als_stage(h, val))) return rc;
     h->has_train = true;
     topn_tc_invalidate(h);
     return LRK_OK;
@@ -432,9 +393,10 @@ int lrk_set_factors(lrk_handle_t h, const double* P, const double* Q, const doub
     if (h->multi) return multi_set_factors(h, P, Q, bu, bi, mu);
     LRK_REQUIRE(h, h->has_train, "call lrk_set_train_csr first (it fixes numUsers / numItems)");
     LRK_REQUIRE(h, P && Q, "P and Q are required");
-    const bool biased = lrk_has_bias(h);
-    LRK_REQUIRE(h, (h->cfg.model != LRK_MODEL_BIASEDMF && h->cfg.model != LRK_MODEL_SVDPP) || (bu && bi), "BiasedMF / SVD++ need userBiases and itemBiases");
-    LRK_REQUIRE(h, h->cfg.model != LRK_MODEL_GBPR || bi, "GBPR needs itemBiases");
+    const LrkModelInfo m = lrk_model_info(h->cfg);
+    const bool biased = m.biases > 0;
+    LRK_REQUIRE(h, m.biases < 2 || (bu && bi), "BiasedMF / SVD++ need userBiases and itemBiases");
+    LRK_REQUIRE(h, m.biases < 1 || bi, "GBPR needs itemBiases");
     LRK_CUDA(h, cudaSetDevice(h->cfg.device));
     if (h->world > 1) return dsgd_set_factors(h, P, Q, bu, bi, mu);
     cudaStream_t st = h->stream;
@@ -459,7 +421,7 @@ int lrk_set_factors(lrk_handle_t h, const double* P, const double* Q, const doub
     f64_to_f32_rows_kernel<<<lrk_ceil_div(I * ld, 256), 256, 0, st>>>(h->Q64, h->Q32, I, k, ld); LRK_LAUNCH_CHECK(h);
     f64_to_f32_rows_kernel<<<lrk_ceil_div(U, 256), 256, 0, st>>>(h->bu64, h->bu32, U, 1, 1); LRK_LAUNCH_CHECK(h);
     f64_to_f32_rows_kernel<<<lrk_ceil_div(I, 256), 256, 0, st>>>(h->bi64, h->bi32, I, 1, 1); LRK_LAUNCH_CHECK(h);
-    if (h->cfg.model != LRK_MODEL_BPR && h->cfg.model != LRK_MODEL_GBPR && h->cfg.model != LRK_MODEL_SVDPP && h->cfg.model != LRK_MODEL_AOBPR && !lrk_is_als(h) && (rc = refresh_user_norm2(h, true))) return rc;
+    if (m.damped && (rc = refresh_user_norm2(h, true))) return rc;
     if (h->aobpr) ((AobprState*)h->aobpr)->count = 0;                 // a new trainModel(): countIter starts at 0 (AoBPRRecommender.java:88)
     if (h->h_pnorm2) { h->pnorm2_prev = 0.f; h->pnorm2_host = *h->h_pnorm2; }
     LRK_CUDA(h, cudaStreamSynchronize(st));   // host buffers may be reused by the caller on return
@@ -504,16 +466,8 @@ int lrk_get_factors(lrk_handle_t h, double* P, double* Q, double* bu, double* bi
 }
 
 // -------------------------------------------------------------------------------------------
-// read-only with respect to the handle (lrk_bpr_peek_samples uses it too)
-static void fill_sgd_params(const lrk_handle_s* h, SgdParams& sp, float lr, float reg_u, float reg_i, double reg_b, int32_t epoch_idx) {
-    memset(&sp, 0, sizeof sp);
-    sp.su = h->d_su; sp.si = h->d_si; sp.sr = h->d_sr; sp.n = h->nnz;
-    sp.P = h->P32; sp.Q = h->Q32; sp.bu = h->bu32; sp.bi = h->bi32;
-    sp.mu = (float)h->mu; sp.lr = lr; sp.reg_u = reg_u; sp.reg_i = reg_i; sp.reg_b = (float)reg_b;
-    sp.loss = h->d_loss; sp.ld = h->ld;
-    sp.hot_share = lrk_is_rating_model(h) ? h->hot_share : 0.0;
-    sp.item_deg = (lrk_is_rating_model(h) || h->cfg.model == LRK_MODEL_RANKSGD) ? h->d_item_deg : nullptr;
-    sp.item_cum = h->cfg.model == LRK_MODEL_RANKSGD ? h->d_item_cum : nullptr;
+// stability cap of the SGD grid (sgd_grid_for; it applies to launches without the staleness-aware step)
+static double sgd_hot_share(const lrk_handle_s* h) {
     // RankSGD: squared loss without regularisation -- B concurrent updates of one item act like ONE step lr * B * |p_u|^2
     // where the sequential walk contracts by exp(-lr * B * |p_u|^2).  Popular items are hit as positives and, by
     // construction of the sampler, as negatives (2 x share), and the two only agree while that product is small: the grid
@@ -521,7 +475,20 @@ static void fill_sgd_params(const lrk_handle_s* h, SgdParams& sp, float lr, floa
     // reached the oracle's loss but Precision@10 0.140 against 0.176 (sequential) / 0.214 (sequential, shuffled order).
     // r02: the RankSGD kernel scales its item-side steps for the samples in flight (sgd.cuh), so the cap is only the fallback of
     // LRK_SGD_NODAMP=1 (r01: it left a handful of CTAs on the ML-20M shape, 0.48 G updates/s)
-    if (h->cfg.model == LRK_MODEL_RANKSGD) sp.hot_share = 8.0 * h->hot_share * (double)std::max(1.f, h->pnorm2_host);
+    if (h->cfg.model == LRK_MODEL_RANKSGD) return 8.0 * h->hot_share * (double)std::max(1.f, h->pnorm2_host);
+    return k_lrk_models[h->cfg.model].rating ? h->hot_share : 0.0;
+}
+
+// read-only with respect to the handle (lrk_bpr_peek_samples uses it too)
+static void fill_sgd_params(const lrk_handle_s* h, SgdParams& sp, float lr, float reg_u, float reg_i, double reg_b, int32_t epoch_idx) {
+    memset(&sp, 0, sizeof sp);
+    sp.su = h->d_su; sp.si = h->d_si; sp.sr = h->d_sr; sp.n = h->nnz;
+    sp.P = h->P32; sp.Q = h->Q32; sp.bu = h->bu32; sp.bi = h->bi32;
+    sp.mu = (float)h->mu; sp.lr = lr; sp.reg_u = reg_u; sp.reg_i = reg_i; sp.reg_b = (float)reg_b;
+    sp.loss = h->d_loss; sp.ld = h->ld;
+    sp.hot_share = sgd_hot_share(h);
+    sp.item_deg = k_lrk_models[h->cfg.model].damped ? h->d_item_deg : nullptr;
+    sp.item_cum = h->cfg.model == LRK_MODEL_RANKSGD ? h->d_item_cum : nullptr;
     sp.rowptr = h->d_rowptr; sp.col = h->d_col; sp.U = h->U; sp.I = h->I;
     sp.seed_lo = (uint32_t)h->cfg.seed; sp.seed_hi = (uint32_t)(h->cfg.seed >> 32); sp.epoch = (uint32_t)epoch_idx;
 }
@@ -534,25 +501,14 @@ int lrk_sgd_epoch(lrk_handle_t h, float lr, float reg_u, float reg_i, double reg
     if (h->world > 1) return dsgd_epoch(h, lr, reg_u, reg_i, reg_b, epoch_idx, loss_out);
     if (h->cfg.model == LRK_MODEL_GBPR) return gbpr_epoch(h, lr, reg_u, reg_i, reg_b, epoch_idx, loss_out);
     if (h->cfg.model == LRK_MODEL_SVDPP) return svdpp_epoch(h, lr, reg_u, reg_i, reg_b, loss_out);
-    if (lrk_is_als(h)) { topn_tc_invalidate(h); return als_epoch(h, reg_u, reg_i, loss_out); }
-    cudaStream_t st = h->stream;
+    if (k_lrk_models[h->cfg.model].als) { topn_tc_invalidate(h); return als_epoch(h, reg_u, reg_i, loss_out); }
+    LrkEpoch e;
     if (h->cfg.update_mode == LRK_UPDATE_REFERENCE_ORDER) {
         // fp64 masters are the working set in this mode
         int rc = refresh_masters(h);
         if (rc) return rc;
-        LRK_CUDA(h, cudaMemsetAsync(h->d_loss, 0, sizeof(double), st));
-        LRK_CUDA(h, cudaEventRecord(h->ev0, st));
-        if (h->nnz > 0 && (rc = exact_epoch(h, (ExactSchedule*)h->exact, lr, reg_u, reg_i, reg_b))) return rc;
-        LRK_CUDA(h, cudaEventRecord(h->ev1, st));
-        topn_tc_invalidate(h);
-        LRK_CUDA(h, cudaMemcpyAsync(h->h_loss, h->d_loss, sizeof(double), cudaMemcpyDeviceToHost, st));
-        LRK_CUDA(h, cudaStreamSynchronize(st));
-        LRK_CUDA(h, cudaEventElapsedTime(&h->last_epoch_ms, h->ev0, h->ev1));
-        const double loss = 0.5 * h->h_loss[0];
-        if (loss_out) *loss_out = loss;
-        if (std::isnan(loss) || std::isinf(loss))
-            return lrk_fail(h, LRK_ERR_DIVERGED, "lrk_sgd_epoch", "Loss = NaN or Infinity: current settings does not fit the recommender!", __FILE__, __LINE__);
-        return LRK_OK;
+        e.enqueue = [&](int) { return h->nnz > 0 ? exact_epoch(h, (ExactSchedule*)h->exact, lr, reg_u, reg_i, reg_b) : (int)LRK_OK; };
+        return lrk_epoch(h, e, loss_out);
     }
     // curvature estimate of the epoch: the value the last norm refresh left in pinned memory (once per epoch call, so that a
     // lrk_bpr_peek_samples between two epochs cannot change which kernel variant the next epoch picks)
@@ -567,86 +523,52 @@ int lrk_sgd_epoch(lrk_handle_t h, float lr, float reg_u, float reg_i, double reg
         if (rc_a) return rc_a;
         sp.ao_rank = ao->d_rank; sp.ao_var = ao->d_var; sp.ao_cum = ao->d_cum; sp.n_entries = h->nnz;
     }
-    const bool biased = h->cfg.model == LRK_MODEL_BIASEDMF;
-    const size_t np_ = (size_t)h->U * h->ld, nq_ = (size_t)h->I * h->ld;
-    int rc;
-    if ((rc = lrk_dev_alloc(h, &h->bk_P, np_))) return rc;
-    if ((rc = lrk_dev_alloc(h, &h->bk_Q, nq_))) return rc;
-    if (biased) {
-        if ((rc = lrk_dev_alloc(h, &h->bk_bu, (size_t)h->U))) return rc;
-        if ((rc = lrk_dev_alloc(h, &h->bk_bi, (size_t)h->I))) return rc;
-    }
-    LRK_CUDA(h, cudaMemcpyAsync(h->bk_P, h->P32, sizeof(float) * np_, cudaMemcpyDeviceToDevice, st));
-    LRK_CUDA(h, cudaMemcpyAsync(h->bk_Q, h->Q32, sizeof(float) * nq_, cudaMemcpyDeviceToDevice, st));
-    if (biased) {
-        LRK_CUDA(h, cudaMemcpyAsync(h->bk_bu, h->bu32, sizeof(float) * (size_t)h->U, cudaMemcpyDeviceToDevice, st));
-        LRK_CUDA(h, cudaMemcpyAsync(h->bk_bi, h->bi32, sizeof(float) * (size_t)h->I, cudaMemcpyDeviceToDevice, st));
-    }
     if (sp.item_deg) sp.pnorm2 = h->d_pnorm2;          // refreshed by refresh_user_norm2 at set_factors and after every epoch
-    // the group kernel takes the curvature from the rows it holds; the stream kernels need mean |p_u|^2 refreshed per epoch
-    const bool track_norm = !h->group && (sp.item_deg != nullptr || h->cfg.model == LRK_MODEL_RANKSGD);
-    double loss = 0.0;
-    for (int attempt = 0;; ++attempt) {
+    e.saved = [&] {
+        std::vector<LrkSaved> v{{h->P32, &h->bk_P, (size_t)h->U * h->ld}, {h->Q32, &h->bk_Q, (size_t)h->I * h->ld}};
+        if (lrk_has_bias(h)) { v.push_back({h->bu32, &h->bk_bu, (size_t)h->U}); v.push_back({h->bi32, &h->bk_bi, (size_t)h->I}); }
+        return v;
+    };
+    e.enqueue = [&](int attempt) -> int {
         sp.conc_div = h->conc_div;
-        LRK_CUDA(h, cudaMemsetAsync(h->d_loss, 0, sizeof(double), st));
-        LRK_CUDA(h, cudaEventRecord(h->ev0, st));
-        if (h->nnz > 0 && h->group) {
+        if (h->nnz == 0) return LRK_OK;
+        int rc;
+        if (h->group) {
             GroupUnits* gu = (GroupUnits*)h->group;
             SgdGroupParams gp;
             memset(&gp, 0, sizeof gp);
             gp.su = sp.su; gp.si = sp.si; gp.sr = sp.sr; gp.units = gu->d_units; gp.n_units = (int32_t)gu->n_units; gp.counter = gu->d_counter;
             gp.P = sp.P; gp.Q = sp.Q; gp.bu = sp.bu; gp.bi = sp.bi; gp.mu = sp.mu; gp.lr = sp.lr; gp.reg_u = sp.reg_u; gp.reg_i = sp.reg_i;
             gp.reg_b = sp.reg_b; gp.loss = sp.loss; gp.ld = sp.ld; gp.item_deg = sp.item_deg;
-            LRK_CUDA(h, cudaMemsetAsync(gu->d_counter, 0, sizeof(unsigned int), st));
-            if ((rc = sgd_group_launch(h, gp, h->nnz, h->conc_div))) return rc;
-        } else if (h->nnz > 0 && ao) {
-            // AoBPR: the epoch in windows of loopNumber samples, the factor rankings refreshed between them (countIter runs across
-            // iterations and restarts at every refresh, AoBPRRecommender.java:92-97)
-            int64_t count = ao->count, done = 0;
-            while (done < h->nnz) {
-                if (count % ao->loop == 0) { if ((rc = aobpr_refresh(h, ao))) return rc; count = 0; }
-                const int64_t w = std::min<int64_t>(h->nnz - done, (int64_t)ao->loop - count);
-                SgdParams wp = sp;
-                wp.n = w; wp.sample_base = done;
-                if ((rc = sgd_launch(h, wp))) return rc;
-                done += w; count += w;
-            }
-            if (attempt == 0) ao->count = count;          // a rolled-back attempt replays the same windows
-        } else if (h->nnz > 0 && (rc = sgd_launch(h, sp))) return rc;
-        LRK_CUDA(h, cudaEventRecord(h->ev1, st));
-        if (track_norm && (rc = refresh_user_norm2(h, false))) return rc;
-        LRK_CUDA(h, cudaMemcpyAsync(h->h_loss, h->d_loss, sizeof(double), cudaMemcpyDeviceToHost, st));
-        LRK_CUDA(h, cudaStreamSynchronize(st));
-        loss = h->h_loss[0];
-        if (h->cfg.model != LRK_MODEL_BPR && h->cfg.model != LRK_MODEL_AOBPR) loss *= 0.5;   // BiasedMFRecommender.java:101 ; BPR / AoBPR have no 0.5
-        const bool bad = !std::isfinite(loss) || (h->prev_loss > 0.0 && loss > 10.0 * h->prev_loss);
-        if (!bad || attempt >= 6 || h->conc_div >= 4096) break;
-        // roll the epoch back and retry with fewer ratings in flight
-        LRK_CUDA(h, cudaMemcpyAsync(h->P32, h->bk_P, sizeof(float) * np_, cudaMemcpyDeviceToDevice, st));
-        LRK_CUDA(h, cudaMemcpyAsync(h->Q32, h->bk_Q, sizeof(float) * nq_, cudaMemcpyDeviceToDevice, st));
-        if (biased) {
-            LRK_CUDA(h, cudaMemcpyAsync(h->bu32, h->bk_bu, sizeof(float) * (size_t)h->U, cudaMemcpyDeviceToDevice, st));
-            LRK_CUDA(h, cudaMemcpyAsync(h->bi32, h->bk_bi, sizeof(float) * (size_t)h->I, cudaMemcpyDeviceToDevice, st));
+            LRK_CUDA(h, cudaMemsetAsync(gu->d_counter, 0, sizeof(unsigned int), h->stream));
+            return sgd_group_launch(h, gp, h->nnz, h->conc_div);
         }
-        h->conc_div *= 4; h->good_epochs = 0; h->rollbacks++;
-        if (track_norm) {
-            if ((rc = refresh_user_norm2(h, true))) return rc;          // the restored factors' norm, visible to the host now
-            h->pnorm2_host = *h->h_pnorm2;
-            // r02: the RankSGD kernel scales its item-side steps for the samples in flight (sgd.cuh), so the cap is only the fallback of
-    // LRK_SGD_NODAMP=1 (r01: it left a handful of CTAs on the ML-20M shape, 0.48 G updates/s)
-    if (h->cfg.model == LRK_MODEL_RANKSGD) sp.hot_share = 8.0 * h->hot_share * (double)std::max(1.f, h->pnorm2_host);
+        if (!ao) return sgd_launch(h, sp);
+        // AoBPR: the epoch in windows of loopNumber samples, the factor rankings refreshed between them (countIter runs across
+        // iterations and restarts at every refresh, AoBPRRecommender.java:92-97)
+        int64_t count = ao->count, done = 0;
+        while (done < h->nnz) {
+            if (count % ao->loop == 0) { if ((rc = aobpr_refresh(h, ao))) return rc; count = 0; }
+            const int64_t w = std::min<int64_t>(h->nnz - done, (int64_t)ao->loop - count);
+            SgdParams wp = sp;
+            wp.n = w; wp.sample_base = done;
+            if ((rc = sgd_launch(h, wp))) return rc;
+            done += w; count += w;
         }
-    }
-    h->f64_valid = false;
-    topn_tc_invalidate(h);
-    LRK_CUDA(h, cudaEventElapsedTime(&h->last_epoch_ms, h->ev0, h->ev1));
-    if (loss_out) *loss_out = loss;
-    if (std::isnan(loss) || std::isinf(loss))
-        return lrk_fail(h, LRK_ERR_DIVERGED, "lrk_sgd_epoch", "Loss = NaN or Infinity: current settings does not fit the recommender!", __FILE__, __LINE__);
-    h->prev_loss = loss;
-    h->epochs_done++;
-    if (h->conc_div > 1 && ++h->good_epochs >= 8) { h->conc_div /= 2; h->good_epochs = 0; }
-    return LRK_OK;
+        if (attempt == 0) ao->count = count;          // a rolled-back attempt replays the same windows
+        return LRK_OK;
+    };
+    // the group kernel takes the curvature from the rows it holds; the stream kernels need mean |p_u|^2 refreshed per epoch
+    e.refresh_norm = !h->group && (sp.item_deg != nullptr || h->cfg.model == LRK_MODEL_RANKSGD);
+    e.rolled_back = [&]() -> int {
+        if (!e.refresh_norm) return LRK_OK;
+        const int rc = refresh_user_norm2(h, true);     // the restored factors' norm, visible to the host now
+        if (rc) return rc;
+        h->pnorm2_host = *h->h_pnorm2;
+        sp.hot_share = sgd_hot_share(h);
+        return LRK_OK;
+    };
+    return lrk_epoch(h, e, loss_out);
 }
 
 int lrk_set_param(lrk_handle_t h, const char* name, double value) {
@@ -1084,8 +1006,7 @@ int lrk_comm_unique_id(uint8_t out[128]) { return dsgd_unique_id(out); }
 int lrk_comm_init(lrk_handle_t h, int32_t rank, int32_t world, const uint8_t unique_id[128]) {
     LRK_REQUIRE(h, h != nullptr, "handle is NULL");
     LRK_NOT_MULTI(h, "lrk_comm_init");
-    LRK_REQUIRE(h, h->cfg.update_mode != LRK_UPDATE_REFERENCE_ORDER, "reference-order mode is single-GPU");
-    LRK_REQUIRE(h, h->cfg.model != LRK_MODEL_RANKSGD && h->cfg.model != LRK_MODEL_GBPR && h->cfg.model != LRK_MODEL_SVDPP && h->cfg.model != LRK_MODEL_AOBPR && !lrk_is_als(h), "RankSGD, GBPR, SVD++, AoBPR, WRMF and eALS are single-GPU in this build");
+    LRK_REQUIRE(h, lrk_model_info(h->cfg).multi_gpu, k_lrk_single_gpu);
     return dsgd_comm_init(h, rank, world, unique_id);
 }
 
@@ -1095,8 +1016,8 @@ int lrk_create_multi(const lrk_config_t* cfg, const int32_t* devices, int32_t n_
     if (n_devices < 1 || n_devices > 8) return lrk_fail(nullptr, LRK_ERR_INVALID, "lrk_create_multi", "1 to 8 devices", __FILE__, __LINE__);
     for (int a = 0; a < n_devices; ++a) for (int b = a + 1; b < n_devices; ++b)
         if (devices[a] == devices[b]) return lrk_fail(nullptr, LRK_ERR_INVALID, "lrk_create_multi", "a device is listed twice", __FILE__, __LINE__);
-    if (n_devices > 1 && (cfg->update_mode == LRK_UPDATE_REFERENCE_ORDER || cfg->model == LRK_MODEL_RANKSGD || cfg->model == LRK_MODEL_GBPR || cfg->model == LRK_MODEL_SVDPP || cfg->model == LRK_MODEL_AOBPR || cfg->model == LRK_MODEL_WRMF || cfg->model == LRK_MODEL_EALS))
-        return lrk_fail(nullptr, LRK_ERR_INVALID, "lrk_create_multi", "reference-order mode, RankSGD, GBPR, SVD++ and AoBPR are single-GPU", __FILE__, __LINE__);
+    if (n_devices > 1 && lrk_model_known(cfg->model) && !lrk_model_info(*cfg).multi_gpu)     // an unknown model fails in lrk_create
+        return lrk_fail(nullptr, LRK_ERR_INVALID, "lrk_create_multi", k_lrk_single_gpu, __FILE__, __LINE__);
     lrk_handle_s* h = new (std::nothrow) lrk_handle_s();
     MultiState* ms = new (std::nothrow) MultiState();
     if (!h || !ms) { delete h; delete ms; return lrk_fail(nullptr, LRK_ERR_NOMEM, "lrk_create_multi", "host allocation failed", __FILE__, __LINE__); }

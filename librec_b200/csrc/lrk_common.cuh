@@ -5,6 +5,7 @@
 #include <cstdio>
 #include <cstring>
 #include <string>
+#include <type_traits>
 #include <unordered_map>
 #include "../../include/librec_b200.h"
 
@@ -49,7 +50,7 @@ struct lrk_handle_s {
     bool has_factors = false;
     bool f64_valid = false;   // masters are in sync with the fp32 working copies
 
-    // Safeguard of the fast SGD mode: factors are snapshotted before an epoch; a non-finite (or exploding) loss
+    // Safeguard of the fast SGD mode (lrk_epoch.cuh): factors are snapshotted before an epoch; a non-finite (or exploding) loss
     // rolls the epoch back and re-runs it with 4x fewer ratings in flight (sticky, relaxed again after 8 good epochs)
     float *bk_P = nullptr, *bk_Q = nullptr, *bk_bu = nullptr, *bk_bi = nullptr;
     int conc_div = 1;           // divisor of the SGD grid
@@ -175,9 +176,55 @@ static inline int lrk_scratch_begin(lrk_handle_s* h, size_t bytes, LrkScratch* o
 }
 
 static inline int lrk_ceil_div(int64_t a, int64_t b) { return (int)((a + b - 1) / b); }
-// models whose prediction adds biases (GBPR: item biases only, its user biases stay zero): b_i + p_u.q_i (+ b_u + mu)
-static inline bool lrk_has_bias(const lrk_handle_s* h) { return h->cfg.model == LRK_MODEL_BIASEDMF || h->cfg.model == LRK_MODEL_GBPR || h->cfg.model == LRK_MODEL_SVDPP; }
-// WRMF / eALS: alternating least squares on the fp64 masters (als.cuh); lrk_sgd_epoch = one ALS iteration
-static inline bool lrk_is_als(const lrk_handle_s* h) { return h->cfg.model == LRK_MODEL_WRMF || h->cfg.model == LRK_MODEL_EALS; }
-// BiasedMF / PMF: one update per train rating with the rating as target (item-run tiles, staleness-aware step)
-static inline bool lrk_is_rating_model(const lrk_handle_s* h) { return h->cfg.model == LRK_MODEL_BIASEDMF || h->cfg.model == LRK_MODEL_PMF; }
+
+// What the host code needs to know about each model: one row per lrk_model value, in enum order
+struct LrkModelInfo {
+    double loss_scale;  // reported loss = loss_scale * the kernels' sum (the references' 0.5 of the squared error); 0: no loss (ALS)
+    bool safeguard;     // the epoch runs under the rollback safeguard (lrk_epoch.cuh)
+    bool damped;        // staleness-aware item step: the SGD kernels read the item degrees and mean |p_u|^2
+    bool multi_gpu;     // DSGD / multi-device handle
+    int biases;         // 0: none; 1: item biases (lrk_set_factors requires bi; user biases stay zero); 2: user and item biases.
+                        // Predictions add b_i + p_u.q_i (+ b_u + mu) when > 0
+    bool rating;        // BiasedMF / PMF: the rating is the target (item-run tiles, reference-order mode, user-group kernel)
+    bool als;           // WRMF / eALS: alternating least squares on the fp64 masters (als.cuh); lrk_sgd_epoch = one ALS iteration
+    bool f64_working;   // the fp64 masters are the working set: an epoch leaves them valid (lrk_model_info sets it)
+};
+static const LrkModelInfo k_lrk_models[] = {
+    //                scale  guard  damped multi  biases rating als
+    /* BiasedMF */ {0.5, true,  true,  true,  2, true,  false},
+    /* PMF      */ {0.5, true,  true,  true,  0, true,  false},
+    /* BPR      */ {1.0, true,  false, true,  0, false, false},
+    /* RankSGD  */ {0.5, true,  true,  false, 0, false, false},
+    /* GBPR     */ {1.0, false, false, false, 1, false, false},
+    /* SVD++    */ {0.5, false, false, false, 2, false, false},
+    /* AoBPR    */ {1.0, true,  false, false, 0, false, false},
+    /* WRMF     */ {0.0, false, false, false, 0, false, true},
+    /* eALS     */ {0.0, false, false, false, 0, false, true},
+};
+static inline bool lrk_model_known(int model) { return model >= 0 && model < (int)(sizeof k_lrk_models / sizeof k_lrk_models[0]); }
+// the row of cfg.model, for cfg.update_mode: the reference-order mode works on the fp64 masters, single-GPU, without the safeguard
+static inline LrkModelInfo lrk_model_info(const lrk_config_t& cfg) {
+    LrkModelInfo m = k_lrk_models[cfg.model];
+    m.f64_working = m.als;
+    if (cfg.update_mode == LRK_UPDATE_REFERENCE_ORDER) { m.safeguard = false; m.multi_gpu = false; m.f64_working = true; }
+    return m;
+}
+static const char* const k_lrk_single_gpu = "reference-order mode, RankSGD, GBPR, SVD++, AoBPR, WRMF and eALS are single-GPU in this build";
+static inline bool lrk_has_bias(const lrk_handle_s* h) { return k_lrk_models[h->cfg.model].biases > 0; }
+
+// Calls f(G, V) with the handle's layout (layout_for_k) as std::integral_constant arguments: a generic lambda instantiates its
+// kernel for each layout, e.g. [&](auto g, auto v) { return launch_gv<decltype(g)::value, decltype(v)::value>(h, p); }
+template <class F>
+static int lrk_with_layout(lrk_handle_s* h, F&& f) {
+    using std::integral_constant;
+    switch (h->G * 100 + h->V) {
+        case 101: return f(integral_constant<int, 1>{}, integral_constant<int, 1>{});
+        case 201: return f(integral_constant<int, 2>{}, integral_constant<int, 1>{});
+        case 401: return f(integral_constant<int, 4>{}, integral_constant<int, 1>{});
+        case 801: return f(integral_constant<int, 8>{}, integral_constant<int, 1>{});
+        case 1601: return f(integral_constant<int, 16>{}, integral_constant<int, 1>{});
+        case 3201: return f(integral_constant<int, 32>{}, integral_constant<int, 1>{});
+        case 3202: return f(integral_constant<int, 32>{}, integral_constant<int, 2>{});
+        default: return lrk_fail(h, LRK_ERR_INVALID, "lrk_with_layout", "unsupported factor layout", __FILE__, __LINE__);
+    }
+}

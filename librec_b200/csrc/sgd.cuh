@@ -59,7 +59,7 @@ struct SgdParams {
     // [item-run tiles | shuffled remainder], the multiplicative walk interleaves the two evenly in time
     int64_t tile_mul;
     double hot_share;       // largest share one item has of this launch's ratings (0 = unknown): stability cap of the grid
-    int conc_div;           // >= 1: divisor of the grid (rollback safeguard, lrk_common.cuh)
+    int conc_div;           // >= 1: divisor of the grid (rollback safeguard, lrk_epoch.cuh)
     // staleness-aware step of item-run tiles: item_deg[i] = ratings of item i in this launch (NULL = off),
     // inflight_frac = (ratings in flight) / n, filled in by the launcher
     const uint32_t* item_deg;
@@ -75,11 +75,7 @@ struct SgdParams {
     const int32_t* __restrict__ col;
     int32_t U, I;
     uint32_t seed_lo, seed_hi, epoch;
-    // BPR under DSGD: positives and negatives are drawn inside the item block [blk_lo, blk_hi) the rank holds
-    // (blk_hi == 0: whole catalogue); Q then addresses the block buffer (row = item - blk_lo); sample_base keeps the
-    // Philox counters of the strata of one epoch apart
-    int32_t blk_lo, blk_hi;
-    int64_t sample_base;
+    int64_t sample_base;    // first Philox sample counter of this launch (the windows of one epoch draw from disjoint ranges)
     // AoBPR only (adaptive oversampling, AoBPRRecommender.java:100-138): per-factor item rankings, factor variances and the
     // cumulative rank distribution, refreshed by the host every |I| ln |I| samples (sgd_aobpr.cuh)
     const int32_t* __restrict__ ao_rank;   // [k][I]: ao_rank[f * I + r] = item of rank r in factor f (descending value)
@@ -202,49 +198,6 @@ __device__ __forceinline__ void bpr_draw(const SgdParams& p, int64_t s_in, int32
     u = -1; pi = 0; nj = 0;
 }
 
-// first index in [b, e) with col >= x
-__device__ __forceinline__ int64_t row_lower_bound(const int32_t* __restrict__ col, int64_t b, int64_t e, int32_t x) {
-    while (b < e) {
-        const int64_t m = (b + e) >> 1;
-        if (__ldg(col + m) < x) b = m + 1; else e = m;
-    }
-    return b;
-}
-// Stratified BPR draw for DSGD (SURVEY.md 8e): user uniform over local users that have at least one and not all
-// items of the held block [blk_lo, blk_hi) in their train row; positive uniform over the row's items in the
-// block; negative uniform over the block's items outside the row (rejection).  Same structure as
-// BPRRecommender.java:54-67 restricted to the stratum.
-__device__ __forceinline__ void bpr_draw_block(const SgdParams& p, int64_t s, int32_t& u, int32_t& pi, int32_t& nj) {
-    const uint2 key = make_uint2(p.seed_lo, p.seed_hi);
-    const uint32_t width = (uint32_t)(p.blk_hi - p.blk_lo);
-    const int64_t sc = s + p.sample_base;
-    uint32_t attempt = 0;
-    // bounded like bpr_draw: a block in which no local user has both a positive and a free negative (width 1, or every user
-    // with ratings in the block has rated all of it) is skipped by the host (DsgdState::bpr_qualify); the cap covers the rest
-    while (attempt < LRK_BPR_MAX_ATTEMPTS) {
-        uint4 x = philox4x32_10(make_uint4((uint32_t)sc, (uint32_t)(sc >> 32), p.epoch, attempt++), key);
-        u = (int32_t)__umulhi(x.x, (uint32_t)p.U);
-        const int64_t rb = __ldg(p.rowptr + u), re = __ldg(p.rowptr + u + 1);
-        const int64_t b = row_lower_bound(p.col, rb, re, p.blk_lo), e = row_lower_bound(p.col, b, re, p.blk_hi);
-        const int64_t len = e - b;
-        if (len == 0 || len == (int64_t)width) continue;
-        pi = __ldg(p.col + b + (int64_t)__umulhi(x.y, (uint32_t)len));
-        nj = p.blk_lo + (int32_t)__umulhi(x.z, width);
-        if (!row_contains(p.col, b, e, nj)) return;
-        nj = p.blk_lo + (int32_t)__umulhi(x.w, width);
-        if (!row_contains(p.col, b, e, nj)) return;
-        for (const uint32_t stop = attempt + LRK_BPR_MAX_ATTEMPTS; attempt < stop;) {
-            x = philox4x32_10(make_uint4((uint32_t)sc, (uint32_t)(sc >> 32), p.epoch, attempt++), key);
-            nj = p.blk_lo + (int32_t)__umulhi(x.x, width); if (!row_contains(p.col, b, e, nj)) return;
-            nj = p.blk_lo + (int32_t)__umulhi(x.y, width); if (!row_contains(p.col, b, e, nj)) return;
-            nj = p.blk_lo + (int32_t)__umulhi(x.z, width); if (!row_contains(p.col, b, e, nj)) return;
-            nj = p.blk_lo + (int32_t)__umulhi(x.w, width); if (!row_contains(p.col, b, e, nj)) return;
-        }
-        break;
-    }
-    u = -1; pi = p.blk_lo; nj = p.blk_lo;
-}
-
 // AoBPR draw (AoBPRRecommender.java:100-138): a train ENTRY uniformly (u, i) -- the staged stream is a permutation of the entries, so
 // a uniform stream position is a uniform entry --, then the negative by adaptive oversampling: rank r from the geometric-like step
 // distribution exp(-((r + 1) / lambda)), factor f with probability |p_uf| var_f / sum, item = the r-th item of factor f's ranking
@@ -297,9 +250,7 @@ __global__ void bpr_peek_kernel(SgdParams p, int64_t first, int64_t n, int32_t* 
     out[3 * t] = u; out[3 * t + 1] = pi; out[3 * t + 2] = nj;
 }
 
-// BLOCKED: DSGD stratum (positives and negatives inside the held item block); a separate instantiation so that the
-// single-GPU kernel does not carry the second sampler (it cost 32 % of its throughput as a run-time branch)
-template <int G, int V, bool ATOMIC, bool BLOCKED = false, bool AOBPR = false>
+template <int G, int V, bool ATOMIC, bool AOBPR = false>
 __global__ void __launch_bounds__(256) sgd_bpr_epoch_kernel(SgdParams p) {
     constexpr int RPS = 32 / G;
     constexpr int STEPS = G;
@@ -317,8 +268,7 @@ __global__ void __launch_bounds__(256) sgd_bpr_epoch_kernel(SgdParams p) {
         {
             const int64_t s = (tile << 5) + lane;
             if (s < p.n) {
-                if (BLOCKED) { bpr_draw_block(p, s, u_l, i_l, j_l); i_l -= p.blk_lo; j_l -= p.blk_lo; }
-                else if (AOBPR) aobpr_draw(p, s, u_l, i_l, j_l);
+                if (AOBPR) aobpr_draw(p, s, u_l, i_l, j_l);
                 else bpr_draw(p, s, u_l, i_l, j_l);
             }
         }
@@ -628,8 +578,7 @@ static int sgd_launch_gv(lrk_handle_s* h, const SgdParams& sp_in) {
     } else if (h->cfg.model == LRK_MODEL_RANKSGD) {
         if (atomic) LRK_GO((sgd_ranksgd_epoch_kernel<G, V, true>)); else LRK_GO((sgd_ranksgd_epoch_kernel<G, V, false>));
     } else {
-        if (sp.ao_rank) { if (atomic) LRK_GO((sgd_bpr_epoch_kernel<G, V, true, false, true>)); else LRK_GO((sgd_bpr_epoch_kernel<G, V, false, false, true>)); }
-        else if (sp.blk_hi > 0) { if (atomic) LRK_GO((sgd_bpr_epoch_kernel<G, V, true, true>)); else LRK_GO((sgd_bpr_epoch_kernel<G, V, false, true>)); }
+        if (sp.ao_rank) { if (atomic) LRK_GO((sgd_bpr_epoch_kernel<G, V, true, true>)); else LRK_GO((sgd_bpr_epoch_kernel<G, V, false, true>)); }
         else if (atomic) LRK_GO((sgd_bpr_epoch_kernel<G, V, true>)); else LRK_GO((sgd_bpr_epoch_kernel<G, V, false>));
     }
 #undef LRK_GO
@@ -638,14 +587,5 @@ static int sgd_launch_gv(lrk_handle_s* h, const SgdParams& sp_in) {
 }
 
 static int sgd_launch(lrk_handle_s* h, const SgdParams& sp) {
-    switch (h->G * 100 + h->V) {
-        case 101: return sgd_launch_gv<1, 1>(h, sp);
-        case 201: return sgd_launch_gv<2, 1>(h, sp);
-        case 401: return sgd_launch_gv<4, 1>(h, sp);
-        case 801: return sgd_launch_gv<8, 1>(h, sp);
-        case 1601: return sgd_launch_gv<16, 1>(h, sp);
-        case 3201: return sgd_launch_gv<32, 1>(h, sp);
-        case 3202: return sgd_launch_gv<32, 2>(h, sp);
-        default: return lrk_fail(h, LRK_ERR_INVALID, "sgd_launch", "unsupported factor layout", __FILE__, __LINE__);
-    }
+    return lrk_with_layout(h, [&](auto G, auto V) { return sgd_launch_gv<decltype(G)::value, decltype(V)::value>(h, sp); });
 }

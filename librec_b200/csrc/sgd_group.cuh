@@ -349,7 +349,7 @@ static bool sgd_group_layout_supported(const lrk_handle_s* h) { return h->V == 1
 static bool lrk_use_group_kernel(const lrk_handle_s* h) {
     const char* env = getenv("LRK_SGD_GROUP");
     if (!env || atoi(env) == 0) return false;
-    return lrk_is_rating_model(h) && h->cfg.update_mode == LRK_UPDATE_ATOMIC && sgd_group_layout_supported(h);
+    return k_lrk_models[h->cfg.model].rating && h->cfg.update_mode == LRK_UPDATE_ATOMIC && sgd_group_layout_supported(h);
 }
 
 static int sgd_group_resident_workers(lrk_handle_s* h, int* ctas_out) {
