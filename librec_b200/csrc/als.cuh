@@ -24,23 +24,17 @@
 #include "lrk_epoch.cuh"
 
 struct AlsState {
-    double* d_val = nullptr;        // weighted train values, CSR order (fp64: the weights are log / affine functions of the rating)
-    int64_t* d_colptr = nullptr;    // the same matrix by columns: users ascending (SequentialAccessSparseMatrix.viewColumn)
-    int32_t* d_cusers = nullptr;
-    double* d_cval = nullptr;
-    double* d_gram = nullptr;       // k x k
-    double* d_conf = nullptr;       // eALS: confidences[numItems] (lrk_set_matrix "eals.confidences")
-    double* d_pred = nullptr;       // eALS: per-entry predictions
-    double *d_tn = nullptr, *d_td = nullptr;   // eALS heavy rows: per-entry terms
-    unsigned int* d_counter = nullptr;
+    LrkBuf<double> d_val;           // weighted train values, CSR order (fp64: the weights are log / affine functions of the rating)
+    LrkBuf<int64_t> d_colptr;       // the same matrix by columns: users ascending (SequentialAccessSparseMatrix.viewColumn)
+    LrkBuf<int32_t> d_cusers;
+    LrkBuf<double> d_cval;
+    LrkBuf<double> d_gram;          // k x k
+    LrkBuf<double> d_conf;          // eALS: confidences[numItems] (lrk_set_matrix "eals.confidences")
+    LrkBuf<double> d_pred;          // eALS: per-entry predictions
+    LrkBuf<double> d_tn, d_td;      // eALS heavy rows: per-entry terms
+    LrkBuf<unsigned int> d_counter;
     bool has_conf = false;
 };
-
-static void als_release(AlsState* a) {
-    if (!a) return;
-    cudaFree(a->d_val); cudaFree(a->d_colptr); cudaFree(a->d_cusers); cudaFree(a->d_cval); cudaFree(a->d_gram); cudaFree(a->d_conf); cudaFree(a->d_pred); cudaFree(a->d_tn); cudaFree(a->d_td); cudaFree(a->d_counter);
-    delete a;
-}
 
 #define ALS_MAX_K 112          // [A | I] of the Gauss-Jordan step must fit the 227 KB of shared memory: k (2k + 2) doubles
 
@@ -400,8 +394,8 @@ __global__ void __launch_bounds__(256) als_eals_heavy_kernel(AlsEalsParams p) {
 // the train matrix by columns + the fp64 values (lrk_set_train_csr tail for WRMF / eALS)
 static int als_stage(lrk_handle_s* h, const double* h_val) {
     cudaStream_t st = h->stream;
-    AlsState* a = (AlsState*)h->als;
-    if (!a) { a = new AlsState(); h->als = a; }
+    if (!h->als) h->als.reset(new AlsState());
+    AlsState* a = h->als.get();
     a->has_conf = false;               // confidences belong to a train matrix (EALSRecommender.java:65-83)
     const int64_t nnz = h->nnz;
     const int32_t U = h->U, I = h->I;
@@ -514,7 +508,7 @@ static int als_eals_side(lrk_handle_s* h, const AlsEalsParams& p) {
 
 // one iteration of WRMFRecommender.trainModel / EALSRecommender.trainModel on the fp64 masters; the models have no loss (0 is returned)
 static int als_epoch(lrk_handle_s* h, float reg_u, float reg_i, double* loss_out) {
-    AlsState* a = (AlsState*)h->als;
+    AlsState* a = h->als.get();
     LRK_REQUIRE(h, a != nullptr, "ALS state missing: call lrk_set_train_csr first");
     const bool eals = h->cfg.model == LRK_MODEL_EALS;
     LRK_REQUIRE(h, !eals || a->has_conf, "eALS needs the item confidences: lrk_set_matrix(h, \"eals.confidences\", c)");

@@ -86,18 +86,22 @@ struct DsgdState {
     std::vector<double> seg_hot_share;  // per segment: largest share one item has of its ratings
     int32_t max_blk = 0;                // rows of the largest item block
     size_t buf_floats = 0;              // floats per rotating buffer: max_blk*ld + max_blk
-    float* qbuf[2] = {nullptr, nullptr};
+    LrkBuf<float> qbuf[2];
     int cur = 0;                        // which buffer holds the current block
     int cur_block = 0;                  // item block id currently held
-    int32_t* d_bounds = nullptr;
+    LrkBuf<int32_t> d_bounds;
     // LRK_DSGD_TRACE=1: events around every sub-epoch kernel / ring exchange of the last epoch
     std::vector<cudaEvent_t> trace_ev;
     int trace = -1;
-    float* gather_buf = nullptr;        // lrk_get_factors: all ranks' ring buffers (world * buf_floats)
-    float* q_ref = nullptr;             // BPR: the item factors at the start of the current window (delta all-reduce)
-    float* q_delta = nullptr;
+    LrkBuf<float> gather_buf;           // lrk_get_factors: all ranks' ring buffers (world * buf_floats)
+    LrkBuf<float> q_ref;                // BPR: the item factors at the start of the current window (delta all-reduce)
+    LrkBuf<float> q_delta;
     int64_t bpr_samples = 0;            // BPR: samples this rank draws per epoch = numRates * (its users / all users)
     DsgdFused fused;                    // experimental one-kernel epoch (dsgd_fused.cuh), LRK_DSGD_FUSED=1
+    ~DsgdState() {
+        dsgd_fused_unmap(&fused);       // the IPC mappings go before the ring buffers
+        for (cudaEvent_t ev : trace_ev) if (ev) cudaEventDestroy(ev);
+    }
 };
 
 __global__ void flag_bits_kernel(const int* __restrict__ flags, int* __restrict__ bits) {
@@ -135,17 +139,6 @@ __global__ void dsgd_unpack_block_kernel(float* __restrict__ Q, float* __restric
     const int64_t nq = (int64_t)rows * ld;
     if (t < nq) Q[(int64_t)first * ld + t] = buf[t];
     else if (t < nq + rows && bi) bi[first + (t - nq)] = buf[(int64_t)max_blk * ld + (t - nq)];
-}
-
-static void dsgd_release(lrk_handle_s* h) {
-    DsgdState* s = (DsgdState*)h->dsgd;
-    if (s) {
-        dsgd_fused_release(&s->fused);
-        cudaFree(s->qbuf[0]); cudaFree(s->qbuf[1]); cudaFree(s->d_bounds); cudaFree(s->q_ref); cudaFree(s->q_delta); cudaFree(s->gather_buf);
-        delete s;
-        h->dsgd = nullptr;
-    }
-    if (h->comm && nccl_api()) { nccl_api()->CommDestroy((ncclComm_t)h->comm); h->comm = nullptr; }
 }
 
 static int dsgd_unique_id(uint8_t* out) {
@@ -195,8 +188,8 @@ static int dsgd_set_train_csr(lrk_handle_s* h, int32_t U, int32_t I, const int64
     cudaStream_t st = h->stream;
     const int world = h->world;
     const int64_t nnz = rowptr[U];
-    DsgdState* s = (DsgdState*)h->dsgd;
-    if (!s) { s = new DsgdState(); h->dsgd = s; }
+    if (!h->dsgd) h->dsgd.reset(new DsgdState());
+    DsgdState* s = h->dsgd.get();
     h->has_train = false;
     int rc;
     if ((rc = lrk_dev_alloc(h, &h->d_rowptr, (size_t)U + 1))) return rc;
@@ -276,15 +269,12 @@ static int dsgd_set_train_csr(lrk_handle_s* h, int32_t U, int32_t I, const int64
     s->seg_off.assign((size_t)world + 1, 0);
     s->seg_hot_share.assign((size_t)world, 0.0);
     dsgd_block_counts_kernel<<<ib, 256, 0, st>>>(h->d_item_deg, I, s->d_bounds, world, d_small); LRK_LAUNCH_CHECK(h);
-    group_units_release((GroupUnits*)h->group);
-    h->group = nullptr;
+    h->group.reset();
     const bool want_group = lrk_use_group_kernel(h) && group_order_supported(U, I, nnz, world);
     if (nnz > 0 && want_group) {
-        GroupUnits* gu = nullptr;
         LRK_CUDA(h, cudaMemsetAsync(w.max_deg, 0, sizeof(uint32_t) * 64, st));
         if ((rc = stage_group_stream(h, h->d_rowptr, h->d_col, row_of, d_val, U, I, nnz, s->d_bounds, world, sgd_group_resident_workers(h, nullptr),
-                                     h->cfg.seed + 977u * h->rank, sc, w.tmp, tmp_bytes, keys, keys2, idx, perm, h->d_su, h->d_si, h->d_sr, &gu))) return rc;
-        h->group = gu;
+                                     h->cfg.seed + 977u * h->rank, sc, w.tmp, tmp_bytes, keys, keys2, idx, perm, h->d_su, h->d_si, h->d_sr, &h->group))) return rc;
     } else if (nnz > 0) {
         if ((rc = stage_tile_keys(h, h->d_col, I, nnz, s->d_bounds, world, h->cfg.seed + 977u * h->rank, w, keys, idx))) return rc;
         size_t tb = tmp_bytes;
@@ -328,7 +318,7 @@ static int dsgd_set_train_csr(lrk_handle_s* h, int32_t U, int32_t I, const int64
 
 // P/bu: the rank's user block; Q/bi: the FULL item factors (identical on every rank)
 static int dsgd_set_factors(lrk_handle_s* h, const double* P, const double* Q, const double* bu, const double* bi, double mu) {
-    DsgdState* s = (DsgdState*)h->dsgd;
+    DsgdState* s = h->dsgd.get();
     cudaStream_t st = h->stream;
     const int k = h->k, ld = h->ld;
     const int64_t U = h->U, I = h->I;
@@ -380,9 +370,10 @@ static int dsgd_fused_map(lrk_handle_s* h, DsgdState* s) {
     cudaStream_t st = h->stream;
     const int world = h->world, rank = h->rank;
     if (f->mapped && f->my_qbuf[0] == s->qbuf[0] && f->my_qbuf[1] == s->qbuf[1]) return LRK_OK;
-    dsgd_fused_release(f);
-    LRK_CUDA(h, cudaMalloc((void**)&f->d_flags, sizeof(unsigned long long) * 4));
-    LRK_CUDA(h, cudaMalloc((void**)&f->d_abort, sizeof(int)));
+    dsgd_fused_unmap(f);
+    int rc;
+    if ((rc = lrk_dev_alloc(h, &f->d_flags, 4))) return rc;
+    if ((rc = lrk_dev_alloc(h, &f->d_abort, 1))) return rc;
     LRK_CUDA(h, cudaMemsetAsync(f->d_flags, 0, sizeof(unsigned long long) * 4, st));
     LRK_CUDA(h, cudaMemsetAsync(f->d_abort, 0, sizeof(int), st));
     // handles of (qbuf[0], qbuf[1], flags) of every rank.  A rank on which CUDA IPC does not work (other container, allocator without
@@ -395,16 +386,15 @@ static int dsgd_fused_map(lrk_handle_s* h, DsgdState* s) {
                         cudaIpcGetMemHandle(&mine[2], f->d_flags) == cudaSuccess);
     cudaGetLastError();
     const size_t hb = sizeof(cudaIpcMemHandle_t) * 3;
-    uint8_t *d_mine = nullptr, *d_all = nullptr;
-    LRK_CUDA(h, cudaMalloc((void**)&d_mine, hb));
-    LRK_CUDA(h, cudaMalloc((void**)&d_all, hb * (size_t)world));
+    LrkBuf<uint8_t> d_mine, d_all;
+    if ((rc = lrk_dev_alloc(h, &d_mine, hb))) return rc;
+    if ((rc = lrk_dev_alloc(h, &d_all, hb * (size_t)world))) return rc;
     std::vector<uint8_t> all(hb * (size_t)world);
     cudaError_t e = cudaMemcpyAsync(d_mine, mine, hb, cudaMemcpyHostToDevice, st);
     ncclResult_t nr = ncclSuccess;
     if (e == cudaSuccess) nr = n->AllGather(d_mine, d_all, hb, ncclUint8, (ncclComm_t)h->comm, st);
     if (e == cudaSuccess && nr == ncclSuccess) e = cudaMemcpyAsync(all.data(), d_all, all.size(), cudaMemcpyDeviceToHost, st);
     if (e == cudaSuccess && nr == ncclSuccess) e = cudaStreamSynchronize(st);
-    cudaFree(d_mine); cudaFree(d_all);
     LRK_NCCL(h, nr);
     LRK_CUDA(h, e);
     auto handle_of = [&](int r, int which) {
@@ -430,8 +420,8 @@ static int dsgd_fused_map(lrk_handle_s* h, DsgdState* s) {
             cudaGetLastError();
             return true;
         };
-        DsgdState* ps = (DsgdState*)h->siblings[prev]->dsgd;
-        DsgdState* ns = (DsgdState*)h->siblings[next]->dsgd;
+        DsgdState* ps = h->siblings[prev]->dsgd.get();
+        DsgdState* ns = h->siblings[next]->dsgd.get();
         ok = ps && ns && ps->fused.d_flags && ns->fused.d_flags && peer(prev) && peer(next);
         if (ok) { q0 = ps->qbuf[0]; q1 = ps->qbuf[1]; pf = ps->fused.d_flags; nf = ns->fused.d_flags; }
     } else {
@@ -446,7 +436,7 @@ static int dsgd_fused_map(lrk_handle_s* h, DsgdState* s) {
     LRK_CUDA(h, cudaMemsetAsync(f->d_abort, 0, sizeof(int), st));
     LRK_CUDA(h, cudaStreamSynchronize(st));
     if (!verdict) {
-        dsgd_fused_release(f);
+        dsgd_fused_unmap(f);
         f->enabled = 0;                  // this communicator keeps the NCCL ring
         return LRK_OK;
     }
@@ -535,7 +525,7 @@ static int dsgd_fused_epoch(lrk_handle_s* h, DsgdState* s, float lr, float reg_u
         f->needs_reset = false;
     }
     if (h->group) {
-        GroupUnits* gu = (GroupUnits*)h->group;
+        GroupUnits* gu = h->group.get();
         DsgdFusedGroupParams gp;
         memset(&gp, 0, sizeof gp);
         int ctas = 0;
@@ -590,7 +580,7 @@ static int dsgd_fused_epoch(lrk_handle_s* h, DsgdState* s, float lr, float reg_u
         sp.tile_mul = sgd_tile_mul(cnt);
         sp.conc_div = h->conc_div;
         sp.item_deg = h->d_item_deg ? h->d_item_deg + s->bounds[(size_t)b] : nullptr;
-        sp.pnorm2 = sp.item_deg ? h->d_pnorm2 : nullptr;
+        sp.pnorm2 = sp.item_deg ? h->d_pnorm2.ptr : nullptr;
         sp.hot_flush_deg = hf ? (atoi(hf) > 0 ? (uint32_t)atoi(hf) : 0xffffffffu) : 512u;
     }
     fp.qbuf[0] = s->qbuf[0]; fp.qbuf[1] = s->qbuf[1];
@@ -656,7 +646,7 @@ static int dsgd_bpr_epoch(lrk_handle_s* h, DsgdState* s, float lr, float reg_u, 
 
 static int dsgd_epoch(lrk_handle_s* h, float lr, float reg_u, float reg_i, double reg_b, int32_t epoch_idx, double* loss_out) {
     NcclApi* n = nccl_api();
-    DsgdState* s = (DsgdState*)h->dsgd;
+    DsgdState* s = h->dsgd.get();
     cudaStream_t st = h->stream;
     const int world = h->world, rank = h->rank;
     const bool bpr_ = h->cfg.model == LRK_MODEL_BPR;
@@ -673,7 +663,7 @@ static int dsgd_epoch(lrk_handle_s* h, float lr, float reg_u, float reg_i, doubl
     if (h->h_pnorm2) { h->pnorm2_prev = h->pnorm2_host; h->pnorm2_host = *h->h_pnorm2; }
     bool fused_done = false;
     e.enqueue = [&](int) -> int {
-        if (h->group) LRK_CUDA(h, cudaMemsetAsync(((GroupUnits*)h->group)->d_counter, 0, sizeof(unsigned int) * 64, st));
+        if (h->group) LRK_CUDA(h, cudaMemsetAsync(h->group->d_counter, 0, sizeof(unsigned int) * 64, st));
         if (s->trace < 0) { const char* t = getenv("LRK_DSGD_TRACE"); s->trace = t && atoi(t) ? 1 : 0; }
         if (s->trace && s->trace_ev.empty()) {
             s->trace_ev.resize((size_t)2 * world + 1);
@@ -698,8 +688,8 @@ static int dsgd_epoch(lrk_handle_s* h, float lr, float reg_u, float reg_i, doubl
                 sp.hot_share = (size_t)b < s->seg_hot_share.size() ? s->seg_hot_share[(size_t)b] : 0.0;
                 sp.conc_div = h->conc_div;
                 sp.item_deg = h->d_item_deg ? h->d_item_deg + s->bounds[(size_t)b] : nullptr;   // block-local item ids
-                sp.pnorm2 = sp.item_deg ? h->d_pnorm2 : nullptr;
-                GroupUnits* gu = (GroupUnits*)h->group;
+                sp.pnorm2 = sp.item_deg ? h->d_pnorm2.ptr : nullptr;
+                GroupUnits* gu = h->group.get();
                 if (gu) {
                     SgdGroupParams gp;
                     memset(&gp, 0, sizeof gp);
@@ -758,7 +748,7 @@ static int dsgd_epoch(lrk_handle_s* h, float lr, float reg_u, float reg_i, doubl
 // P/bu: the rank's user block; Q/bi: the full item factors, gathered from the ring
 static int dsgd_get_factors(lrk_handle_s* h, double* P, double* Q, double* bu, double* bi) {
     NcclApi* n = nccl_api();
-    DsgdState* s = (DsgdState*)h->dsgd;
+    DsgdState* s = h->dsgd.get();
     cudaStream_t st = h->stream;
     const int world = h->world;
     const int64_t U = h->U, I = h->I;
@@ -778,7 +768,7 @@ static int dsgd_get_factors(lrk_handle_s* h, double* P, double* Q, double* bu, d
             const int32_t first = s->bounds[b], rows = s->bounds[b + 1] - first;
             if (rows > 0) {
                 dsgd_unpack_block_kernel<<<lrk_ceil_div((int64_t)rows * h->ld + rows, 256), 256, 0, st>>>(
-                    h->Q32, biased ? h->bi32 : nullptr, first, rows, h->ld, s->max_blk, all + s->buf_floats * (size_t)r);
+                    h->Q32, biased ? h->bi32.ptr : nullptr, first, rows, h->ld, s->max_blk, all + s->buf_floats * (size_t)r);
                 h->launches++;
                 e = cudaGetLastError();
             }

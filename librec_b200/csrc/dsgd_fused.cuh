@@ -168,8 +168,8 @@ struct DsgdFused {
     int enabled = -1;                        // -1: environment not read yet
     bool mapped = false;
     float* my_qbuf[2] = {nullptr, nullptr};  // the buffers the mappings were made for
-    unsigned long long* d_flags = nullptr;   // [0,1] ready, [2,3] peer_free
-    int* d_abort = nullptr;
+    LrkBuf<unsigned long long> d_flags;      // [0,1] ready, [2,3] peer_free
+    LrkBuf<int> d_abort;
     float* peer_qbuf[2] = {nullptr, nullptr};
     unsigned long long* prev_flags = nullptr;
     unsigned long long* next_flags = nullptr;
@@ -179,9 +179,8 @@ struct DsgdFused {
     bool needs_reset = false;                // lrk_set_factors re-packed the ring (buffer 0 holds the block again): restart the flag sequence
 };
 
-static void dsgd_fused_release(DsgdFused* f) {
+static void dsgd_fused_unmap(DsgdFused* f) {
     for (int i = 0; i < f->n_opened; ++i) if (f->opened[i]) cudaIpcCloseMemHandle(f->opened[i]);
     f->n_opened = 0;
-    cudaFree(f->d_flags); cudaFree(f->d_abort);
-    f->d_flags = nullptr; f->d_abort = nullptr; f->mapped = false;
+    f->d_flags.reset(); f->d_abort.reset(); f->mapped = false;
 }

@@ -46,11 +46,11 @@ static int l2_probe_run(lrk_handle_s* h, size_t working_set_bytes, int row_float
     const int G = row_floats / 4;
     const uint32_t rows = (uint32_t)(working_set_bytes / (sizeof(float) * (size_t)row_floats));
     LRK_REQUIRE(h, rows >= 1024, "working set too small");
-    float* buf = nullptr;
-    float* sink = nullptr;
-    LRK_CUDA(h, cudaMalloc((void**)&buf, sizeof(float) * (size_t)rows * row_floats));
-    cudaError_t e = cudaMalloc((void**)&sink, sizeof(float));
-    if (e == cudaSuccess) e = cudaMemsetAsync(buf, 0, sizeof(float) * (size_t)rows * row_floats, st);
+    LrkBuf<float> buf, sink;
+    int rc;
+    if ((rc = lrk_dev_alloc(h, &buf, (size_t)rows * row_floats))) return rc;
+    if ((rc = lrk_dev_alloc(h, &sink, 1))) return rc;
+    cudaError_t e = cudaMemsetAsync(buf, 0, sizeof(float) * (size_t)rows * row_floats, st);
     cudaEvent_t e0 = nullptr, e1 = nullptr;
     if (e == cudaSuccess) e = cudaEventCreate(&e0);
     if (e == cudaSuccess) e = cudaEventCreate(&e1);
@@ -82,7 +82,6 @@ static int l2_probe_run(lrk_handle_s* h, size_t working_set_bytes, int row_float
     }
     if (e0) cudaEventDestroy(e0);
     if (e1) cudaEventDestroy(e1);
-    cudaFree(buf); cudaFree(sink);
     LRK_CUDA(h, e);
     return LRK_OK;
 }

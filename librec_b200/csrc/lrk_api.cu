@@ -35,8 +35,8 @@ static int multi_topn(lrk_handle_s* h, const int32_t* users, int32_t nq, int32_t
 // GBPR: train CSC (users of every item, ascending) next to the CSR -- the group draws of GBPRRecommender.java:104-116 walk an item's column
 static int gbpr_stage(lrk_handle_s* h) {
     cudaStream_t st = h->stream;
-    GbprState* g = (GbprState*)h->gbpr;
-    if (!g) { g = new GbprState(); h->gbpr = g; }
+    if (!h->gbpr) h->gbpr.reset(new GbprState());
+    GbprState* g = h->gbpr.get();
     const int64_t nnz = h->nnz;
     const int32_t U = h->U, I = h->I;
     int rc;
@@ -65,13 +65,13 @@ static int gbpr_stage(lrk_handle_s* h) {
     LRK_CUDA(h, cub::DeviceScan::ExclusiveSum(tmp, t1, deg, deg_ex, (int)I, st));
     gbpr_colptr_kernel<<<lrk_ceil_div(I, 256), 256, 0, st>>>(deg_ex, deg, I, g->d_colptr); LRK_LAUNCH_CHECK(h);
     t1 = tb;
-    LRK_CUDA(h, cub::DeviceRadixSort::SortPairs(tmp, t1, k_in, k_out, rows, g->d_cusers, (int)nnz, 0, end_bit, st));   // stable: users ascending
+    LRK_CUDA(h, cub::DeviceRadixSort::SortPairs(tmp, t1, k_in, k_out, rows, g->d_cusers.ptr, (int)nnz, 0, end_bit, st));   // stable: users ascending
     LRK_CUDA(h, cudaStreamSynchronize(st));
     return LRK_OK;
 }
 
 static int gbpr_fill(lrk_handle_s* h, GbprParams& p, float lr, float reg_u, float reg_i, double reg_b, int32_t epoch_idx) {
-    GbprState* g = (GbprState*)h->gbpr;
+    GbprState* g = h->gbpr.get();
     memset(&p, 0, sizeof p);
     p.n = h->nnz; p.P = h->P32; p.Q = h->Q32; p.tP = g->tP; p.tQ = g->tQ; p.bi = h->bi32;
     p.lr = lr; p.reg_u = reg_u; p.reg_i = reg_i; p.reg_b = (float)reg_b; p.rho = g->rho; p.glen = g->glen;
@@ -98,7 +98,7 @@ static int gbpr_launch_gv(lrk_handle_s* h, const GbprParams& p) {
 
 // one GBPR iteration: GBPRRecommender.java:84-168
 static int gbpr_epoch(lrk_handle_s* h, float lr, float reg_u, float reg_i, double reg_b, int32_t epoch_idx, double* loss_out) {
-    GbprState* g = (GbprState*)h->gbpr;
+    GbprState* g = h->gbpr.get();
     LRK_REQUIRE(h, g != nullptr, "GBPR state missing: call lrk_set_train_csr first");
     cudaStream_t st = h->stream;
     const size_t np_ = (size_t)h->U * h->ld, nq_ = (size_t)h->I * h->ld;
@@ -124,8 +124,8 @@ static int gbpr_epoch(lrk_handle_s* h, float lr, float reg_u, float reg_i, doubl
 // SVD++: train values in CSR order + users by descending degree
 static int svdpp_stage(lrk_handle_s* h, const double* h_val) {
     cudaStream_t st = h->stream;
-    SvdppState* g = (SvdppState*)h->svdpp;
-    if (!g) { g = new SvdppState(); h->svdpp = g; }
+    if (!h->svdpp) h->svdpp.reset(new SvdppState());
+    SvdppState* g = h->svdpp.get();
     const int64_t nnz = h->nnz;
     const int32_t U = h->U;
     int rc;
@@ -146,7 +146,7 @@ static int svdpp_stage(lrk_handle_s* h, const double* h_val) {
         f64_to_f32_kernel<<<lrk_ceil_div(nnz, 256), 256, 0, st>>>(d_val, g->d_cval, nnz); LRK_LAUNCH_CHECK(h);
     }
     svdpp_deg_kernel<<<lrk_ceil_div(U, 256), 256, 0, st>>>(h->d_rowptr, U, deg, ids); LRK_LAUNCH_CHECK(h);
-    LRK_CUDA(h, cub::DeviceRadixSort::SortPairsDescending(tmp, tb, deg, deg2, ids, g->d_uorder, (int)U, 0, 32, st));
+    LRK_CUDA(h, cub::DeviceRadixSort::SortPairsDescending(tmp, tb, deg, deg2, ids, g->d_uorder.ptr, (int)U, 0, 32, st));
     LRK_CUDA(h, cudaStreamSynchronize(st));
     return LRK_OK;
 }
@@ -169,7 +169,7 @@ static int svdpp_launch_gv(lrk_handle_s* h, const SvdppParams& p) {
 
 // one SVD++ iteration: SVDPlusPlusRecommender.java:63-109
 static int svdpp_epoch(lrk_handle_s* h, float lr, float reg_u, float reg_i, double reg_b, double* loss_out) {
-    SvdppState* g = (SvdppState*)h->svdpp;
+    SvdppState* g = h->svdpp.get();
     LRK_REQUIRE(h, g != nullptr && g->has_y, "SVD++ needs impItemFactors: lrk_set_matrix(h, \"svdpp.y\", Y) after lrk_set_factors");
     cudaStream_t st = h->stream;
     SvdppParams p;
@@ -260,7 +260,7 @@ int lrk_create(const lrk_config_t* cfg, lrk_handle_t* out) {
         if (cudaStreamCreateWithFlags(&h->own_stream, cudaStreamNonBlocking) != cudaSuccess) { rc = LRK_ERR_CUDA; break; }
         h->stream = h->own_stream;
         if (cudaEventCreate(&h->ev0) != cudaSuccess || cudaEventCreate(&h->ev1) != cudaSuccess) { rc = LRK_ERR_CUDA; break; }
-        if (cudaMalloc((void**)&h->d_loss, 64) != cudaSuccess) { rc = LRK_ERR_NOMEM; break; }
+        if (lrk_dev_alloc(h, &h->d_loss, 8) != LRK_OK) { rc = LRK_ERR_NOMEM; break; }
         if (cudaMallocHost((void**)&h->h_loss, 64) != cudaSuccess) { rc = LRK_ERR_NOMEM; break; }
     } while (0);
     if (rc != LRK_OK) {
@@ -277,31 +277,6 @@ int lrk_destroy(lrk_handle_t h) {
     if (h->multi) return multi_destroy(h);
     cudaSetDevice(h->cfg.device);
     if (h->stream) cudaStreamSynchronize(h->stream);
-    group_units_release((GroupUnits*)h->group);
-    gbpr_release((GbprState*)h->gbpr);
-    svdpp_release((SvdppState*)h->svdpp);
-    aobpr_release((AobprState*)h->aobpr);
-    als_release((AlsState*)h->als);
-    dsgd_release(h);
-    topn_tc_release(h);
-    exact_release((ExactSchedule*)h->exact);
-    lrk_dev_free(&h->d_rowptr); lrk_dev_free(&h->d_col);
-    lrk_dev_free(&h->d_su); lrk_dev_free(&h->d_si); lrk_dev_free(&h->d_sr);
-    lrk_dev_free(&h->P32); lrk_dev_free(&h->Q32); lrk_dev_free(&h->bu32); lrk_dev_free(&h->bi32);
-    lrk_dev_free(&h->P64); lrk_dev_free(&h->Q64); lrk_dev_free(&h->bu64); lrk_dev_free(&h->bi64);
-    lrk_dev_free(&h->d_loss);
-    lrk_dev_free(&h->d_item_deg); lrk_dev_free(&h->d_item_cum); lrk_dev_free(&h->d_pnorm2);
-    lrk_dev_free(&h->bk_P); lrk_dev_free(&h->bk_Q); lrk_dev_free(&h->bk_bu); lrk_dev_free(&h->bk_bi);
-    lrk_dev_free(&h->tn_users); lrk_dev_free(&h->tn_items); lrk_dev_free(&h->tn_scores); lrk_dev_free(&h->tn_counts);
-    if (h->scratch) cudaFree(h->scratch);
-    if (h->h_loss) cudaFreeHost(h->h_loss);
-    if (h->h_pnorm2) cudaFreeHost(h->h_pnorm2);
-    if (h->ev0) cudaEventDestroy(h->ev0);
-    if (h->ev1) cudaEventDestroy(h->ev1);
-    if (h->copy_stream) cudaStreamDestroy(h->copy_stream);
-    if (h->ev_copy0) cudaEventDestroy(h->ev_copy0);
-    if (h->ev_copy1) cudaEventDestroy(h->ev_copy1);
-    if (h->own_stream) cudaStreamDestroy(h->own_stream);
     delete h;
     return LRK_OK;
 }
@@ -352,33 +327,25 @@ int lrk_set_train_csr(lrk_handle_t h, int32_t U, int32_t I, const int64_t* rowpt
     }
     // BiasedMF / PMF in the default (atomic) mode train with the user-group kernel over a unit-ordered stream (sgd_group.cuh);
     // Hogwild mode, the reference-order mode, BPR / RankSGD and layouts outside 32 < ld <= 128 keep the shuffled stream of sgd.cuh
-    group_units_release((GroupUnits*)h->group);
-    h->group = nullptr;
+    h->group.reset();
     const bool want_group = lrk_use_group_kernel(h) && group_order_supported(U, I, nnz, 1);
-    GroupUnits* gu = nullptr;
     rc = stage_coo_from_csr(h, h->d_rowptr, h->d_col, val, U, I, nnz, h->d_su, h->d_si, h->d_sr, /*validate=*/true,
-                            want_group ? sgd_group_resident_workers(h, nullptr) : 0, &gu);
+                            want_group ? sgd_group_resident_workers(h, nullptr) : 0, &h->group);
     if (rc) return rc;
-    h->group = gu;
     if (h->cfg.model == LRK_MODEL_RANKSGD && nnz > 0) {
         // sampling table of the negatives: inclusive prefix sums of the item degrees (RankSGDRecommender.java:47-57)
         if ((rc = lrk_dev_alloc(h, &h->d_item_cum, (size_t)I))) return rc;
         size_t tb = 0;
-        LRK_CUDA(h, cub::DeviceScan::InclusiveSum(nullptr, tb, h->d_item_deg, h->d_item_cum, (int)I, st));
-        void* tmp = nullptr;
-        LRK_CUDA(h, cudaMalloc(&tmp, tb + 16));
-        cudaError_t e = cub::DeviceScan::InclusiveSum(tmp, tb, h->d_item_deg, h->d_item_cum, (int)I, st);
-        if (e == cudaSuccess) e = cudaStreamSynchronize(st);
-        cudaFree(tmp);
-        LRK_CUDA(h, e);
+        LRK_CUDA(h, cub::DeviceScan::InclusiveSum(nullptr, tb, h->d_item_deg.ptr, h->d_item_cum.ptr, (int)I, st));
+        LrkScratch sc;
+        if ((rc = lrk_scratch_begin(h, tb + 256, &sc))) return rc;
+        LRK_CUDA(h, cub::DeviceScan::InclusiveSum(sc.take<char>(tb), tb, h->d_item_deg.ptr, h->d_item_cum.ptr, (int)I, st));
+        LRK_CUDA(h, cudaStreamSynchronize(st));
         h->launches++;
     }
     if (h->cfg.update_mode == LRK_UPDATE_REFERENCE_ORDER) {
-        exact_release((ExactSchedule*)h->exact);
-        h->exact = nullptr;
-        ExactSchedule* es = nullptr;
-        if ((rc = exact_build_schedule(h, &es, U, I, rowptr, col, val))) return rc;
-        h->exact = es;
+        h->exact.reset();
+        if ((rc = exact_build_schedule(h, &h->exact, U, I, rowptr, col, val))) return rc;
     }
     if (h->cfg.model == LRK_MODEL_GBPR && (rc = gbpr_stage(h))) return rc;
     if (h->cfg.model == LRK_MODEL_SVDPP && (rc = svdpp_stage(h, val))) return rc;
@@ -422,7 +389,7 @@ int lrk_set_factors(lrk_handle_t h, const double* P, const double* Q, const doub
     f64_to_f32_rows_kernel<<<lrk_ceil_div(U, 256), 256, 0, st>>>(h->bu64, h->bu32, U, 1, 1); LRK_LAUNCH_CHECK(h);
     f64_to_f32_rows_kernel<<<lrk_ceil_div(I, 256), 256, 0, st>>>(h->bi64, h->bi32, I, 1, 1); LRK_LAUNCH_CHECK(h);
     if (m.damped && (rc = refresh_user_norm2(h, true))) return rc;
-    if (h->aobpr) ((AobprState*)h->aobpr)->count = 0;                 // a new trainModel(): countIter starts at 0 (AoBPRRecommender.java:88)
+    if (h->aobpr) h->aobpr->count = 0;                 // a new trainModel(): countIter starts at 0 (AoBPRRecommender.java:88)
     if (h->h_pnorm2) { h->pnorm2_prev = 0.f; h->pnorm2_host = *h->h_pnorm2; }
     LRK_CUDA(h, cudaStreamSynchronize(st));   // host buffers may be reused by the caller on return
     h->mu = mu;
@@ -487,8 +454,8 @@ static void fill_sgd_params(const lrk_handle_s* h, SgdParams& sp, float lr, floa
     sp.mu = (float)h->mu; sp.lr = lr; sp.reg_u = reg_u; sp.reg_i = reg_i; sp.reg_b = (float)reg_b;
     sp.loss = h->d_loss; sp.ld = h->ld;
     sp.hot_share = sgd_hot_share(h);
-    sp.item_deg = k_lrk_models[h->cfg.model].damped ? h->d_item_deg : nullptr;
-    sp.item_cum = h->cfg.model == LRK_MODEL_RANKSGD ? h->d_item_cum : nullptr;
+    sp.item_deg = k_lrk_models[h->cfg.model].damped ? h->d_item_deg.ptr : nullptr;
+    sp.item_cum = h->cfg.model == LRK_MODEL_RANKSGD ? h->d_item_cum.ptr : nullptr;
     sp.rowptr = h->d_rowptr; sp.col = h->d_col; sp.U = h->U; sp.I = h->I;
     sp.seed_lo = (uint32_t)h->cfg.seed; sp.seed_hi = (uint32_t)(h->cfg.seed >> 32); sp.epoch = (uint32_t)epoch_idx;
 }
@@ -507,7 +474,7 @@ int lrk_sgd_epoch(lrk_handle_t h, float lr, float reg_u, float reg_i, double reg
         // fp64 masters are the working set in this mode
         int rc = refresh_masters(h);
         if (rc) return rc;
-        e.enqueue = [&](int) { return h->nnz > 0 ? exact_epoch(h, (ExactSchedule*)h->exact, lr, reg_u, reg_i, reg_b) : (int)LRK_OK; };
+        e.enqueue = [&](int) { return h->nnz > 0 ? exact_epoch(h, h->exact.get(), lr, reg_u, reg_i, reg_b) : (int)LRK_OK; };
         return lrk_epoch(h, e, loss_out);
     }
     // curvature estimate of the epoch: the value the last norm refresh left in pinned memory (once per epoch call, so that a
@@ -517,7 +484,7 @@ int lrk_sgd_epoch(lrk_handle_t h, float lr, float reg_u, float reg_i, double reg
     fill_sgd_params(h, sp, lr, reg_u, reg_i, reg_b, epoch_idx);
     AobprState* ao = nullptr;
     if (h->cfg.model == LRK_MODEL_AOBPR) {
-        ao = (AobprState*)h->aobpr;
+        ao = h->aobpr.get();
         LRK_REQUIRE(h, ao != nullptr, "AoBPR needs rec.item.distribution.parameter: lrk_set_param(h, \"aobpr.lambda\", value)");
         int rc_a = aobpr_prepare(h, ao);
         if (rc_a) return rc_a;
@@ -534,7 +501,7 @@ int lrk_sgd_epoch(lrk_handle_t h, float lr, float reg_u, float reg_i, double reg
         if (h->nnz == 0) return LRK_OK;
         int rc;
         if (h->group) {
-            GroupUnits* gu = (GroupUnits*)h->group;
+            GroupUnits* gu = h->group.get();
             SgdGroupParams gp;
             memset(&gp, 0, sizeof gp);
             gp.su = sp.su; gp.si = sp.si; gp.sr = sp.sr; gp.units = gu->d_units; gp.n_units = (int32_t)gu->n_units; gp.counter = gu->d_counter;
@@ -576,8 +543,8 @@ int lrk_set_param(lrk_handle_t h, const char* name, double value) {
     LRK_NOT_MULTI(h, "lrk_set_param");
     if (!strcmp(name, "gbpr.rho") || !strcmp(name, "gbpr.gsize")) {
         LRK_REQUIRE(h, h->cfg.model == LRK_MODEL_GBPR, "gbpr.* parameters need a GBPR handle");
-        GbprState* g = (GbprState*)h->gbpr;
-        if (!g) { g = new GbprState(); h->gbpr = g; }
+        if (!h->gbpr) h->gbpr.reset(new GbprState());
+        GbprState* g = h->gbpr.get();
         if (!strcmp(name, "gbpr.rho")) g->rho = (float)value;
         else {
             LRK_REQUIRE(h, value >= 1.0 && value <= (double)LRK_GBPR_MAX_GROUP, "rec.gpbr.gsize must be in 1..8");
@@ -587,17 +554,15 @@ int lrk_set_param(lrk_handle_t h, const char* name, double value) {
     }
     if (!strcmp(name, "aobpr.lambda")) {
         LRK_REQUIRE(h, h->cfg.model == LRK_MODEL_AOBPR, "aobpr.* parameters need an AoBPR handle");
-        AobprState* a = (AobprState*)h->aobpr;
-        if (!a) { a = new AobprState(); h->aobpr = a; }
-        a->dist_param = (float)value;
-        a->I = 0;                                 // the rank distribution is rebuilt at the next epoch
+        if (!h->aobpr) h->aobpr.reset(new AobprState());
+        h->aobpr->dist_param = (float)value;
+        h->aobpr->I = 0;                                // the rank distribution is rebuilt at the next epoch
         return LRK_OK;
     }
     if (!strcmp(name, "svdpp.reg_imp")) {
         LRK_REQUIRE(h, h->cfg.model == LRK_MODEL_SVDPP, "svdpp.* parameters need an SVD++ handle");
-        SvdppState* g = (SvdppState*)h->svdpp;
-        if (!g) { g = new SvdppState(); h->svdpp = g; }
-        g->reg_imp = value;
+        if (!h->svdpp) h->svdpp.reset(new SvdppState());
+        h->svdpp->reg_imp = value;
         return LRK_OK;
     }
     return lrk_fail(h, LRK_ERR_INVALID, "lrk_set_param", "unknown parameter name", __FILE__, __LINE__);
@@ -609,7 +574,7 @@ int lrk_set_matrix(lrk_handle_t h, const char* name, const double* values) {
     if (!strcmp(name, "eals.confidences") && h->cfg.model == LRK_MODEL_EALS) {
         LRK_REQUIRE(h, h->has_train, "call lrk_set_train_csr first (it fixes numItems)");
         LRK_CUDA(h, cudaSetDevice(h->cfg.device));
-        AlsState* a = (AlsState*)h->als;
+        AlsState* a = h->als.get();
         LRK_REQUIRE(h, a != nullptr, "ALS state missing");
         int rc_a;
         if ((rc_a = lrk_dev_alloc(h, &a->d_conf, (size_t)h->I))) return rc_a;
@@ -621,8 +586,8 @@ int lrk_set_matrix(lrk_handle_t h, const char* name, const double* values) {
     LRK_REQUIRE(h, !strcmp(name, "svdpp.y") && h->cfg.model == LRK_MODEL_SVDPP, "unknown matrix name for this model");
     LRK_REQUIRE(h, h->has_factors, "call lrk_set_factors first");
     LRK_CUDA(h, cudaSetDevice(h->cfg.device));
-    SvdppState* g = (SvdppState*)h->svdpp;
-    if (!g) { g = new SvdppState(); h->svdpp = g; }
+    if (!h->svdpp) h->svdpp.reset(new SvdppState());
+    SvdppState* g = h->svdpp.get();
     cudaStream_t st = h->stream;
     const int64_t I = h->I;
     int rc;
@@ -639,7 +604,7 @@ int lrk_get_matrix(lrk_handle_t h, const char* name, double* values) {
     LRK_REQUIRE(h, h != nullptr && name != nullptr && values != nullptr, "NULL argument");
     LRK_NOT_MULTI(h, "lrk_get_matrix");
     if (!strcmp(name, "eals.confidences") && h->cfg.model == LRK_MODEL_EALS) {
-        AlsState* a = (AlsState*)h->als;
+        AlsState* a = h->als.get();
         LRK_REQUIRE(h, a != nullptr && a->has_conf, "matrix not set");
         LRK_CUDA(h, cudaSetDevice(h->cfg.device));
         LRK_CUDA(h, cudaMemcpyAsync(values, a->d_conf, sizeof(double) * (size_t)h->I, cudaMemcpyDeviceToHost, h->stream));
@@ -647,7 +612,7 @@ int lrk_get_matrix(lrk_handle_t h, const char* name, double* values) {
         return LRK_OK;
     }
     LRK_REQUIRE(h, !strcmp(name, "svdpp.y") && h->cfg.model == LRK_MODEL_SVDPP, "unknown matrix name for this model");
-    SvdppState* g = (SvdppState*)h->svdpp;
+    SvdppState* g = h->svdpp.get();
     LRK_REQUIRE(h, g != nullptr && g->has_y, "matrix not set");
     LRK_CUDA(h, cudaSetDevice(h->cfg.device));
     cudaStream_t st = h->stream;
@@ -697,7 +662,7 @@ int lrk_debug_stream(lrk_handle_t h, int32_t* su, int32_t* si, float* sr, int32_
     LRK_REQUIRE(h, h->has_train, "no train CSR");
     LRK_CUDA(h, cudaSetDevice(h->cfg.device));
     cudaStream_t st = h->stream;
-    GroupUnits* gu = (GroupUnits*)h->group;
+    GroupUnits* gu = h->group.get();
     *n_units_out = gu ? gu->n_units : 0;
     const size_t n = (size_t)h->nnz;
     if (su && n) LRK_CUDA(h, cudaMemcpyAsync(su, h->d_su, sizeof(int32_t) * n, cudaMemcpyDeviceToHost, st));
@@ -748,42 +713,33 @@ int lrk_bpr_peek_samples(lrk_handle_t h, int32_t epoch_idx, int64_t first, int64
     fill_sgd_params(h, sp, 0.f, 0.f, 0.f, 0.0, epoch_idx);
     if (h->cfg.model == LRK_MODEL_AOBPR) {
         // the draws depend on the factor rankings: those of the current item factors (what the first window of an epoch uses)
-        AobprState* ao = (AobprState*)h->aobpr;
+        AobprState* ao = h->aobpr.get();
         LRK_REQUIRE(h, ao != nullptr && h->has_factors, "AoBPR: set the factors and rec.item.distribution.parameter first");
         int rc_a = aobpr_prepare(h, ao);
         if (rc_a == LRK_OK) rc_a = aobpr_refresh(h, ao);
         if (rc_a) return rc_a;
         sp.ao_rank = ao->d_rank; sp.ao_var = ao->d_var; sp.ao_cum = ao->d_cum; sp.n_entries = h->nnz;
     }
-    int32_t* d_out = nullptr;
-    LRK_CUDA(h, cudaMalloc((void**)&d_out, sizeof(int32_t) * 3 * (size_t)n));
-    if (h->cfg.model == LRK_MODEL_GBPR) {
-        // 11 ints per sample: {u, i, j, group[8] padded with -1}
-        cudaFree(d_out);
+    const bool gbpr = h->cfg.model == LRK_MODEL_GBPR;
+    const size_t n_out = (gbpr ? 3 + LRK_GBPR_MAX_GROUP : 3) * (size_t)n;    // GBPR: 11 ints per sample {u, i, j, group[8] padded with -1}
+    LrkScratch sc;
+    int rc;
+    if ((rc = lrk_scratch_begin(h, sizeof(int32_t) * n_out + 256, &sc))) return rc;
+    int32_t* d_out = sc.take<int32_t>(n_out);
+    if (!d_out) return lrk_fail(h, LRK_ERR_NOMEM, "lrk_bpr_peek_samples", "scratch arena too small", __FILE__, __LINE__);
+    if (gbpr) {
         LRK_REQUIRE(h, h->gbpr != nullptr, "GBPR state missing");
-        LRK_CUDA(h, cudaMalloc((void**)&d_out, sizeof(int32_t) * (3 + LRK_GBPR_MAX_GROUP) * (size_t)n));
         GbprParams gp;
         gbpr_fill(h, gp, 0.f, 0.f, 0.f, 0.0, epoch_idx);
         gbpr_peek_kernel<<<lrk_ceil_div(n, 256), 256, 0, h->stream>>>(gp, first, n, d_out);
-        h->launches++;
-        cudaError_t ge = cudaGetLastError();
-        if (ge == cudaSuccess) ge = cudaMemcpyAsync(out, d_out, sizeof(int32_t) * (3 + LRK_GBPR_MAX_GROUP) * (size_t)n, cudaMemcpyDeviceToHost, h->stream);
-        if (ge == cudaSuccess) ge = cudaStreamSynchronize(h->stream);
-        cudaFree(d_out);
-        LRK_CUDA(h, ge);
-        return LRK_OK;
-    }
-    if (h->cfg.model == LRK_MODEL_RANKSGD) {
-        if (first + n > h->nnz) { cudaFree(d_out); return lrk_fail(h, LRK_ERR_INVALID, "lrk_bpr_peek_samples", "RankSGD has one sample per train entry: first + n exceeds nnz", __FILE__, __LINE__); }
+    } else if (h->cfg.model == LRK_MODEL_RANKSGD) {
+        if (first + n > h->nnz) return lrk_fail(h, LRK_ERR_INVALID, "lrk_bpr_peek_samples", "RankSGD has one sample per train entry: first + n exceeds nnz", __FILE__, __LINE__);
         ranksgd_peek_kernel<<<lrk_ceil_div(n, 256), 256, 0, h->stream>>>(sp, first, n, d_out);
     } else
-    bpr_peek_kernel<<<lrk_ceil_div(n, 256), 256, 0, h->stream>>>(sp, first, n, d_out);
-    h->launches++;
-    cudaError_t e = cudaGetLastError();
-    if (e == cudaSuccess) e = cudaMemcpyAsync(out, d_out, sizeof(int32_t) * 3 * (size_t)n, cudaMemcpyDeviceToHost, h->stream);
-    if (e == cudaSuccess) e = cudaStreamSynchronize(h->stream);
-    cudaFree(d_out);
-    LRK_CUDA(h, e);
+        bpr_peek_kernel<<<lrk_ceil_div(n, 256), 256, 0, h->stream>>>(sp, first, n, d_out);
+    LRK_LAUNCH_CHECK(h);
+    LRK_CUDA(h, cudaMemcpyAsync(out, d_out, sizeof(int32_t) * n_out, cudaMemcpyDeviceToHost, h->stream));
+    LRK_CUDA(h, cudaStreamSynchronize(h->stream));
     return LRK_OK;
 }
 
@@ -839,28 +795,26 @@ int lrk_eval_rating(lrk_handle_t h, int32_t U, const int64_t* t_rowptr, const in
     if (rc) return rc;
     cudaStream_t st = h->stream;
     const int nb = lrk_ceil_div(nnz, 256);
-    int64_t* d_rp = nullptr; int32_t* d_c = nullptr; double *d_v = nullptr, *d_p = nullptr, *d_part = nullptr;
+    LrkScratch sc;
+    if ((rc = lrk_scratch_begin(h, sizeof(int64_t) * ((size_t)U + 1) + (size_t)nnz * 20 + sizeof(double) * ((size_t)nb * 2 + 2) + 5 * 256, &sc))) return rc;
+    int64_t* d_rp = sc.take<int64_t>((size_t)U + 1);
+    int32_t* d_c = sc.take<int32_t>((size_t)nnz);
+    double* d_v = sc.take<double>((size_t)nnz);
+    double* d_p = sc.take<double>((size_t)nnz);
+    double* d_part = sc.take<double>((size_t)nb * 2 + 2);
+    if (!d_rp || !d_c || !d_v || !d_p || !d_part) return lrk_fail(h, LRK_ERR_NOMEM, "lrk_eval_rating", "scratch arena too small", __FILE__, __LINE__);
+    LRK_CUDA(h, cudaMemcpyAsync(d_rp, t_rowptr, sizeof(int64_t) * ((size_t)U + 1), cudaMemcpyHostToDevice, st));
+    LRK_CUDA(h, cudaMemcpyAsync(d_c, t_col, sizeof(int32_t) * (size_t)nnz, cudaMemcpyHostToDevice, st));
+    LRK_CUDA(h, cudaMemcpyAsync(d_v, t_val, sizeof(double) * (size_t)nnz, cudaMemcpyHostToDevice, st));
+    eval_rating_kernel<<<nb, 256, 0, st>>>(h->P64, h->Q64, h->bu64, h->bi64, h->mu, lrk_has_bias(h),
+                                           h->k, U, d_rp, d_c, d_v, min_rate, max_rate, d_p, d_part, d_part + nb);
+    eval_rating_final_kernel<<<1, 32, 0, st>>>(d_part, d_part + nb, nb, nnz, d_part + 2 * (size_t)nb);
+    h->launches += 2;
+    LRK_CUDA(h, cudaGetLastError());
     double res[2] = {0, 0};
-    cudaError_t e = cudaMalloc((void**)&d_rp, sizeof(int64_t) * ((size_t)U + 1));
-    if (e == cudaSuccess) e = cudaMalloc((void**)&d_c, sizeof(int32_t) * (size_t)nnz);
-    if (e == cudaSuccess) e = cudaMalloc((void**)&d_v, sizeof(double) * (size_t)nnz);
-    if (e == cudaSuccess) e = cudaMalloc((void**)&d_p, sizeof(double) * (size_t)nnz);
-    if (e == cudaSuccess) e = cudaMalloc((void**)&d_part, sizeof(double) * ((size_t)nb * 2 + 2));
-    if (e == cudaSuccess) e = cudaMemcpyAsync(d_rp, t_rowptr, sizeof(int64_t) * ((size_t)U + 1), cudaMemcpyHostToDevice, st);
-    if (e == cudaSuccess) e = cudaMemcpyAsync(d_c, t_col, sizeof(int32_t) * (size_t)nnz, cudaMemcpyHostToDevice, st);
-    if (e == cudaSuccess) e = cudaMemcpyAsync(d_v, t_val, sizeof(double) * (size_t)nnz, cudaMemcpyHostToDevice, st);
-    if (e == cudaSuccess) {
-        eval_rating_kernel<<<nb, 256, 0, st>>>(h->P64, h->Q64, h->bu64, h->bi64, h->mu, lrk_has_bias(h),
-                                               h->k, U, d_rp, d_c, d_v, min_rate, max_rate, d_p, d_part, d_part + nb);
-        eval_rating_final_kernel<<<1, 32, 0, st>>>(d_part, d_part + nb, nb, nnz, d_part + 2 * (size_t)nb);
-        h->launches += 2;
-        e = cudaGetLastError();
-    }
-    if (e == cudaSuccess && pred_out) e = cudaMemcpyAsync(pred_out, d_p, sizeof(double) * (size_t)nnz, cudaMemcpyDeviceToHost, st);
-    if (e == cudaSuccess) e = cudaMemcpyAsync(res, d_part + 2 * (size_t)nb, sizeof(double) * 2, cudaMemcpyDeviceToHost, st);
-    if (e == cudaSuccess) e = cudaStreamSynchronize(st);
-    cudaFree(d_rp); cudaFree(d_c); cudaFree(d_v); cudaFree(d_p); cudaFree(d_part);
-    LRK_CUDA(h, e);
+    if (pred_out) LRK_CUDA(h, cudaMemcpyAsync(pred_out, d_p, sizeof(double) * (size_t)nnz, cudaMemcpyDeviceToHost, st));
+    LRK_CUDA(h, cudaMemcpyAsync(res, d_part + 2 * (size_t)nb, sizeof(double) * 2, cudaMemcpyDeviceToHost, st));
+    LRK_CUDA(h, cudaStreamSynchronize(st));
     if (rmse_out) *rmse_out = res[0];
     if (mae_out) *mae_out = res[1];
     return LRK_OK;
@@ -1051,6 +1005,16 @@ int lrk_create_multi(const lrk_config_t* cfg, const int32_t* devices, int32_t n_
 }
 
 }  // extern "C"
+
+lrk_handle_s::~lrk_handle_s() {
+    dsgd.reset();                                       // the ring buffers and their IPC mappings go before the communicator
+    if (comm && nccl_api()) nccl_api()->CommDestroy((ncclComm_t)comm);
+    if (h_loss) cudaFreeHost(h_loss);
+    if (h_pnorm2) cudaFreeHost(h_pnorm2);
+    for (cudaEvent_t ev : {ev0, ev1, ev_copy0, ev_copy1}) if (ev) cudaEventDestroy(ev);
+    if (copy_stream) cudaStreamDestroy(copy_stream);
+    if (own_stream) cudaStreamDestroy(own_stream);
+}
 
 static int multi_destroy(lrk_handle_s* h) {
     MultiState* ms = (MultiState*)h->multi;

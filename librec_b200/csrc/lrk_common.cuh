@@ -4,13 +4,32 @@
 #include <cstdint>
 #include <cstdio>
 #include <cstring>
+#include <memory>
 #include <string>
 #include <type_traits>
-#include <unordered_map>
+#include <utility>
 #include "../../include/librec_b200.h"
 
 #define LRK_MAX_FACTORS 256
 #define LRK_MAX_TOPN 512
+
+// Owning device buffer: cudaFree on destruction, reused by lrk_dev_alloc while its capacity suffices.  It converts to T*, so
+// kernel arguments and parameter structs take it as they would a raw pointer.
+template <typename T>
+struct LrkBuf {
+    T* ptr = nullptr;
+    size_t cap = 0;   // bytes
+    LrkBuf() = default;
+    LrkBuf(LrkBuf&& o) noexcept { swap(o); }
+    LrkBuf& operator=(LrkBuf&& o) noexcept { swap(o); return *this; }
+    ~LrkBuf() { reset(); }
+    void swap(LrkBuf& o) noexcept { std::swap(ptr, o.ptr); std::swap(cap, o.cap); }
+    void reset() { if (ptr) cudaFree(ptr); ptr = nullptr; cap = 0; }
+    operator T*() const { return ptr; }
+};
+
+// model states (one translation unit: lrk_api.cu includes their headers and defines ~lrk_handle_s after them)
+struct GroupUnits; struct TcState; struct GbprState; struct SvdppState; struct AobprState; struct AlsState; struct ExactSchedule; struct DsgdState;
 
 struct lrk_handle_s {
     lrk_config_t cfg{};
@@ -26,39 +45,39 @@ struct lrk_handle_s {
     cudaEvent_t ev_copy0 = nullptr, ev_copy1 = nullptr;
 
     // train CSR (device): membership for BPR sampling and the top-N train mask
-    int64_t* d_rowptr = nullptr;
-    int32_t* d_col = nullptr;
+    LrkBuf<int64_t> d_rowptr;
+    LrkBuf<int32_t> d_col;
     // shuffled COO stream for the SGD epoch (SoA, 12 B / rating)
-    int32_t* d_su = nullptr;
-    int32_t* d_si = nullptr;
-    float* d_sr = nullptr;
+    LrkBuf<int32_t> d_su;
+    LrkBuf<int32_t> d_si;
+    LrkBuf<float> d_sr;
     bool has_train = false;
-    void* group = nullptr;    // GroupUnits*: the stream is unit-ordered (staging_group.cuh) and the epoch runs sgd_group_epoch_kernel
+    std::unique_ptr<GroupUnits> group;   // the stream is unit-ordered (staging_group.cuh) and the epoch runs sgd_group_epoch_kernel
     int64_t run_tiles = 0;    // 32-rating item-run tiles in the staged stream (lrk_stage_stats)
     uint32_t max_item_deg = 0;
     double hot_share = 0.0;   // largest share one item has of the train ratings (stability cap of the SGD grid)
-    float* d_pnorm2 = nullptr;        // mean |p_u|^2 at the start of the epoch (curvature term of that step)
+    LrkBuf<float> d_pnorm2;           // mean |p_u|^2 at the start of the epoch (curvature term of that step)
     float pnorm2_host = 0.f;          // its host copy, refreshed with every loss read-back (picks the kernel variant)
     float pnorm2_prev = 0.f;          // the value one epoch earlier (growth of the user factors, sgd_launch_gv)
-    uint32_t* d_item_deg = nullptr;   // ratings per item in this handle's shard (staleness-aware step of run tiles, sgd.cuh)
-    uint32_t* d_item_cum = nullptr;   // RankSGD: inclusive prefix sums of d_item_deg (negative sampling table)
+    LrkBuf<uint32_t> d_item_deg;      // ratings per item in this handle's shard (staleness-aware step of run tiles, sgd.cuh)
+    LrkBuf<uint32_t> d_item_cum;      // RankSGD: inclusive prefix sums of d_item_deg (negative sampling table)
 
     // factors: fp32 working copies (padded rows) + fp64 masters (dense rows, what Java sees)
-    float *P32 = nullptr, *Q32 = nullptr, *bu32 = nullptr, *bi32 = nullptr;
-    double *P64 = nullptr, *Q64 = nullptr, *bu64 = nullptr, *bi64 = nullptr;
+    LrkBuf<float> P32, Q32, bu32, bi32;
+    LrkBuf<double> P64, Q64, bu64, bi64;
     double mu = 0.0;
     bool has_factors = false;
     bool f64_valid = false;   // masters are in sync with the fp32 working copies
 
     // Safeguard of the fast SGD mode (lrk_epoch.cuh): factors are snapshotted before an epoch; a non-finite (or exploding) loss
     // rolls the epoch back and re-runs it with 4x fewer ratings in flight (sticky, relaxed again after 8 good epochs)
-    float *bk_P = nullptr, *bk_Q = nullptr, *bk_bu = nullptr, *bk_bi = nullptr;
+    LrkBuf<float> bk_P, bk_Q, bk_bu, bk_bi;
     int conc_div = 1;           // divisor of the SGD grid
     int good_epochs = 0;
     double prev_loss = -1.0;    // loss of the last accepted epoch (< 0: none yet)
     int64_t rollbacks = 0;
     int epochs_done = 0;        // accepted epochs since lrk_set_factors (picks the kernel variant of the first epochs)
-    double* d_loss = nullptr;   // device accumulator
+    LrkBuf<double> d_loss;      // device accumulator
     double* h_loss = nullptr;   // pinned
     float* h_pnorm2 = nullptr;  // pinned
     cudaEvent_t ev0 = nullptr, ev1 = nullptr;
@@ -71,18 +90,18 @@ struct lrk_handle_s {
     float topn_phase_ms[4] = {0.f, 0.f, 0.f, 0.f};
     float topn_err_ratio = 0.f;   // largest observed |fp16 sweep score - exact score| / certificate bound (must be < 1)
     // result buffers of lrk_topn, reused across calls (cudaMalloc/cudaFree of 130 MB cost 20-400 ms per call)
-    int32_t *tn_users = nullptr, *tn_items = nullptr, *tn_counts = nullptr;
-    double* tn_scores = nullptr;
+    LrkBuf<int32_t> tn_users, tn_items, tn_counts;
+    LrkBuf<double> tn_scores;
     // tensor-core top-N state (bf16 copies, norms); see topn_tc.cuh
-    void* tc = nullptr;
+    std::unique_ptr<TcState> tc;
 
-    void* gbpr = nullptr;     // GbprState* (sgd_gbpr.cuh)
-    void* svdpp = nullptr;    // SvdppState* (sgd_svdpp.cuh)
-    void* aobpr = nullptr;    // AobprState* (sgd_aobpr.cuh)
-    void* als = nullptr;      // AlsState* (als.cuh): WRMF / eALS
+    std::unique_ptr<GbprState> gbpr;     // sgd_gbpr.cuh
+    std::unique_ptr<SvdppState> svdpp;   // sgd_svdpp.cuh
+    std::unique_ptr<AobprState> aobpr;   // sgd_aobpr.cuh
+    std::unique_ptr<AlsState> als;       // als.cuh: WRMF / eALS
 
     // reference-order (wavefront) schedule, see sgd_exact.cuh
-    void* exact = nullptr;
+    std::unique_ptr<ExactSchedule> exact;
 
     // single-process multi-GPU parent (multi.cuh): no device state of its own, forwards to one child per device
     void* multi = nullptr;
@@ -94,14 +113,14 @@ struct lrk_handle_s {
     // DSGD
     void* comm = nullptr;   // ncclComm_t
     int rank = 0, world = 1;
-    void* dsgd = nullptr;   // DsgdState*
+    std::unique_ptr<DsgdState> dsgd;
 
-    // allocation bookkeeping: device buffers are reused across calls when they are large enough
-    std::unordered_map<void*, size_t> caps;
-    void* scratch = nullptr;      // staging workspace (temporaries of lrk_set_train_csr), grown on demand
-    size_t scratch_bytes = 0;
+    LrkBuf<char> scratch;   // staging arena (lrk_scratch_begin)
 
     std::string err;
+
+    // frees everything above; safe on a handle without device state (a multi-device parent, a half-created handle)
+    ~lrk_handle_s();
 };
 
 extern thread_local std::string g_lrk_tls_error;
@@ -133,26 +152,17 @@ static inline int lrk_fail(lrk_handle_s* h, int code, const char* what, const ch
         LRK_CUDA((h), cudaGetLastError());   \
     } while (0)
 
+// at least `count` elements in *b (one when count is 0): kept when large enough, otherwise reallocated without its contents
 template <typename T>
-static inline int lrk_dev_alloc(lrk_handle_s* h, T** p, size_t count) {
-    if (count == 0) count = 1;
-    const size_t bytes = count * sizeof(T);
-    if (*p) {
-        auto it = h->caps.find((void*)*p);
-        if (it != h->caps.end() && it->second >= bytes) return LRK_OK;   // reuse
-        if (it != h->caps.end()) h->caps.erase(it);
-        cudaFree(*p);
-        *p = nullptr;
-    }
-    LRK_CUDA(h, cudaMalloc((void**)p, bytes));
-    h->caps[(void*)*p] = bytes;
+static inline int lrk_dev_alloc(lrk_handle_s* h, LrkBuf<T>* b, size_t count) {
+    const size_t bytes = (count ? count : 1) * sizeof(T);
+    if (b->cap >= bytes) return LRK_OK;
+    b->reset();
+    LRK_CUDA(h, cudaMalloc((void**)&b->ptr, bytes));
+    b->cap = bytes;
     return LRK_OK;
 }
-template <typename T>
-static inline void lrk_dev_free(T** p) {
-    if (*p) { cudaFree(*p); *p = nullptr; }
-}
-// bump allocator over the handle's staging workspace
+// bump allocator over the handle's staging arena
 struct LrkScratch {
     char* base = nullptr;
     size_t used = 0, cap = 0;
@@ -165,13 +175,13 @@ struct LrkScratch {
         return r;
     }
 };
+// The staging arena serves the outermost level of one C-ABI call: a call takes it once and everything it hands out is
+// overwritten by the next lrk_scratch_begin.  A helper that runs inside another helper's use of the arena keeps its
+// temporaries in LrkBufs of the state it belongs to instead.
 static inline int lrk_scratch_begin(lrk_handle_s* h, size_t bytes, LrkScratch* out) {
-    if (h->scratch_bytes < bytes) {
-        if (h->scratch) { cudaFree(h->scratch); h->scratch = nullptr; h->scratch_bytes = 0; }
-        LRK_CUDA(h, cudaMalloc(&h->scratch, bytes));
-        h->scratch_bytes = bytes;
-    }
-    out->base = (char*)h->scratch; out->used = 0; out->cap = h->scratch_bytes;
+    const int rc = lrk_dev_alloc(h, &h->scratch, bytes);
+    if (rc) return rc;
+    out->base = h->scratch; out->used = 0; out->cap = h->scratch.cap;
     return LRK_OK;
 }
 

@@ -8,7 +8,7 @@
 #include <vector>
 
 // A float array under the rollback safeguard: copied to *bk before the epoch, copied back after a rejected attempt
-struct LrkSaved { float* live; float** bk; size_t n; };
+struct LrkSaved { float* live; LrkBuf<float>* bk; size_t n; };
 
 struct LrkEpoch {
     std::function<int(int attempt)> enqueue;   // the attempt's work on h->stream, between the timing events ev0 and ev1

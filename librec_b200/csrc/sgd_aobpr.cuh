@@ -15,22 +15,17 @@
 #include <vector>
 
 struct AobprState {
-    int32_t* d_rank = nullptr;     // [ld][I]
-    float* d_var = nullptr;        // [ld] (padded factors: 0)
-    float* d_cum = nullptr;        // [I]
-    uint64_t *d_keys = nullptr, *d_keys2 = nullptr;
-    int32_t *d_vals = nullptr;
-    void* d_tmp = nullptr; size_t tmp_bytes = 0;
+    LrkBuf<int32_t> d_rank;        // [ld][I]
+    LrkBuf<float> d_var;           // [ld] (padded factors: 0)
+    LrkBuf<float> d_cum;           // [I]
+    LrkBuf<uint64_t> d_keys, d_keys2;
+    LrkBuf<int32_t> d_vals;
+    LrkBuf<char> d_tmp; size_t tmp_bytes = 0;
     int32_t I = 0; int ld = 0;
     float dist_param = 0.f;        // rec.item.distribution.parameter (no default in the reference: setup() throws without it)
     int32_t lambda = 0, loop = 0;
     int64_t count = 0;             // countIter (:92-97)
 };
-static void aobpr_release(AobprState* a) {
-    if (!a) return;
-    cudaFree(a->d_rank); cudaFree(a->d_var); cudaFree(a->d_cum); cudaFree(a->d_keys); cudaFree(a->d_keys2); cudaFree(a->d_vals); cudaFree(a->d_tmp);
-    delete a;
-}
 // key of (item i, factor f): f in the high word, the factor value mapped to an unsigned that sorts DESCENDING in the low word
 __global__ void aobpr_keys_kernel(const float* __restrict__ Q, int32_t I, int ld, int k, uint64_t* __restrict__ keys, int32_t* __restrict__ vals) {
     const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -69,18 +64,17 @@ static int aobpr_prepare(lrk_handle_s* h, AobprState* a) {
     a->loop = (int32_t)((double)I * log((double)I));                            // :65
     LRK_REQUIRE(h, a->lambda > 0 && a->loop > 0, "rec.item.distribution.parameter * numItems must be at least 1");
     if (a->I == I && a->ld == h->ld && a->d_rank) return LRK_OK;
-    cudaFree(a->d_rank); cudaFree(a->d_var); cudaFree(a->d_cum); cudaFree(a->d_keys); cudaFree(a->d_keys2); cudaFree(a->d_vals); cudaFree(a->d_tmp);
-    a->d_rank = nullptr; a->d_var = nullptr; a->d_cum = nullptr; a->d_keys = nullptr; a->d_keys2 = nullptr; a->d_vals = nullptr; a->d_tmp = nullptr;
     const size_t n = (size_t)I * h->k;
-    LRK_CUDA(h, cudaMalloc((void**)&a->d_rank, sizeof(int32_t) * (size_t)I * h->ld));
-    LRK_CUDA(h, cudaMalloc((void**)&a->d_var, sizeof(float) * (size_t)h->ld));
-    LRK_CUDA(h, cudaMalloc((void**)&a->d_cum, sizeof(float) * (size_t)I));
-    LRK_CUDA(h, cudaMalloc((void**)&a->d_keys, sizeof(uint64_t) * n));
-    LRK_CUDA(h, cudaMalloc((void**)&a->d_keys2, sizeof(uint64_t) * n));
-    LRK_CUDA(h, cudaMalloc((void**)&a->d_vals, sizeof(int32_t) * n));
+    int rc;
+    if ((rc = lrk_dev_alloc(h, &a->d_rank, (size_t)I * h->ld))) return rc;
+    if ((rc = lrk_dev_alloc(h, &a->d_var, (size_t)h->ld))) return rc;
+    if ((rc = lrk_dev_alloc(h, &a->d_cum, (size_t)I))) return rc;
+    if ((rc = lrk_dev_alloc(h, &a->d_keys, n))) return rc;
+    if ((rc = lrk_dev_alloc(h, &a->d_keys2, n))) return rc;
+    if ((rc = lrk_dev_alloc(h, &a->d_vals, n))) return rc;
     a->tmp_bytes = 0;
-    LRK_CUDA(h, cub::DeviceRadixSort::SortPairs(nullptr, a->tmp_bytes, a->d_keys, a->d_keys2, a->d_vals, a->d_rank, (int)n, 0, 40, st));
-    LRK_CUDA(h, cudaMalloc(&a->d_tmp, a->tmp_bytes + 16));
+    LRK_CUDA(h, cub::DeviceRadixSort::SortPairs(nullptr, a->tmp_bytes, a->d_keys.ptr, a->d_keys2.ptr, a->d_vals.ptr, a->d_rank.ptr, (int)n, 0, 40, st));
+    if ((rc = lrk_dev_alloc(h, &a->d_tmp, a->tmp_bytes + 16))) return rc;
     LRK_CUDA(h, cudaMemsetAsync(a->d_var, 0, sizeof(float) * (size_t)h->ld, st));
     LRK_CUDA(h, cudaMemsetAsync(a->d_rank, 0, sizeof(int32_t) * (size_t)I * h->ld, st));   // padded factors (never drawn unless p_u is all zero) rank item 0
     // cumulative rank distribution in double on the host (I values), float on the device
@@ -105,7 +99,7 @@ static int aobpr_refresh(lrk_handle_s* h, AobprState* a) {
     size_t tb = a->tmp_bytes;
     int hi_bits = 1;
     while ((1 << hi_bits) < h->k) ++hi_bits;
-    LRK_CUDA(h, cub::DeviceRadixSort::SortPairs(a->d_tmp, tb, a->d_keys, a->d_keys2, a->d_vals, a->d_rank, (int)n, 0, 32 + hi_bits, st));
+    LRK_CUDA(h, cub::DeviceRadixSort::SortPairs(a->d_tmp, tb, a->d_keys.ptr, a->d_keys2.ptr, a->d_vals.ptr, a->d_rank.ptr, (int)n, 0, 32 + hi_bits, st));
     h->launches++;
     aobpr_var_kernel<<<h->k, 256, 0, st>>>(h->Q32, h->I, h->ld, a->d_var); LRK_LAUNCH_CHECK(h);
     return LRK_OK;

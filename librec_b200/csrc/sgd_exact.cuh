@@ -19,11 +19,11 @@ struct ExactSchedule {
     int64_t nnz = 0;
     int32_t num_levels = 0;
     int64_t max_width = 0;
-    int64_t* d_level_ptr = nullptr;   // num_levels + 1
-    int32_t* d_u = nullptr;
-    int32_t* d_i = nullptr;
-    double* d_r = nullptr;
-    unsigned long long* d_bar = nullptr;
+    LrkBuf<int64_t> d_level_ptr;      // num_levels + 1
+    LrkBuf<int32_t> d_u;
+    LrkBuf<int32_t> d_i;
+    LrkBuf<double> d_r;
+    LrkBuf<unsigned long long> d_bar;
     unsigned long long generation = 0;   // arrivals counted by d_bar so far; lives and dies with d_bar (a re-staged schedule starts at 0)
 };
 
@@ -112,17 +112,11 @@ __global__ void __launch_bounds__(256) sgd_reference_order_kernel(ExactParams p)
     if (lane == 0) atomicAdd(p.loss, loss_acc);
 }
 
-static void exact_release(ExactSchedule* s) {
-    if (!s) return;
-    cudaFree(s->d_level_ptr); cudaFree(s->d_u); cudaFree(s->d_i); cudaFree(s->d_r); cudaFree(s->d_bar);
-    delete s;
-}
-
 // Host scheduling: one O(nnz) pass in CSR order computes the levels, a counting sort groups the
 // ratings by level.  (Host logic, like the reference's own CSR construction; no arithmetic on ratings.)
-static int exact_build_schedule(lrk_handle_s* h, ExactSchedule** out, int32_t U, int32_t I, const int64_t* rowptr,
+static int exact_build_schedule(lrk_handle_s* h, std::unique_ptr<ExactSchedule>* out, int32_t U, int32_t I, const int64_t* rowptr,
                                 const int32_t* col, const double* val) {
-    ExactSchedule* s = new ExactSchedule();
+    std::unique_ptr<ExactSchedule> s(new ExactSchedule());
     const int64_t nnz = rowptr[U];
     s->nnz = nnz;
     std::vector<int32_t> row_level((size_t)U, 0), col_level((size_t)I, 0), level((size_t)nnz);
@@ -149,18 +143,18 @@ static int exact_build_schedule(lrk_handle_s* h, ExactSchedule** out, int32_t U,
             const int64_t pos = cursor[(size_t)level[(size_t)e] - 1]++;
             lu[(size_t)pos] = u; li[(size_t)pos] = col[e]; lr[(size_t)pos] = val[e];
         }
-    cudaError_t e = cudaMalloc((void**)&s->d_level_ptr, sizeof(int64_t) * ((size_t)L + 1));
-    if (e == cudaSuccess) e = cudaMalloc((void**)&s->d_u, sizeof(int32_t) * (size_t)(nnz ? nnz : 1));
-    if (e == cudaSuccess) e = cudaMalloc((void**)&s->d_i, sizeof(int32_t) * (size_t)(nnz ? nnz : 1));
-    if (e == cudaSuccess) e = cudaMalloc((void**)&s->d_r, sizeof(double) * (size_t)(nnz ? nnz : 1));
-    if (e == cudaSuccess) e = cudaMalloc((void**)&s->d_bar, sizeof(unsigned long long));
-    if (e == cudaSuccess) e = cudaMemset(s->d_bar, 0, sizeof(unsigned long long));
-    if (e == cudaSuccess) e = cudaMemcpy(s->d_level_ptr, start.data(), sizeof(int64_t) * ((size_t)L + 1), cudaMemcpyHostToDevice);
-    if (e == cudaSuccess && nnz) e = cudaMemcpy(s->d_u, lu.data(), sizeof(int32_t) * (size_t)nnz, cudaMemcpyHostToDevice);
-    if (e == cudaSuccess && nnz) e = cudaMemcpy(s->d_i, li.data(), sizeof(int32_t) * (size_t)nnz, cudaMemcpyHostToDevice);
-    if (e == cudaSuccess && nnz) e = cudaMemcpy(s->d_r, lr.data(), sizeof(double) * (size_t)nnz, cudaMemcpyHostToDevice);
-    if (e != cudaSuccess) { exact_release(s); LRK_CUDA(h, e); }
-    *out = s;
+    int rc;
+    if ((rc = lrk_dev_alloc(h, &s->d_level_ptr, (size_t)L + 1))) return rc;
+    if ((rc = lrk_dev_alloc(h, &s->d_u, (size_t)nnz))) return rc;
+    if ((rc = lrk_dev_alloc(h, &s->d_i, (size_t)nnz))) return rc;
+    if ((rc = lrk_dev_alloc(h, &s->d_r, (size_t)nnz))) return rc;
+    if ((rc = lrk_dev_alloc(h, &s->d_bar, 1))) return rc;
+    LRK_CUDA(h, cudaMemset(s->d_bar, 0, sizeof(unsigned long long)));
+    LRK_CUDA(h, cudaMemcpy(s->d_level_ptr, start.data(), sizeof(int64_t) * ((size_t)L + 1), cudaMemcpyHostToDevice));
+    if (nnz) LRK_CUDA(h, cudaMemcpy(s->d_u, lu.data(), sizeof(int32_t) * (size_t)nnz, cudaMemcpyHostToDevice));
+    if (nnz) LRK_CUDA(h, cudaMemcpy(s->d_i, li.data(), sizeof(int32_t) * (size_t)nnz, cudaMemcpyHostToDevice));
+    if (nnz) LRK_CUDA(h, cudaMemcpy(s->d_r, lr.data(), sizeof(double) * (size_t)nnz, cudaMemcpyHostToDevice));
+    *out = std::move(s);
     return LRK_OK;
 }
 

@@ -215,14 +215,9 @@ __global__ void gbpr_colptr_kernel(const uint32_t* __restrict__ deg_excl, const 
 }
 
 struct GbprState {
-    int64_t* d_colptr = nullptr;
-    int32_t* d_cusers = nullptr;
-    float* tP = nullptr; float* tQ = nullptr;
+    LrkBuf<int64_t> d_colptr;
+    LrkBuf<int32_t> d_cusers;
+    LrkBuf<float> tP, tQ;
     float rho = 1.5f;            // rec.gpbr.rho   (GBPRRecommender.java:71)
     int glen = 2;                // rec.gpbr.gsize (GBPRRecommender.java:72)
 };
-static void gbpr_release(GbprState* g) {
-    if (!g) return;
-    cudaFree(g->d_colptr); cudaFree(g->d_cusers); cudaFree(g->tP); cudaFree(g->tQ);
-    delete g;
-}

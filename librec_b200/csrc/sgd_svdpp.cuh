@@ -168,19 +168,14 @@ __global__ void __launch_bounds__(256) sgd_svdpp_epoch_kernel(SvdppParams p) {
 }
 
 struct SvdppState {
-    float* d_cval = nullptr;       // train values in CSR order
-    int32_t* d_uorder = nullptr;   // users by descending degree
-    unsigned int* d_counter = nullptr;
-    float* Y32 = nullptr;          // impItemFactors, padded rows like Q32
-    double* Y64 = nullptr;
+    LrkBuf<float> d_cval;          // train values in CSR order
+    LrkBuf<int32_t> d_uorder;      // users by descending degree
+    LrkBuf<unsigned int> d_counter;
+    LrkBuf<float> Y32;             // impItemFactors, padded rows like Q32
+    LrkBuf<double> Y64;
     bool has_y = false;
     double reg_imp = 0.015;        // rec.impItem.regularization (SVDPlusPlusRecommender.java:52)
 };
-static void svdpp_release(SvdppState* s) {
-    if (!s) return;
-    cudaFree(s->d_cval); cudaFree(s->d_uorder); cudaFree(s->d_counter); cudaFree(s->Y32); cudaFree(s->Y64);
-    delete s;
-}
 __global__ void svdpp_deg_kernel(const int64_t* __restrict__ rowptr, int32_t U, uint32_t* __restrict__ deg, int32_t* __restrict__ ids) {
     const int32_t u = blockIdx.x * blockDim.x + threadIdx.x;
     if (u < U) { deg[u] = (uint32_t)(rowptr[u + 1] - rowptr[u]); ids[u] = u; }

@@ -173,11 +173,11 @@ struct GroupUnits;
 static int stage_group_stream(lrk_handle_s* h, const int64_t* d_rowptr, const int32_t* d_col, const int32_t* row_of, const double* d_val,
                               int32_t U, int32_t I, int64_t nnz, const int32_t* d_bounds, int world, int workers, uint64_t seed,
                               LrkScratch& sc, void* tmp, size_t tmp_bytes, uint64_t* keys, uint64_t* keys2, uint32_t* idx, uint32_t* perm,
-                              int32_t* su, int32_t* si, float* sr, GroupUnits** out);
+                              int32_t* su, int32_t* si, float* sr, std::unique_ptr<GroupUnits>* out);
 // group_workers > 0: stage the unit-ordered stream of the user-group kernel (staging_group.cuh) for that many resident workers
 static int stage_coo_from_csr(lrk_handle_s* h, const int64_t* d_rowptr, const int32_t* d_col, const double* h_val,
                               int32_t U, int32_t I, int64_t nnz, int32_t* su, int32_t* si, float* sr, bool validate,
-                              int group_workers = 0, GroupUnits** group_out = nullptr) {
+                              int group_workers = 0, std::unique_ptr<GroupUnits>* group_out = nullptr) {
     cudaStream_t st = h->stream;
     if (nnz == 0) { LRK_CUDA(h, cudaStreamSynchronize(st)); return LRK_OK; }
     size_t tmp64 = 0;

@@ -22,8 +22,8 @@
 #define LRK_GROUP_MAX_UNITS (1 << 27)
 
 struct GroupUnits {               // device unit table of a staged stream + host-side block ranges
-    int4* d_units = nullptr;      // {stream start, ratings, first user, users | slices << 16 (0: the unit owns its users exclusively)}
-    unsigned int* d_counter = nullptr;   // one work counter per item block (dynamic unit fetch)
+    LrkBuf<int4> d_units;         // {stream start, ratings, first user, users | slices << 16 (0: the unit owns its users exclusively)}
+    LrkBuf<unsigned int> d_counter;      // one work counter per item block (dynamic unit fetch)
     int64_t n_units = 0;
     uint32_t target = 0;
     std::vector<int64_t> unit_base;      // world + 1: units of block b are [unit_base[b], unit_base[b+1])
@@ -121,12 +121,6 @@ __global__ void group_gather_kernel(const uint32_t* __restrict__ perm, const int
     su[t] = row_of[e]; si[t] = i - (bounds ? bounds[b] : 0); sr[t] = (float)val[e];
 }
 
-static void group_units_release(GroupUnits* g) {
-    if (!g) return;
-    cudaFree(g->d_units); cudaFree(g->d_counter);
-    delete g;
-}
-
 static bool group_order_supported(int32_t U, int32_t I, int64_t nnz, int world) {
     return I <= LRK_GROUP_MAX_ITEMS && (int64_t)U * world < (int64_t)0x7fffffff && nnz < (int64_t)0xffffffffLL && nnz > 0;
 }
@@ -136,13 +130,13 @@ static bool group_order_supported(int32_t U, int32_t I, int64_t nnz, int world) 
 static int stage_group_stream(lrk_handle_s* h, const int64_t* d_rowptr, const int32_t* d_col, const int32_t* row_of, const double* d_val,
                               int32_t U, int32_t I, int64_t nnz, const int32_t* d_bounds, int world, int workers, uint64_t seed,
                               LrkScratch& sc, void* tmp, size_t tmp_bytes, uint64_t* keys, uint64_t* keys2, uint32_t* idx, uint32_t* perm,
-                              int32_t* su, int32_t* si, float* sr, GroupUnits** out) {
+                              int32_t* su, int32_t* si, float* sr, std::unique_ptr<GroupUnits>* out) {
     cudaStream_t st = h->stream;
     const int64_t nv = (int64_t)U * world;
     uint32_t *degv = sc.take<uint32_t>((size_t)nv), *rowlo = sc.take<uint32_t>((size_t)nv), *S = sc.take<uint32_t>((size_t)nv);
     uint32_t *started = sc.take<uint32_t>((size_t)nv), *incl = sc.take<uint32_t>((size_t)nv);
     if (!degv || !rowlo || !S || !started || !incl) return lrk_fail(h, LRK_ERR_NOMEM, "stage_group_stream", "scratch arena too small", __FILE__, __LINE__);
-    GroupUnits* g = new GroupUnits();
+    std::unique_ptr<GroupUnits> g(new GroupUnits());
     // unit size: >= 4 units per worker and stratum so that the dynamic fetch balances the tail; 384 .. 2048 ratings
     int64_t target = (nnz / world) / (4 * (int64_t)(workers > 0 ? workers : 1));
     if (target < 384) target = 384;
@@ -151,55 +145,46 @@ static int stage_group_stream(lrk_handle_s* h, const int64_t* d_rowptr, const in
     const int vb = lrk_ceil_div(nv, 256), nb = lrk_ceil_div(nnz, 256);
     group_block_deg_kernel<<<vb, 256, 0, st>>>(d_rowptr, d_col, U, I, d_bounds, world, degv, rowlo); LRK_LAUNCH_CHECK(h);
     size_t tb = tmp_bytes;
-    cudaError_t e = cub::DeviceScan::ExclusiveSum(tmp, tb, degv, S, (int)nv, st);
-    if (e == cudaSuccess) { group_unit_flags_kernel<<<vb, 256, 0, st>>>(degv, S, U, world, g->target, started); h->launches++; e = cudaGetLastError(); }
+    LRK_CUDA(h, cub::DeviceScan::ExclusiveSum(tmp, tb, degv, S, (int)nv, st));
+    group_unit_flags_kernel<<<vb, 256, 0, st>>>(degv, S, U, world, g->target, started); LRK_LAUNCH_CHECK(h);
     tb = tmp_bytes;
-    if (e == cudaSuccess) e = cub::DeviceScan::InclusiveSum(tmp, tb, started, incl, (int)nv, st);
+    LRK_CUDA(h, cub::DeviceScan::InclusiveSum(tmp, tb, started, incl, (int)nv, st));
     uint32_t n_units = 0;
     std::vector<uint32_t> first_incl((size_t)world), first_started((size_t)world);
-    if (e == cudaSuccess) e = cudaMemcpyAsync(&n_units, incl + (nv - 1), sizeof(uint32_t), cudaMemcpyDeviceToHost, st);
-    for (int b = 0; b < world && e == cudaSuccess; ++b) {
-        e = cudaMemcpyAsync(&first_incl[(size_t)b], incl + (int64_t)b * U, sizeof(uint32_t), cudaMemcpyDeviceToHost, st);
-        if (e == cudaSuccess) e = cudaMemcpyAsync(&first_started[(size_t)b], started + (int64_t)b * U, sizeof(uint32_t), cudaMemcpyDeviceToHost, st);
+    LRK_CUDA(h, cudaMemcpyAsync(&n_units, incl + (nv - 1), sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
+    for (int b = 0; b < world; ++b) {
+        LRK_CUDA(h, cudaMemcpyAsync(&first_incl[(size_t)b], incl + (int64_t)b * U, sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
+        LRK_CUDA(h, cudaMemcpyAsync(&first_started[(size_t)b], started + (int64_t)b * U, sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
     }
-    if (e == cudaSuccess) e = cudaStreamSynchronize(st);
-    if (e != cudaSuccess || n_units == 0 || n_units >= LRK_GROUP_MAX_UNITS) {
-        group_units_release(g);
-        if (e != cudaSuccess) LRK_CUDA(h, e);
+    LRK_CUDA(h, cudaStreamSynchronize(st));
+    if (n_units == 0 || n_units >= LRK_GROUP_MAX_UNITS)
         return lrk_fail(h, LRK_ERR_INVALID, "stage_group_stream", "unit count out of range", __FILE__, __LINE__);
-    }
     g->n_units = n_units;
     g->unit_base.assign((size_t)world + 1, (int64_t)n_units);
     for (int b = 0; b < world; ++b) g->unit_base[(size_t)b] = (int64_t)first_incl[(size_t)b] - (int64_t)first_started[(size_t)b];
-    e = cudaMalloc((void**)&g->d_units, sizeof(int4) * (size_t)n_units);
-    if (e == cudaSuccess) e = cudaMalloc((void**)&g->d_counter, sizeof(unsigned int) * 64);
-    if (e == cudaSuccess) e = cudaMemsetAsync(g->d_units, 0, sizeof(int4) * (size_t)n_units, st);
-    if (e == cudaSuccess) e = cudaMemsetAsync(g->d_counter, 0, sizeof(unsigned int) * 64, st);
-    if (e != cudaSuccess) { group_units_release(g); LRK_CUDA(h, e); }
+    int rc;
+    if ((rc = lrk_dev_alloc(h, &g->d_units, (size_t)n_units))) return rc;
+    if ((rc = lrk_dev_alloc(h, &g->d_counter, 64))) return rc;
+    LRK_CUDA(h, cudaMemsetAsync(g->d_units, 0, sizeof(int4) * (size_t)n_units, st));
+    LRK_CUDA(h, cudaMemsetAsync(g->d_counter, 0, sizeof(unsigned int) * 64, st));
     group_unit_desc_kernel<<<vb, 256, 0, st>>>(started, incl, U, world, g->d_units); h->launches++;
     // LRK_SGD_GROUP_ROTATE=0: every unit walks its items in plain ascending order, exactly like a row of the reference's CSR walk
     // (all concurrently running units then start on the low item ids together; a probe for small matrices)
     const char* rot_env = getenv("LRK_SGD_GROUP_ROTATE");
     const int rotate = (rot_env && atoi(rot_env) == 0) ? 0 : 1;
     group_keys_kernel<<<nb, 256, 0, st>>>(row_of, d_col, nnz, U, I, d_bounds, world, degv, rowlo, started, incl, g->target, seed, rotate, g->d_units, keys, idx);
-    h->launches++;
-    e = cudaGetLastError();
+    LRK_LAUNCH_CHECK(h);
     tb = tmp_bytes;
-    if (e == cudaSuccess) e = cub::DeviceRadixSort::SortPairs(tmp, tb, keys, keys2, idx, perm, (int)nnz, 0, 52, st);
-    if (e == cudaSuccess) {
-        group_gather_kernel<<<nb, 256, 0, st>>>(perm, row_of, d_col, d_val, d_bounds, world, nnz, su, si, sr); h->launches++;
-        // unit starts = exclusive prefix sums of the unit sizes (keys2 is free again: reuse it as two uint32 arrays)
-        uint32_t* cnt = reinterpret_cast<uint32_t*>(keys);
-        uint32_t* start = cnt + n_units;
-        if ((size_t)n_units * 2 * sizeof(uint32_t) > (size_t)nnz * sizeof(uint64_t)) e = cudaErrorInvalidValue;
-        if (e == cudaSuccess) {
-            group_unit_counts_kernel<<<lrk_ceil_div(n_units, 256), 256, 0, st>>>(g->d_units, n_units, cnt); h->launches++;
-            tb = tmp_bytes;
-            e = cub::DeviceScan::ExclusiveSum(tmp, tb, cnt, start, (int)n_units, st);
-            if (e == cudaSuccess) { group_unit_starts_kernel<<<lrk_ceil_div(n_units, 256), 256, 0, st>>>(g->d_units, n_units, start); h->launches++; e = cudaGetLastError(); }
-        }
-    }
-    if (e != cudaSuccess) { group_units_release(g); LRK_CUDA(h, e); }
-    *out = g;
+    LRK_CUDA(h, cub::DeviceRadixSort::SortPairs(tmp, tb, keys, keys2, idx, perm, (int)nnz, 0, 52, st));
+    group_gather_kernel<<<nb, 256, 0, st>>>(perm, row_of, d_col, d_val, d_bounds, world, nnz, su, si, sr); h->launches++;
+    // unit starts = exclusive prefix sums of the unit sizes (keys2 is free again: reuse it as two uint32 arrays)
+    uint32_t* cnt = reinterpret_cast<uint32_t*>(keys);
+    uint32_t* start = cnt + n_units;
+    if ((size_t)n_units * 2 * sizeof(uint32_t) > (size_t)nnz * sizeof(uint64_t)) LRK_CUDA(h, cudaErrorInvalidValue);
+    group_unit_counts_kernel<<<lrk_ceil_div(n_units, 256), 256, 0, st>>>(g->d_units, n_units, cnt); h->launches++;
+    tb = tmp_bytes;
+    LRK_CUDA(h, cub::DeviceScan::ExclusiveSum(tmp, tb, cnt, start, (int)n_units, st));
+    group_unit_starts_kernel<<<lrk_ceil_div(n_units, 256), 256, 0, st>>>(g->d_units, n_units, start); LRK_LAUNCH_CHECK(h);
+    *out = std::move(g);
     return LRK_OK;
 }

@@ -411,7 +411,8 @@ __global__ void topn_scatter_kernel(const int32_t* __restrict__ slots, int n, in
     if (r == 0) out_counts[c] = fc[f];
 }
 
-// d_users: device array of nq user ids (required).  Results to device buffers [nq x topn].
+// d_users: device array of nq user ids (required).  Results to device buffers [nq x topn].  Takes the staging arena: the
+// callers (topn_to_device, topn_tc_run) hold none of it.
 static int topn_exact_parallel_launch(lrk_handle_s* h, const int32_t* d_users, int32_t nq, int topn, int exclude_train,
                                       int32_t* d_items, double* d_scores, int32_t* d_counts) {
     cudaStream_t st = h->stream;
@@ -421,45 +422,42 @@ static int topn_exact_parallel_launch(lrk_handle_s* h, const int32_t* d_users, i
     int32_t part_items = lrk_ceil_div(h->I, n_parts);
     part_items = ((part_items + TOPN_PAR_THREADS - 1) / TOPN_PAR_THREADS) * TOPN_PAR_THREADS;
     n_parts = lrk_ceil_div(h->I, part_items);
-    int32_t *pi = nullptr, *pc = nullptr, *tie = nullptr, *tslots = nullptr, *tusers = nullptr, *fi = nullptr, *fc = nullptr;
-    double *psc = nullptr, *fs = nullptr; int* tcount = nullptr;
-    int ntie = 0, rc = LRK_OK;
-    cudaError_t e = cudaMalloc((void**)&pi, sizeof(int32_t) * (size_t)nq * n_parts * T);
-    if (e == cudaSuccess) e = cudaMalloc((void**)&psc, sizeof(double) * (size_t)nq * n_parts * T);
-    if (e == cudaSuccess) e = cudaMalloc((void**)&pc, sizeof(int32_t) * (size_t)nq * n_parts);
-    if (e == cudaSuccess) e = cudaMalloc((void**)&tie, sizeof(int32_t) * (size_t)nq * 3);
-    if (e == cudaSuccess) e = cudaMalloc((void**)&tcount, sizeof(int));
-    if (e == cudaSuccess) e = cudaMemsetAsync(tcount, 0, sizeof(int), st);
-    do {
-        if (e != cudaSuccess) break;
-        tslots = tie + nq; tusers = tie + 2 * (size_t)nq;
-        const size_t smem = sizeof(double) * ((size_t)h->k + (size_t)T * TOPN_PAR_THREADS + 8) + sizeof(int32_t) * ((size_t)T * TOPN_PAR_THREADS + 16);
-        if ((e = cudaFuncSetAttribute(topn_exact_parts_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)) != cudaSuccess) break;
-        topn_exact_parts_kernel<<<nq * n_parts, TOPN_PAR_THREADS, smem, st>>>(
-            h->P64, h->Q64, h->bu64, h->bi64, h->mu, lrk_has_bias(h), h->k, h->I, h->d_rowptr, h->d_col,
-            exclude_train, d_users, n_parts, part_items, T, pi, psc, pc);
-        h->launches++;
-        if ((e = cudaGetLastError()) != cudaSuccess) break;
-        topn_exact_merge_kernel<<<lrk_ceil_div(nq, 4), 128, 0, st>>>(nq, n_parts, T, topn, pi, psc, pc, d_items, d_scores, d_counts, tie);
-        topn_collect_ties_kernel<<<lrk_ceil_div(nq, 256), 256, 0, st>>>(tie, d_users, nq, tslots, tusers, tcount);
-        h->launches += 2;
-        if ((e = cudaGetLastError()) != cudaSuccess) break;
-        if ((e = cudaMemcpyAsync(&ntie, tcount, sizeof(int), cudaMemcpyDeviceToHost, st)) != cudaSuccess) break;
-        if ((e = cudaStreamSynchronize(st)) != cudaSuccess) break;
-        if (ntie > 0) {
-            if ((e = cudaMalloc((void**)&fi, sizeof(int32_t) * (size_t)ntie * topn)) != cudaSuccess) break;
-            if ((e = cudaMalloc((void**)&fs, sizeof(double) * (size_t)ntie * topn)) != cudaSuccess) break;
-            if ((e = cudaMalloc((void**)&fc, sizeof(int32_t) * (size_t)ntie)) != cudaSuccess) break;
-            if ((rc = topn_exact_launch(h, tusers, ntie, topn, exclude_train, fi, fs, fc))) break;
-            topn_scatter_kernel<<<lrk_ceil_div((int64_t)ntie * topn, 256), 256, 0, st>>>(tslots, ntie, topn, fi, fs, fc, d_items, d_scores, d_counts);
-            h->launches++;
-            if ((e = cudaGetLastError()) != cudaSuccess) break;
-            if ((e = cudaStreamSynchronize(st)) != cudaSuccess) break;
-        }
-    } while (0);
-    cudaFree(pi); cudaFree(psc); cudaFree(pc); cudaFree(tie); cudaFree(tcount); cudaFree(fi); cudaFree(fs); cudaFree(fc);
+    // partial lists, tie flags and the tie replay (at most nq rows) in the staging arena
+    const size_t np = (size_t)nq * n_parts;
+    LrkScratch sc;
+    int rc = lrk_scratch_begin(h, np * T * 12 + np * 4 + (size_t)nq * 16 + (size_t)nq * topn * 12 + 9 * 256, &sc);
     if (rc) return rc;
-    LRK_CUDA(h, e);
+    int32_t* pi = sc.take<int32_t>(np * T);
+    double* psc = sc.take<double>(np * T);
+    int32_t* pc = sc.take<int32_t>(np);
+    int32_t* tie = sc.take<int32_t>((size_t)nq * 3);
+    int* tcount = sc.take<int>(1);
+    int32_t* fi = sc.take<int32_t>((size_t)nq * topn);
+    double* fs = sc.take<double>((size_t)nq * topn);
+    int32_t* fc = sc.take<int32_t>((size_t)nq);
+    if (!pi || !psc || !pc || !tie || !tcount || !fi || !fs || !fc)
+        return lrk_fail(h, LRK_ERR_NOMEM, "topn_exact_parallel_launch", "scratch arena too small", __FILE__, __LINE__);
+    int32_t *tslots = tie + nq, *tusers = tie + 2 * (size_t)nq;
+    LRK_CUDA(h, cudaMemsetAsync(tcount, 0, sizeof(int), st));
+    const size_t smem = sizeof(double) * ((size_t)h->k + (size_t)T * TOPN_PAR_THREADS + 8) + sizeof(int32_t) * ((size_t)T * TOPN_PAR_THREADS + 16);
+    LRK_CUDA(h, cudaFuncSetAttribute(topn_exact_parts_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    topn_exact_parts_kernel<<<nq * n_parts, TOPN_PAR_THREADS, smem, st>>>(
+        h->P64, h->Q64, h->bu64, h->bi64, h->mu, lrk_has_bias(h), h->k, h->I, h->d_rowptr, h->d_col,
+        exclude_train, d_users, n_parts, part_items, T, pi, psc, pc);
+    LRK_LAUNCH_CHECK(h);
+    topn_exact_merge_kernel<<<lrk_ceil_div(nq, 4), 128, 0, st>>>(nq, n_parts, T, topn, pi, psc, pc, d_items, d_scores, d_counts, tie);
+    topn_collect_ties_kernel<<<lrk_ceil_div(nq, 256), 256, 0, st>>>(tie, d_users, nq, tslots, tusers, tcount);
+    h->launches += 2;
+    LRK_CUDA(h, cudaGetLastError());
+    int ntie = 0;
+    LRK_CUDA(h, cudaMemcpyAsync(&ntie, tcount, sizeof(int), cudaMemcpyDeviceToHost, st));
+    LRK_CUDA(h, cudaStreamSynchronize(st));
+    if (ntie > 0) {
+        if ((rc = topn_exact_launch(h, tusers, ntie, topn, exclude_train, fi, fs, fc))) return rc;
+        topn_scatter_kernel<<<lrk_ceil_div((int64_t)ntie * topn, 256), 256, 0, st>>>(tslots, ntie, topn, fi, fs, fc, d_items, d_scores, d_counts);
+        LRK_LAUNCH_CHECK(h);
+        LRK_CUDA(h, cudaStreamSynchronize(st));
+    }
     return LRK_OK;
 }
 

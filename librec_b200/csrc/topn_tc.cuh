@@ -46,35 +46,28 @@
 #define TC_MAX_CHUNKS 16
 
 struct TcState {
-    __half* Bq = nullptr;             // [I x Kp] item operand: fp16(2^eQ * q), BiasedMF: + {hi, lo} split of 2^eQ * b_i
+    LrkBuf<__half> Bq;                // [I x Kp] item operand: fp16(2^eQ * q), BiasedMF: + {hi, lo} split of 2^eQ * b_i
     int Kp = 0;
     bool valid = false;
     bool finite = true;               // false: some item factor / bias is NaN or Inf -> exact path only
     int eQ = 0;                       // power-of-two scale of the item operand
     double qnorm_max = 0.0, bi_max = 0.0, qabs_max = 0.0;
-    unsigned long long* d_stats = nullptr;   // [0] max ||q||^2 bits, [1] max |bi| bits, [2] max |q_f| bits, [3] max err/bound (float bits)
+    LrkBuf<unsigned long long> d_stats;      // [0] max ||q||^2 bits, [1] max |bi| bits, [2] max |q_f| bits, [3] max err/bound (float bits)
     PFN_cuTensorMapEncodeTiled_v12000 encode = nullptr;
-    void* work = nullptr;                    // per-pass scratch (user operand, candidate lists, ...), grown on demand
-    size_t work_bytes = 0;
-    void* lists = nullptr;                   // per-call lists of rows without a certificate
-    size_t lists_bytes = 0;
+    LrkBuf<char> work;                       // per-pass scratch (user operand, candidate lists, ...)
+    LrkBuf<char> lists;                      // per-call lists of rows without a certificate
+    LrkBuf<int32_t> fail_items, fail_counts; // exact results of the rows without a certificate
+    LrkBuf<double> fail_scores;
     cudaEvent_t ev[5] = {nullptr, nullptr, nullptr, nullptr, nullptr};   // phase boundaries of the last call
+    ~TcState() { for (cudaEvent_t e : ev) if (e) cudaEventDestroy(e); }
 };
 
 static inline TcState* tc_state(lrk_handle_s* h) {
-    if (!h->tc) h->tc = new TcState();
-    return (TcState*)h->tc;
-}
-static inline void topn_tc_release(lrk_handle_s* h) {
-    TcState* s = (TcState*)h->tc;
-    if (!s) return;
-    cudaFree(s->Bq); cudaFree(s->d_stats); cudaFree(s->work); cudaFree(s->lists);
-    for (cudaEvent_t e : s->ev) if (e) cudaEventDestroy(e);
-    delete s;
-    h->tc = nullptr;
+    if (!h->tc) h->tc.reset(new TcState());
+    return h->tc.get();
 }
 static inline void topn_tc_invalidate(lrk_handle_s* h) {
-    if (h->tc) ((TcState*)h->tc)->valid = false;
+    if (h->tc) h->tc->valid = false;
 }
 static inline int tc_kp(lrk_handle_s* h) {
     const int kaug = h->k + (lrk_has_bias(h) ? 2 : 0);
@@ -793,13 +786,9 @@ static int tc_pass(lrk_handle_s* h, TcState* s, const int32_t* d_users, int32_t 
     const size_t b_aq = up(sizeof(__half) * (size_t)nq_pad * Kp), b_pn = up(sizeof(double2) * (size_t)nq_pad);
     const size_t b_cs = up(sizeof(uint2) * (size_t)nq_pad * n_chunks * TC_CAP);
     const size_t b_cc = up(sizeof(int32_t) * (size_t)nq_pad * n_chunks), b_ct = up(sizeof(float) * (size_t)nq_pad * n_chunks);
-    const size_t need = b_aq + b_pn + b_cs + b_cc + b_ct + 256;
-    if (s->work_bytes < need) {
-        if (s->work) { cudaFree(s->work); s->work = nullptr; s->work_bytes = 0; }
-        LRK_CUDA(h, cudaMalloc(&s->work, need));
-        s->work_bytes = need;
-    }
-    char* w = (char*)s->work;
+    int rc = lrk_dev_alloc(h, &s->work, b_aq + b_pn + b_cs + b_cc + b_ct + 256);
+    if (rc) return rc;
+    char* w = s->work;
     __half* Aq = (__half*)w; w += b_aq;
     double2* pstat = (double2*)w; w += b_pn;
     uint2* cand = (uint2*)w; w += b_cs;
@@ -810,7 +799,7 @@ static int tc_pass(lrk_handle_s* h, TcState* s, const int32_t* d_users, int32_t 
     tc_build_users_kernel<<<lrk_ceil_div(nq, 8), 256, 0, st>>>(h->P64, biased, h->k, Kp, d_users, nq, Aq, pstat);
     LRK_LAUNCH_CHECK(h);
     CUtensorMap tmB;
-    int rc = tc_make_map(h, s, &tmB, s->Bq, Kp, h->I);
+    rc = tc_make_map(h, s, &tmB, s->Bq, Kp, h->I);
     if (rc) return rc;
     TcParams p;
     memset(&p, 0, sizeof p);
@@ -851,11 +840,11 @@ static int topn_tc_run(lrk_handle_s* h, const int32_t* d_users, int32_t nq, int 
         return lrk_fail(h, LRK_ERR_INVALID, "lrk_topn", "tensor-core path supports k (+2 for BiasedMF) <= 128 and topn <= 26", __FILE__, __LINE__);
     for (cudaEvent_t& ev : s->ev) if (!ev) LRK_CUDA(h, cudaEventCreate(&ev));
     LRK_CUDA(h, cudaEventRecord(s->ev[0], st));
+    int rc;
     // ---- item operand (cached until the factors change)
     if (!s->valid || s->Kp != Kp) {
-        if (s->Bq) { cudaFree(s->Bq); s->Bq = nullptr; }
-        LRK_CUDA(h, cudaMalloc((void**)&s->Bq, sizeof(__half) * (size_t)h->I * Kp));
-        if (!s->d_stats) LRK_CUDA(h, cudaMalloc((void**)&s->d_stats, 32));
+        if ((rc = lrk_dev_alloc(h, &s->Bq, (size_t)h->I * Kp))) return rc;
+        if ((rc = lrk_dev_alloc(h, &s->d_stats, 4))) return rc;
         LRK_CUDA(h, cudaMemsetAsync(s->d_stats, 0, 32, st));
         tc_item_stats_kernel<<<lrk_ceil_div(h->I, 8), 256, 0, st>>>(h->Q64, h->bi64, biased, h->k, h->I, s->d_stats);
         LRK_LAUNCH_CHECK(h);
@@ -875,23 +864,15 @@ static int topn_tc_run(lrk_handle_s* h, const int32_t* d_users, int32_t nq, int 
     }
     if (!s->finite) {
         // NaN / Inf among the item factors: Double.compareTo semantics for those need the exact kernel
-        int rc0 = topn_exact_launch(h, d_users, nq, topn, exclude_train, d_items, d_scores, d_counts);
-        if (rc0) return rc0;
+        if ((rc = topn_exact_launch(h, d_users, nq, topn, exclude_train, d_items, d_scores, d_counts))) return rc;
         LRK_CUDA(h, cudaStreamSynchronize(st));
         h->topn_fast_users = 0; h->topn_fallback_users = nq;
         return LRK_OK;
     }
     // ---- fail lists of the call (outside the per-pass scratch, which a second pass may regrow)
-    {
-        const size_t need_l = sizeof(int32_t) * 5 * (size_t)nq + 64;
-        if (s->lists_bytes < need_l) {
-            if (s->lists) { cudaFree(s->lists); s->lists = nullptr; s->lists_bytes = 0; }
-            LRK_CUDA(h, cudaMalloc(&s->lists, need_l));
-            s->lists_bytes = need_l;
-        }
-    }
-    int* counters = (int*)s->lists;                                   // [0] second-sweep rows, [1] exact-kernel rows
-    int32_t* rs_slots = (int32_t*)((char*)s->lists + 64);
+    if ((rc = lrk_dev_alloc(h, &s->lists, sizeof(int32_t) * 5 * (size_t)nq + 64))) return rc;
+    int* counters = (int*)s->lists.ptr;                               // [0] second-sweep rows, [1] exact-kernel rows
+    int32_t* rs_slots = (int32_t*)(s->lists + 64);
     int32_t* rs_users = rs_slots + nq;
     float* rs_tau0 = (float*)(rs_users + nq);
     int32_t* ex_slots = (int32_t*)(rs_tau0 + nq);
@@ -900,7 +881,7 @@ static int topn_tc_run(lrk_handle_s* h, const int32_t* d_users, int32_t nq, int 
     LRK_CUDA(h, cudaMemsetAsync(s->d_stats + 3, 0, 8, st));
     int cnts[2] = {0, 0};
     // pass 1: every queried row from tau = -inf
-    int rc = tc_pass(h, s, d_users, nq, nullptr, nullptr, topn, exclude_train, TC_KEEP_DEFAULT(topn), d_items, d_scores, d_counts,
+    rc = tc_pass(h, s, d_users, nq, nullptr, nullptr, topn, exclude_train, TC_KEEP_DEFAULT(topn), d_items, d_scores, d_counts,
                      rs_slots, rs_users, rs_tau0, counters, ex_slots, ex_users, counters + 1, true);
     if (rc) return rc;
     LRK_CUDA(h, cudaMemcpyAsync(cnts, counters, sizeof cnts, cudaMemcpyDeviceToHost, st));
@@ -919,23 +900,14 @@ static int topn_tc_run(lrk_handle_s* h, const int32_t* d_users, int32_t nq, int 
     const int nfail = cnts[1];
     if (nfail > 0) {
         // rows still without a certificate (exact ties, fewer than N candidates, crowded bands): exact fp64 path
-        int32_t *fi = nullptr, *fc = nullptr; double* fs = nullptr;
-        cudaError_t e = cudaMalloc((void**)&fi, sizeof(int32_t) * (size_t)nfail * topn);
-        if (e == cudaSuccess) e = cudaMalloc((void**)&fs, sizeof(double) * (size_t)nfail * topn);
-        if (e == cudaSuccess) e = cudaMalloc((void**)&fc, sizeof(int32_t) * (size_t)nfail);
-        if (e == cudaSuccess) {
-            rc = topn_exact_parallel_launch(h, ex_users, nfail, topn, exclude_train, fi, fs, fc);
-            if (rc == LRK_OK) {
-                topn_scatter_kernel<<<lrk_ceil_div((int64_t)nfail * topn, 256), 256, 0, st>>>(ex_slots, nfail, topn, fi, fs, fc,
-                                                                                           d_items, d_scores, d_counts);
-                h->launches++;
-                e = cudaGetLastError();
-            }
-        }
-        if (e == cudaSuccess && rc == LRK_OK) e = cudaStreamSynchronize(st);
-        cudaFree(fi); cudaFree(fs); cudaFree(fc);
-        if (rc) return rc;
-        LRK_CUDA(h, e);
+        if ((rc = lrk_dev_alloc(h, &s->fail_items, (size_t)nfail * topn))) return rc;
+        if ((rc = lrk_dev_alloc(h, &s->fail_scores, (size_t)nfail * topn))) return rc;
+        if ((rc = lrk_dev_alloc(h, &s->fail_counts, (size_t)nfail))) return rc;
+        if ((rc = topn_exact_parallel_launch(h, ex_users, nfail, topn, exclude_train, s->fail_items, s->fail_scores, s->fail_counts))) return rc;
+        topn_scatter_kernel<<<lrk_ceil_div((int64_t)nfail * topn, 256), 256, 0, st>>>(ex_slots, nfail, topn, s->fail_items, s->fail_scores,
+                                                                                   s->fail_counts, d_items, d_scores, d_counts);
+        LRK_LAUNCH_CHECK(h);
+        LRK_CUDA(h, cudaStreamSynchronize(st));
     }
     LRK_CUDA(h, cudaEventRecord(s->ev[4], st));
     LRK_CUDA(h, cudaStreamSynchronize(st));
