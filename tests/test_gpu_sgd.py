@@ -57,7 +57,10 @@ def test_item_run_tiles_are_minibatches_for_the_item(O, capi, model_name, k):
     """Items with >= 512 ratings are staged as runs of 32 ratings (staging.cuh) and the kernel applies one item-row
     update per flush period (8, 16 or 32 ratings of a run, sgd.cuh): for users that rate a single item this is a mini-batch step on q_i / b_i.
     To first order in lr the epoch equals one step with every gradient taken at the initial q_i; which chunks see
-    which earlier updates depends on scheduling and moves the result by O(lr^2 * degree) -- hence the tolerances."""
+    which earlier updates depends on scheduling and moves the result by O(lr^2 * degree) -- hence the tolerances.
+    The item-side tolerances are loose on purpose: at lr * degree = 0.026 the item step also carries the staleness damping of
+    run tiles (a few per cent) and second-order terms of the same size, which this test does not model.  The item side is held
+    to derived budgets, and the damping to its formula, in test_gpu_sgd_first_order.py."""
     n_items, per_item = 6, 512
     n = n_items * per_item
     rng = np.random.default_rng(5)
