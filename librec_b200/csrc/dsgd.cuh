@@ -83,7 +83,6 @@ static inline void dsgd_item_bounds(const int64_t* item_count, int32_t I, int wo
 struct DsgdState {
     std::vector<int32_t> bounds;        // world+1 item block bounds
     std::vector<int64_t> seg_off;       // world+1 offsets of the COO segments
-    std::vector<double> seg_hot_share;  // per segment: largest share one item has of its ratings
     int32_t max_blk = 0;                // rows of the largest item block
     size_t buf_floats = 0;              // floats per rotating buffer: max_blk*ld + max_blk
     LrkBuf<float> qbuf[2];
@@ -97,7 +96,7 @@ struct DsgdState {
     LrkBuf<float> q_ref;                // BPR: the item factors at the start of the current window (delta all-reduce)
     LrkBuf<float> q_delta;
     int64_t bpr_samples = 0;            // BPR: samples this rank draws per epoch = numRates * (its users / all users)
-    DsgdFused fused;                    // experimental one-kernel epoch (dsgd_fused.cuh), LRK_DSGD_FUSED=1
+    DsgdFused fused;                    // the in-kernel ring of the rating models (dsgd_fused.cuh); LRK_DSGD_FUSED=0 turns it off
     ~DsgdState() {
         dsgd_fused_unmap(&fused);       // the IPC mappings go before the ring buffers
         for (cudaEvent_t ev : trace_ev) if (ev) cudaEventDestroy(ev);
@@ -267,13 +266,12 @@ static int dsgd_set_train_csr(lrk_handle_s* h, int32_t U, int32_t I, const int64
 
     // bucket by item block; inside a block: item-run tiles, then the shuffled rest (staging.cuh, stage_tile_keys)
     s->seg_off.assign((size_t)world + 1, 0);
-    s->seg_hot_share.assign((size_t)world, 0.0);
     dsgd_block_counts_kernel<<<ib, 256, 0, st>>>(h->d_item_deg, I, s->d_bounds, world, d_small); LRK_LAUNCH_CHECK(h);
     h->group.reset();
     const bool want_group = lrk_use_group_kernel(h) && group_order_supported(U, I, nnz, world);
     if (nnz > 0 && want_group) {
         LRK_CUDA(h, cudaMemsetAsync(w.max_deg, 0, sizeof(uint32_t) * 64, st));
-        if ((rc = stage_group_stream(h, h->d_rowptr, h->d_col, row_of, d_val, U, I, nnz, s->d_bounds, world, sgd_group_resident_workers(h, nullptr),
+        if ((rc = stage_group_stream(h, h->d_rowptr, h->d_col, row_of, d_val, U, I, nnz, s->d_bounds, world, sgd_group_resident_workers(h),
                                      h->cfg.seed + 977u * h->rank, sc, w.tmp, tmp_bytes, keys, keys2, idx, perm, h->d_su, h->d_si, h->d_sr, &h->group))) return rc;
     } else if (nnz > 0) {
         if ((rc = stage_tile_keys(h, h->d_col, I, nnz, s->d_bounds, world, h->cfg.seed + 977u * h->rank, w, keys, idx))) return rc;
@@ -294,10 +292,7 @@ static int dsgd_set_train_csr(lrk_handle_s* h, int32_t U, int32_t I, const int64
     h->run_tiles = (int64_t)last_base + (int64_t)last_runs;
     h->max_item_deg = 0;
     for (int b = 0; b < world; ++b) h->max_item_deg = std::max(h->max_item_deg, md[b]);
-    for (int b = 0; b < world; ++b) {
-        s->seg_off[(size_t)b + 1] = s->seg_off[(size_t)b] + (int64_t)small[b];
-        if (small[b] > 0) s->seg_hot_share[(size_t)b] = (double)md[b] / (double)small[b];
-    }
+    for (int b = 0; b < world; ++b) s->seg_off[(size_t)b + 1] = s->seg_off[(size_t)b] + (int64_t)small[b];
     if (h->cfg.model == LRK_MODEL_BPR) {
         // BPRRecommender.java:48-58 draws numRates samples per iteration, the user uniformly over ALL users: this rank's share is
         // numRates * (its users / all users)
@@ -363,7 +358,8 @@ static int dsgd_set_factors(lrk_handle_s* h, const double* P, const double* Q, c
     return LRK_OK;
 }
 
-// ---- experimental fused epoch (dsgd_fused.cuh): IPC mapping of the ring neighbours, then one cooperative launch per epoch
+// ---- fused epoch (dsgd_fused.cuh, the default; LRK_DSGD_FUSED=0 turns it off): IPC mapping of the ring neighbours, then one
+// cooperative launch per epoch
 static int dsgd_fused_map(lrk_handle_s* h, DsgdState* s) {
     NcclApi* n = nccl_api();
     DsgdFused* f = &s->fused;
@@ -448,59 +444,43 @@ static int dsgd_fused_map(lrk_handle_s* h, DsgdState* s) {
     return LRK_OK;
 }
 
+// the fused epoch kernel for (model, variant)
 template <int G, int V>
-static int dsgd_fused_launch_gv(lrk_handle_s* h, DsgdState* s, DsgdFusedParams& fp, bool track) {
-    const bool biased = h->cfg.model == LRK_MODEL_BIASEDMF;
-    void* kern = nullptr;
-    if (biased) kern = track ? (void*)dsgd_fused_epoch_kernel<G, V, true, true> : (void*)dsgd_fused_epoch_kernel<G, V, true, false>;
-    else kern = track ? (void*)dsgd_fused_epoch_kernel<G, V, false, true> : (void*)dsgd_fused_epoch_kernel<G, V, false, false>;
-    int per_sm = 0;
-    LRK_CUDA(h, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, 256, 0));
-    if (per_sm < 1) per_sm = 1;
-    int64_t grid = (int64_t)h->sm_count * per_sm;
-    for (int t = 0; t < h->world; ++t) {                       // staleness cap of the smallest non-empty segment (sgd_grid_for)
-        const int64_t n = fp.seg[t].n;
-        if (n <= 0) continue;
-        const int64_t stale_cap = (n / 16) / (8 * (int64_t)(32 / G) * 2);
-        if (stale_cap < grid) grid = stale_cap;
-    }
-    if (h->conc_div > 1) grid /= h->conc_div;
-    if (grid < 1) grid = 1;
-    for (int t = 0; t < h->world; ++t) {
-        const int64_t n = fp.seg[t].n > 0 ? fp.seg[t].n : 1;
-        fp.seg[t].inflight_frac = (float)((double)grid * 8.0 * (double)(32 / G > 8 ? 32 / G : 8) / (double)n);
-    }
+static const void* dsgd_fused_kernel(const lrk_handle_s* h, bool track) {
+    if (h->cfg.model == LRK_MODEL_BIASEDMF)
+        return track ? (const void*)dsgd_fused_epoch_kernel<G, V, true, true> : (const void*)dsgd_fused_epoch_kernel<G, V, true, false>;
+    return track ? (const void*)dsgd_fused_epoch_kernel<G, V, false, true> : (const void*)dsgd_fused_epoch_kernel<G, V, false, false>;
+}
+
+template <int G, int V>
+static int dsgd_fused_launch_gv(lrk_handle_s* h, DsgdFusedParams& fp) {
+    const bool track = sgd_track(h, fp.seg[0]);
+    const void* kern = dsgd_fused_kernel<G, V>(h, track);
+    int grid = 1, rc;
+    if ((rc = sgd_grid(h, kern, 32 / G, track, fp.seg, h->world, &grid))) return rc;
     void* args[] = {(void*)&fp};
     LRK_CUDA(h, cudaLaunchCooperativeKernel(kern, dim3((unsigned)grid), dim3(256), args, 0, h->stream));
     h->launches++;
-    (void)s;
     return LRK_OK;
 }
 
 template <int G, int V>
-static int dsgd_fused_group_launch_gv(lrk_handle_s* h, DsgdFusedGroupParams& fp) {
+static int dsgd_fused_group_launch_gv(lrk_handle_s* h, const SgdParams* seg, DsgdFusedGroupParams& fp) {
     const bool biased = h->cfg.model == LRK_MODEL_BIASEDMF;
     void* kern = biased ? (void*)dsgd_fused_group_epoch_kernel<G, V, true> : (void*)dsgd_fused_group_epoch_kernel<G, V, false>;
     const size_t smem = sgd_group_smem_bytes<G, V>();
     LRK_CUDA(h, cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     int per_sm = 0;
     LRK_CUDA(h, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, 256, smem));
-    if (per_sm < 1) per_sm = 1;
-    constexpr int WPC = 8 * (32 / G);
-    int64_t grid = (int64_t)h->sm_count * per_sm;
-    int64_t most = 1;
-    for (int t = 0; t < h->world; ++t) most = std::max<int64_t>(most, (fp.seg[t].n_units + WPC - 1) / WPC);
-    if (most < grid) grid = most;
-    if (h->conc_div > 1) grid /= h->conc_div;
-    if (grid < 1) grid = 1;
+    const int grid = sgd_group_grid(h, (int64_t)h->sm_count * std::max(per_sm, 1), 8 * (32 / G), seg, fp.seg, h->world);
     void* args[] = {(void*)&fp};
     LRK_CUDA(h, cudaLaunchCooperativeKernel(kern, dim3((unsigned)grid), dim3(256), args, smem, h->stream));
     h->launches++;
-    return (int)grid;
+    return LRK_OK;
 }
 
 // true: the epoch's strata were run by the fused kernel (s->cur advanced like the loop would have); false: not applicable here
-static int dsgd_fused_epoch(lrk_handle_s* h, DsgdState* s, float lr, float reg_u, float reg_i, double reg_b, int32_t epoch_idx, bool* done) {
+static int dsgd_fused_epoch(lrk_handle_s* h, DsgdState* s, const SgdParams& base, bool* done) {
     *done = false;
     DsgdFused* f = &s->fused;
     if (f->enabled < 0) { const char* e = getenv("LRK_DSGD_FUSED"); f->enabled = (e && atoi(e) == 0) ? 0 : 1; }     // default on
@@ -524,79 +504,37 @@ static int dsgd_fused_epoch(lrk_handle_s* h, DsgdState* s, float lr, float reg_u
         f->seq = 0;
         f->needs_reset = false;
     }
-    if (h->group) {
-        GroupUnits* gu = h->group.get();
-        DsgdFusedGroupParams gp;
-        memset(&gp, 0, sizeof gp);
-        int ctas = 0;
-        const int workers = sgd_group_resident_workers(h, &ctas);
-        for (int t = 0; t < world; ++t) {
-            const int b = dsgd_block_at(h->rank, world, t);
-            const int64_t off = s->seg_off[(size_t)b], cnt = s->seg_off[(size_t)b + 1] - off;
-            SgdGroupParams& sp = gp.seg[t];
-            sp.su = h->d_su; sp.si = h->d_si; sp.sr = h->d_sr;
-            sp.units = gu->d_units + gu->unit_base[(size_t)b];
-            sp.n_units = cnt > 0 ? (int32_t)(gu->unit_base[(size_t)b + 1] - gu->unit_base[(size_t)b]) : 0;
-            sp.counter = gu->d_counter + b;
-            sp.P = h->P32; sp.bu = h->bu32;
-            sp.mu = (float)h->mu; sp.lr = lr; sp.reg_u = reg_u; sp.reg_i = reg_i; sp.reg_b = (float)reg_b;
-            sp.loss = h->d_loss; sp.ld = h->ld;
-            sp.item_deg = h->d_item_deg ? h->d_item_deg + s->bounds[(size_t)b] : nullptr;
-            const double w = (double)std::min<int64_t>((int64_t)workers / (h->conc_div > 1 ? h->conc_div : 1), std::max<int64_t>(sp.n_units, 1));
-            sp.inflight_frac = (float)(w / (double)(cnt > 0 ? cnt : 1));
-        }
-        gp.qbuf[0] = s->qbuf[0]; gp.qbuf[1] = s->qbuf[1];
-        gp.peer_qbuf[0] = f->peer_qbuf[0]; gp.peer_qbuf[1] = f->peer_qbuf[1];
-        gp.ready = f->d_flags; gp.peer_free = f->d_flags + 2;
-        gp.prev_ready = f->prev_flags; gp.next_peer_free = f->next_flags + 2;
-        gp.seq0 = f->seq; gp.cur0 = s->cur; gp.world = world;
-        gp.buf_floats = (long long)s->buf_floats; gp.bi_off = (long long)s->max_blk * h->ld;
-        gp.abort = f->d_abort;
-        gp.spin_limit = 4000000000LL;
-        LRK_CUDA(h, cudaMemsetAsync(f->d_abort, 0, sizeof(int), h->stream));
-        switch (h->G) {
-            case 8: rc = dsgd_fused_group_launch_gv<8, 1>(h, gp); break;
-            case 16: rc = dsgd_fused_group_launch_gv<16, 1>(h, gp); break;
-            default: rc = dsgd_fused_group_launch_gv<32, 1>(h, gp); break;
-        }
-        if (rc < 0) return rc;
-        f->seq += (unsigned long long)world;
-        s->cur = (s->cur + world) & 1;
-        s->cur_block = dsgd_block_at(h->rank, world, world);
-        *done = true;
-        return LRK_OK;
-    }
-    DsgdFusedParams fp;
-    memset(&fp, 0, sizeof fp);
-    static const char* hf = getenv("LRK_SGD_HOT_FLUSH");
+    SgdParams seg[LRK_FUSED_MAX_WORLD];
     for (int t = 0; t < world; ++t) {
         const int b = dsgd_block_at(h->rank, world, t);
-        const int64_t off = s->seg_off[(size_t)b], cnt = s->seg_off[(size_t)b + 1] - off;
-        SgdParams& sp = fp.seg[t];
-        sp.su = h->d_su + off; sp.si = h->d_si + off; sp.sr = h->d_sr + off; sp.n = cnt;
-        sp.P = h->P32; sp.bu = h->bu32;
-        sp.mu = (float)h->mu; sp.lr = lr; sp.reg_u = reg_u; sp.reg_i = reg_i; sp.reg_b = (float)reg_b;
-        sp.loss = h->d_loss; sp.ld = h->ld; sp.epoch = (uint32_t)epoch_idx;
-        sp.tile_mul = sgd_tile_mul(cnt);
-        sp.conc_div = h->conc_div;
-        sp.item_deg = h->d_item_deg ? h->d_item_deg + s->bounds[(size_t)b] : nullptr;
-        sp.pnorm2 = sp.item_deg ? h->d_pnorm2.ptr : nullptr;
-        sp.hot_flush_deg = hf ? (atoi(hf) > 0 ? (uint32_t)atoi(hf) : 0xffffffffu) : 512u;
+        const int64_t off = s->seg_off[(size_t)b];
+        seg[t] = sgd_segment(h, base, off, s->seg_off[(size_t)b + 1] - off, nullptr, nullptr, s->bounds[(size_t)b]);   // Q / bi: in-kernel
     }
-    fp.qbuf[0] = s->qbuf[0]; fp.qbuf[1] = s->qbuf[1];
-    fp.peer_qbuf[0] = f->peer_qbuf[0]; fp.peer_qbuf[1] = f->peer_qbuf[1];
-    fp.ready = f->d_flags; fp.peer_free = f->d_flags + 2;
-    fp.prev_ready = f->prev_flags; fp.next_peer_free = f->next_flags + 2;
-    fp.seq0 = f->seq; fp.cur0 = s->cur; fp.world = world;
-    fp.buf_floats = (long long)s->buf_floats; fp.bi_off = (long long)s->max_blk * h->ld;
-    fp.abort = f->d_abort;
-    fp.spin_limit = 4000000000LL;                               // ~2 s at 2 GHz
+    auto ring = [&](auto& p) {
+        p.qbuf[0] = s->qbuf[0]; p.qbuf[1] = s->qbuf[1];
+        p.peer_qbuf[0] = f->peer_qbuf[0]; p.peer_qbuf[1] = f->peer_qbuf[1];
+        p.ready = f->d_flags; p.peer_free = f->d_flags + 2;
+        p.prev_ready = f->prev_flags; p.next_peer_free = f->next_flags + 2;
+        p.seq0 = f->seq; p.cur0 = s->cur; p.world = world;
+        p.buf_floats = (long long)s->buf_floats; p.bi_off = (long long)s->max_blk * h->ld;
+        p.abort = f->d_abort;
+        p.spin_limit = 4000000000LL;                            // ~2 s at 2 GHz
+    };
     LRK_CUDA(h, cudaMemsetAsync(f->d_abort, 0, sizeof(int), h->stream));      // a timeout of an earlier epoch must not silence this one
-    const bool track = fp.seg[0].item_deg && sgd_want_track(h, h->G * h->V);
-    switch (h->G) {
-        case 16: rc = dsgd_fused_launch_gv<16, 1>(h, s, fp, track); break;          // k in 33..64 and 65..128: the benchmark shapes;
-        case 32: rc = dsgd_fused_launch_gv<32, 1>(h, s, fp, track); break;          // smaller k stays on the sub-epoch loop
-        default: return LRK_OK;
+    if (h->group) {
+        DsgdFusedGroupParams gp{};
+        ring(gp);
+        for (int t = 0; t < world; ++t) gp.seg[t] = sgd_group_params(h, seg[t], dsgd_block_at(h->rank, world, t));
+        rc = sgd_with_group_layout(h, [&](auto G, auto V) { return dsgd_fused_group_launch_gv<decltype(G)::value, decltype(V)::value>(h, seg, gp); });
+    } else {
+        DsgdFusedParams fp{};
+        ring(fp);
+        for (int t = 0; t < world; ++t) fp.seg[t] = seg[t];
+        rc = lrk_with_layout(h, [&](auto G, auto V) -> int {
+            // k in 33..64 and 65..128: the benchmark shapes; smaller k stays on the sub-epoch loop (checked above)
+            if constexpr (decltype(G)::value >= 16 && decltype(V)::value == 1) return dsgd_fused_launch_gv<decltype(G)::value, decltype(V)::value>(h, fp);
+            else return lrk_fail(h, LRK_ERR_INVALID, "dsgd_fused_epoch", "unsupported factor layout", __FILE__, __LINE__);
+        });
     }
     if (rc) return rc;
     f->seq += (unsigned long long)world;
@@ -614,7 +552,7 @@ static int dsgd_fused_epoch(lrk_handle_s* h, DsgdState* s, float lr, float reg_u
 // apply the sum -- the one real exchange step of this path.  Within a window a rank does not see the other ranks' item updates
 // (the same kind of staleness as ratings in flight on one GPU, one window long).
 #define LRK_BPR_WINDOWS 8
-static int dsgd_bpr_epoch(lrk_handle_s* h, DsgdState* s, float lr, float reg_u, float reg_i, int32_t epoch_idx) {
+static int dsgd_bpr_epoch(lrk_handle_s* h, DsgdState* s, const SgdParams& base) {
     NcclApi* n = nccl_api();
     cudaStream_t st = h->stream;
     const int64_t nq = (int64_t)h->I * h->ld;
@@ -622,18 +560,12 @@ static int dsgd_bpr_epoch(lrk_handle_s* h, DsgdState* s, float lr, float reg_u, 
     if ((rc = lrk_dev_alloc(h, &s->q_ref, (size_t)nq))) return rc;
     if ((rc = lrk_dev_alloc(h, &s->q_delta, (size_t)nq))) return rc;
     LRK_CUDA(h, cudaMemcpyAsync(s->q_ref, h->Q32, sizeof(float) * (size_t)nq, cudaMemcpyDeviceToDevice, st));
-    const uint64_t seed = h->cfg.seed + 977u * (uint64_t)h->rank;
     int64_t done = 0;
     for (int w = 0; w < LRK_BPR_WINDOWS; ++w) {
         const int64_t cnt = s->bpr_samples * (w + 1) / LRK_BPR_WINDOWS - done;
         if (cnt > 0 && h->U > 0 && h->nnz > 0) {
-            SgdParams sp;
-            memset(&sp, 0, sizeof sp);
-            sp.n = cnt; sp.P = h->P32; sp.Q = h->Q32; sp.lr = lr; sp.reg_u = reg_u; sp.reg_i = reg_i;
-            sp.loss = h->d_loss; sp.ld = h->ld; sp.epoch = (uint32_t)epoch_idx;
-            sp.rowptr = h->d_rowptr; sp.col = h->d_col; sp.U = h->U; sp.I = h->I;
-            sp.seed_lo = (uint32_t)seed; sp.seed_hi = (uint32_t)(seed >> 32);
-            sp.sample_base = done; sp.conc_div = h->conc_div;
+            SgdParams sp = sgd_segment(h, base, 0, cnt, h->Q32, h->bi32, 0);
+            sp.sample_base = done;
             if ((rc = sgd_launch(h, sp))) return rc;
         }
         done += cnt;
@@ -661,6 +593,7 @@ static int dsgd_epoch(lrk_handle_s* h, float lr, float reg_u, float reg_i, doubl
         return v;
     };
     if (h->h_pnorm2) { h->pnorm2_prev = h->pnorm2_host; h->pnorm2_host = *h->h_pnorm2; }
+    const SgdParams base = sgd_params(h, lr, reg_u, reg_i, reg_b, epoch_idx);
     bool fused_done = false;
     e.enqueue = [&](int) -> int {
         if (h->group) LRK_CUDA(h, cudaMemsetAsync(h->group->d_counter, 0, sizeof(unsigned int) * 64, st));
@@ -672,36 +605,15 @@ static int dsgd_epoch(lrk_handle_s* h, float lr, float reg_u, float reg_i, doubl
         if (s->trace) LRK_CUDA(h, cudaEventRecord(s->trace_ev[0], st));
         fused_done = false;
         int rc;
-        if (bpr_) { if ((rc = dsgd_bpr_epoch(h, s, lr, reg_u, reg_i, epoch_idx))) return rc; }
-        else if ((rc = dsgd_fused_epoch(h, s, lr, reg_u, reg_i, reg_b, epoch_idx, &fused_done))) return rc;
+        if (bpr_) { if ((rc = dsgd_bpr_epoch(h, s, base))) return rc; }
+        else if ((rc = dsgd_fused_epoch(h, s, base, &fused_done))) return rc;
         for (int sub = 0; !bpr_ && !fused_done && sub < world; ++sub) {
             const int b = dsgd_block_at(rank, world, sub);
             float* buf = s->qbuf[s->cur];
             const int64_t off = s->seg_off[(size_t)b], cnt = s->seg_off[(size_t)b + 1] - off;
             if (cnt > 0) {
-                SgdParams sp;
-                memset(&sp, 0, sizeof sp);
-                sp.su = h->d_su + off; sp.si = h->d_si + off; sp.sr = h->d_sr + off; sp.n = cnt;
-                sp.P = h->P32; sp.Q = buf; sp.bu = h->bu32; sp.bi = buf + (size_t)s->max_blk * h->ld;
-                sp.mu = (float)h->mu; sp.lr = lr; sp.reg_u = reg_u; sp.reg_i = reg_i; sp.reg_b = (float)reg_b;
-                sp.loss = h->d_loss; sp.ld = h->ld; sp.epoch = (uint32_t)epoch_idx;
-                sp.hot_share = (size_t)b < s->seg_hot_share.size() ? s->seg_hot_share[(size_t)b] : 0.0;
-                sp.conc_div = h->conc_div;
-                sp.item_deg = h->d_item_deg ? h->d_item_deg + s->bounds[(size_t)b] : nullptr;   // block-local item ids
-                sp.pnorm2 = sp.item_deg ? h->d_pnorm2.ptr : nullptr;
-                GroupUnits* gu = h->group.get();
-                if (gu) {
-                    SgdGroupParams gp;
-                    memset(&gp, 0, sizeof gp);
-                    gp.su = h->d_su; gp.si = h->d_si; gp.sr = h->d_sr;                      // unit starts index the whole stream
-                    gp.units = gu->d_units + gu->unit_base[(size_t)b];
-                    gp.n_units = (int32_t)(gu->unit_base[(size_t)b + 1] - gu->unit_base[(size_t)b]);
-                    gp.counter = gu->d_counter + b;
-                    gp.P = sp.P; gp.Q = sp.Q; gp.bu = sp.bu; gp.bi = sp.bi; gp.mu = sp.mu; gp.lr = sp.lr; gp.reg_u = sp.reg_u; gp.reg_i = sp.reg_i;
-                    gp.reg_b = sp.reg_b; gp.loss = sp.loss; gp.ld = sp.ld; gp.item_deg = sp.item_deg;
-                    rc = sgd_group_launch(h, gp, cnt, h->conc_div);
-                } else rc = sgd_launch(h, sp);
-                if (rc) return rc;
+                const SgdParams sp = sgd_segment(h, base, off, cnt, buf, buf + (size_t)s->max_blk * h->ld, s->bounds[(size_t)b]);
+                if ((rc = h->group ? sgd_group_launch(h, sp, b) : sgd_launch(h, sp))) return rc;
             }
             if (s->trace) LRK_CUDA(h, cudaEventRecord(s->trace_ev[(size_t)2 * sub + 1], st));
             if (world > 1) {

@@ -251,7 +251,8 @@ int lrk_create(const lrk_config_t* cfg, lrk_handle_t* out) {
     layout_for_k(h->k, &h->ld, &h->G, &h->V);
     {   // the user-group kernel (LRK_SGD_GROUP=1, sgd_group.cuh) needs at least 8 lanes per rating: small k are padded to 32 columns
         const char* env = getenv("LRK_SGD_GROUP");
-        if (env && atoi(env) != 0 && k_lrk_models[cfg->model].rating && cfg->update_mode == LRK_UPDATE_ATOMIC && h->ld < 32) { h->ld = 32; h->G = 8; h->V = 1; }
+        h->sgd_group = env && atoi(env) != 0 && k_lrk_models[cfg->model].rating && cfg->update_mode == LRK_UPDATE_ATOMIC;
+        if (h->sgd_group && h->ld < 32) { h->ld = 32; h->G = 8; h->V = 1; }
     }
     h->sm_count = prop.multiProcessorCount;
     int rc = LRK_OK;
@@ -325,12 +326,12 @@ int lrk_set_train_csr(lrk_handle_t h, int32_t U, int32_t I, const int64_t* rowpt
         topn_tc_invalidate(h);
         return LRK_OK;
     }
-    // BiasedMF / PMF in the default (atomic) mode train with the user-group kernel over a unit-ordered stream (sgd_group.cuh);
-    // Hogwild mode, the reference-order mode, BPR / RankSGD and layouts outside 32 < ld <= 128 keep the shuffled stream of sgd.cuh
+    // BiasedMF / PMF in atomic mode with LRK_SGD_GROUP=1 train with the user-group kernel over a unit-ordered stream (sgd_group.cuh);
+    // everything else keeps the item-run-tile stream of sgd.cuh
     h->group.reset();
     const bool want_group = lrk_use_group_kernel(h) && group_order_supported(U, I, nnz, 1);
     rc = stage_coo_from_csr(h, h->d_rowptr, h->d_col, val, U, I, nnz, h->d_su, h->d_si, h->d_sr, /*validate=*/true,
-                            want_group ? sgd_group_resident_workers(h, nullptr) : 0, &h->group);
+                            want_group ? sgd_group_resident_workers(h) : 0, &h->group);
     if (rc) return rc;
     if (h->cfg.model == LRK_MODEL_RANKSGD && nnz > 0) {
         // sampling table of the negatives: inclusive prefix sums of the item degrees (RankSGDRecommender.java:47-57)
@@ -433,33 +434,6 @@ int lrk_get_factors(lrk_handle_t h, double* P, double* Q, double* bu, double* bi
 }
 
 // -------------------------------------------------------------------------------------------
-// stability cap of the SGD grid (sgd_grid_for; it applies to launches without the staleness-aware step)
-static double sgd_hot_share(const lrk_handle_s* h) {
-    // RankSGD: squared loss without regularisation -- B concurrent updates of one item act like ONE step lr * B * |p_u|^2
-    // where the sequential walk contracts by exp(-lr * B * |p_u|^2).  Popular items are hit as positives and, by
-    // construction of the sampler, as negatives (2 x share), and the two only agree while that product is small: the grid
-    // is capped at lr * 2 share * |p|^2 * (ratings in flight) <= 1/4 (sgd_grid_for's hot-item cap).  With <= 1 instead, C1
-    // reached the oracle's loss but Precision@10 0.140 against 0.176 (sequential) / 0.214 (sequential, shuffled order).
-    // r02: the RankSGD kernel scales its item-side steps for the samples in flight (sgd.cuh), so the cap is only the fallback of
-    // LRK_SGD_NODAMP=1 (r01: it left a handful of CTAs on the ML-20M shape, 0.48 G updates/s)
-    if (h->cfg.model == LRK_MODEL_RANKSGD) return 8.0 * h->hot_share * (double)std::max(1.f, h->pnorm2_host);
-    return k_lrk_models[h->cfg.model].rating ? h->hot_share : 0.0;
-}
-
-// read-only with respect to the handle (lrk_bpr_peek_samples uses it too)
-static void fill_sgd_params(const lrk_handle_s* h, SgdParams& sp, float lr, float reg_u, float reg_i, double reg_b, int32_t epoch_idx) {
-    memset(&sp, 0, sizeof sp);
-    sp.su = h->d_su; sp.si = h->d_si; sp.sr = h->d_sr; sp.n = h->nnz;
-    sp.P = h->P32; sp.Q = h->Q32; sp.bu = h->bu32; sp.bi = h->bi32;
-    sp.mu = (float)h->mu; sp.lr = lr; sp.reg_u = reg_u; sp.reg_i = reg_i; sp.reg_b = (float)reg_b;
-    sp.loss = h->d_loss; sp.ld = h->ld;
-    sp.hot_share = sgd_hot_share(h);
-    sp.item_deg = k_lrk_models[h->cfg.model].damped ? h->d_item_deg.ptr : nullptr;
-    sp.item_cum = h->cfg.model == LRK_MODEL_RANKSGD ? h->d_item_cum.ptr : nullptr;
-    sp.rowptr = h->d_rowptr; sp.col = h->d_col; sp.U = h->U; sp.I = h->I;
-    sp.seed_lo = (uint32_t)h->cfg.seed; sp.seed_hi = (uint32_t)(h->cfg.seed >> 32); sp.epoch = (uint32_t)epoch_idx;
-}
-
 int lrk_sgd_epoch(lrk_handle_t h, float lr, float reg_u, float reg_i, double reg_b, int32_t epoch_idx, double* loss_out) {
     LRK_REQUIRE(h, h != nullptr, "handle is NULL");
     if (h->multi) return multi_sgd_epoch(h, lr, reg_u, reg_i, reg_b, epoch_idx, loss_out);
@@ -480,8 +454,7 @@ int lrk_sgd_epoch(lrk_handle_t h, float lr, float reg_u, float reg_i, double reg
     // curvature estimate of the epoch: the value the last norm refresh left in pinned memory (once per epoch call, so that a
     // lrk_bpr_peek_samples between two epochs cannot change which kernel variant the next epoch picks)
     if (h->h_pnorm2) { h->pnorm2_prev = h->pnorm2_host; h->pnorm2_host = *h->h_pnorm2; }
-    SgdParams sp;
-    fill_sgd_params(h, sp, lr, reg_u, reg_i, reg_b, epoch_idx);
+    SgdParams sp = sgd_segment(h, sgd_params(h, lr, reg_u, reg_i, reg_b, epoch_idx), 0, h->nnz, h->Q32, h->bi32, 0);
     AobprState* ao = nullptr;
     if (h->cfg.model == LRK_MODEL_AOBPR) {
         ao = h->aobpr.get();
@@ -490,25 +463,17 @@ int lrk_sgd_epoch(lrk_handle_t h, float lr, float reg_u, float reg_i, double reg
         if (rc_a) return rc_a;
         sp.ao_rank = ao->d_rank; sp.ao_var = ao->d_var; sp.ao_cum = ao->d_cum; sp.n_entries = h->nnz;
     }
-    if (sp.item_deg) sp.pnorm2 = h->d_pnorm2;          // refreshed by refresh_user_norm2 at set_factors and after every epoch
     e.saved = [&] {
         std::vector<LrkSaved> v{{h->P32, &h->bk_P, (size_t)h->U * h->ld}, {h->Q32, &h->bk_Q, (size_t)h->I * h->ld}};
         if (lrk_has_bias(h)) { v.push_back({h->bu32, &h->bk_bu, (size_t)h->U}); v.push_back({h->bi32, &h->bk_bi, (size_t)h->I}); }
         return v;
     };
     e.enqueue = [&](int attempt) -> int {
-        sp.conc_div = h->conc_div;
         if (h->nnz == 0) return LRK_OK;
         int rc;
         if (h->group) {
-            GroupUnits* gu = h->group.get();
-            SgdGroupParams gp;
-            memset(&gp, 0, sizeof gp);
-            gp.su = sp.su; gp.si = sp.si; gp.sr = sp.sr; gp.units = gu->d_units; gp.n_units = (int32_t)gu->n_units; gp.counter = gu->d_counter;
-            gp.P = sp.P; gp.Q = sp.Q; gp.bu = sp.bu; gp.bi = sp.bi; gp.mu = sp.mu; gp.lr = sp.lr; gp.reg_u = sp.reg_u; gp.reg_i = sp.reg_i;
-            gp.reg_b = sp.reg_b; gp.loss = sp.loss; gp.ld = sp.ld; gp.item_deg = sp.item_deg;
-            LRK_CUDA(h, cudaMemsetAsync(gu->d_counter, 0, sizeof(unsigned int), h->stream));
-            return sgd_group_launch(h, gp, h->nnz, h->conc_div);
+            LRK_CUDA(h, cudaMemsetAsync(h->group->d_counter, 0, sizeof(unsigned int), h->stream));
+            return sgd_group_launch(h, sp, 0);
         }
         if (!ao) return sgd_launch(h, sp);
         // AoBPR: the epoch in windows of loopNumber samples, the factor rankings refreshed between them (countIter runs across
@@ -517,8 +482,8 @@ int lrk_sgd_epoch(lrk_handle_t h, float lr, float reg_u, float reg_i, double reg
         while (done < h->nnz) {
             if (count % ao->loop == 0) { if ((rc = aobpr_refresh(h, ao))) return rc; count = 0; }
             const int64_t w = std::min<int64_t>(h->nnz - done, (int64_t)ao->loop - count);
-            SgdParams wp = sp;
-            wp.n = w; wp.sample_base = done;
+            SgdParams wp = sgd_segment(h, sp, 0, w, h->Q32, h->bi32, 0);
+            wp.sample_base = done;
             if ((rc = sgd_launch(h, wp))) return rc;
             done += w; count += w;
         }
@@ -532,7 +497,6 @@ int lrk_sgd_epoch(lrk_handle_t h, float lr, float reg_u, float reg_i, double reg
         const int rc = refresh_user_norm2(h, true);     // the restored factors' norm, visible to the host now
         if (rc) return rc;
         h->pnorm2_host = *h->h_pnorm2;
-        sp.hot_share = sgd_hot_share(h);
         return LRK_OK;
     };
     return lrk_epoch(h, e, loss_out);
@@ -709,8 +673,7 @@ int lrk_bpr_peek_samples(lrk_handle_t h, int32_t epoch_idx, int64_t first, int64
     LRK_REQUIRE(h, h->world == 1, "not available in DSGD mode");
     LRK_CUDA(h, cudaSetDevice(h->cfg.device));
     if (n == 0) return LRK_OK;
-    SgdParams sp;
-    fill_sgd_params(h, sp, 0.f, 0.f, 0.f, 0.0, epoch_idx);
+    SgdParams sp = sgd_params(h, 0.f, 0.f, 0.f, 0.0, epoch_idx);
     if (h->cfg.model == LRK_MODEL_AOBPR) {
         // the draws depend on the factor rankings: those of the current item factors (what the first window of an epoch uses)
         AobprState* ao = h->aobpr.get();

@@ -52,13 +52,13 @@ struct lrk_handle_s {
     LrkBuf<int32_t> d_si;
     LrkBuf<float> d_sr;
     bool has_train = false;
+    bool sgd_group = false;              // LRK_SGD_GROUP=1 at lrk_create: BiasedMF / PMF in atomic mode use the user-group kernel
     std::unique_ptr<GroupUnits> group;   // the stream is unit-ordered (staging_group.cuh) and the epoch runs sgd_group_epoch_kernel
     int64_t run_tiles = 0;    // 32-rating item-run tiles in the staged stream (lrk_stage_stats)
     uint32_t max_item_deg = 0;
-    double hot_share = 0.0;   // largest share one item has of the train ratings (stability cap of the SGD grid)
     LrkBuf<float> d_pnorm2;           // mean |p_u|^2 at the start of the epoch (curvature term of that step)
     float pnorm2_host = 0.f;          // its host copy, refreshed with every loss read-back (picks the kernel variant)
-    float pnorm2_prev = 0.f;          // the value one epoch earlier (growth of the user factors, sgd_launch_gv)
+    float pnorm2_prev = 0.f;          // the value one epoch earlier (growth of the user factors, the LRK_SGD_TRACE line)
     LrkBuf<uint32_t> d_item_deg;      // ratings per item in this handle's shard (staleness-aware step of run tiles, sgd.cuh)
     LrkBuf<uint32_t> d_item_cum;      // RankSGD: inclusive prefix sums of d_item_deg (negative sampling table)
 

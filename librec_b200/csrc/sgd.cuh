@@ -38,7 +38,7 @@
 // (user_norm2_kernel, read from device memory) for a warp's first run tile, then the mean over the 32 users of
 // the warp's previous run tile (the factors grow fast in the first epochs; 5 shuffles per tile).  Config C4 (PMF k=128, lr 0.01, Netflix
 // shape) ran at 1.2 G updates/s behind the rollback safeguard (grid / 8) before this, at 6.6 G without a rollback after.  (Without it the grid had to be capped at lr * s * in-flight <= 1, s = share of the hottest item,
-// which left 142 of 592 CTAs at 8 DSGD strata; sgd_grid_for keeps that cap for launches without degrees.)
+// which left 142 of 592 CTAs at 8 DSGD strata; that cap is gone.)
 #pragma once
 #include "lrk_common.cuh"
 
@@ -58,10 +58,9 @@ struct SgdParams {
     // tile t of the epoch is read from stream position (t * tile_mul) % ntiles: the staged stream is
     // [item-run tiles | shuffled remainder], the multiplicative walk interleaves the two evenly in time
     int64_t tile_mul;
-    double hot_share;       // largest share one item has of this launch's ratings (0 = unknown): stability cap of the grid
-    int conc_div;           // >= 1: divisor of the grid (rollback safeguard, lrk_epoch.cuh)
+    int conc_div;           // >= 1: divisor of the grid (rollback safeguard, lrk_epoch.cuh), filled in by sgd_grid
     // staleness-aware step of item-run tiles: item_deg[i] = ratings of item i in this launch (NULL = off),
-    // inflight_frac = (ratings in flight) / n, filled in by the launcher
+    // inflight_frac = (ratings in flight) / n, filled in by sgd_grid
     const uint32_t* item_deg;
     float inflight_frac;
     // run tiles of items with at least this many ratings flush every 16 ratings, from twice this on once per tile
@@ -133,7 +132,7 @@ __device__ __forceinline__ void block_loss_commit(double v, double* out) {
 // BiasedMF / PMF.  G lanes per rating, V float4 per lane (row length ld = 4*G*V floats).
 // ---------------------------------------------------------------------------------------------
 // TRACK: refresh the curvature estimate max(1, mean |p_u|^2) from every run tile (a few registers and 5 shuffles per
-// tile; chosen by the launcher when the user factors are no longer small, see sgd_launch_gv)
+// tile; chosen by the launcher when the user factors are no longer small, see sgd_want_track)
 template <int G, int V, bool BIASED, bool ATOMIC, bool TRACK = false>
 __global__ void __launch_bounds__(256, (G * V <= 16 && !TRACK) ? 4 : ((G * V <= 32) ? 3 : 1)) sgd_rating_epoch_kernel(SgdParams p) {
 #include "sgd_rating_body.inc"
@@ -470,36 +469,6 @@ __global__ void __launch_bounds__(256) sgd_ranksgd_epoch_kernel(SgdParams p) {
     block_loss_commit(loss_d, p.loss);
 }
 
-// ---------------------------------------------------------------------------------------------
-// launch plumbing
-// ---------------------------------------------------------------------------------------------
-// Grid: whole multiples of the SM count for big inputs.  For small inputs the number of ratings in
-// flight is capped at nnz/16 (8 warps x ratings-per-step x 2 pipeline stages per block): with the
-// whole matrix in flight at once the epoch degenerates into one full-batch gradient step, which is
-// unstable at SGD learning rates (observed: PMF on ml-100k diverges) -- DESIGN.md "staleness cap".
-template <typename K>
-static int sgd_grid_for(lrk_handle_s* h, K kernel, int64_t n, int rps, int* grid_out, double lr = 0.0, double hot_share = 0.0,
-                        int conc_div = 1) {
-    int per_sm = 0;
-    LRK_CUDA(h, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, 256, 0));
-    if (per_sm < 1) per_sm = 1;
-    int64_t grid = (int64_t)h->sm_count * per_sm;           // whole multiples of the SM count
-    const int64_t need = ((n + 31) / 32 + 7) / 8;           // 8 warps per block, one tile per warp
-    if (need < grid) grid = need;
-    const int64_t stale_cap = (n / 16) / (8 * (int64_t)rps * 2);
-    if (stale_cap < grid) grid = stale_cap;
-    if (lr > 0.0 && hot_share > 0.0) {      // only for launches without per-item degrees (no staleness-aware step)
-        // a warp keeps at most 8 ratings of one item in flight (run-tile chunk; 2 steps of the general path)
-        const double in_flight_max = 1.0 / (lr * hot_share);
-        const int64_t hot_cap = (int64_t)(in_flight_max / (8.0 * (double)(rps > 8 ? rps : 8)));
-        if (hot_cap < grid) grid = hot_cap;
-    }
-    if (conc_div > 1) grid /= conc_div;
-    if (grid < 1) grid = 1;
-    *grid_out = (int)grid;
-    return LRK_OK;
-}
-
 // mean |p_u|^2 over the rank's users -> out[0] (float); out must be zeroed before
 __global__ void user_norm2_kernel(const float* __restrict__ P, int64_t U, int ld, float* __restrict__ out) {
     float acc = 0.f;
@@ -525,6 +494,45 @@ static int refresh_user_norm2(lrk_handle_s* h, bool sync) {
     return LRK_OK;
 }
 
+// ---------------------------------------------------------------------------------------------
+// Launch plan of the stream kernels: every launcher (one GPU, the DSGD sub-epoch loop, the fused DSGD epoch, the sample
+// windows of BPR / AoBPR) takes its parameters, kernel variant, grid and in-flight share from the functions below.
+// ---------------------------------------------------------------------------------------------
+// A/B probes of the plan, read once per process (DESIGN.md §6.1)
+struct SgdProbes {
+    uint32_t hot_flush_deg = 512u;  // LRK_SGD_HOT_FLUSH: degree from which run tiles flush every 16 ratings (0 = always every 8)
+    int track = -1;                 // LRK_SGD_TRACK=0/1: forces the TRACK variant of the damped atomic launches off / on
+    bool trace = false;             // LRK_SGD_TRACE=1: one line per launched segment on stderr (sgd_trace)
+};
+static const SgdProbes& sgd_probes() {
+    static const SgdProbes probes = [] {
+        SgdProbes p;
+        if (const char* e = getenv("LRK_SGD_HOT_FLUSH")) p.hot_flush_deg = atoi(e) > 0 ? (uint32_t)atoi(e) : 0xffffffffu;
+        if (const char* e = getenv("LRK_SGD_TRACK")) p.track = atoi(e) != 0;
+        if (const char* e = getenv("LRK_SGD_TRACE")) p.trace = atoi(e) != 0;
+        return p;
+    }();
+    return probes;
+}
+
+// The handle's whole stream and model; read-only with respect to the handle (lrk_bpr_peek_samples uses it too).  DSGD ranks
+// draw their samples from seeds of their own.
+static SgdParams sgd_params(const lrk_handle_s* h, float lr, float reg_u, float reg_i, double reg_b, int32_t epoch_idx) {
+    SgdParams sp;
+    memset(&sp, 0, sizeof sp);
+    sp.su = h->d_su; sp.si = h->d_si; sp.sr = h->d_sr; sp.n = h->nnz;
+    sp.P = h->P32; sp.Q = h->Q32; sp.bu = h->bu32; sp.bi = h->bi32;
+    sp.mu = (float)h->mu; sp.lr = lr; sp.reg_u = reg_u; sp.reg_i = reg_i; sp.reg_b = (float)reg_b;
+    sp.loss = h->d_loss; sp.ld = h->ld;
+    sp.item_deg = k_lrk_models[h->cfg.model].damped ? h->d_item_deg.ptr : nullptr;
+    sp.hot_flush_deg = sgd_probes().hot_flush_deg;
+    sp.item_cum = h->cfg.model == LRK_MODEL_RANKSGD ? h->d_item_cum.ptr : nullptr;
+    sp.rowptr = h->d_rowptr; sp.col = h->d_col; sp.U = h->U; sp.I = h->I;
+    const uint64_t seed = h->cfg.seed + 977u * (uint64_t)h->rank;
+    sp.seed_lo = (uint32_t)seed; sp.seed_hi = (uint32_t)(seed >> 32); sp.epoch = (uint32_t)epoch_idx;
+    return sp;
+}
+
 // multiplier of the tile walk: close to the golden-ratio fraction of the tile count and coprime with it
 static int64_t sgd_tile_mul(int64_t n) {
     const int64_t T = (n + 31) / 32;
@@ -536,6 +544,54 @@ static int64_t sgd_tile_mul(int64_t n) {
     return a % T ? a % T : 1;
 }
 
+// base narrowed to ratings [off, off + n) of the staged stream, trained against the item rows Q / bi of the item block that
+// starts at item0 (the stream's item ids are block-local): one GPU passes the whole stream, DSGD one stratum, the sample
+// windows of BPR / AoBPR their length (with sample_base set by the caller)
+static SgdParams sgd_segment(const lrk_handle_s* h, const SgdParams& base, int64_t off, int64_t n, float* Q, float* bi, int32_t item0) {
+    SgdParams sp = base;
+    sp.su = base.su + off; sp.si = base.si + off; sp.sr = base.sr + off; sp.n = n;
+    sp.tile_mul = sgd_tile_mul(n);
+    sp.Q = Q; sp.bi = bi;
+    sp.item_deg = base.item_deg ? base.item_deg + item0 : nullptr;
+    sp.pnorm2 = sp.item_deg ? h->d_pnorm2.ptr : nullptr;
+    return sp;
+}
+
+// LRK_SGD_TRACE=1: the plan of one segment (the prefix up to `track` is what tests parse)
+static void sgd_trace(const lrk_handle_s* h, const SgdParams& sp, bool track, int grid, float inflight_frac) {
+    if (!sgd_probes().trace) return;
+    fprintf(stderr, "[sgd] epoch %u n %lld mean|p|^2 %.5f (prev %.5f) track %d conc_div %d grid %d inflight_frac %.9g tile_mul %lld hot_flush_deg %u\n",
+            sp.epoch, (long long)sp.n, h->pnorm2_host, h->pnorm2_prev, (int)track, h->conc_div, grid, inflight_frac, (long long)sp.tile_mul,
+            sp.hot_flush_deg);
+}
+
+// Grid of one launch over the segments seg[0..nseg) -- one, or the strata of a fused DSGD epoch -- for a kernel with rps
+// ratings per warp step: whole multiples of the SM count for big inputs, no more blocks than the tiles need (8 warps per
+// block, one tile per warp), and at most nnz/16 ratings in flight (8 warps x ratings-per-step x 2 pipeline stages per block)
+// for the smallest segment: with the whole matrix in flight at once the epoch degenerates into one full-batch gradient
+// step, which is unstable at SGD learning rates (observed: PMF on ml-100k diverges) -- DESIGN.md "staleness cap".  The
+// rollback safeguard divides the result.  Writes each segment's conc_div and inflight_frac = (ratings in flight) / n.
+static int sgd_grid(lrk_handle_s* h, const void* kernel, int rps, bool track, SgdParams* seg, int nseg, int* grid_out) {
+    int per_sm = 0;
+    LRK_CUDA(h, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, 256, 0));
+    int64_t grid = (int64_t)h->sm_count * std::max(per_sm, 1);
+    for (int t = 0; t < nseg; ++t) {
+        const int64_t n = seg[t].n;
+        if (n <= 0) continue;
+        grid = std::min(grid, ((n + 31) / 32 + 7) / 8);
+        grid = std::min(grid, (n / 16) / (8 * (int64_t)rps * 2));
+    }
+    if (h->conc_div > 1) grid /= h->conc_div;
+    if (grid < 1) grid = 1;
+    for (int t = 0; t < nseg; ++t) {
+        seg[t].conc_div = h->conc_div;
+        seg[t].inflight_frac = (float)((double)grid * 8.0 * (double)std::max(rps, 8) / (double)std::max<int64_t>(seg[t].n, 1));
+        sgd_trace(h, seg[t], track, (int)grid, seg[t].inflight_frac);
+    }
+    *grid_out = (int)grid;
+    return LRK_OK;
+}
+
 // Which epoch kernel variant: TRACK follows mean |p_u|^2 of the rows in flight (curvature of the item-side step) instead of taking the
 // epoch-start value.  It is needed as soon as the user factors are no longer small, and whenever they may grow within the epoch:
 // PMF on un-centred ratings takes mean |p_u|^2 from 1e-4 to ~2 inside the FIRST epoch, so an epoch that starts far below any
@@ -545,47 +601,44 @@ static int64_t sgd_tile_mul(int64_t n) {
 static bool sgd_want_track(const lrk_handle_s* h, int gv) {
     return gv >= 32 || h->epochs_done < 2 || h->pnorm2_host > 0.02f;
 }
+// the variant of a launch: only the damped atomic launches have a TRACK variant; LRK_SGD_TRACK overrides the rule above
+static bool sgd_track(const lrk_handle_s* h, const SgdParams& sp) {
+    if (h->cfg.update_mode != LRK_UPDATE_ATOMIC || !sp.item_deg) return false;
+    return sgd_probes().track >= 0 ? sgd_probes().track != 0 : sgd_want_track(h, h->G * h->V);
+}
+
+// the stream kernel for (model, update mode, variant)
+template <int G, int V>
+static const void* sgd_kernel(const lrk_handle_s* h, const SgdParams& sp, bool track) {
+    const bool atomic = h->cfg.update_mode == LRK_UPDATE_ATOMIC;
+    switch (h->cfg.model) {
+        case LRK_MODEL_BIASEDMF:
+            return track ? (const void*)sgd_rating_epoch_kernel<G, V, true, true, true>
+                         : atomic ? (const void*)sgd_rating_epoch_kernel<G, V, true, true> : (const void*)sgd_rating_epoch_kernel<G, V, true, false>;
+        case LRK_MODEL_PMF:
+            return track ? (const void*)sgd_rating_epoch_kernel<G, V, false, true, true>
+                         : atomic ? (const void*)sgd_rating_epoch_kernel<G, V, false, true> : (const void*)sgd_rating_epoch_kernel<G, V, false, false>;
+        case LRK_MODEL_RANKSGD:
+            return atomic ? (const void*)sgd_ranksgd_epoch_kernel<G, V, true> : (const void*)sgd_ranksgd_epoch_kernel<G, V, false>;
+        default:    // BPR, AoBPR
+            if (sp.ao_rank) return atomic ? (const void*)sgd_bpr_epoch_kernel<G, V, true, true> : (const void*)sgd_bpr_epoch_kernel<G, V, false, true>;
+            return atomic ? (const void*)sgd_bpr_epoch_kernel<G, V, true> : (const void*)sgd_bpr_epoch_kernel<G, V, false>;
+    }
+}
 
 template <int G, int V>
-static int sgd_launch_gv(lrk_handle_s* h, const SgdParams& sp_in) {
-    SgdParams sp = sp_in;
-    static const bool no_damp = getenv("LRK_SGD_NODAMP") && atoi(getenv("LRK_SGD_NODAMP"));    // A/B probe: fall back to the grid cap
-    if (no_damp) sp.item_deg = nullptr;
-    sp.tile_mul = sgd_tile_mul(sp.n);
-    {   // LRK_SGD_HOT_FLUSH: A/B probe of the degree from which run tiles flush every 16 ratings (0 = always every 8)
-        static const char* env = getenv("LRK_SGD_HOT_FLUSH");
-        sp.hot_flush_deg = env ? (atoi(env) > 0 ? (uint32_t)atoi(env) : 0xffffffffu) : 512u;
-    }
-    const bool atomic = h->cfg.update_mode == LRK_UPDATE_ATOMIC;
-    int grid = 1;
-#define LRK_GO(KERN)                                                          \
-    do {                                                                      \
-        int rc__ = sgd_grid_for(h, KERN, sp.n, 32 / G, &grid, (double)sp.lr, sp.item_deg ? 0.0 : sp.hot_share, sp.conc_div); \
-        if (rc__) return rc__;                                                \
-        sp.inflight_frac = (float)((double)grid * 8.0 * (double)(32 / G > 8 ? 32 / G : 8) / (double)(sp.n > 0 ? sp.n : 1)); \
-        KERN<<<grid, 256, 0, h->stream>>>(sp);                                \
-    } while (0)
-    bool track = atomic && sp.item_deg && sgd_want_track(h, G * V);
-    { static const bool trace = getenv("LRK_SGD_TRACE") && atoi(getenv("LRK_SGD_TRACE"));
-      if (trace) fprintf(stderr, "[sgd] epoch %u n %lld mean|p|^2 %.5f (prev %.5f) track %d conc_div %d\n", sp.epoch, (long long)sp.n, h->pnorm2_host, h->pnorm2_prev, (int)track, sp.conc_div); }
-    { static const char* env = getenv("LRK_SGD_TRACK"); if (env && atomic && sp.item_deg) track = atoi(env) != 0; }    // A/B probe
-    if (h->cfg.model == LRK_MODEL_BIASEDMF) {
-        if (track) LRK_GO((sgd_rating_epoch_kernel<G, V, true, true, true>));
-        else if (atomic) LRK_GO((sgd_rating_epoch_kernel<G, V, true, true>)); else LRK_GO((sgd_rating_epoch_kernel<G, V, true, false>));
-    } else if (h->cfg.model == LRK_MODEL_PMF) {
-        if (track) LRK_GO((sgd_rating_epoch_kernel<G, V, false, true, true>));
-        else if (atomic) LRK_GO((sgd_rating_epoch_kernel<G, V, false, true>)); else LRK_GO((sgd_rating_epoch_kernel<G, V, false, false>));
-    } else if (h->cfg.model == LRK_MODEL_RANKSGD) {
-        if (atomic) LRK_GO((sgd_ranksgd_epoch_kernel<G, V, true>)); else LRK_GO((sgd_ranksgd_epoch_kernel<G, V, false>));
-    } else {
-        if (sp.ao_rank) { if (atomic) LRK_GO((sgd_bpr_epoch_kernel<G, V, true, true>)); else LRK_GO((sgd_bpr_epoch_kernel<G, V, false, true>)); }
-        else if (atomic) LRK_GO((sgd_bpr_epoch_kernel<G, V, true>)); else LRK_GO((sgd_bpr_epoch_kernel<G, V, false>));
-    }
-#undef LRK_GO
-    LRK_LAUNCH_CHECK(h);
+static int sgd_launch_gv(lrk_handle_s* h, const SgdParams& seg) {
+    SgdParams sp = seg;
+    const bool track = sgd_track(h, sp);
+    const void* kernel = sgd_kernel<G, V>(h, sp, track);
+    int grid = 1, rc;
+    if ((rc = sgd_grid(h, kernel, 32 / G, track, &sp, 1, &grid))) return rc;
+    void* args[] = {(void*)&sp};
+    LRK_CUDA(h, cudaLaunchKernel(kernel, dim3((unsigned)grid), dim3(256), args, 0, h->stream));
+    h->launches++;
     return LRK_OK;
 }
 
-static int sgd_launch(lrk_handle_s* h, const SgdParams& sp) {
-    return lrk_with_layout(h, [&](auto G, auto V) { return sgd_launch_gv<decltype(G)::value, decltype(V)::value>(h, sp); });
+static int sgd_launch(lrk_handle_s* h, const SgdParams& seg) {
+    return lrk_with_layout(h, [&](auto G, auto V) { return sgd_launch_gv<decltype(G)::value, decltype(V)::value>(h, seg); });
 }

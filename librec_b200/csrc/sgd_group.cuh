@@ -325,9 +325,19 @@ __global__ void __launch_bounds__(256, 2) sgd_group_epoch_kernel(SgdGroupParams 
 template <int G, int V>
 static size_t sgd_group_smem_bytes() { return sizeof(float) * (size_t)(8 * (32 / G)) * sgd_group_smem_floats_per_worker<G, V>(); }
 
-// resident workers of the group kernel for a layout (sets the unit size at staging and the in-flight estimate at launch)
+static bool sgd_group_layout_supported(const lrk_handle_s* h) { return h->V == 1 && (h->G == 8 || h->G == 16 || h->G == 32); }
+// f(G, V) for the layouts the user-group kernels are built for (sgd_group_layout_supported)
+template <class F>
+static int sgd_with_group_layout(lrk_handle_s* h, F&& f) {
+    return lrk_with_layout(h, [&](auto G, auto V) -> int {
+        if constexpr (decltype(G)::value >= 8 && decltype(V)::value == 1) return f(G, V);
+        else return lrk_fail(h, LRK_ERR_INVALID, "sgd_with_group_layout", "unsupported factor layout", __FILE__, __LINE__);
+    });
+}
+
+// CTAs of the group kernel resident at once (sets the unit size at staging and bounds the grid at launch)
 template <int G, int V>
-static int sgd_group_resident_workers_gv(lrk_handle_s* h, int* ctas_out) {
+static int sgd_group_ctas(lrk_handle_s* h) {
     const size_t smem = sgd_group_smem_bytes<G, V>();
     cudaFuncSetAttribute(sgd_group_epoch_kernel<G, V, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     cudaFuncSetAttribute(sgd_group_epoch_kernel<G, V, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
@@ -336,54 +346,63 @@ static int sgd_group_resident_workers_gv(lrk_handle_s* h, int* ctas_out) {
         cudaGetLastError();
         per_sm = 1;
     }
-    if (ctas_out) *ctas_out = per_sm * h->sm_count;
-    return per_sm * h->sm_count * 8 * (32 / G);
+    return per_sm * h->sm_count;
 }
-static bool sgd_group_layout_supported(const lrk_handle_s* h) { return h->V == 1 && (h->G == 8 || h->G == 16 || h->G == 32); }
-// Selected with LRK_SGD_GROUP=1 (read at every lrk_set_train_csr).  r02 measurement on one B200 (ML-20M shape, BiasedMF k=64): this
+static int sgd_group_resident_workers(lrk_handle_s* h) {
+    return sgd_with_group_layout(h, [&](auto G, auto V) { return sgd_group_ctas<decltype(G)::value, decltype(V)::value>(h) * 8 * (32 / decltype(G)::value); });
+}
+// Selected with LRK_SGD_GROUP=1 (read at lrk_create).  r02 measurement on one B200 (ML-20M shape, BiasedMF k=64): this
 // kernel is bit-for-bit the closer one to the reference (held-out RMSE within 1.3e-5 of the sequential oracle, first-epoch loss of
 // config C4 92.9 M vs the oracle's 94.6 M against 134 M for the item-run-tile kernel), but it is INSTRUCTION bound, not L2 bound:
 // 140 warp-instructions per rating (ncu, profiles/r02_group_kernel_ncu_summary.md) against 53 for the item-run-tile kernel -- the
 // sequential chain needs per-rating control flow (pair heads, look-ahead, ring slots) and the two workers of a warp diverge on it --
 // 4.0-4.8 ms per epoch against 1.5 ms.  So the item-run-tile kernel stays the default and this one is the order-faithful option.
-static bool lrk_use_group_kernel(const lrk_handle_s* h) {
-    const char* env = getenv("LRK_SGD_GROUP");
-    if (!env || atoi(env) == 0) return false;
-    return k_lrk_models[h->cfg.model].rating && h->cfg.update_mode == LRK_UPDATE_ATOMIC && sgd_group_layout_supported(h);
+static bool lrk_use_group_kernel(const lrk_handle_s* h) { return h->sgd_group && sgd_group_layout_supported(h); }
+
+// The group kernel's parameters for item block b (0 on one GPU): those of the block's stream segment (sgd_segment), with the
+// block's units in place of its ratings (unit starts index the whole stream).  A block without ratings gets no units.
+static SgdGroupParams sgd_group_params(const lrk_handle_s* h, const SgdParams& seg, int b) {
+    const GroupUnits* gu = h->group.get();
+    SgdGroupParams gp;
+    memset(&gp, 0, sizeof gp);
+    gp.su = h->d_su; gp.si = h->d_si; gp.sr = h->d_sr;
+    gp.units = gu->d_units + gu->unit_base[(size_t)b];
+    gp.n_units = seg.n > 0 ? (int32_t)(gu->unit_base[(size_t)b + 1] - gu->unit_base[(size_t)b]) : 0;
+    gp.counter = gu->d_counter + b;
+    gp.P = seg.P; gp.Q = seg.Q; gp.bu = seg.bu; gp.bi = seg.bi;
+    gp.mu = seg.mu; gp.lr = seg.lr; gp.reg_u = seg.reg_u; gp.reg_i = seg.reg_i; gp.reg_b = seg.reg_b;
+    gp.loss = seg.loss; gp.ld = seg.ld; gp.item_deg = seg.item_deg;
+    return gp;
 }
 
-static int sgd_group_resident_workers(lrk_handle_s* h, int* ctas_out) {
-    switch (h->G) {
-        case 8: return sgd_group_resident_workers_gv<8, 1>(h, ctas_out);
-        case 16: return sgd_group_resident_workers_gv<16, 1>(h, ctas_out);
-        default: return sgd_group_resident_workers_gv<32, 1>(h, ctas_out);
+// Grid of one group-kernel launch over the blocks gseg[0..nseg) (one, or the strata of a fused DSGD epoch; seg: their stream
+// segments): at most `ctas`, no more CTAs than the block with the most units can keep busy, divided by the rollback safeguard.
+// Per block the workers in flight are min(grid * WPC, units) and inflight_frac = those workers / the block's ratings.
+static int sgd_group_grid(lrk_handle_s* h, int64_t ctas, int wpc, const SgdParams* seg, SgdGroupParams* gseg, int nseg) {
+    int64_t most = 1;
+    for (int t = 0; t < nseg; ++t) most = std::max<int64_t>(most, (gseg[t].n_units + wpc - 1) / wpc);
+    int64_t grid = std::min(ctas, most);
+    if (h->conc_div > 1) grid /= h->conc_div;
+    if (grid < 1) grid = 1;
+    for (int t = 0; t < nseg; ++t) {
+        const double workers = (double)std::min<int64_t>(grid * wpc, gseg[t].n_units);
+        gseg[t].inflight_frac = (float)(workers / (double)std::max<int64_t>(seg[t].n, 1));
+        sgd_trace(h, seg[t], false, (int)grid, gseg[t].inflight_frac);
     }
+    return (int)grid;
 }
 
 template <int G, int V>
-static int sgd_group_launch_gv(lrk_handle_s* h, SgdGroupParams& gp, int64_t n_ratings, int conc_div) {
-    int ctas = 0;
-    const int workers_full = sgd_group_resident_workers_gv<G, V>(h, &ctas);
-    (void)workers_full;
-    constexpr int WPC = 8 * (32 / G);
-    int64_t grid = ctas;
-    const int64_t need = (gp.n_units + WPC - 1) / WPC;
-    if (need < grid) grid = need;
-    if (conc_div > 1) grid /= conc_div;                      // rollback safeguard: fewer units in flight
-    if (grid < 1) grid = 1;
-    const double workers = (double)std::min<int64_t>(grid * WPC, gp.n_units);
-    gp.inflight_frac = (float)(workers / (double)(n_ratings > 0 ? n_ratings : 1));
+static int sgd_group_launch_gv(lrk_handle_s* h, const SgdParams& seg, int b) {
+    SgdGroupParams gp = sgd_group_params(h, seg, b);
+    const int grid = sgd_group_grid(h, sgd_group_ctas<G, V>(h), 8 * (32 / G), &seg, &gp, 1);
     const size_t smem = sgd_group_smem_bytes<G, V>();
     if (h->cfg.model == LRK_MODEL_BIASEDMF) sgd_group_epoch_kernel<G, V, true><<<(unsigned)grid, 256, smem, h->stream>>>(gp);
     else sgd_group_epoch_kernel<G, V, false><<<(unsigned)grid, 256, smem, h->stream>>>(gp);
     LRK_LAUNCH_CHECK(h);
     return LRK_OK;
 }
-static int sgd_group_launch(lrk_handle_s* h, SgdGroupParams& gp, int64_t n_ratings, int conc_div) {
-    switch (h->G) {
-        case 8: return sgd_group_launch_gv<8, 1>(h, gp, n_ratings, conc_div);
-        case 16: return sgd_group_launch_gv<16, 1>(h, gp, n_ratings, conc_div);
-        case 32: return sgd_group_launch_gv<32, 1>(h, gp, n_ratings, conc_div);
-        default: return lrk_fail(h, LRK_ERR_INVALID, "sgd_group_launch", "unsupported factor layout", __FILE__, __LINE__);
-    }
+// the epoch (one GPU) or one sub-epoch (DSGD) of item block b over the stream segment seg of that block
+static int sgd_group_launch(lrk_handle_s* h, const SgdParams& seg, int b) {
+    return sgd_with_group_layout(h, [&](auto G, auto V) { return sgd_group_launch_gv<decltype(G)::value, decltype(V)::value>(h, seg, b); });
 }

@@ -71,7 +71,7 @@ __global__ void f32_to_f64_rows_kernel(const float* __restrict__ src, double* __
 // of ONE item (items with >= LRK_RUN_MIN_DEGREE ratings in the block's shard give floor(deg/32) of
 // them, the CSR-order remainder joins the shuffled part); tiles are shuffled among themselves.  The
 // kernel flushes the item-side delta of a run every 8 ratings (16 / 32 for hot items, sgd.cuh), so a flush of
-// a 128-rating item is a mini-batch of 1/16 of its ratings -- the share the staleness cap of sgd_grid_for
+// a 128-rating item is a mini-batch of 1/16 of its ratings -- the share the staleness cap of sgd_grid
 // allows in flight -- and its step is damped by the staleness-aware factor.  (Before that factor existed,
 // runs from 64 ratings up made PMF at lr 0.01 diverge on ml-100k and the threshold was 512; 512 -> 128 moves
 // half of the remaining ratings into run tiles: C2 epoch 1.65 -> 1.50 ms.)  The
@@ -87,7 +87,7 @@ __global__ void item_degree_kernel(const int32_t* __restrict__ col, int64_t nnz,
     const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (t < nnz) atomicAdd(deg + col[t], 1u);
 }
-// runs per item; max_deg[b] = largest item degree of block b (stability cap of the SGD grid, sgd.cuh)
+// runs per item; max_deg[b] = largest item degree of block b (lrk_stage_stats)
 __global__ void item_runs_kernel(const uint32_t* __restrict__ deg, int32_t I, uint32_t* __restrict__ runs,
                                  const int32_t* __restrict__ bounds, int world, uint32_t* __restrict__ max_deg) {
     const int32_t i = blockIdx.x * blockDim.x + threadIdx.x;
@@ -238,7 +238,7 @@ static int stage_coo_from_csr(lrk_handle_s* h, const int64_t* d_rowptr, const in
         if ((rc = stage_group_stream(h, d_rowptr, d_col, row_of, d_val, U, I, nnz, nullptr, 1, group_workers, h->cfg.seed, sc, w.tmp, tmp_bytes,
                                      keys, keys2, idx, perm, su, si, sr, group_out))) return rc;
         LRK_CUDA(h, cudaStreamSynchronize(st));
-        h->hot_share = 0.0; h->run_tiles = 0; h->max_item_deg = 0;
+        h->run_tiles = 0; h->max_item_deg = 0;
     } else if (!flags) {
         if ((rc = stage_tile_keys(h, d_col, I, nnz, nullptr, 1, h->cfg.seed, w, keys, idx))) return rc;
         size_t tb = tmp_bytes;
@@ -253,7 +253,6 @@ static int stage_coo_from_csr(lrk_handle_s* h, const int64_t* d_rowptr, const in
         LRK_CUDA(h, cudaMemcpyAsync(h->d_item_deg, w.deg, sizeof(uint32_t) * (size_t)I, cudaMemcpyDeviceToDevice, st));
         LRK_CUDA(h, cudaMemcpyAsync(&max_deg, w.max_deg, sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
         LRK_CUDA(h, cudaStreamSynchronize(st));
-        h->hot_share = (double)max_deg / (double)nnz;
         h->run_tiles = (int64_t)last_base + (int64_t)last_runs;
         h->max_item_deg = max_deg;
     }

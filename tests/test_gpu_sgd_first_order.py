@@ -30,7 +30,7 @@ EPS32 = float(np.finfo(np.float32).eps)
 KAPPA = 2.0              # a row's path length under the real dynamics exceeds its first-order path length by a second-order share (<< 1)
 K_LAYOUTS = (3, 8, 16, 20, 64, 128, 200)       # G = 1, 2, 4, 8, 16, 32 and 32 x 2 (layout_for_k, lrk_api.cu)
 RUN_DEGREES = (224, 704, 2048)                 # run-tile items: 8-rating, 16-rating and whole-tile flush periods
-RUN_MIN_DEGREE, HOT_FLUSH_DEG = 128, 512       # staging.cuh, sgd_launch_gv
+RUN_MIN_DEGREE, HOT_FLUSH_DEG = 128, 512       # staging.cuh, sgd_probes
 
 
 def f32(a):
@@ -354,8 +354,8 @@ def run_flush_steps(G, deg, lr, pn2=1.0):
 
 
 def inflight_frac_range(G, n):
-    """inflight_frac of sgd_launch_gv: grid * 8 * max(rps, 8) / n for a grid of at least 1 and at most the staleness cap of
-    sgd_grid_for (the cap binds below ~37 k * rps ratings; it is <= 1/4 whenever it is >= 1)"""
+    """inflight_frac of sgd_grid: grid * 8 * max(rps, 8) / n for a grid of at least 1 and at most the staleness cap of
+    sgd_grid (the cap binds below ~37 k * rps ratings; it is <= 1/4 whenever it is >= 1)"""
     rps = 32 // G
     grid_hi = max(1, (n // 16) // (8 * rps * 2))
     f = lambda grid: grid * 8.0 * max(rps, 8) / n
@@ -573,7 +573,7 @@ def test_rating_epoch_is_first_order(O, capi, model, k, variant):
 def test_run_tile_item_step_is_damped_by_the_staleness_factor(O, capi, k, variant):
     """PMF at a learning rate where the damping of run tiles is visible: the item delta of every item is ONE scalar c_i times
     its first-order delta, c_i = (1 - e^-x) / x with x inside the range sgd_rating_body.inc:52-66 allows (inflight_frac
-    between its value for a one-block grid and the staleness cap of sgd_grid_for), c_i clearly below 1 for run-tile items
+    between its value for a one-block grid and the staleness cap of sgd_grid), c_i clearly below 1 for run-tile items
     and 1 for items below the run threshold.  |p_u|^2 ~ 1e-4 keeps the item rows first order although lr * degree is up to
     6 (the damping uses max(1, |p|^2) = 1); reg_i = 0, whose contraction lr * degree * reg_i would otherwise act like a
     second damping.  The user rows are checked by the first-order test above."""
