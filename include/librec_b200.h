@@ -74,7 +74,7 @@ typedef enum {
      * reference's Gauss-Jordan inverse (math/structure/DenseMatrix.java:362-437).  lrk_set_train_csr takes the WEIGHTED values
      * (weightMatrix() stays in the shim's setup()); lrk_sgd_epoch = one iteration (lr and reg_b ignored, loss 0 -- the class
      * never assigns it); fp64 in the reference's operation order: factors BIT-identical to the reference's; rec.factor.number <= 112;
-     * single GPU; scoring as for PMF */
+     * several GPUs through lrk_create_multi (bit-identical to one GPU), not as a DSGD rank (lrk_comm_init); scoring as for PMF */
     LRK_MODEL_WRMF = 7,
     /* eals -> recommender/cf/ranking/EALSRecommender.java:114-214 (SURVEY.md 8f row N3): element-wise ALS.  Weighted values as
      * for WRMF; the item confidences (:65-83, computed in the shim's setup()) through lrk_set_matrix("eals.confidences");
@@ -114,7 +114,11 @@ LRK_API int lrk_create(const lrk_config_t* cfg, lrk_handle_t* out);
  * job/RecommenderJob.java:121-143 runs, that trains on all listed GPUs.  It takes and returns the FULL matrices exactly like a
  * single-device handle; inside, users are cut into contiguous blocks, one per device, each device runs a DSGD rank on its own host
  * thread (NCCL communicator created inside this process; item blocks rotate over NVLink), and lrk_topn shards the queried users over
- * the devices with the full item matrix on each (no collective).  cfg->device is ignored.  Supported on a multi handle:
+ * the devices with the full item matrix on each (no collective).  BiasedMF, PMF, BPR and WRMF; the other models take one device.
+ * WRMF needs no communicator: every device stages the full train matrix and holds full copies of both factor matrices, solves its
+ * own range of users and of items (contiguous ranges of about equal solve cost), and the devices exchange the new rows after each
+ * half-iteration (peer copies); the factors are bit-identical to a single device's, and lrk_last_epoch_ms is the wall time of the
+ * whole iteration.  With one device a multi handle is a plain handle.  cfg->device is ignored.  Supported on a multi handle:
  * lrk_set_train_csr, lrk_set_factors, lrk_sgd_epoch(s), lrk_get_factors, lrk_topn, lrk_topn_stats, lrk_stage_stats, lrk_last_epoch_ms,
  * lrk_sgd_safeguard_state, lrk_launch_count, lrk_synchronize, lrk_probe_l2, lrk_last_error, lrk_destroy; the remaining entry points
  * return LRK_ERR_INVALID (gather the factors with lrk_get_factors and use a single-device handle for them). */
@@ -135,7 +139,8 @@ LRK_API int lrk_host_free(void* p);
  * (recommender/MatrixRecommender.java:90) -- the per-row int[]/double[] pieces
  * (math/structure/RowSequentialAccessSparseMatrix.java:19, OrderedIntDoubleMapping) flattened to
  * rowptr[U+1], col[nnz] (ascending inside a row), val[nnz].  Builds the device CSR and a
- * device-shuffled COO stream for the SGD epoch.  nnz < 2^31 per handle (under DSGD / a multi handle: per rank). */
+ * device-shuffled COO stream for the SGD epoch.  nnz < 2^31 per handle (under DSGD / a multi handle: per rank; a WRMF multi handle
+ * stages the whole matrix on every device, so there the limit is on the full matrix). */
 LRK_API int lrk_set_train_csr(lrk_handle_t h, int32_t num_users, int32_t num_items,
                       const int64_t* rowptr, const int32_t* col, const double* val);
 /* replaces: DenseMatrix userFactors/itemFactors (double[][], math/structure/DenseMatrix.java:20),

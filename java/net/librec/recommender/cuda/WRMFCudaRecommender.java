@@ -1,6 +1,8 @@
 // NOT COMPILED HERE.  rec.recommender.class=net.librec.recommender.cuda.WRMFCudaRecommender
 // Replaces the trainModel() of recommender/cf/ranking/WRMFRecommender.java:74-166 (alternating least squares, one Gauss-Jordan
-// inverse per user and per item and iteration); single GPU, rec.factor.number <= 112.  setup() keeps the reference's
+// inverse per user and per item and iteration); rec.factor.number <= 112.  rec.cuda.devices=0,1,... trains on several GPUs of one
+// box through one multi-device handle (each device solves a range of users and of items, the new rows are exchanged between the
+// devices after each half-iteration), with the same bit-identical factors as one GPU.  setup() keeps the reference's
 // weightMatrix() (:63-72) in Java -- Math.log / Math.pow are evaluated by the JVM exactly as before -- and the native side receives
 // the weighted values.  The native iteration performs the reference's floating-point operations in the reference's order in fp64,
 // so userFactors / itemFactors come back bit-identical to what WRMFRecommender would have computed; recommendRank is the native

@@ -8,8 +8,8 @@
 // on the fp64 masters and perform every floating-point operation of the reference in the reference's order (explicit
 // __dmul_rn / __dadd_rn / __dsub_rn, never an FMA; IEEE double division), so the factors are BIT-identical to the oracle's
 // (tests/test_gpu_als.py).  Parallelism comes from what the reference leaves independent:
-//   * Gram matrices (Y^T Y, X^T X, Sq): k^2 independent accumulation chains over the rows, one thread per entry, rows staged
-//     through shared memory;
+//   * Gram matrices (Y^T Y, X^T X, Sq): k^2 independent accumulation chains over the rows, one thread per entry, an 8 x 8 tile of
+//     entries per CTA, the tile's columns of the rows staged through shared memory;
 //   * WRMF: one CTA per row.  Thread (tr, tc) of a 16 x 16 grid keeps a TILE x TILE block of A in registers while the row's entries
 //     stream through shared memory in order (each entry of A has its own chain), then the CTA runs the reference's Gauss-Jordan
 //     on [A | I] in shared memory (k pivot steps, every step parallel over rows x columns) and the final W . b;
@@ -53,28 +53,55 @@ __global__ void als_iota_kernel(int32_t* __restrict__ out, int64_t n) {
 
 // out[r][c] = sum_i M[i][c] * M[i][r] (w == nullptr; DenseMatrix.times over the transpose) or, with weights, the eALS cache
 // sum_i (w[i] * M[i][max(r,c)]) * M[i][min(r,c)] (EALSRecommender.java:128-137 computes the lower triangle and mirrors it).
-// One thread per entry, rows i in order; `stage` (<= 32) rows per shared-memory stage.
-__global__ void __launch_bounds__(256) als_gram_kernel(const double* __restrict__ M, int64_t n, int k, int stage, const double* __restrict__ w, double* __restrict__ out) {
-    extern __shared__ double gs[];
-    double* rows = gs;                 // stage x k
-    double* ws = gs + stage * k;       // stage
-    const int id = blockIdx.x * 256 + threadIdx.x;
-    const bool live = id < k * k;
-    const int r = live ? id / k : 0, c = live ? id % k : 0;
-    const int a = w ? (r > c ? r : c) : c, b = w ? (r > c ? c : r) : r;
+// One thread per entry, rows i in order: every entry is one chain of n dependent adds, so the kernel's time is that chain as long
+// as the rows arrive fast enough.  A CTA owns an 8 x 8 tile of `out` and stages only the 16 columns the tile reads (columns
+// r0.. and c0..), so the ceil(k/8)^2 tiles spread over the SMs and no SM has to stream whole rows; the next stage's rows travel
+// in registers while the current one is consumed.
+#define ALS_GRAM_TILE 8
+#define ALS_GRAM_STAGE 128
+__global__ void __launch_bounds__(ALS_GRAM_TILE * ALS_GRAM_TILE) als_gram_kernel(const double* __restrict__ M, int64_t n, int k, const double* __restrict__ w, double* __restrict__ out) {
+    constexpr int T = ALS_GRAM_TILE, S = ALS_GRAM_STAGE, NT = T * T, W = 2 * T, NPT = S * W / NT, NPW = S / NT;
+    __shared__ double rs[S * W];       // stage rows x {columns r0 .. r0+T-1, columns c0 .. c0+T-1}
+    __shared__ double ws[S];
+    const int tiles = (k + T - 1) / T;
+    const int r0 = (blockIdx.x / tiles) * T, c0 = (blockIdx.x % tiles) * T;
+    const int tid = threadIdx.x, tr = tid / T, tc = tid % T;
+    const int r = r0 + tr, c = c0 + tc;
+    const bool live = r < k && c < k;
+    // slots of M[i][a] and M[i][b] in a staged row: a = c, b = r without weights; a = max(r, c), b = min(r, c) with them
+    const int sa = (w && r > c) ? tr : T + tc, sb = (w && r > c) ? T + tc : tr;
+    double pre[NPT], prew[NPW];
+    auto fetch = [&](int64_t base) {
+#pragma unroll
+        for (int j = 0; j < NPT; ++j) {
+            const int t = tid + NT * j, e = t / W, f = t % W, col = f < T ? r0 + f : c0 + f - T;
+            pre[j] = (base + e < n && col < k) ? M[(base + e) * k + col] : 0.0;
+        }
+#pragma unroll
+        for (int j = 0; j < NPW; ++j) { const int e = tid + NT * j; prew[j] = (w && base + e < n) ? w[base + e] : 0.0; }
+    };
     double v = 0.0;
-    for (int64_t base = 0; base < n; base += stage) {
-        const int cnt = (int)((n - base) < stage ? (n - base) : stage);
+    if (n > 0) fetch(0);
+    for (int64_t base = 0; base < n; base += S) {
+        const int cnt = (int)((n - base) < S ? (n - base) : S);
         __syncthreads();
-        for (int t = threadIdx.x; t < cnt * k; t += 256) rows[t] = M[base * k + t];
-        if (w && threadIdx.x < cnt) ws[threadIdx.x] = w[base + threadIdx.x];
+#pragma unroll
+        for (int j = 0; j < NPT; ++j) rs[tid + NT * j] = pre[j];
+#pragma unroll
+        for (int j = 0; j < NPW; ++j) ws[tid + NT * j] = prew[j];
         __syncthreads();
+        if (base + S < n) fetch(base + S);
         if (live) {
-            if (w) for (int j = 0; j < cnt; ++j) v = __dadd_rn(v, __dmul_rn(__dmul_rn(ws[j], rows[j * k + a]), rows[j * k + b]));
-            else for (int j = 0; j < cnt; ++j) v = __dadd_rn(v, __dmul_rn(rows[j * k + a], rows[j * k + b]));
+            if (w) {
+#pragma unroll 8
+                for (int j = 0; j < cnt; ++j) v = __dadd_rn(v, __dmul_rn(__dmul_rn(ws[j], rs[j * W + sa]), rs[j * W + sb]));
+            } else {
+#pragma unroll 8
+                for (int j = 0; j < cnt; ++j) v = __dadd_rn(v, __dmul_rn(rs[j * W + sa], rs[j * W + sb]));
+            }
         }
     }
-    if (live) out[id] = v;
+    if (live) out[r * k + c] = v;
 }
 
 struct AlsSolveParams {
@@ -85,6 +112,7 @@ struct AlsSolveParams {
     const double* G;          // F^T F
     double* OUT;              // this side's factors
     double reg;
+    int32_t row0;             // the rows [row0, row0 + n_rows) are solved (a device's range on a multi-device handle)
     int32_t n_rows;
     int k;
 };
@@ -105,7 +133,7 @@ __global__ void __launch_bounds__(256) als_wrmf_solve_kernel(AlsSolveParams p) {
     double* colp = bs + k;                         // k
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const int tr = tid >> 4, tc = tid & 15;
-    for (int32_t row = blockIdx.x; row < p.n_rows; row += gridDim.x) {
+    for (int32_t row = p.row0 + blockIdx.x; row < p.row0 + p.n_rows; row += gridDim.x) {
         const int64_t b0 = p.ptr[row], e0 = p.ptr[row + 1];
         double acc[TILE][TILE];
 #pragma unroll
@@ -444,10 +472,8 @@ static int als_stage(lrk_handle_s* h, const double* h_val) {
 }
 
 static int als_gram(lrk_handle_s* h, const double* M, int64_t n, const double* w, double* out) {
-    const int k = h->k;
-    const int stage = k <= 128 ? 32 : 16;                 // 33 KB of shared memory at most
-    const size_t smem = sizeof(double) * ((size_t)stage * k + stage);
-    als_gram_kernel<<<lrk_ceil_div((int64_t)k * k, 256), 256, smem, h->stream>>>(M, n, k, stage, w, out);
+    const int tiles = lrk_ceil_div(h->k, ALS_GRAM_TILE);
+    als_gram_kernel<<<tiles * tiles, ALS_GRAM_TILE * ALS_GRAM_TILE, 0, h->stream>>>(M, n, h->k, w, out);
     LRK_LAUNCH_CHECK(h);
     h->launches++;
     return LRK_OK;
@@ -506,6 +532,30 @@ static int als_eals_side(lrk_handle_s* h, const AlsEalsParams& p) {
     return LRK_OK;
 }
 
+// the Gram matrix a WRMF half-iteration reads: Q^T Q before the user side, P^T P before the item side
+static int als_wrmf_gram(lrk_handle_s* h, bool item_side) {
+    return item_side ? als_gram(h, h->P64, h->U, nullptr, h->als->d_gram) : als_gram(h, h->Q64, h->I, nullptr, h->als->d_gram);
+}
+
+// the user side (rows of the CSR, solved against Q) or the item side (rows of the CSC, solved against P), rows [row0, row0 + n_rows)
+static AlsSolveParams als_wrmf_params(lrk_handle_s* h, bool item_side, float reg, int32_t row0, int32_t n_rows) {
+    AlsState* a = h->als.get();
+    AlsSolveParams p;
+    memset(&p, 0, sizeof p);
+    p.k = h->k; p.G = a->d_gram; p.reg = (double)reg; p.row0 = row0; p.n_rows = n_rows;
+    if (item_side) { p.ptr = a->d_colptr; p.idx = a->d_cusers; p.w = a->d_cval; p.F = h->P64; p.OUT = h->Q64; }
+    else { p.ptr = h->d_rowptr; p.idx = h->d_col; p.w = a->d_val; p.F = h->Q64; p.OUT = h->P64; }
+    return p;
+}
+
+// keep the fp32 working copies in step (nothing on the ALS path reads them, the scoring entry points use the masters)
+static int als_refresh_f32(lrk_handle_s* h) {
+    cudaStream_t st = h->stream;
+    f64_to_f32_rows_kernel<<<lrk_ceil_div((int64_t)h->U * h->ld, 256), 256, 0, st>>>(h->P64, h->P32, h->U, h->k, h->ld); LRK_LAUNCH_CHECK(h);
+    f64_to_f32_rows_kernel<<<lrk_ceil_div((int64_t)h->I * h->ld, 256), 256, 0, st>>>(h->Q64, h->Q32, h->I, h->k, h->ld); LRK_LAUNCH_CHECK(h);
+    return LRK_OK;
+}
+
 // one iteration of WRMFRecommender.trainModel / EALSRecommender.trainModel on the fp64 masters; the models have no loss (0 is returned)
 static int als_epoch(lrk_handle_s* h, float reg_u, float reg_i, double* loss_out) {
     AlsState* a = h->als.get();
@@ -515,19 +565,11 @@ static int als_epoch(lrk_handle_s* h, float reg_u, float reg_i, double* loss_out
     LRK_REQUIRE(h, h->f64_valid, "internal: fp64 masters out of date");
     LrkEpoch e;
     e.enqueue = [&](int) -> int {
-        cudaStream_t st = h->stream;
         const int k = h->k;
         int rc;
         if (!eals) {
-            AlsSolveParams p;
-            memset(&p, 0, sizeof p);
-            p.k = k; p.G = a->d_gram;
-            if ((rc = als_gram(h, h->Q64, h->I, nullptr, a->d_gram))) return rc;
-            p.ptr = h->d_rowptr; p.idx = h->d_col; p.w = a->d_val; p.F = h->Q64; p.OUT = h->P64; p.reg = (double)reg_u; p.n_rows = h->U;
-            if ((rc = als_wrmf_side(h, p))) return rc;
-            if ((rc = als_gram(h, h->P64, h->U, nullptr, a->d_gram))) return rc;
-            p.ptr = a->d_colptr; p.idx = a->d_cusers; p.w = a->d_cval; p.F = h->P64; p.OUT = h->Q64; p.reg = (double)reg_i; p.n_rows = h->I;
-            if ((rc = als_wrmf_side(h, p))) return rc;
+            if ((rc = als_wrmf_gram(h, false)) || (rc = als_wrmf_side(h, als_wrmf_params(h, false, reg_u, 0, h->U)))) return rc;
+            if ((rc = als_wrmf_gram(h, true)) || (rc = als_wrmf_side(h, als_wrmf_params(h, true, reg_i, 0, h->I)))) return rc;
         } else {
             AlsEalsParams p;
             memset(&p, 0, sizeof p);
@@ -543,10 +585,7 @@ static int als_epoch(lrk_handle_s* h, float reg_u, float reg_i, double* loss_out
             p.ptr = a->d_colptr; p.idx = a->d_cusers; p.w = a->d_cval; p.Fself = h->Q64; p.Fother = h->P64; p.reg = (double)reg_i; p.n_rows = h->I;
             if ((rc = als_eals_side<true>(h, p))) return rc;
         }
-        // keep the fp32 working copies in step (nothing on this path reads them, the scoring entry points use the masters)
-        f64_to_f32_rows_kernel<<<lrk_ceil_div((int64_t)h->U * h->ld, 256), 256, 0, st>>>(h->P64, h->P32, h->U, k, h->ld); LRK_LAUNCH_CHECK(h);
-        f64_to_f32_rows_kernel<<<lrk_ceil_div((int64_t)h->I * h->ld, 256), 256, 0, st>>>(h->Q64, h->Q32, h->I, k, h->ld); LRK_LAUNCH_CHECK(h);
-        return LRK_OK;
+        return als_refresh_f32(h);
     };
     return lrk_epoch(h, e, loss_out);             // loss 0: trainModel never assigns `loss` in either class
 }

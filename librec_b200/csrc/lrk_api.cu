@@ -604,6 +604,12 @@ int lrk_sgd_epochs(lrk_handle_t h, int32_t n_epochs, float lr, float decay, floa
 
 int lrk_stage_stats(lrk_handle_t h, int64_t out[4]) {
     LRK_REQUIRE(h, h != nullptr && out != nullptr, "NULL argument");
+    if (h->multi && ((MultiState*)h->multi)->als) {            // every child stages the whole matrix: count it once
+        lrk_handle_s* c = ((MultiState*)h->multi)->child[0];
+        const int rc = lrk_stage_stats(c, out);
+        if (rc) h->err = c->err;
+        return rc;
+    }
     if (h->multi) {
         int64_t acc[4] = {0, 0, 0, 0};
         for (lrk_handle_s* c : ((MultiState*)h->multi)->child) {
@@ -649,7 +655,11 @@ int lrk_sgd_safeguard_state(lrk_handle_t h, int32_t* conc_div, int64_t* rollback
 }
 int lrk_last_epoch_ms(lrk_handle_t h, float* ms_out) {
     LRK_REQUIRE(h, h != nullptr && ms_out != nullptr, "NULL argument");
-    if (h->multi) { *ms_out = 0.f; for (lrk_handle_s* c : ((MultiState*)h->multi)->child) *ms_out = std::max(*ms_out, c->last_epoch_ms); return LRK_OK; }
+    if (h->multi && !((MultiState*)h->multi)->als) {
+        *ms_out = 0.f;
+        for (lrk_handle_s* c : ((MultiState*)h->multi)->child) *ms_out = std::max(*ms_out, c->last_epoch_ms);
+        return LRK_OK;
+    }
     *ms_out = h->last_epoch_ms;
     return LRK_OK;
 }
@@ -923,7 +933,7 @@ int lrk_comm_unique_id(uint8_t out[128]) { return dsgd_unique_id(out); }
 int lrk_comm_init(lrk_handle_t h, int32_t rank, int32_t world, const uint8_t unique_id[128]) {
     LRK_REQUIRE(h, h != nullptr, "handle is NULL");
     LRK_NOT_MULTI(h, "lrk_comm_init");
-    LRK_REQUIRE(h, lrk_model_info(h->cfg).multi_gpu, k_lrk_single_gpu);
+    LRK_REQUIRE(h, lrk_model_info(h->cfg).dsgd, k_lrk_single_gpu);
     return dsgd_comm_init(h, rank, world, unique_id);
 }
 
@@ -933,7 +943,7 @@ int lrk_create_multi(const lrk_config_t* cfg, const int32_t* devices, int32_t n_
     if (n_devices < 1 || n_devices > 8) return lrk_fail(nullptr, LRK_ERR_INVALID, "lrk_create_multi", "1 to 8 devices", __FILE__, __LINE__);
     for (int a = 0; a < n_devices; ++a) for (int b = a + 1; b < n_devices; ++b)
         if (devices[a] == devices[b]) return lrk_fail(nullptr, LRK_ERR_INVALID, "lrk_create_multi", "a device is listed twice", __FILE__, __LINE__);
-    if (n_devices > 1 && lrk_model_known(cfg->model) && !lrk_model_info(*cfg).multi_gpu)     // an unknown model fails in lrk_create
+    if (n_devices > 1 && lrk_model_known(cfg->model) && !lrk_model_info(*cfg).multi_device)     // an unknown model fails in lrk_create
         return lrk_fail(nullptr, LRK_ERR_INVALID, "lrk_create_multi", k_lrk_single_gpu, __FILE__, __LINE__);
     lrk_handle_s* h = new (std::nothrow) lrk_handle_s();
     MultiState* ms = new (std::nothrow) MultiState();
@@ -941,19 +951,38 @@ int lrk_create_multi(const lrk_config_t* cfg, const int32_t* devices, int32_t n_
     h->cfg = *cfg; h->cfg.device = devices[0]; h->k = cfg->num_factors; h->multi = ms;
     ms->n = n_devices; ms->devices.assign(devices, devices + n_devices);
     ms->child.assign((size_t)n_devices, nullptr); ms->scorer.assign((size_t)n_devices, nullptr);
+    ms->als = n_devices > 1 && lrk_model_known(cfg->model) && !lrk_model_info(*cfg).dsgd;     // WRMF: plain children, no DSGD
     int rc = LRK_OK;
     for (int g = 0; g < n_devices && rc == LRK_OK; ++g) {
         lrk_config_t c = *cfg;
         c.device = devices[g];
         rc = lrk_create(&c, &ms->child[(size_t)g]);
-        if (rc == LRK_OK) { ms->child[(size_t)g]->same_process = true; ms->child[(size_t)g]->siblings = ms->child.data(); }   // peer pointers instead of CUDA IPC
+        if (rc == LRK_OK && !ms->als) { ms->child[(size_t)g]->same_process = true; ms->child[(size_t)g]->siblings = ms->child.data(); }   // peer pointers instead of CUDA IPC
     }
     for (int g = 0; g < n_devices; ++g) {
         LrkWorker* w = new LrkWorker();
         w->th = std::thread([w] { w->loop(); });
         ms->workers.push_back(w);
     }
-    if (rc == LRK_OK && n_devices > 1) {
+    if (rc == LRK_OK && ms->als) {
+        // the row exchange copies device to device: direct peer access where the pair has it (cudaMemcpyPeerAsync stages
+        // through the host otherwise), and the events of the phase split
+        ms->als_ev.assign((size_t)n_devices * LRK_ALS_EVENTS, nullptr);
+        for (int a = 0; a < n_devices && rc == LRK_OK; ++a) {
+            if (cudaSetDevice(devices[a]) != cudaSuccess) { rc = lrk_fail(h, LRK_ERR_CUDA, "cudaSetDevice", cudaGetErrorString(cudaGetLastError()), __FILE__, __LINE__); break; }
+            for (int b = 0; b < n_devices && rc == LRK_OK; ++b) {
+                int can = 0;
+                if (b == a || cudaDeviceCanAccessPeer(&can, devices[a], devices[b]) != cudaSuccess || !can) { cudaGetLastError(); continue; }
+                const cudaError_t pe = cudaDeviceEnablePeerAccess(devices[b], 0);
+                if (pe != cudaSuccess && pe != cudaErrorPeerAccessAlreadyEnabled) rc = lrk_fail(h, LRK_ERR_CUDA, "cudaDeviceEnablePeerAccess", cudaGetErrorString(pe), __FILE__, __LINE__);
+                cudaGetLastError();
+            }
+            for (int e = 0; e < LRK_ALS_EVENTS && rc == LRK_OK; ++e) {
+                const cudaError_t ce = cudaEventCreate(&ms->als_ev[(size_t)a * LRK_ALS_EVENTS + e]);
+                if (ce != cudaSuccess) rc = lrk_fail(h, LRK_ERR_CUDA, "cudaEventCreate", cudaGetErrorString(ce), __FILE__, __LINE__);
+            }
+        }
+    } else if (rc == LRK_OK && n_devices > 1) {
         uint8_t uid[128];
         rc = lrk_comm_unique_id(uid);
         if (rc == LRK_OK) rc = multi_run(h, ms, [&](int g) { return lrk_comm_init(ms->child[(size_t)g], g, ms->n, uid); });
@@ -986,6 +1015,8 @@ static int multi_destroy(lrk_handle_s* h) {
         multi_run(h, ms, [&](int g) -> int { return ms->child[(size_t)g] ? lrk_destroy(ms->child[(size_t)g]) : (int)LRK_OK; });
     else for (lrk_handle_s* c : ms->child) if (c) lrk_destroy(c);
     for (lrk_handle_s* c : ms->scorer) if (c) lrk_destroy(c);
+    for (size_t e = 0; e < ms->als_ev.size(); ++e)
+        if (ms->als_ev[e]) { cudaSetDevice(ms->devices[e / LRK_ALS_EVENTS]); cudaEventDestroy(ms->als_ev[e]); }
     for (LrkWorker* w : ms->workers) { w->stop(); delete w; }
     delete ms;
     h->multi = nullptr;
@@ -997,13 +1028,28 @@ static int multi_set_train_csr(lrk_handle_s* h, int32_t U, int32_t I, const int6
     MultiState* ms = (MultiState*)h->multi;
     LRK_REQUIRE(h, U >= ms->n, "fewer users than devices");
     ms->U = U; ms->I = I;
-    ms->ub.assign((size_t)ms->n + 1, 0);
-    for (int g = 0; g <= ms->n; ++g) ms->ub[(size_t)g] = (int64_t)g * U / ms->n;
     const int64_t nnz = rowptr[U];
+    if (ms->als) {
+        // every child stages the whole matrix; the rows are split by the estimated solve cost: the entries' rank-one updates
+        // (k^2 each) plus the row's Gauss-Jordan inverse (k^3)
+        LRK_REQUIRE(h, nnz >= 0 && nnz < (int64_t)0x7fffffffLL, "nnz out of range (the staging sorts take an int count: at most 2^31 - 1 train entries; every device of a WRMF multi-device handle stages all of them)");
+        const double k = (double)h->k, row_cost = k * k * k;
+        std::vector<int64_t> deg((size_t)I, 0);
+        for (int64_t e = 0; e < nnz; ++e) {
+            LRK_REQUIRE(h, col[e] >= 0 && col[e] < I, "column index out of range");
+            deg[(size_t)col[e]]++;
+        }
+        ms->ub = multi_cost_bounds(U, ms->n, true, [&](int64_t u) { return (double)(rowptr[u + 1] - rowptr[u]) * k * k + row_cost; });
+        ms->ib = multi_cost_bounds(I, ms->n, false, [&](int64_t i) { return (double)deg[(size_t)i] * k * k + row_cost; });
+    } else {
+        ms->ub.assign((size_t)ms->n + 1, 0);
+        for (int g = 0; g <= ms->n; ++g) ms->ub[(size_t)g] = (int64_t)g * U / ms->n;
+    }
     ms->rowptr.assign(rowptr, rowptr + U + 1);                 // kept for the scoring handles (top-N train mask)
     ms->col.assign(col, col + nnz);
     ms->scorer_csr = false; ms->scorer_factors = false;
     const int rc = multi_run(h, ms, [&](int g) -> int {
+        if (ms->als) return lrk_set_train_csr(ms->child[(size_t)g], U, I, rowptr, col, val);
         const int64_t lo = ms->ub[(size_t)g], hi = ms->ub[(size_t)g + 1], off = rowptr[lo];
         std::vector<int64_t> rp((size_t)(hi - lo) + 1);
         for (int64_t u = lo; u <= hi; ++u) rp[(size_t)(u - lo)] = rowptr[u] - off;
@@ -1020,6 +1066,7 @@ static int multi_set_factors(lrk_handle_s* h, const double* P, const double* Q, 
     ms->mu = mu; ms->scorer_factors = false;
     const int k = h->k;
     const int rc = multi_run(h, ms, [&](int g) {
+        if (ms->als) return lrk_set_factors(ms->child[(size_t)g], P, Q, bu, bi, mu);   // full replicas
         const int64_t lo = ms->ub[(size_t)g];
         return lrk_set_factors(ms->child[(size_t)g], P + lo * k, Q, bu ? bu + lo : nullptr, bi, mu);
     });
@@ -1030,6 +1077,11 @@ static int multi_set_factors(lrk_handle_s* h, const double* P, const double* Q, 
 static int multi_get_factors(lrk_handle_s* h, double* P, double* Q, double* bu, double* bi) {
     MultiState* ms = (MultiState*)h->multi;
     LRK_REQUIRE(h, h->has_factors, "no factors set");
+    if (ms->als) {                             // the replicas are equal after every iteration
+        const int rc = lrk_get_factors(ms->child[0], P, Q, bu, bi);
+        if (rc) h->err = ms->child[0]->err;
+        return rc;
+    }
     const int k = h->k;
     return multi_run(h, ms, [&](int g) {       // every rank enters the ring gather; rank 0 delivers the item side
         const int64_t lo = ms->ub[(size_t)g];
@@ -1037,9 +1089,96 @@ static int multi_get_factors(lrk_handle_s* h, double* P, double* Q, double* bu, 
     });
 }
 
+// One WRMF iteration over the devices.  Every child holds the full train matrix and full replicas of P and Q; device g solves the
+// users [ub[g], ub[g+1]) and the items [ib[g], ib[g+1]).  Per half: the Gram matrix of the fixed side on every device (each
+// computes the same full sum, so nothing depends on the partition), the device's row range, then every device pulls the other
+// ranges' new rows straight from their owners' replicas.  multi_run is the host barrier between the phases: a device's rows are
+// final before anyone copies them, and a Gram starts only after all blocks of its side have arrived.
+static int multi_als_epoch(lrk_handle_s* h, MultiState* ms, float reg_u, float reg_i, double* loss_out) {
+    const auto t0 = std::chrono::steady_clock::now();
+    const int k = h->k;
+    auto ev = [&](int g, int e) { return ms->als_ev[(size_t)g * LRK_ALS_EVENTS + e]; };
+    // the other devices' ranges of one side into device g's replica, on g's stream
+    auto pull = [&](int g, bool item_side) -> int {
+        lrk_handle_s* c = ms->child[(size_t)g];
+        const std::vector<int64_t>& b = item_side ? ms->ib : ms->ub;
+        for (int s = 0; s < ms->n; ++s) {
+            const int64_t lo = b[(size_t)s], cnt = b[(size_t)s + 1] - lo;
+            if (s == g || cnt == 0) continue;
+            lrk_handle_s* src = ms->child[(size_t)s];
+            double* dst = item_side ? c->Q64.ptr : c->P64.ptr;
+            const double* from = item_side ? src->Q64.ptr : src->P64.ptr;
+            LRK_CUDA(c, cudaMemcpyPeerAsync(dst + lo * k, c->cfg.device, from + lo * k, src->cfg.device, sizeof(double) * (size_t)(cnt * k), c->stream));
+        }
+        return LRK_OK;
+    };
+    int rc = multi_run(h, ms, [&](int g) -> int {
+        lrk_handle_s* c = ms->child[(size_t)g];
+        LRK_CUDA(c, cudaSetDevice(c->cfg.device));
+        LRK_REQUIRE(c, c->als != nullptr && c->f64_valid, "ALS state missing: call lrk_set_train_csr and lrk_set_factors first");
+        const int64_t lo = ms->ub[(size_t)g], hi = ms->ub[(size_t)g + 1];
+        int r;
+        LRK_CUDA(c, cudaEventRecord(ev(g, 0), c->stream));
+        if ((r = als_wrmf_gram(c, false))) return r;
+        LRK_CUDA(c, cudaEventRecord(ev(g, 1), c->stream));
+        if ((r = als_wrmf_side(c, als_wrmf_params(c, false, reg_u, (int32_t)lo, (int32_t)(hi - lo))))) return r;
+        LRK_CUDA(c, cudaEventRecord(ev(g, 2), c->stream));
+        LRK_CUDA(c, cudaStreamSynchronize(c->stream));
+        return LRK_OK;
+    });
+    if (rc == LRK_OK) rc = multi_run(h, ms, [&](int g) -> int {
+        lrk_handle_s* c = ms->child[(size_t)g];
+        LRK_CUDA(c, cudaSetDevice(c->cfg.device));
+        const int64_t lo = ms->ib[(size_t)g], hi = ms->ib[(size_t)g + 1];
+        int r;
+        LRK_CUDA(c, cudaEventRecord(ev(g, 3), c->stream));
+        if ((r = pull(g, false))) return r;
+        LRK_CUDA(c, cudaEventRecord(ev(g, 4), c->stream));
+        if ((r = als_wrmf_gram(c, true))) return r;
+        LRK_CUDA(c, cudaEventRecord(ev(g, 5), c->stream));
+        if ((r = als_wrmf_side(c, als_wrmf_params(c, true, reg_i, (int32_t)lo, (int32_t)(hi - lo))))) return r;
+        LRK_CUDA(c, cudaEventRecord(ev(g, 6), c->stream));
+        LRK_CUDA(c, cudaStreamSynchronize(c->stream));
+        return LRK_OK;
+    });
+    if (rc == LRK_OK) rc = multi_run(h, ms, [&](int g) -> int {
+        lrk_handle_s* c = ms->child[(size_t)g];
+        LRK_CUDA(c, cudaSetDevice(c->cfg.device));
+        int r;
+        LRK_CUDA(c, cudaEventRecord(ev(g, 7), c->stream));
+        if ((r = pull(g, true))) return r;
+        LRK_CUDA(c, cudaEventRecord(ev(g, 8), c->stream));
+        if ((r = als_refresh_f32(c))) return r;
+        LRK_CUDA(c, cudaStreamSynchronize(c->stream));
+        return LRK_OK;
+    });
+    if (rc) return rc;
+    h->last_epoch_ms = std::chrono::duration<float, std::milli>(std::chrono::steady_clock::now() - t0).count();
+    if (loss_out) *loss_out = 0.0;                    // trainModel never assigns `loss`
+    const char* trace = getenv("LRK_ALS_TRACE");
+    if (trace && atoi(trace)) {
+        // per device, ms between consecutive events: Gram(Q), users, waiting for the slowest device, P exchange, Gram(P), items,
+        // waiting, Q exchange
+        static const char* const names[] = {"gram_q", "solve_u", "wait_p", "xchg_p", "gram_p", "solve_i", "wait_q", "xchg_q"};
+        for (int g = 0; g < ms->n; ++g) {
+            std::string line = "[als] device " + std::to_string(ms->devices[(size_t)g]);
+            for (int e = 0; e + 1 < LRK_ALS_EVENTS; ++e) {
+                float t = 0.f;
+                cudaEventElapsedTime(&t, ev(g, e), ev(g, e + 1));
+                char buf[48];
+                snprintf(buf, sizeof buf, " %s %.3f", names[e], t);
+                line += buf;
+            }
+            fprintf(stderr, "%s total %.3f ms\n", line.c_str(), h->last_epoch_ms);
+        }
+    }
+    return LRK_OK;
+}
+
 static int multi_sgd_epoch(lrk_handle_s* h, float lr, float reg_u, float reg_i, double reg_b, int32_t epoch_idx, double* loss_out) {
     MultiState* ms = (MultiState*)h->multi;
     LRK_REQUIRE(h, h->has_train && h->has_factors, "set the train CSR and the factors before training");
+    if (ms->als) { ms->scorer_factors = false; return multi_als_epoch(h, ms, reg_u, reg_i, loss_out); }
     std::vector<double> loss((size_t)ms->n, 0.0);
     const int rc = multi_run(h, ms, [&](int g) { return lrk_sgd_epoch(ms->child[(size_t)g], lr, reg_u, reg_i, reg_b, epoch_idx, &loss[(size_t)g]); });
     if (loss_out) *loss_out = loss[0];          // all-reduced: the same on every rank

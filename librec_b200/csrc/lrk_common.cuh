@@ -192,7 +192,8 @@ struct LrkModelInfo {
     double loss_scale;  // reported loss = loss_scale * the kernels' sum (the references' 0.5 of the squared error); 0: no loss (ALS)
     bool safeguard;     // the epoch runs under the rollback safeguard (lrk_epoch.cuh)
     bool damped;        // staleness-aware item step: the SGD kernels read the item degrees and mean |p_u|^2
-    bool multi_gpu;     // DSGD / multi-device handle
+    bool dsgd;          // a DSGD rank: lrk_comm_init (process per GPU) and the DSGD children of a multi-device handle
+    bool multi_device;  // lrk_create_multi with more than one device (DSGD children, or for WRMF full replicas that split the rows)
     int biases;         // 0: none; 1: item biases (lrk_set_factors requires bi; user biases stay zero); 2: user and item biases.
                         // Predictions add b_i + p_u.q_i (+ b_u + mu) when > 0
     bool rating;        // BiasedMF / PMF: the rating is the target (item-run tiles, reference-order mode, user-group kernel)
@@ -200,26 +201,27 @@ struct LrkModelInfo {
     bool f64_working;   // the fp64 masters are the working set: an epoch leaves them valid (lrk_model_info sets it)
 };
 static const LrkModelInfo k_lrk_models[] = {
-    //                scale  guard  damped multi  biases rating als
-    /* BiasedMF */ {0.5, true,  true,  true,  2, true,  false},
-    /* PMF      */ {0.5, true,  true,  true,  0, true,  false},
-    /* BPR      */ {1.0, true,  false, true,  0, false, false},
-    /* RankSGD  */ {0.5, true,  true,  false, 0, false, false},
-    /* GBPR     */ {1.0, false, false, false, 1, false, false},
-    /* SVD++    */ {0.5, false, false, false, 2, false, false},
-    /* AoBPR    */ {1.0, true,  false, false, 0, false, false},
-    /* WRMF     */ {0.0, false, false, false, 0, false, true},
-    /* eALS     */ {0.0, false, false, false, 0, false, true},
+    //                scale  guard  damped dsgd   multi  biases rating als
+    /* BiasedMF */ {0.5, true,  true,  true,  true,  2, true,  false},
+    /* PMF      */ {0.5, true,  true,  true,  true,  0, true,  false},
+    /* BPR      */ {1.0, true,  false, true,  true,  0, false, false},
+    /* RankSGD  */ {0.5, true,  true,  false, false, 0, false, false},
+    /* GBPR     */ {1.0, false, false, false, false, 1, false, false},
+    /* SVD++    */ {0.5, false, false, false, false, 2, false, false},
+    /* AoBPR    */ {1.0, true,  false, false, false, 0, false, false},
+    /* WRMF     */ {0.0, false, false, false, true,  0, false, true},
+    /* eALS     */ {0.0, false, false, false, false, 0, false, true},
 };
 static inline bool lrk_model_known(int model) { return model >= 0 && model < (int)(sizeof k_lrk_models / sizeof k_lrk_models[0]); }
 // the row of cfg.model, for cfg.update_mode: the reference-order mode works on the fp64 masters, single-GPU, without the safeguard
 static inline LrkModelInfo lrk_model_info(const lrk_config_t& cfg) {
     LrkModelInfo m = k_lrk_models[cfg.model];
     m.f64_working = m.als;
-    if (cfg.update_mode == LRK_UPDATE_REFERENCE_ORDER) { m.safeguard = false; m.multi_gpu = false; m.f64_working = true; }
+    if (cfg.update_mode == LRK_UPDATE_REFERENCE_ORDER) { m.safeguard = false; m.dsgd = false; m.multi_device = false; m.f64_working = true; }
     return m;
 }
-static const char* const k_lrk_single_gpu = "reference-order mode, RankSGD, GBPR, SVD++, AoBPR, WRMF and eALS are single-GPU in this build";
+static const char* const k_lrk_single_gpu = "reference-order mode, RankSGD, GBPR, SVD++, AoBPR and eALS are single-GPU in this build; "
+                                            "WRMF runs on several GPUs through lrk_create_multi only, not as a DSGD rank";
 static inline bool lrk_has_bias(const lrk_handle_s* h) { return k_lrk_models[h->cfg.model].biases > 0; }
 
 // Calls f(G, V) with the handle's layout (layout_for_k) as std::integral_constant arguments: a generic lambda instantiates its

@@ -7,14 +7,23 @@
 // collectives that all ranks must enter together.  Training = the children's DSGD epoch (csrc/dsgd.cuh; the in-kernel ring takes the
 // neighbours' buffers by peer pointers, CUDA IPC cannot map memory of the same process); top-N = one scoring
 // handle per device over its user block with the full item matrix, no collective (SURVEY.md 8e).
+//
+// WRMF takes another route (`als` below): no DSGD and no communicator.  Every device gets a plain child handle that stages the FULL
+// train matrix and holds full replicas of P and Q; users and, separately, items are cut into contiguous ranges of about equal
+// solve cost, and one iteration solves each device's ranges and exchanges the new rows between the devices (multi_als_epoch in
+// lrk_api.cu).  A row's solve reads only the full other side, its Gram matrix and the row's own entries, so the split changes no
+// floating-point operation: the factors are bit-identical to a single device's.
 #pragma once
 #include "lrk_common.cuh"
+#include <algorithm>
 #include <condition_variable>
 #include <functional>
 #include <new>
 #include <mutex>
 #include <thread>
 #include <vector>
+
+#define LRK_ALS_EVENTS 9   // per device and WRMF iteration: start, Gram(Q), users, P pull start / end, Gram(P), items, Q pull start / end
 
 struct LrkWorker {
     std::thread th;
@@ -60,6 +69,9 @@ struct MultiState {
     std::vector<lrk_handle_s*> scorer;    // top-N handle per device over its user block (created on first use)
     std::vector<LrkWorker*> workers;
     std::vector<int64_t> ub;              // n + 1 user bounds
+    bool als = false;                     // WRMF on n > 1 devices: plain children with the full matrices, rows split by solve cost
+    std::vector<int64_t> ib;              // als: n + 1 item bounds (a range may be empty)
+    std::vector<cudaEvent_t> als_ev;      // als: LRK_ALS_EVENTS per device (the phase split of the LRK_ALS_TRACE line)
     int32_t U = 0, I = 0;
     double mu = 0.0;
     // host copies the scoring handles are staged from
@@ -87,4 +99,24 @@ static int multi_run(lrk_handle_s* h, MultiState* ms, const std::function<int(in
         }
     }
     return rc;
+}
+
+// n + 1 bounds that cut the rows [0, rows) into n contiguous ranges of about equal total cost; with `nonempty` (rows >= n) every
+// range keeps at least one row
+static std::vector<int64_t> multi_cost_bounds(int64_t rows, int n, bool nonempty, const std::function<double(int64_t)>& cost) {
+    std::vector<int64_t> b((size_t)n + 1, rows);
+    b[0] = 0;
+    double total = 0.0;
+    for (int64_t r = 0; r < rows; ++r) total += cost(r);
+    double acc = 0.0;
+    int g = 1;
+    for (int64_t r = 0; r < rows && g < n; ++r) {
+        while (g < n && acc >= total * g / n) b[(size_t)g++] = r;
+        acc += cost(r);
+    }
+    if (nonempty) {
+        for (int q = 1; q < n; ++q) b[(size_t)q] = std::max(b[(size_t)q], b[(size_t)q - 1] + 1);
+        for (int q = n - 1; q >= 1; --q) b[(size_t)q] = std::min(b[(size_t)q], b[(size_t)q + 1] - 1);
+    }
+    return b;
 }
