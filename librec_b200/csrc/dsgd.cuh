@@ -308,6 +308,7 @@ static int dsgd_set_train_csr(lrk_handle_s* h, int32_t U, int32_t I, const int64
     s->buf_floats = (s->buf_floats + 3) & ~(size_t)3;                       // float4-copyable
     for (int j = 0; j < 2; ++j) if ((rc = lrk_dev_alloc(h, &s->qbuf[j], s->buf_floats))) return rc;
     h->has_train = true;
+    topn_tc_invalidate(h);
     return LRK_OK;
 }
 
@@ -355,6 +356,7 @@ static int dsgd_set_factors(lrk_handle_s* h, const double* P, const double* Q, c
     LRK_CUDA(h, cudaStreamSynchronize(st));
     h->prev_loss = -1.0; h->conc_div = 1; h->good_epochs = 0; h->epochs_done = 0;
     h->mu = mu; h->has_factors = true; h->f64_valid = false;
+    topn_tc_invalidate(h);
     return LRK_OK;
 }
 
@@ -657,13 +659,12 @@ static int dsgd_epoch(lrk_handle_s* h, float lr, float reg_u, float reg_i, doubl
     return rc;
 }
 
-// P/bu: the rank's user block; Q/bi: the full item factors, gathered from the ring
-static int dsgd_get_factors(lrk_handle_s* h, double* P, double* Q, double* bu, double* bi) {
+// the full item factors into Q32 / bi32 (lrk_get_factors then refreshes the masters and copies them out); the masters are stale after it
+static int dsgd_gather_items(lrk_handle_s* h) {
     NcclApi* n = nccl_api();
     DsgdState* s = h->dsgd.get();
     cudaStream_t st = h->stream;
     const int world = h->world;
-    const int64_t U = h->U, I = h->I;
     const bool biased = h->cfg.model == LRK_MODEL_BIASEDMF;
     // all-gather the rotating buffers (every rank holds block `cur_block`), then unpack into Q32 / bi32
     // (BPR keeps the full item matrix on every rank: nothing to gather)
@@ -689,16 +690,6 @@ static int dsgd_get_factors(lrk_handle_s* h, double* P, double* Q, double* bu, d
     if (nr == ncclSuccess && e == cudaSuccess) e = cudaStreamSynchronize(st);
     LRK_NCCL(h, nr);
     LRK_CUDA(h, e);
-    f32_to_f64_rows_kernel<<<lrk_ceil_div(U * h->k, 256), 256, 0, st>>>(h->P32, h->P64, U, h->k, h->ld); LRK_LAUNCH_CHECK(h);
-    f32_to_f64_rows_kernel<<<lrk_ceil_div(I * h->k, 256), 256, 0, st>>>(h->Q32, h->Q64, I, h->k, h->ld); LRK_LAUNCH_CHECK(h);
-    if (biased) {
-        f32_to_f64_rows_kernel<<<lrk_ceil_div(U, 256), 256, 0, st>>>(h->bu32, h->bu64, U, 1, 1); LRK_LAUNCH_CHECK(h);
-        f32_to_f64_rows_kernel<<<lrk_ceil_div(I, 256), 256, 0, st>>>(h->bi32, h->bi64, I, 1, 1); LRK_LAUNCH_CHECK(h);
-    }
-    if (P) LRK_CUDA(h, cudaMemcpyAsync(P, h->P64, sizeof(double) * (size_t)U * h->k, cudaMemcpyDeviceToHost, st));
-    if (Q) LRK_CUDA(h, cudaMemcpyAsync(Q, h->Q64, sizeof(double) * (size_t)I * h->k, cudaMemcpyDeviceToHost, st));
-    if (bu && biased) LRK_CUDA(h, cudaMemcpyAsync(bu, h->bu64, sizeof(double) * (size_t)U, cudaMemcpyDeviceToHost, st));
-    if (bi && biased) LRK_CUDA(h, cudaMemcpyAsync(bi, h->bi64, sizeof(double) * (size_t)I, cudaMemcpyDeviceToHost, st));
-    LRK_CUDA(h, cudaStreamSynchronize(st));
+    h->f64_valid = false;
     return LRK_OK;
 }

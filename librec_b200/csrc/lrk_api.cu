@@ -11,7 +11,6 @@
 #include "sgd_aobpr.cuh"
 #include "als.cuh"
 #include "lrk_epoch.cuh"
-#include <chrono>
 #include "topn_exact.cuh"
 #include "topn_tc.cuh"
 #include "dsgd.cuh"
@@ -23,13 +22,6 @@
 
 thread_local std::string g_lrk_tls_error;
 
-static int multi_destroy(lrk_handle_s* h);
-static int multi_set_train_csr(lrk_handle_s* h, int32_t U, int32_t I, const int64_t* rowptr, const int32_t* col, const double* val);
-static int multi_set_factors(lrk_handle_s* h, const double* P, const double* Q, const double* bu, const double* bi, double mu);
-static int multi_get_factors(lrk_handle_s* h, double* P, double* Q, double* bu, double* bi);
-static int multi_sgd_epoch(lrk_handle_s* h, float lr, float reg_u, float reg_i, double reg_b, int32_t epoch_idx, double* loss_out);
-static int multi_topn(lrk_handle_s* h, const int32_t* users, int32_t nq, int32_t topn, int32_t exclude_train, int32_t* out_items,
-                      double* out_scores, int32_t* out_counts);
 #define LRK_NOT_MULTI(h, what) LRK_REQUIRE(h, !(h)->multi, what " is not available on a multi-device handle: call lrk_get_factors and use a single-device handle")
 
 // GBPR: train CSC (users of every item, ascending) next to the CSR -- the group draws of GBPRRecommender.java:104-116 walk an item's column
@@ -275,9 +267,10 @@ int lrk_create(const lrk_config_t* cfg, lrk_handle_t* out) {
 
 int lrk_destroy(lrk_handle_t h) {
     if (!h) return LRK_OK;
-    if (h->multi) return multi_destroy(h);
-    cudaSetDevice(h->cfg.device);
-    if (h->stream) cudaStreamSynchronize(h->stream);
+    if (!h->multi) {                                    // a multi-device parent has no stream of its own; ~MultiState destroys its children
+        cudaSetDevice(h->cfg.device);
+        if (h->stream) cudaStreamSynchronize(h->stream);
+    }
     delete h;
     return LRK_OK;
 }
@@ -291,7 +284,7 @@ int lrk_set_stream(lrk_handle_t h, void* cuda_stream) {
 }
 int lrk_synchronize(lrk_handle_t h) {
     LRK_REQUIRE(h, h != nullptr, "handle is NULL");
-    if (h->multi) { for (lrk_handle_s* c : ((MultiState*)h->multi)->child) { const int rc = lrk_synchronize(c); if (rc) return rc; } return LRK_OK; }
+    if (h->multi) { for (const LrkChild& c : h->multi->child) { const int rc = lrk_synchronize(c.get()); if (rc) return rc; } return LRK_OK; }
     LRK_CUDA(h, cudaSetDevice(h->cfg.device));
     LRK_CUDA(h, cudaStreamSynchronize(h->stream));
     return LRK_OK;
@@ -300,7 +293,7 @@ int lrk_synchronize(lrk_handle_t h) {
 // -------------------------------------------------------------------------------------------
 int lrk_set_train_csr(lrk_handle_t h, int32_t U, int32_t I, const int64_t* rowptr, const int32_t* col, const double* val) {
     LRK_REQUIRE(h, h != nullptr, "handle is NULL");
-    LRK_REQUIRE(h, U > 0 && I > 0 && rowptr && (col || rowptr[U] == 0) && (val || rowptr[U] == 0 || h->score_only), "bad CSR arguments");
+    LRK_REQUIRE(h, U > 0 && I > 0 && rowptr && (col || rowptr[U] == 0) && (val || rowptr[U] == 0), "bad CSR arguments");
     if (h->multi) return multi_set_train_csr(h, U, I, rowptr, col, val);
     LRK_REQUIRE(h, !h->has_factors || (h->U == U && h->I == I), "CSR shape differs from the factors already set");
     const int64_t nnz = rowptr[U];
@@ -312,20 +305,12 @@ int lrk_set_train_csr(lrk_handle_t h, int32_t U, int32_t I, const int64_t* rowpt
     int rc;
     if ((rc = lrk_dev_alloc(h, &h->d_rowptr, (size_t)U + 1))) return rc;
     if ((rc = lrk_dev_alloc(h, &h->d_col, (size_t)nnz))) return rc;
-    if (!h->score_only) {
-        if ((rc = lrk_dev_alloc(h, &h->d_su, (size_t)nnz))) return rc;
-        if ((rc = lrk_dev_alloc(h, &h->d_si, (size_t)nnz))) return rc;
-        if ((rc = lrk_dev_alloc(h, &h->d_sr, (size_t)nnz))) return rc;
-    }
+    if ((rc = lrk_dev_alloc(h, &h->d_su, (size_t)nnz))) return rc;
+    if ((rc = lrk_dev_alloc(h, &h->d_si, (size_t)nnz))) return rc;
+    if ((rc = lrk_dev_alloc(h, &h->d_sr, (size_t)nnz))) return rc;
     LRK_CUDA(h, cudaMemcpyAsync(h->d_rowptr, rowptr, sizeof(int64_t) * ((size_t)U + 1), cudaMemcpyHostToDevice, st));
     LRK_CUDA(h, cudaMemcpyAsync(h->d_col, col, sizeof(int32_t) * (size_t)nnz, cudaMemcpyHostToDevice, st));
     h->U = U; h->I = I; h->nnz = nnz;
-    if (h->score_only) {            // top-N mask only (scoring child of a multi handle; its DSGD sibling validated the shard)
-        LRK_CUDA(h, cudaStreamSynchronize(st));
-        h->has_train = true;
-        topn_tc_invalidate(h);
-        return LRK_OK;
-    }
     // BiasedMF / PMF in atomic mode with LRK_SGD_GROUP=1 train with the user-group kernel over a unit-ordered stream (sgd_group.cuh);
     // everything else keeps the item-run-tile stream of sgd.cuh
     h->group.reset();
@@ -421,9 +406,12 @@ int lrk_get_factors(lrk_handle_t h, double* P, double* Q, double* bu, double* bi
     if (h->multi) return multi_get_factors(h, P, Q, bu, bi);
     LRK_REQUIRE(h, h->has_factors, "no factors set");
     LRK_CUDA(h, cudaSetDevice(h->cfg.device));
-    if (h->world > 1) return dsgd_get_factors(h, P, Q, bu, bi);
-    int rc = refresh_masters(h);
-    if (rc) return rc;
+    int rc;
+    if (h->world > 1) {
+        if ((rc = dsgd_gather_items(h))) return rc;
+        if (!lrk_has_bias(h)) bu = bi = nullptr;        // a PMF / BPR rank leaves the caller's bias buffers untouched
+    }
+    if ((rc = refresh_masters(h))) return rc;
     cudaStream_t st = h->stream;
     if (P) LRK_CUDA(h, cudaMemcpyAsync(P, h->P64, sizeof(double) * (size_t)h->U * h->k, cudaMemcpyDeviceToHost, st));
     if (Q) LRK_CUDA(h, cudaMemcpyAsync(Q, h->Q64, sizeof(double) * (size_t)h->I * h->k, cudaMemcpyDeviceToHost, st));
@@ -604,23 +592,7 @@ int lrk_sgd_epochs(lrk_handle_t h, int32_t n_epochs, float lr, float decay, floa
 
 int lrk_stage_stats(lrk_handle_t h, int64_t out[4]) {
     LRK_REQUIRE(h, h != nullptr && out != nullptr, "NULL argument");
-    if (h->multi && ((MultiState*)h->multi)->als) {            // every child stages the whole matrix: count it once
-        lrk_handle_s* c = ((MultiState*)h->multi)->child[0];
-        const int rc = lrk_stage_stats(c, out);
-        if (rc) h->err = c->err;
-        return rc;
-    }
-    if (h->multi) {
-        int64_t acc[4] = {0, 0, 0, 0};
-        for (lrk_handle_s* c : ((MultiState*)h->multi)->child) {
-            int64_t v[4];
-            const int rc = lrk_stage_stats(c, v);
-            if (rc) { h->err = c->err; return rc; }
-            acc[0] += v[0]; acc[1] += v[1]; acc[2] = std::max(acc[2], v[2]); acc[3] = v[3];
-        }
-        for (int i = 0; i < 4; ++i) out[i] = acc[i];
-        return LRK_OK;
-    }
+    if (h->multi) return multi_stage_stats(h, out);
     LRK_REQUIRE(h, h->has_train, "no train CSR");
     out[0] = h->nnz; out[1] = 32 * h->run_tiles; out[2] = (int64_t)h->max_item_deg; out[3] = LRK_RUN_MIN_DEGREE;
     return LRK_OK;
@@ -648,16 +620,16 @@ int lrk_debug_stream(lrk_handle_t h, int32_t* su, int32_t* si, float* sr, int32_
 
 int lrk_sgd_safeguard_state(lrk_handle_t h, int32_t* conc_div, int64_t* rollbacks) {
     LRK_REQUIRE(h, h != nullptr, "handle is NULL");
-    if (h->multi) return lrk_sgd_safeguard_state(((MultiState*)h->multi)->child[0], conc_div, rollbacks);   // the ranks decide alike
+    if (h->multi) return lrk_sgd_safeguard_state(h->multi->child[0].get(), conc_div, rollbacks);   // the ranks decide alike
     if (conc_div) *conc_div = h->conc_div;
     if (rollbacks) *rollbacks = h->rollbacks;
     return LRK_OK;
 }
 int lrk_last_epoch_ms(lrk_handle_t h, float* ms_out) {
     LRK_REQUIRE(h, h != nullptr && ms_out != nullptr, "NULL argument");
-    if (h->multi && !((MultiState*)h->multi)->als) {
+    if (h->multi && !h->multi->als) {
         *ms_out = 0.f;
-        for (lrk_handle_s* c : ((MultiState*)h->multi)->child) *ms_out = std::max(*ms_out, c->last_epoch_ms);
+        for (const LrkChild& c : h->multi->child) *ms_out = std::max(*ms_out, c->last_epoch_ms);
         return LRK_OK;
     }
     *ms_out = h->last_epoch_ms;
@@ -666,10 +638,8 @@ int lrk_last_epoch_ms(lrk_handle_t h, float* ms_out) {
 int lrk_launch_count(lrk_handle_t h, uint64_t* out) {
     LRK_REQUIRE(h, h != nullptr && out != nullptr, "NULL argument");
     if (h->multi) {
-        MultiState* ms = (MultiState*)h->multi;
         *out = 0;
-        for (lrk_handle_s* c : ms->child) *out += c->launches;
-        for (lrk_handle_s* c : ms->scorer) if (c) *out += c->launches;
+        for (const LrkChild& c : h->multi->child) *out += c->launches;
         return LRK_OK;
     }
     *out = h->launches;
@@ -801,7 +771,7 @@ static int topn_to_device(lrk_handle_s* h, const int32_t* users, int32_t nq, int
     LRK_REQUIRE(h, topn > 0, "rec.recommender.ranking.topn should be more than 0!");   // AbstractRecommender.java:115-117
     LRK_REQUIRE(h, topn <= LRK_MAX_TOPN, "topn above LRK_MAX_TOPN (512)");
     LRK_REQUIRE(h, !exclude_train || h->has_train, "exclude_train needs the train CSR");
-    LRK_REQUIRE(h, h->world == 1, "gather the factors with lrk_get_factors in DSGD mode; top-N shards by user block");
+    LRK_REQUIRE(h, h->world == 1 || h->same_process, "gather the factors with lrk_get_factors in DSGD mode; top-N shards by user block");
     LRK_CUDA(h, cudaSetDevice(h->cfg.device));
     h->topn_fast_users = 0; h->topn_fallback_users = 0; h->topn_ms = 0.f;
     for (int i = 0; i < 4; ++i) h->topn_phase_ms[i] = 0.f;
@@ -908,14 +878,7 @@ int lrk_topn_phase_ms(lrk_handle_t h, float out[6]) {
 
 int lrk_topn_stats(lrk_handle_t h, int64_t* fast_users, int64_t* fallback_users, float* ms_out) {
     LRK_REQUIRE(h, h != nullptr, "handle is NULL");
-    if (h->multi) {
-        int64_t a = 0, b = 0; float ms = 0.f;
-        for (lrk_handle_s* c : ((MultiState*)h->multi)->scorer) if (c) { a += c->topn_fast_users; b += c->topn_fallback_users; ms = std::max(ms, c->topn_ms); }
-        if (fast_users) *fast_users = a;
-        if (fallback_users) *fallback_users = b;
-        if (ms_out) *ms_out = ms;
-        return LRK_OK;
-    }
+    if (h->multi) return multi_topn_stats(h, fast_users, fallback_users, ms_out);
     if (fast_users) *fast_users = h->topn_fast_users;
     if (fallback_users) *fallback_users = h->topn_fallback_users;
     if (ms_out) *ms_out = h->topn_ms;
@@ -924,7 +887,7 @@ int lrk_topn_stats(lrk_handle_t h, int64_t* fast_users, int64_t* fallback_users,
 
 int lrk_probe_l2(lrk_handle_t h, uint64_t working_set_bytes, int32_t row_floats, double out_gbps[3]) {
     LRK_REQUIRE(h, h != nullptr && out_gbps != nullptr, "NULL argument");
-    if (h->multi) h = ((MultiState*)h->multi)->child[0];
+    if (h->multi) h = h->multi->child[0].get();
     LRK_CUDA(h, cudaSetDevice(h->cfg.device));
     return l2_probe_run(h, (size_t)working_set_bytes, row_floats, out_gbps);
 }
@@ -938,62 +901,7 @@ int lrk_comm_init(lrk_handle_t h, int32_t rank, int32_t world, const uint8_t uni
 }
 
 int lrk_create_multi(const lrk_config_t* cfg, const int32_t* devices, int32_t n_devices, lrk_handle_t* out) {
-    if (!cfg || !out || !devices) return lrk_fail(nullptr, LRK_ERR_INVALID, "lrk_create_multi", "NULL argument", __FILE__, __LINE__);
-    *out = nullptr;
-    if (n_devices < 1 || n_devices > 8) return lrk_fail(nullptr, LRK_ERR_INVALID, "lrk_create_multi", "1 to 8 devices", __FILE__, __LINE__);
-    for (int a = 0; a < n_devices; ++a) for (int b = a + 1; b < n_devices; ++b)
-        if (devices[a] == devices[b]) return lrk_fail(nullptr, LRK_ERR_INVALID, "lrk_create_multi", "a device is listed twice", __FILE__, __LINE__);
-    if (n_devices > 1 && lrk_model_known(cfg->model) && !lrk_model_info(*cfg).multi_device)     // an unknown model fails in lrk_create
-        return lrk_fail(nullptr, LRK_ERR_INVALID, "lrk_create_multi", k_lrk_single_gpu, __FILE__, __LINE__);
-    lrk_handle_s* h = new (std::nothrow) lrk_handle_s();
-    MultiState* ms = new (std::nothrow) MultiState();
-    if (!h || !ms) { delete h; delete ms; return lrk_fail(nullptr, LRK_ERR_NOMEM, "lrk_create_multi", "host allocation failed", __FILE__, __LINE__); }
-    h->cfg = *cfg; h->cfg.device = devices[0]; h->k = cfg->num_factors; h->multi = ms;
-    ms->n = n_devices; ms->devices.assign(devices, devices + n_devices);
-    ms->child.assign((size_t)n_devices, nullptr); ms->scorer.assign((size_t)n_devices, nullptr);
-    ms->als = n_devices > 1 && lrk_model_known(cfg->model) && !lrk_model_info(*cfg).dsgd;     // WRMF: plain children, no DSGD
-    int rc = LRK_OK;
-    for (int g = 0; g < n_devices && rc == LRK_OK; ++g) {
-        lrk_config_t c = *cfg;
-        c.device = devices[g];
-        rc = lrk_create(&c, &ms->child[(size_t)g]);
-        if (rc == LRK_OK && !ms->als) { ms->child[(size_t)g]->same_process = true; ms->child[(size_t)g]->siblings = ms->child.data(); }   // peer pointers instead of CUDA IPC
-    }
-    for (int g = 0; g < n_devices; ++g) {
-        LrkWorker* w = new LrkWorker();
-        w->th = std::thread([w] { w->loop(); });
-        ms->workers.push_back(w);
-    }
-    if (rc == LRK_OK && ms->als) {
-        // the row exchange copies device to device: direct peer access where the pair has it (cudaMemcpyPeerAsync stages
-        // through the host otherwise), and the events of the phase split
-        ms->als_ev.assign((size_t)n_devices * LRK_ALS_EVENTS, nullptr);
-        for (int a = 0; a < n_devices && rc == LRK_OK; ++a) {
-            if (cudaSetDevice(devices[a]) != cudaSuccess) { rc = lrk_fail(h, LRK_ERR_CUDA, "cudaSetDevice", cudaGetErrorString(cudaGetLastError()), __FILE__, __LINE__); break; }
-            for (int b = 0; b < n_devices && rc == LRK_OK; ++b) {
-                int can = 0;
-                if (b == a || cudaDeviceCanAccessPeer(&can, devices[a], devices[b]) != cudaSuccess || !can) { cudaGetLastError(); continue; }
-                const cudaError_t pe = cudaDeviceEnablePeerAccess(devices[b], 0);
-                if (pe != cudaSuccess && pe != cudaErrorPeerAccessAlreadyEnabled) rc = lrk_fail(h, LRK_ERR_CUDA, "cudaDeviceEnablePeerAccess", cudaGetErrorString(pe), __FILE__, __LINE__);
-                cudaGetLastError();
-            }
-            for (int e = 0; e < LRK_ALS_EVENTS && rc == LRK_OK; ++e) {
-                const cudaError_t ce = cudaEventCreate(&ms->als_ev[(size_t)a * LRK_ALS_EVENTS + e]);
-                if (ce != cudaSuccess) rc = lrk_fail(h, LRK_ERR_CUDA, "cudaEventCreate", cudaGetErrorString(ce), __FILE__, __LINE__);
-            }
-        }
-    } else if (rc == LRK_OK && n_devices > 1) {
-        uint8_t uid[128];
-        rc = lrk_comm_unique_id(uid);
-        if (rc == LRK_OK) rc = multi_run(h, ms, [&](int g) { return lrk_comm_init(ms->child[(size_t)g], g, ms->n, uid); });
-    }
-    if (rc != LRK_OK) {
-        const std::string why = h->err.empty() ? g_lrk_tls_error : h->err;
-        multi_destroy(h);
-        return lrk_fail(nullptr, rc, "lrk_create_multi", why.c_str(), __FILE__, __LINE__);
-    }
-    *out = h;
-    return LRK_OK;
+    return multi_create(cfg, devices, n_devices, out);
 }
 
 }  // extern "C"
@@ -1006,245 +914,4 @@ lrk_handle_s::~lrk_handle_s() {
     for (cudaEvent_t ev : {ev0, ev1, ev_copy0, ev_copy1}) if (ev) cudaEventDestroy(ev);
     if (copy_stream) cudaStreamDestroy(copy_stream);
     if (own_stream) cudaStreamDestroy(own_stream);
-}
-
-static int multi_destroy(lrk_handle_s* h) {
-    MultiState* ms = (MultiState*)h->multi;
-    // the children's communicators are destroyed together, each on its own thread
-    if (!ms->workers.empty() && (int)ms->workers.size() == ms->n)
-        multi_run(h, ms, [&](int g) -> int { return ms->child[(size_t)g] ? lrk_destroy(ms->child[(size_t)g]) : (int)LRK_OK; });
-    else for (lrk_handle_s* c : ms->child) if (c) lrk_destroy(c);
-    for (lrk_handle_s* c : ms->scorer) if (c) lrk_destroy(c);
-    for (size_t e = 0; e < ms->als_ev.size(); ++e)
-        if (ms->als_ev[e]) { cudaSetDevice(ms->devices[e / LRK_ALS_EVENTS]); cudaEventDestroy(ms->als_ev[e]); }
-    for (LrkWorker* w : ms->workers) { w->stop(); delete w; }
-    delete ms;
-    h->multi = nullptr;
-    delete h;
-    return LRK_OK;
-}
-
-static int multi_set_train_csr(lrk_handle_s* h, int32_t U, int32_t I, const int64_t* rowptr, const int32_t* col, const double* val) {
-    MultiState* ms = (MultiState*)h->multi;
-    LRK_REQUIRE(h, U >= ms->n, "fewer users than devices");
-    ms->U = U; ms->I = I;
-    const int64_t nnz = rowptr[U];
-    if (ms->als) {
-        // every child stages the whole matrix; the rows are split by the estimated solve cost: the entries' rank-one updates
-        // (k^2 each) plus the row's Gauss-Jordan inverse (k^3)
-        LRK_REQUIRE(h, nnz >= 0 && nnz < (int64_t)0x7fffffffLL, "nnz out of range (the staging sorts take an int count: at most 2^31 - 1 train entries; every device of a WRMF multi-device handle stages all of them)");
-        const double k = (double)h->k, row_cost = k * k * k;
-        std::vector<int64_t> deg((size_t)I, 0);
-        for (int64_t e = 0; e < nnz; ++e) {
-            LRK_REQUIRE(h, col[e] >= 0 && col[e] < I, "column index out of range");
-            deg[(size_t)col[e]]++;
-        }
-        ms->ub = multi_cost_bounds(U, ms->n, true, [&](int64_t u) { return (double)(rowptr[u + 1] - rowptr[u]) * k * k + row_cost; });
-        ms->ib = multi_cost_bounds(I, ms->n, false, [&](int64_t i) { return (double)deg[(size_t)i] * k * k + row_cost; });
-    } else {
-        ms->ub.assign((size_t)ms->n + 1, 0);
-        for (int g = 0; g <= ms->n; ++g) ms->ub[(size_t)g] = (int64_t)g * U / ms->n;
-    }
-    ms->rowptr.assign(rowptr, rowptr + U + 1);                 // kept for the scoring handles (top-N train mask)
-    ms->col.assign(col, col + nnz);
-    ms->scorer_csr = false; ms->scorer_factors = false;
-    const int rc = multi_run(h, ms, [&](int g) -> int {
-        if (ms->als) return lrk_set_train_csr(ms->child[(size_t)g], U, I, rowptr, col, val);
-        const int64_t lo = ms->ub[(size_t)g], hi = ms->ub[(size_t)g + 1], off = rowptr[lo];
-        std::vector<int64_t> rp((size_t)(hi - lo) + 1);
-        for (int64_t u = lo; u <= hi; ++u) rp[(size_t)(u - lo)] = rowptr[u] - off;
-        return lrk_set_train_csr(ms->child[(size_t)g], (int32_t)(hi - lo), I, rp.data(), col + off, val + off);
-    });
-    if (rc == LRK_OK) { h->U = U; h->I = I; h->nnz = nnz; h->has_train = true; }
-    return rc;
-}
-
-static int multi_set_factors(lrk_handle_s* h, const double* P, const double* Q, const double* bu, const double* bi, double mu) {
-    MultiState* ms = (MultiState*)h->multi;
-    LRK_REQUIRE(h, h->has_train, "call lrk_set_train_csr first (it fixes numUsers / numItems)");
-    LRK_REQUIRE(h, P && Q, "P and Q are required");
-    ms->mu = mu; ms->scorer_factors = false;
-    const int k = h->k;
-    const int rc = multi_run(h, ms, [&](int g) {
-        if (ms->als) return lrk_set_factors(ms->child[(size_t)g], P, Q, bu, bi, mu);   // full replicas
-        const int64_t lo = ms->ub[(size_t)g];
-        return lrk_set_factors(ms->child[(size_t)g], P + lo * k, Q, bu ? bu + lo : nullptr, bi, mu);
-    });
-    if (rc == LRK_OK) { h->has_factors = true; h->mu = mu; }
-    return rc;
-}
-
-static int multi_get_factors(lrk_handle_s* h, double* P, double* Q, double* bu, double* bi) {
-    MultiState* ms = (MultiState*)h->multi;
-    LRK_REQUIRE(h, h->has_factors, "no factors set");
-    if (ms->als) {                             // the replicas are equal after every iteration
-        const int rc = lrk_get_factors(ms->child[0], P, Q, bu, bi);
-        if (rc) h->err = ms->child[0]->err;
-        return rc;
-    }
-    const int k = h->k;
-    return multi_run(h, ms, [&](int g) {       // every rank enters the ring gather; rank 0 delivers the item side
-        const int64_t lo = ms->ub[(size_t)g];
-        return lrk_get_factors(ms->child[(size_t)g], P ? P + lo * k : nullptr, g == 0 ? Q : nullptr, bu ? bu + lo : nullptr, g == 0 ? bi : nullptr);
-    });
-}
-
-// One WRMF iteration over the devices.  Every child holds the full train matrix and full replicas of P and Q; device g solves the
-// users [ub[g], ub[g+1]) and the items [ib[g], ib[g+1]).  Per half: the Gram matrix of the fixed side on every device (each
-// computes the same full sum, so nothing depends on the partition), the device's row range, then every device pulls the other
-// ranges' new rows straight from their owners' replicas.  multi_run is the host barrier between the phases: a device's rows are
-// final before anyone copies them, and a Gram starts only after all blocks of its side have arrived.
-static int multi_als_epoch(lrk_handle_s* h, MultiState* ms, float reg_u, float reg_i, double* loss_out) {
-    const auto t0 = std::chrono::steady_clock::now();
-    const int k = h->k;
-    auto ev = [&](int g, int e) { return ms->als_ev[(size_t)g * LRK_ALS_EVENTS + e]; };
-    // the other devices' ranges of one side into device g's replica, on g's stream
-    auto pull = [&](int g, bool item_side) -> int {
-        lrk_handle_s* c = ms->child[(size_t)g];
-        const std::vector<int64_t>& b = item_side ? ms->ib : ms->ub;
-        for (int s = 0; s < ms->n; ++s) {
-            const int64_t lo = b[(size_t)s], cnt = b[(size_t)s + 1] - lo;
-            if (s == g || cnt == 0) continue;
-            lrk_handle_s* src = ms->child[(size_t)s];
-            double* dst = item_side ? c->Q64.ptr : c->P64.ptr;
-            const double* from = item_side ? src->Q64.ptr : src->P64.ptr;
-            LRK_CUDA(c, cudaMemcpyPeerAsync(dst + lo * k, c->cfg.device, from + lo * k, src->cfg.device, sizeof(double) * (size_t)(cnt * k), c->stream));
-        }
-        return LRK_OK;
-    };
-    int rc = multi_run(h, ms, [&](int g) -> int {
-        lrk_handle_s* c = ms->child[(size_t)g];
-        LRK_CUDA(c, cudaSetDevice(c->cfg.device));
-        LRK_REQUIRE(c, c->als != nullptr && c->f64_valid, "ALS state missing: call lrk_set_train_csr and lrk_set_factors first");
-        const int64_t lo = ms->ub[(size_t)g], hi = ms->ub[(size_t)g + 1];
-        int r;
-        LRK_CUDA(c, cudaEventRecord(ev(g, 0), c->stream));
-        if ((r = als_wrmf_gram(c, false))) return r;
-        LRK_CUDA(c, cudaEventRecord(ev(g, 1), c->stream));
-        if ((r = als_wrmf_side(c, als_wrmf_params(c, false, reg_u, (int32_t)lo, (int32_t)(hi - lo))))) return r;
-        LRK_CUDA(c, cudaEventRecord(ev(g, 2), c->stream));
-        LRK_CUDA(c, cudaStreamSynchronize(c->stream));
-        return LRK_OK;
-    });
-    if (rc == LRK_OK) rc = multi_run(h, ms, [&](int g) -> int {
-        lrk_handle_s* c = ms->child[(size_t)g];
-        LRK_CUDA(c, cudaSetDevice(c->cfg.device));
-        const int64_t lo = ms->ib[(size_t)g], hi = ms->ib[(size_t)g + 1];
-        int r;
-        LRK_CUDA(c, cudaEventRecord(ev(g, 3), c->stream));
-        if ((r = pull(g, false))) return r;
-        LRK_CUDA(c, cudaEventRecord(ev(g, 4), c->stream));
-        if ((r = als_wrmf_gram(c, true))) return r;
-        LRK_CUDA(c, cudaEventRecord(ev(g, 5), c->stream));
-        if ((r = als_wrmf_side(c, als_wrmf_params(c, true, reg_i, (int32_t)lo, (int32_t)(hi - lo))))) return r;
-        LRK_CUDA(c, cudaEventRecord(ev(g, 6), c->stream));
-        LRK_CUDA(c, cudaStreamSynchronize(c->stream));
-        return LRK_OK;
-    });
-    if (rc == LRK_OK) rc = multi_run(h, ms, [&](int g) -> int {
-        lrk_handle_s* c = ms->child[(size_t)g];
-        LRK_CUDA(c, cudaSetDevice(c->cfg.device));
-        int r;
-        LRK_CUDA(c, cudaEventRecord(ev(g, 7), c->stream));
-        if ((r = pull(g, true))) return r;
-        LRK_CUDA(c, cudaEventRecord(ev(g, 8), c->stream));
-        if ((r = als_refresh_f32(c))) return r;
-        LRK_CUDA(c, cudaStreamSynchronize(c->stream));
-        return LRK_OK;
-    });
-    if (rc) return rc;
-    h->last_epoch_ms = std::chrono::duration<float, std::milli>(std::chrono::steady_clock::now() - t0).count();
-    if (loss_out) *loss_out = 0.0;                    // trainModel never assigns `loss`
-    const char* trace = getenv("LRK_ALS_TRACE");
-    if (trace && atoi(trace)) {
-        // per device, ms between consecutive events: Gram(Q), users, waiting for the slowest device, P exchange, Gram(P), items,
-        // waiting, Q exchange
-        static const char* const names[] = {"gram_q", "solve_u", "wait_p", "xchg_p", "gram_p", "solve_i", "wait_q", "xchg_q"};
-        for (int g = 0; g < ms->n; ++g) {
-            std::string line = "[als] device " + std::to_string(ms->devices[(size_t)g]);
-            for (int e = 0; e + 1 < LRK_ALS_EVENTS; ++e) {
-                float t = 0.f;
-                cudaEventElapsedTime(&t, ev(g, e), ev(g, e + 1));
-                char buf[48];
-                snprintf(buf, sizeof buf, " %s %.3f", names[e], t);
-                line += buf;
-            }
-            fprintf(stderr, "%s total %.3f ms\n", line.c_str(), h->last_epoch_ms);
-        }
-    }
-    return LRK_OK;
-}
-
-static int multi_sgd_epoch(lrk_handle_s* h, float lr, float reg_u, float reg_i, double reg_b, int32_t epoch_idx, double* loss_out) {
-    MultiState* ms = (MultiState*)h->multi;
-    LRK_REQUIRE(h, h->has_train && h->has_factors, "set the train CSR and the factors before training");
-    if (ms->als) { ms->scorer_factors = false; return multi_als_epoch(h, ms, reg_u, reg_i, loss_out); }
-    std::vector<double> loss((size_t)ms->n, 0.0);
-    const int rc = multi_run(h, ms, [&](int g) { return lrk_sgd_epoch(ms->child[(size_t)g], lr, reg_u, reg_i, reg_b, epoch_idx, &loss[(size_t)g]); });
-    if (loss_out) *loss_out = loss[0];          // all-reduced: the same on every rank
-    ms->scorer_factors = false;
-    return rc;
-}
-
-// top-N: users shard by block, every device holds the full item matrix, no collective (SURVEY.md 8e)
-static int multi_topn(lrk_handle_s* h, const int32_t* users, int32_t nq, int32_t topn, int32_t exclude_train, int32_t* out_items,
-                      double* out_scores, int32_t* out_counts) {
-    MultiState* ms = (MultiState*)h->multi;
-    LRK_REQUIRE(h, h->has_factors, "no factors set");
-    LRK_REQUIRE(h, topn > 0 && topn <= LRK_MAX_TOPN, "rec.recommender.ranking.topn should be more than 0!");
-    if (nq == 0) return LRK_OK;
-    if (users) for (int32_t c = 0; c < nq; ++c) LRK_REQUIRE(h, users[c] >= 0 && users[c] < ms->U, "user index out of range");
-    else LRK_REQUIRE(h, nq <= ms->U, "nq exceeds numUsers");
-    const int k = h->k;
-    const bool biased = lrk_has_bias(h);
-    int rc;
-    if (!ms->scorer_factors) {
-        ms->P.resize((size_t)ms->U * k); ms->Q.resize((size_t)ms->I * k);
-        if (biased) { ms->bu.resize((size_t)ms->U); ms->bi.resize((size_t)ms->I); }
-        if ((rc = multi_get_factors(h, ms->P.data(), ms->Q.data(), biased ? ms->bu.data() : nullptr, biased ? ms->bi.data() : nullptr))) return rc;
-    }
-    // queries by shard
-    std::vector<std::vector<int32_t>> local((size_t)ms->n), pos((size_t)ms->n);
-    for (int32_t c = 0; c < nq; ++c) {
-        const int32_t u = users ? users[c] : c;
-        int g = (int)(((int64_t)u * ms->n) / ms->U);
-        while (g > 0 && u < ms->ub[(size_t)g]) --g;
-        while (g + 1 < ms->n && u >= ms->ub[(size_t)g + 1]) ++g;
-        local[(size_t)g].push_back((int32_t)(u - ms->ub[(size_t)g]));
-        pos[(size_t)g].push_back(c);
-    }
-    const bool stage_csr = !ms->scorer_csr, stage_fac = !ms->scorer_factors;
-    rc = multi_run(h, ms, [&](int g) -> int {
-        int r = LRK_OK;
-        lrk_handle_s*& sc = ms->scorer[(size_t)g];
-        if (!sc) {
-            lrk_config_t c = h->cfg;
-            c.device = ms->devices[(size_t)g];
-            if ((r = lrk_create(&c, &sc))) return r;
-            sc->score_only = true;
-        }
-        const int64_t lo = ms->ub[(size_t)g], hi = ms->ub[(size_t)g + 1];
-        if (stage_csr) {
-            const int64_t off = ms->rowptr[(size_t)lo];
-            std::vector<int64_t> rp((size_t)(hi - lo) + 1);
-            for (int64_t u = lo; u <= hi; ++u) rp[(size_t)(u - lo)] = ms->rowptr[(size_t)u] - off;
-            if ((r = lrk_set_train_csr(sc, (int32_t)(hi - lo), ms->I, rp.data(), ms->col.data() + off, nullptr))) return r;
-        }
-        if (stage_csr || stage_fac)
-            if ((r = lrk_set_factors(sc, ms->P.data() + lo * k, ms->Q.data(), biased ? ms->bu.data() + lo : nullptr, biased ? ms->bi.data() : nullptr, ms->mu))) return r;
-        const size_t m = local[(size_t)g].size();
-        if (m == 0) return LRK_OK;
-        std::vector<int32_t> it(m * (size_t)topn), cn(m);
-        std::vector<double> sc_(m * (size_t)topn);
-        if ((r = lrk_topn(sc, local[(size_t)g].data(), (int32_t)m, topn, exclude_train, it.data(), sc_.data(), cn.data()))) return r;
-        for (size_t t = 0; t < m; ++t) {
-            const size_t c = (size_t)pos[(size_t)g][t];
-            memcpy(out_items + c * topn, it.data() + t * topn, sizeof(int32_t) * (size_t)topn);
-            memcpy(out_scores + c * topn, sc_.data() + t * topn, sizeof(double) * (size_t)topn);
-            out_counts[c] = cn[t];
-        }
-        return LRK_OK;
-    }, &ms->scorer);
-    if (rc == LRK_OK) { ms->scorer_csr = true; ms->scorer_factors = true; }
-    return rc;
 }

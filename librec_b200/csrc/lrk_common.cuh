@@ -30,6 +30,11 @@ struct LrkBuf {
 
 // model states (one translation unit: lrk_api.cu includes their headers and defines ~lrk_handle_s after them)
 struct GroupUnits; struct TcState; struct GbprState; struct SvdppState; struct AobprState; struct AlsState; struct ExactSchedule; struct DsgdState;
+struct MultiState;
+
+// owning pointer of a child handle of a multi-device parent (multi.cuh): lrk_destroy selects its device, syncs and deletes it
+struct LrkChildDelete { void operator()(lrk_handle_s* c) const { lrk_destroy(c); } };
+using LrkChild = std::unique_ptr<lrk_handle_s, LrkChildDelete>;
 
 struct lrk_handle_s {
     lrk_config_t cfg{};
@@ -104,11 +109,10 @@ struct lrk_handle_s {
     std::unique_ptr<ExactSchedule> exact;
 
     // single-process multi-GPU parent (multi.cuh): no device state of its own, forwards to one child per device
-    void* multi = nullptr;
+    std::unique_ptr<MultiState> multi;
     bool same_process = false; // DSGD child of a multi handle: its ring neighbours live in this process (CUDA IPC cannot map them;
-                               // the in-kernel ring takes their buffers by plain peer pointers instead)
-    lrk_handle_s** siblings = nullptr;   // same_process: the handles of all ranks, indexed by rank
-    bool score_only = false;   // scoring child of a multi handle: the train CSR is kept for the top-N mask only (no COO stream)
+                               // the in-kernel ring takes their buffers by plain peer pointers instead), and it serves top-N
+    const LrkChild* siblings = nullptr;  // same_process: the handles of all ranks, indexed by rank (the parent's child table)
 
     // DSGD
     void* comm = nullptr;   // ncclComm_t

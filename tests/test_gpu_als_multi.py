@@ -1,7 +1,9 @@
 """GPU: WRMF on several devices through one multi-device handle (lrk_create_multi, rec.cuda.devices in the Java shim).  Every device
 holds the full matrices, solves its own range of users and of items, and the devices exchange the new rows after each half-iteration
-(csrc/multi.cuh, multi_als_epoch in csrc/lrk_api.cu).  A row's solve reads only the full other side, so the split changes no
+(multi_als_epoch in csrc/multi.cuh).  A row's solve reads only the full other side, so the split changes no
 floating-point operation: the bar is BIT equality with the single-device handle and with the oracle, whatever the partition."""
+import ctypes as C
+
 import numpy as np
 import pytest
 
@@ -195,3 +197,35 @@ def test_wrmf_is_not_a_dsgd_rank(capi):
             with pytest.raises(capi.LibrecException) as e:
                 h.comm_init(0, 2, bytes(128))
             assert e.value.status == capi.ERR_INVALID
+
+
+def _topn_users(capi, h):
+    """(fast, fallback) users of the last top-N call, read without lrk_topn_phase_ms (a multi handle refuses that one)"""
+    a, b = C.c_int64(), C.c_int64()
+    assert capi.load().lrk_topn_stats(h._h, C.byref(a), C.byref(b), None) == capi.OK
+    return a.value, b.value
+
+
+def test_wrmf_multi_topn_after_each_iteration(O, capi):
+    """top-N of every user after iteration 1 and again after iteration 2, served by the children on the tensor-core path: each list
+    equals recommendRank on the oracle's factors, so the iteration must have dropped each child's cached item operand"""
+    devs = _all_devices(capi)
+    U, I, k, N, per_row = 600 * len(devs), 8200, 16, 10, 10     # equal rows: >= 512 users per device; I >= 8192, N <= 26
+    rng = np.random.default_rng(31)
+    col = np.concatenate([np.sort(rng.choice(I, per_row, replace=False)) for _ in range(U)]).astype(np.int32)
+    tr = O.Csr(U, I, np.arange(U + 1, dtype=np.int64) * per_row, col, rng.choice([1.0, 2.0, 3.0, 4.0, 5.0], U * per_row))
+    val = _wrmf_weights(O, tr.val)
+    P, Q = _factors(tr, k, 32)
+    oP, oQ = P.copy(), Q.copy()
+    with capi.Handle(capi.MODEL_WRMF, k, seed=1, devices=devs) as h:
+        h.set_train_csr(tr.U, tr.I, tr.rowptr, tr.col, val)
+        h.set_factors(P, Q)
+        for it in range(2):
+            h.sgd_epoch(0.0, 0.01, 0.01, 0.0, it + 1)
+            O.lib().lro_wrmf_epoch(tr.U, tr.I, tr.rowptr, tr.col, val, k, oP, oQ, 0.01, 0.01)
+            items, scores, counts = h.topn(N)
+            fast, fallback = _topn_users(capi, h)
+            oi, os_, oc = O.recommend_rank(1, U, I, k, oP, oQ, None, None, 0.0, tr, N)
+            assert np.array_equal(items, oi) and np.array_equal(scores.view(np.int64), os_.view(np.int64)), it
+            assert np.array_equal(counts, oc), it
+            assert fast > 0 and fast + fallback == U, it
