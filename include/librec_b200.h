@@ -57,8 +57,9 @@ typedef enum {
      * against a negative drawn by item popularity; single GPU; lrk_sgd_epoch ignores the regularisation arguments */
     LRK_MODEL_RANKSGD = 3,
     /* gbpr -> recommender/cf/ranking/GBPRRecommender.java:82-172 (SURVEY.md 8f row N3): group-preference BPR.  Item biases only
-     * (lrk_set_factors: bu may be NULL, bi is required); rec.gpbr.rho / rec.gpbr.gsize through lrk_set_param; single GPU;
-     * lrk_sgd_epoch's reg_b is rec.bias.regularization */
+     * (lrk_set_factors: bi is required; it ignores bu and global_mean and keeps zero user biases and a zero mean, so every
+     * prediction and top-N score is predict() = b_i + p_u.q_i, GBPRRecommender.java:194-196; training reads no global mean);
+     * rec.gpbr.rho / rec.gpbr.gsize through lrk_set_param; single GPU; lrk_sgd_epoch's reg_b is rec.bias.regularization */
     LRK_MODEL_GBPR = 4,
     /* svdpp -> recommender/cf/rating/SVDPlusPlusRecommender.java:62-123 (SURVEY.md 8f row N3): BiasedMF plus the implicit-feedback
      * factors impItemFactors (I x k) -- handed over / read back with lrk_set_matrix / lrk_get_matrix("svdpp.y"),

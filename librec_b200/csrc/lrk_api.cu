@@ -247,6 +247,7 @@ int lrk_create(const lrk_config_t* cfg, lrk_handle_t* out) {
         if (h->sgd_group && h->ld < 32) { h->ld = 32; h->G = 8; h->V = 1; }
     }
     h->sm_count = prop.multiProcessorCount;
+    h->smem_optin = prop.sharedMemPerBlockOptin;        // = cudaDevAttrMaxSharedMemoryPerBlockOptin
     int rc = LRK_OK;
     do {
         if (cudaSetDevice(cfg->device) != cudaSuccess) { rc = LRK_ERR_CUDA; break; }
@@ -350,6 +351,9 @@ int lrk_set_factors(lrk_handle_t h, const double* P, const double* Q, const doub
     const bool biased = m.biases > 0;
     LRK_REQUIRE(h, m.biases < 2 || (bu && bi), "BiasedMF / SVD++ need userBiases and itemBiases");
     LRK_REQUIRE(h, m.biases < 1 || bi, "GBPR needs itemBiases");
+    // GBPR predicts b_i + p_u.q_i (GBPRRecommender.java:194-196): the scoring kernels' ((p.q + b_u) + b_i) + mu equals that
+    // bit for bit with b_u = mu = 0, whatever global mean or user biases the caller passes
+    if (h->cfg.model == LRK_MODEL_GBPR) { bu = nullptr; mu = 0.0; }
     LRK_CUDA(h, cudaSetDevice(h->cfg.device));
     if (h->world > 1) return dsgd_set_factors(h, P, Q, bu, bi, mu);
     cudaStream_t st = h->stream;
@@ -794,7 +798,7 @@ static int topn_to_device(lrk_handle_s* h, const int32_t* users, int32_t nq, int
     cudaEventRecord(h->ev0, st);
     const bool want_tc = h->cfg.topn_path == 2 || (h->cfg.topn_path == 0 && topn_tc_profitable(h, nq, topn));
     if (want_tc) rc = topn_tc_run(h, d_users, nq, topn, exclude_train, h->tn_items, h->tn_scores, h->tn_counts);
-    else if (d_users && h->cfg.topn_path != 1 && nq <= 4 * h->sm_count && h->I >= 32768) {
+    else if (d_users && h->cfg.topn_path != 1 && nq <= 4 * h->sm_count && h->I >= 32768 && topn_parts_fit(h, topn)) {
         rc = topn_exact_parallel_launch(h, d_users, nq, topn, exclude_train, h->tn_items, h->tn_scores, h->tn_counts);
         h->topn_fallback_users = nq;
     } else { rc = topn_exact_launch(h, d_users, nq, topn, exclude_train, h->tn_items, h->tn_scores, h->tn_counts); h->topn_fallback_users = nq; }

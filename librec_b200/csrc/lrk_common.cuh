@@ -45,6 +45,7 @@ struct lrk_handle_s {
     int32_t U = 0, I = 0;
     int64_t nnz = 0;
     int sm_count = 0;
+    size_t smem_optin = 0;    // largest dynamic shared memory a block can opt in to (cudaDevAttrMaxSharedMemoryPerBlockOptin)
     cudaStream_t own_stream = nullptr, stream = nullptr;
     cudaStream_t copy_stream = nullptr;          // second stream: the H2D copy of the rating values overlaps the sort of the staging
     cudaEvent_t ev_copy0 = nullptr, ev_copy1 = nullptr;
@@ -97,6 +98,9 @@ struct lrk_handle_s {
     // result buffers of lrk_topn, reused across calls (cudaMalloc/cudaFree of 130 MB cost 20-400 ms per call)
     LrkBuf<int32_t> tn_users, tn_items, tn_counts;
     LrkBuf<double> tn_scores;
+    // heaps of the warp-per-user top-N kernel when they do not fit in shared memory (topn_exact_launch).  Not the staging arena:
+    // the tie replay of the item-parallel path runs while that path holds it
+    LrkBuf<char> tn_heaps;
     // tensor-core top-N state (bf16 copies, norms); see topn_tc.cuh
     std::unique_ptr<TcState> tc;
 
@@ -137,12 +141,16 @@ static inline int lrk_fail(lrk_handle_s* h, int code, const char* what, const ch
     return code;
 }
 
+// A failed call also clears the runtime's last error: a non-sticky error (an out-of-memory cudaMalloc, a rejected launch
+// attribute) is returned once, here, and not again by the next call on any handle that checks cudaGetLastError.
 #define LRK_CUDA(h, call)                                                                        \
     do {                                                                                         \
         cudaError_t e__ = (call);                                                                \
-        if (e__ != cudaSuccess)                                                                  \
+        if (e__ != cudaSuccess) {                                                                \
+            cudaGetLastError();                                                                  \
             return lrk_fail((h), e__ == cudaErrorMemoryAllocation ? LRK_ERR_NOMEM : LRK_ERR_CUDA, \
                             #call, cudaGetErrorString(e__), __FILE__, __LINE__);                 \
+        }                                                                                        \
     } while (0)
 
 #define LRK_REQUIRE(h, cond, msg)                                                         \

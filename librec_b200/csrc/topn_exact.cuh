@@ -9,7 +9,7 @@
 //                the heap ARRAY order followed by a stable descending sort.
 // The heap walk is inherently sequential per user, so one warp owns a user: lanes score 32
 // consecutive items in parallel (each lane a full left-to-right dot), then the warp replays the
-// 32 offers in item order against the heap kept in shared memory.
+// 32 offers in item order against the heap kept in shared memory (in global memory when the block's heaps do not fit).
 // This kernel is the exact path for every catalogue and the fallback of the tensor-core
 // candidate path (topn_tc.cuh) when its exactness certificate fails.
 #pragma once
@@ -121,23 +121,34 @@ __device__ __forceinline__ void heap_replace_min(HeapRef h, int size, double xv,
 #define TOPN_UPW 4                      // users per warp
 #define TOPN_UPB (TOPN_WARPS * TOPN_UPW)  // users per block
 
-// smem layout (doubles first): Qs[32][k+1] | Ps[UPB][k] | hv[UPB][topn] | hk[UPB][topn] (int32)
-static inline size_t topn_exact_smem(int k, int topn) {
-    return sizeof(double) * ((size_t)32 * (k + 1) + (size_t)TOPN_UPB * k + (size_t)TOPN_UPB * topn) +
-           sizeof(int32_t) * (size_t)TOPN_UPB * topn;
+// smem layout (doubles first): Qs[32][k+1] | Ps[UPB][k] | hv[UPB][topn] | hk[UPB][topn] (int32).  Without `heaps` the last
+// two live in global memory (kHeapsInSmem = false): at k = 256 the heaps fit in shared memory up to N = 263 only.
+static inline size_t topn_exact_smem(int k, int topn, bool heaps) {
+    return sizeof(double) * ((size_t)32 * (k + 1) + (size_t)TOPN_UPB * k) +
+           (heaps ? (sizeof(double) + sizeof(int32_t)) * (size_t)TOPN_UPB * topn : 0);
 }
 
+// heap_v / heap_k: [gridDim.x * UPB][topn] heaps in global memory, read only when !kHeapsInSmem
+template <bool kHeapsInSmem>
 __global__ void __launch_bounds__(TOPN_WARPS * 32) topn_exact_kernel(
     const double* __restrict__ P, const double* __restrict__ Q, const double* __restrict__ bu,
     const double* __restrict__ bi, double mu, int biased, int k, int32_t I,
     const int64_t* __restrict__ rowptr, const int32_t* __restrict__ col, int exclude_train,
     const int32_t* __restrict__ users, int32_t nq, int topn,
-    int32_t* __restrict__ out_items, double* __restrict__ out_scores, int32_t* __restrict__ out_counts) {
+    int32_t* __restrict__ out_items, double* __restrict__ out_scores, int32_t* __restrict__ out_counts,
+    double* heap_v, int32_t* heap_k) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     double* Qs = reinterpret_cast<double*>(smem_raw);
     double* Ps = Qs + (size_t)32 * (k + 1);
-    double* hv_all = Ps + (size_t)TOPN_UPB * k;
-    int32_t* hk_all = reinterpret_cast<int32_t*>(hv_all + (size_t)TOPN_UPB * topn);
+    double* hv_all;
+    int32_t* hk_all;
+    if (kHeapsInSmem) {
+        hv_all = Ps + (size_t)TOPN_UPB * k;
+        hk_all = reinterpret_cast<int32_t*>(hv_all + (size_t)TOPN_UPB * topn);
+    } else {
+        hv_all = heap_v + (size_t)blockIdx.x * TOPN_UPB * topn;
+        hk_all = heap_k + (size_t)blockIdx.x * TOPN_UPB * topn;
+    }
 
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const int qs_ld = k + 1;
@@ -259,12 +270,23 @@ __global__ void __launch_bounds__(TOPN_WARPS * 32) topn_exact_kernel(
 // results to device buffers
 static int topn_exact_launch(lrk_handle_s* h, const int32_t* d_users, int32_t nq, int topn, int exclude_train,
                              int32_t* d_items, double* d_scores, int32_t* d_counts) {
-    const size_t smem = topn_exact_smem(h->k, topn);
-    LRK_CUDA(h, cudaFuncSetAttribute(topn_exact_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    const bool heaps_in_smem = topn_exact_smem(h->k, topn, true) <= h->smem_optin;
+    const size_t smem = topn_exact_smem(h->k, topn, heaps_in_smem);
     const int grid = lrk_ceil_div(nq, TOPN_UPB);
-    topn_exact_kernel<<<grid, TOPN_WARPS * 32, smem, h->stream>>>(
+    double* heap_v = nullptr;
+    int32_t* heap_k = nullptr;
+    if (!heaps_in_smem) {
+        const size_t slots = (size_t)grid * TOPN_UPB * topn;
+        const int rc = lrk_dev_alloc(h, &h->tn_heaps, slots * (sizeof(double) + sizeof(int32_t)));
+        if (rc) return rc;
+        heap_v = reinterpret_cast<double*>(h->tn_heaps.ptr);
+        heap_k = reinterpret_cast<int32_t*>(heap_v + slots);
+    }
+    auto kernel = heaps_in_smem ? topn_exact_kernel<true> : topn_exact_kernel<false>;
+    LRK_CUDA(h, cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    kernel<<<grid, TOPN_WARPS * 32, smem, h->stream>>>(
         h->P64, h->Q64, h->bu64, h->bi64, h->mu, lrk_has_bias(h), h->k, h->I,
-        h->d_rowptr, h->d_col, exclude_train, d_users, nq, topn, d_items, d_scores, d_counts);
+        h->d_rowptr, h->d_col, exclude_train, d_users, nq, topn, d_items, d_scores, d_counts, heap_v, heap_k);
     LRK_LAUNCH_CHECK(h);
     return LRK_OK;
 }
@@ -280,6 +302,15 @@ static int topn_exact_launch(lrk_handle_s* h, const int32_t* d_users, int32_t nq
 // first N+1 (rare) are replayed by topn_exact_kernel.
 // ---------------------------------------------------------------------------------------------
 #define TOPN_PAR_THREADS 256
+// smem of topn_exact_parts_kernel: the user row [k] | T = topn+1 sorted lists per thread [T][256] (doubles, then int32) | the
+// block reduction (8 doubles, 16 int32).  3072 B per list slot: from N = 74 (k > 240) or N = 75 the lists exceed a B200 block.
+static inline size_t topn_parts_smem(int k, int topn) {
+    const size_t T = (size_t)topn + 1;
+    return sizeof(double) * ((size_t)k + T * TOPN_PAR_THREADS + 8) + sizeof(int32_t) * (T * TOPN_PAR_THREADS + 16);
+}
+// the one predicate of every choice of the item-parallel path: otherwise the warp-per-user kernel serves the call
+static inline bool topn_parts_fit(const lrk_handle_s* h, int topn) { return topn_parts_smem(h->k, topn) <= h->smem_optin; }
+
 __global__ void __launch_bounds__(TOPN_PAR_THREADS) topn_exact_parts_kernel(
     const double* __restrict__ P, const double* __restrict__ Q, const double* __restrict__ bu, const double* __restrict__ bi,
     double mu, int biased, int k, int32_t I, const int64_t* __restrict__ rowptr, const int32_t* __restrict__ col,
@@ -412,7 +443,7 @@ __global__ void topn_scatter_kernel(const int32_t* __restrict__ slots, int n, in
 }
 
 // d_users: device array of nq user ids (required).  Results to device buffers [nq x topn].  Takes the staging arena: the
-// callers (topn_to_device, topn_tc_run) hold none of it.
+// callers (topn_to_device, topn_tc_run) hold none of it.  They call it only when topn_parts_fit(h, topn).
 static int topn_exact_parallel_launch(lrk_handle_s* h, const int32_t* d_users, int32_t nq, int topn, int exclude_train,
                                       int32_t* d_items, double* d_scores, int32_t* d_counts) {
     cudaStream_t st = h->stream;
@@ -439,7 +470,7 @@ static int topn_exact_parallel_launch(lrk_handle_s* h, const int32_t* d_users, i
         return lrk_fail(h, LRK_ERR_NOMEM, "topn_exact_parallel_launch", "scratch arena too small", __FILE__, __LINE__);
     int32_t *tslots = tie + nq, *tusers = tie + 2 * (size_t)nq;
     LRK_CUDA(h, cudaMemsetAsync(tcount, 0, sizeof(int), st));
-    const size_t smem = sizeof(double) * ((size_t)h->k + (size_t)T * TOPN_PAR_THREADS + 8) + sizeof(int32_t) * ((size_t)T * TOPN_PAR_THREADS + 16);
+    const size_t smem = topn_parts_smem(h->k, topn);
     LRK_CUDA(h, cudaFuncSetAttribute(topn_exact_parts_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     topn_exact_parts_kernel<<<nq * n_parts, TOPN_PAR_THREADS, smem, st>>>(
         h->P64, h->Q64, h->bu64, h->bi64, h->mu, lrk_has_bias(h), h->k, h->I, h->d_rowptr, h->d_col,

@@ -903,7 +903,9 @@ static int topn_tc_run(lrk_handle_s* h, const int32_t* d_users, int32_t nq, int 
         if ((rc = lrk_dev_alloc(h, &s->fail_items, (size_t)nfail * topn))) return rc;
         if ((rc = lrk_dev_alloc(h, &s->fail_scores, (size_t)nfail * topn))) return rc;
         if ((rc = lrk_dev_alloc(h, &s->fail_counts, (size_t)nfail))) return rc;
-        if ((rc = topn_exact_parallel_launch(h, ex_users, nfail, topn, exclude_train, s->fail_items, s->fail_scores, s->fail_counts))) return rc;
+        rc = topn_parts_fit(h, topn) ? topn_exact_parallel_launch(h, ex_users, nfail, topn, exclude_train, s->fail_items, s->fail_scores, s->fail_counts)
+                                     : topn_exact_launch(h, ex_users, nfail, topn, exclude_train, s->fail_items, s->fail_scores, s->fail_counts);
+        if (rc) return rc;
         topn_scatter_kernel<<<lrk_ceil_div((int64_t)nfail * topn, 256), 256, 0, st>>>(ex_slots, nfail, topn, s->fail_items, s->fail_scores,
                                                                                    s->fail_counts, d_items, d_scores, d_counts);
         LRK_LAUNCH_CHECK(h);

@@ -6,6 +6,7 @@ import numpy as np
 
 from conftest import rng_csr
 from test_oracle_aobpr import JavaRandom
+from test_oracle_pins import _py_topk
 from test_oracle_ranking_eval import JavaHashSet
 
 
@@ -107,3 +108,33 @@ def test_gbpr_matches_python_replay(O):
     raters = {i: set(np.flatnonzero([(i in tr.col[tr.rowptr[u]:tr.rowptr[u + 1]]) for u in range(tr.U)]).tolist()) for i in range(tr.I)}
     for (u, i, j), g in zip(etrips, egroups):
         assert set(g) <= raters[i] and (u in g or len(raters[i]) <= g_len) and 1 <= len(g) <= g_len
+
+
+def test_gbpr_ranking_is_biasedmf_with_zero_user_bias_and_mean(O):
+    """GBPR's predict() is b_i + p_u.q_i (GBPRRecommender.java:194-196); the oracle and the device score it as BiasedMF does,
+    ((d + b_u) + b_i) + mu with d the left-to-right dot product, given b_u = 0 and mu = 0.  The two agree bit for bit: the dot
+    product starts from +0.0, and a round-to-nearest sum is -0.0 only when both terms are -0.0, so d is never -0.0.  Hence
+    d + 0.0 == d, d + b_i is never -0.0 either, and ((d + 0) + b_i) + 0 == d + b_i == b_i + d.  This replays recommendRank
+    with b_i + d in plain Python floats (sign-carrying zeros, exact ties) and compares the lists bit for bit."""
+    U, I, k, N = 14, 60, 4, 8
+    rng = np.random.default_rng(21)
+    P, Q = rng.normal(size=(U, k)), rng.normal(size=(I, k))
+    bi = rng.normal(size=I)
+    P[0] = 0.0; P[1] = -0.0                               # d = +0.0 for every item: the score is b_i (or +0.0)
+    Q[7] = -0.0; Q[8] = 0.0                               # d = +0.0 for every user
+    bi[[7, 8, 9]] = -0.0; bi[[20, 21]] = bi[19]; Q[[20, 21]] = Q[19]   # -0.0 biases, exact ties
+    tr = rng_csr(O, U, I, 0.2, 22)
+    items, scores, counts = O.recommend_rank(O.BIASEDMF, U, I, k, P, Q, np.zeros(U), bi, 0.0, tr, N, nthreads=2)
+    for u in range(U):
+        row = set(tr.col[tr.rowptr[u]:tr.rowptr[u + 1]].tolist())
+        cand = [i for i in range(I) if i not in row]
+        vals = []
+        for i in cand:
+            d = 0.0
+            for f in range(k):
+                d += P[u, f] * Q[i, f]
+            vals.append(float(bi[i]) + d)
+        _, order = _py_topk(vals, N)
+        assert counts[u] == len(order)
+        assert items[u, :counts[u]].tolist() == [cand[t] for t in order]
+        assert scores[u, :counts[u]].view(np.int64).tolist() == np.array([vals[t] for t in order]).view(np.int64).tolist()
