@@ -46,11 +46,6 @@ __global__ void als_csc_gather_kernel(const int32_t* __restrict__ perm, const in
     cusers[t] = rows[e];
     cval[t] = val[e];
 }
-__global__ void als_iota_kernel(int32_t* __restrict__ out, int64_t n) {
-    const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (t < n) out[t] = (int32_t)t;
-}
-
 // out[r][c] = sum_i M[i][c] * M[i][r] (w == nullptr; DenseMatrix.times over the transpose) or, with weights, the eALS cache
 // sum_i (w[i] * M[i][max(r,c)]) * M[i][min(r,c)] (EALSRecommender.java:128-137 computes the lower triangle and mirrors it).
 // One thread per entry, rows i in order: every entry is one chain of n dependent adds, so the kernel's time is that chain as long
@@ -441,31 +436,22 @@ static int als_stage(lrk_handle_s* h, const double* h_val) {
     }
     if (nnz == 0) { LRK_CUDA(h, cudaMemsetAsync(a->d_colptr, 0, sizeof(int64_t) * ((size_t)I + 1), st)); return LRK_OK; }
     LRK_CUDA(h, cudaMemcpyAsync(a->d_val, h_val, sizeof(double) * (size_t)nnz, cudaMemcpyHostToDevice, st));
-    size_t tb_sort = 0, tb_scan = 0;
-    int end_bit = 1;
-    while (end_bit < 32 && ((int64_t)1 << end_bit) < (int64_t)I) ++end_bit;
-    LRK_CUDA(h, cub::DeviceRadixSort::SortPairs(nullptr, tb_sort, (uint32_t*)nullptr, (uint32_t*)nullptr, (int32_t*)nullptr, (int32_t*)nullptr, (int)nnz, 0, end_bit, st));
-    LRK_CUDA(h, cub::DeviceScan::ExclusiveSum(nullptr, tb_scan, (uint32_t*)nullptr, (uint32_t*)nullptr, (int)I, st));
-    const size_t tb = std::max(tb_sort, tb_scan) + 256;
+    const size_t tb = by_item_order_tmp_bytes(I, nnz);
     LrkScratch sc;
     if ((rc = lrk_scratch_begin(h, (size_t)nnz * 20 + (size_t)I * 8 + tb + 16 * 256, &sc))) return rc;
-    uint32_t *k_in = sc.take<uint32_t>((size_t)nnz), *k_out = sc.take<uint32_t>((size_t)nnz);
-    int32_t *rows = sc.take<int32_t>((size_t)nnz), *iota = sc.take<int32_t>((size_t)nnz), *perm = sc.take<int32_t>((size_t)nnz);
+    uint32_t *keys = sc.take<uint32_t>((size_t)nnz), *keys_out = sc.take<uint32_t>((size_t)nnz), *ids = sc.take<uint32_t>((size_t)nnz);
+    uint32_t* perm = sc.take<uint32_t>((size_t)nnz);
+    int32_t* rows = sc.take<int32_t>((size_t)nnz);
     uint32_t *deg = sc.take<uint32_t>((size_t)I), *deg_ex = sc.take<uint32_t>((size_t)I);
     void* tmp = sc.take<char>(tb);
-    if (!k_in || !k_out || !rows || !iota || !perm || !deg || !deg_ex || !tmp) return lrk_fail(h, LRK_ERR_NOMEM, "als_stage", "scratch arena too small", __FILE__, __LINE__);
+    if (!keys || !keys_out || !ids || !perm || !rows || !deg || !deg_ex || !tmp) return lrk_fail(h, LRK_ERR_NOMEM, "als_stage", "scratch arena too small", __FILE__, __LINE__);
     const int nb = lrk_ceil_div(nnz, 256);
     coo_rows_kernel<<<nb, 256, 0, st>>>(h->d_rowptr, U, nnz, rows); LRK_LAUNCH_CHECK(h);
-    als_iota_kernel<<<nb, 256, 0, st>>>(iota, nnz); LRK_LAUNCH_CHECK(h);
-    LRK_CUDA(h, cudaMemcpyAsync(k_in, h->d_col, sizeof(uint32_t) * (size_t)nnz, cudaMemcpyDeviceToDevice, st));
-    LRK_CUDA(h, cudaMemsetAsync(deg, 0, sizeof(uint32_t) * (size_t)I, st));
-    item_degree_kernel<<<nb, 256, 0, st>>>(h->d_col, nnz, deg); LRK_LAUNCH_CHECK(h);
-    size_t t1 = tb;
-    LRK_CUDA(h, cub::DeviceScan::ExclusiveSum(tmp, t1, deg, deg_ex, (int)I, st));
-    gbpr_colptr_kernel<<<lrk_ceil_div(I, 256), 256, 0, st>>>(deg_ex, deg, I, a->d_colptr); LRK_LAUNCH_CHECK(h);
-    t1 = tb;
-    LRK_CUDA(h, cub::DeviceRadixSort::SortPairs(tmp, t1, k_in, k_out, iota, perm, (int)nnz, 0, end_bit, st));   // stable: users ascending within an item
-    als_csc_gather_kernel<<<nb, 256, 0, st>>>(perm, rows, a->d_val, nnz, a->d_cusers, a->d_cval); LRK_LAUNCH_CHECK(h);
+    if ((rc = by_item_order(h, h->d_col, I, nnz, deg, deg_ex, perm, keys, keys_out, ids, tmp, tb))) return rc;
+    csc_colptr_kernel<<<lrk_ceil_div(I, 256), 256, 0, st>>>(deg_ex, deg, I, a->d_colptr); LRK_LAUNCH_CHECK(h);
+    // users ascending within an item
+    als_csc_gather_kernel<<<nb, 256, 0, st>>>(reinterpret_cast<const int32_t*>(perm), rows, a->d_val, nnz, a->d_cusers, a->d_cval);
+    LRK_LAUNCH_CHECK(h);
     LRK_CUDA(h, cudaStreamSynchronize(st));
     h->launches += 6;
     return LRK_OK;

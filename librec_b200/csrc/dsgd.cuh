@@ -10,7 +10,7 @@
 //     (g+s+1) mod G from rank g+1 (grouped ncclSend/ncclRecv on the handle's stream, NVLink 5);
 //   * strata of one sub-epoch touch disjoint users AND items, so there is no cross-GPU race;
 //   * one fp64 ncclAllReduce of the loss per epoch.
-// NCCL is dlopen'ed lazily so that the single-GPU path has no NCCL dependency.
+// NCCL is dlopen'ed lazily so that the single-GPU path has no NCCL dependency (lrk_nccl.cuh).
 #pragma once
 #include "lrk_common.cuh"
 #include "staging.cuh"
@@ -18,77 +18,19 @@
 #include "sgd_group.cuh"
 #include "dsgd_fused.cuh"
 #include "lrk_epoch.cuh"
-#include <nccl.h>
-#include <dlfcn.h>
+#include "lrk_nccl.cuh"
 #include <vector>
 #include <algorithm>
-
-struct NcclApi {
-    void* lib = nullptr;
-    ncclResult_t (*GetUniqueId)(ncclUniqueId*) = nullptr;
-    ncclResult_t (*CommInitRank)(ncclComm_t*, int, ncclUniqueId, int) = nullptr;
-    ncclResult_t (*CommDestroy)(ncclComm_t) = nullptr;
-    ncclResult_t (*Send)(const void*, size_t, ncclDataType_t, int, ncclComm_t, cudaStream_t) = nullptr;
-    ncclResult_t (*Recv)(void*, size_t, ncclDataType_t, int, ncclComm_t, cudaStream_t) = nullptr;
-    ncclResult_t (*AllReduce)(const void*, void*, size_t, ncclDataType_t, ncclRedOp_t, ncclComm_t, cudaStream_t) = nullptr;
-    ncclResult_t (*AllGather)(const void*, void*, size_t, ncclDataType_t, ncclComm_t, cudaStream_t) = nullptr;
-    ncclResult_t (*GroupStart)() = nullptr;
-    ncclResult_t (*GroupEnd)() = nullptr;
-    const char* (*GetErrorString)(ncclResult_t) = nullptr;
-};
-
-static NcclApi* nccl_api() {
-    static NcclApi api;
-    static bool tried = false;
-    if (tried) return api.lib ? &api : nullptr;
-    tried = true;
-    const char* names[] = {"libnccl.so.2", "libnccl.so"};
-    for (const char* n : names) { api.lib = dlopen(n, RTLD_NOW | RTLD_GLOBAL); if (api.lib) break; }
-    if (!api.lib) return nullptr;
-#define LRK_SYM(field, sym) *(void**)(&api.field) = dlsym(api.lib, sym); if (!api.field) { api.lib = nullptr; return nullptr; }
-    LRK_SYM(GetUniqueId, "ncclGetUniqueId") LRK_SYM(CommInitRank, "ncclCommInitRank") LRK_SYM(CommDestroy, "ncclCommDestroy")
-    LRK_SYM(Send, "ncclSend") LRK_SYM(Recv, "ncclRecv") LRK_SYM(AllReduce, "ncclAllReduce") LRK_SYM(AllGather, "ncclAllGather")
-    LRK_SYM(GroupStart, "ncclGroupStart") LRK_SYM(GroupEnd, "ncclGroupEnd") LRK_SYM(GetErrorString, "ncclGetErrorString")
-#undef LRK_SYM
-    return &api;
-}
-
-#define LRK_NCCL(h, call)                                                                                         \
-    do {                                                                                                          \
-        ncclResult_t r__ = (call);                                                                                \
-        if (r__ != ncclSuccess) return lrk_fail((h), LRK_ERR_NCCL, #call, nccl_api()->GetErrorString(r__), __FILE__, __LINE__); \
-    } while (0)
 
 // ---- the DSGD plan: pure functions of (rank, world, sub-epoch); mirrored by librec_b200/dsgd_plan.py
 static inline int dsgd_block_at(int rank, int world, int sub) { return (rank + sub) % world; }
 static inline int dsgd_send_peer(int rank, int world) { return (rank - 1 + world) % world; }
 static inline int dsgd_recv_peer(int rank, int world) { return (rank + 1) % world; }
-// contiguous item blocks balanced by rating count: block b = [bounds[b], bounds[b+1])
-static inline void dsgd_item_bounds(const int64_t* item_count, int32_t I, int world, std::vector<int32_t>& bounds) {
-    int64_t total = 0;
-    for (int32_t i = 0; i < I; ++i) total += item_count[i];
-    bounds.assign(world + 1, I);
-    bounds[0] = 0;
-    int64_t acc = 0;
-    int b = 1;
-    for (int32_t i = 0; i < I && b < world; ++i) {
-        acc += item_count[i];
-        // close block b-1 after item i once it holds its share; keep at least one item per remaining block
-        while (b < world && (acc * world >= total * b || I - (i + 1) <= world - b)) { bounds[b] = i + 1; ++b; }
-    }
-    for (int j = 1; j <= world; ++j) if (bounds[j] < bounds[j - 1]) bounds[j] = bounds[j - 1];
-    bounds[world] = I;
-}
-
-struct DsgdState {
-    std::vector<int32_t> bounds;        // world+1 item block bounds
-    std::vector<int64_t> seg_off;       // world+1 offsets of the COO segments
-    int32_t max_blk = 0;                // rows of the largest item block
+struct DsgdState : ItemBlocks {          // the item blocks and segments of the stream: staging.cuh
     size_t buf_floats = 0;              // floats per rotating buffer: max_blk*ld + max_blk
     LrkBuf<float> qbuf[2];
     int cur = 0;                        // which buffer holds the current block
     int cur_block = 0;                  // item block id currently held
-    LrkBuf<int32_t> d_bounds;
     // LRK_DSGD_TRACE=1: events around every sub-epoch kernel / ring exchange of the last epoch
     std::vector<cudaEvent_t> trace_ev;
     int trace = -1;
@@ -103,19 +45,6 @@ struct DsgdState {
     }
 };
 
-__global__ void flag_bits_kernel(const int* __restrict__ flags, int* __restrict__ bits) {
-    if (threadIdx.x < 3) bits[threadIdx.x] = (flags[0] >> threadIdx.x) & 1;
-}
-__global__ void dsgd_gather_kernel(const uint32_t* __restrict__ perm, const uint64_t* __restrict__ keys_sorted,
-                                   const int32_t* __restrict__ row_of, const int32_t* __restrict__ col,
-                                   const double* __restrict__ val, const int32_t* __restrict__ bounds, int64_t nnz,
-                                   int32_t* __restrict__ su, int32_t* __restrict__ si, float* __restrict__ sr) {
-    const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (t >= nnz) return;
-    const uint32_t e = perm[t];
-    const int b = (int)(keys_sorted[t] >> 58);
-    su[t] = row_of[e]; si[t] = col[e] - bounds[b]; sr[t] = (float)val[e];
-}
 // BPR windows: delta = Q - Qref ; after the all-reduce Q = Qref + sum of all ranks' deltas
 __global__ void dsgd_delta_kernel(const float* __restrict__ q, const float* __restrict__ ref, float* __restrict__ delta, int64_t n) {
     const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -166,197 +95,45 @@ static int dsgd_comm_init(lrk_handle_s* h, int rank, int world, const uint8_t* u
     return LRK_OK;
 }
 
-// local ratings per item block from the local item degrees (one thread per item)
-__global__ void dsgd_block_counts_kernel(const uint32_t* __restrict__ deg, int32_t I, const int32_t* __restrict__ bounds, int world,
-                                         unsigned long long* __restrict__ cnt) {
-    const int32_t i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= I || deg[i] == 0) return;
-    int b = 0;
-    while (b + 1 < world && i >= bounds[b + 1]) ++b;
-    atomicAdd(cnt + b, (unsigned long long)deg[i]);
-}
-__global__ void u32_to_u64_kernel(const uint32_t* __restrict__ in, int32_t n, unsigned long long* __restrict__ out) {
-    const int32_t i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i < n) out[i] = in[i];
-}
-
-// rank-local user block: CSR with U_local rows and GLOBAL item ids.  Everything that walks the nnz entries runs on the device and
-// takes its temporaries from the handle's staging arena (the host only sees O(numItems) and O(world) arrays).
-static int dsgd_set_train_csr(lrk_handle_s* h, int32_t U, int32_t I, const int64_t* rowptr, const int32_t* col, const double* val) {
-    NcclApi* n = nccl_api();
-    cudaStream_t st = h->stream;
-    const int world = h->world;
-    const int64_t nnz = rowptr[U];
-    if (!h->dsgd) h->dsgd.reset(new DsgdState());
+// the rest of lrk_set_train_csr on a rank (stage_train_csr staged the stream and the item blocks)
+static int dsgd_set_train_csr(lrk_handle_s* h) {
     DsgdState* s = h->dsgd.get();
-    h->has_train = false;
+    cudaStream_t st = h->stream;
     int rc;
-    if ((rc = lrk_dev_alloc(h, &h->d_rowptr, (size_t)U + 1))) return rc;
-    if ((rc = lrk_dev_alloc(h, &h->d_col, (size_t)nnz))) return rc;
-    if ((rc = lrk_dev_alloc(h, &h->d_su, (size_t)nnz))) return rc;
-    if ((rc = lrk_dev_alloc(h, &h->d_si, (size_t)nnz))) return rc;
-    if ((rc = lrk_dev_alloc(h, &h->d_sr, (size_t)nnz))) return rc;
-    if ((rc = lrk_dev_alloc(h, &s->d_bounds, (size_t)world + 1))) return rc;
-    if ((rc = lrk_dev_alloc(h, &h->d_item_deg, (size_t)I + 4))) return rc;
-    LRK_CUDA(h, cudaMemcpyAsync(h->d_rowptr, rowptr, sizeof(int64_t) * ((size_t)U + 1), cudaMemcpyHostToDevice, st));
-    if (nnz > 0) LRK_CUDA(h, cudaMemcpyAsync(h->d_col, col, sizeof(int32_t) * (size_t)nnz, cudaMemcpyHostToDevice, st));
-    h->U = U; h->I = I; h->nnz = nnz;
-
-    size_t tmp64 = 0;
-    LRK_CUDA(h, cub::DeviceRadixSort::SortPairs(nullptr, tmp64, (uint64_t*)nullptr, (uint64_t*)nullptr, (uint32_t*)nullptr,
-                                                (uint32_t*)nullptr, (int)std::max<int64_t>(nnz, 1), 0, 64, st));
-    const size_t tmp_bytes = std::max(tmp64, stage_tile_keys_tmp_bytes(I, std::max<int64_t>(nnz, 1)));
-    const size_t nn = (size_t)std::max<int64_t>(nnz, 1);
-    LrkScratch sc;
-    if ((rc = lrk_scratch_begin(h, nn * (8 + 4 + 8 + 8 + 4 * 6) + (size_t)I * (16 + 8) + (size_t)U * world * 20 + tmp_bytes + 80 * 256, &sc))) return rc;
-    double* d_val = sc.take<double>(nn);
-    int32_t* row_of = sc.take<int32_t>(nn);
-    uint64_t *keys = sc.take<uint64_t>(nn), *keys2 = sc.take<uint64_t>(nn);
-    uint32_t *idx = sc.take<uint32_t>(nn), *perm = sc.take<uint32_t>(nn);
-    TileKeyWork w;
-    w.k32 = sc.take<uint32_t>(nn); w.v32 = sc.take<uint32_t>(nn); w.k32_out = sc.take<uint32_t>(nn); w.sorted_e = sc.take<uint32_t>(nn);
-    w.deg = sc.take<uint32_t>((size_t)I); w.item_start = sc.take<uint32_t>((size_t)I);
-    w.runs = sc.take<uint32_t>((size_t)I); w.run_base = sc.take<uint32_t>((size_t)I);
-    w.max_deg = sc.take<uint32_t>(64);
-    w.tmp = sc.take<char>(tmp_bytes); w.tmp_bytes = tmp_bytes;
-    unsigned long long* d_cnt = sc.take<unsigned long long>((size_t)I);
-    unsigned long long* d_small = sc.take<unsigned long long>(128);        // [0,64) block counts, [64] flags
-    if (!d_val || !row_of || !keys || !keys2 || !idx || !perm || !w.k32 || !w.v32 || !w.k32_out || !w.sorted_e || !w.deg || !w.item_start ||
-        !w.runs || !w.run_base || !w.max_deg || !w.tmp || !d_cnt || !d_small)
-        return lrk_fail(h, LRK_ERR_NOMEM, "dsgd_set_train_csr", "scratch arena too small", __FILE__, __LINE__);
-    int* d_flags = reinterpret_cast<int*>(d_small + 64);
-    const int nb = lrk_ceil_div(nn, 256), ib = lrk_ceil_div(I, 256);
-
-    // validate the shard BEFORE anything indexes by column (same checks and messages as the single-GPU path); the flag is
-    // all-reduced so that every rank fails together and nobody is left waiting in a collective
-    LRK_CUDA(h, cudaMemsetAsync(d_small, 0, sizeof(unsigned long long) * 128, st));
-    if (nnz > 0) {
-        LRK_CUDA(h, cudaMemcpyAsync(d_val, val, sizeof(double) * (size_t)nnz, cudaMemcpyHostToDevice, st));
-        coo_rows_kernel<<<nb, 256, 0, st>>>(h->d_rowptr, U, nnz, row_of); LRK_LAUNCH_CHECK(h);
-    }
-    {
-        const int64_t m = nnz > U ? nnz : U;
-        csr_validate_kernel<<<lrk_ceil_div(m, 256), 256, 0, st>>>(h->d_rowptr, h->d_col, U, I, nnz, d_flags); LRK_LAUNCH_CHECK(h);
-        if (nnz > 0) { csr_validate_rows_kernel<<<nb, 256, 0, st>>>(h->d_rowptr, h->d_col, row_of, nnz, d_flags); LRK_LAUNCH_CHECK(h); }
-    }
-    int flags[4] = {0, 0, 0, 0};
-    {   // bit-wise OR across ranks: three counters (one per bit) summed
-        int* d_bits = d_flags + 4;
-        flag_bits_kernel<<<1, 32, 0, st>>>(d_flags, d_bits); LRK_LAUNCH_CHECK(h);
-        LRK_NCCL(h, n->AllReduce(d_bits, d_bits, 3, ncclInt32, ncclSum, (ncclComm_t)h->comm, st));
-        LRK_CUDA(h, cudaMemcpyAsync(flags, d_bits, sizeof(int) * 3, cudaMemcpyDeviceToHost, st));
-        LRK_CUDA(h, cudaStreamSynchronize(st));
-    }
-    if (flags[0]) return lrk_fail(h, LRK_ERR_INVALID, "lrk_set_train_csr", "rowptr is not a monotone prefix sum ending at nnz", __FILE__, __LINE__);
-    if (flags[1]) return lrk_fail(h, LRK_ERR_INVALID, "lrk_set_train_csr", "column index out of range", __FILE__, __LINE__);
-    if (flags[2]) return lrk_fail(h, LRK_ERR_INVALID, "lrk_set_train_csr", "columns must be strictly ascending inside a row", __FILE__, __LINE__);
-
-    // global item popularity -> identical block bounds on every rank (host work is O(numItems))
-    LRK_CUDA(h, cudaMemsetAsync(h->d_item_deg, 0, sizeof(uint32_t) * (size_t)I, st));
-    if (nnz > 0) { item_degree_kernel<<<nb, 256, 0, st>>>(h->d_col, nnz, h->d_item_deg); LRK_LAUNCH_CHECK(h); }
-    u32_to_u64_kernel<<<ib, 256, 0, st>>>(h->d_item_deg, I, d_cnt); LRK_LAUNCH_CHECK(h);
-    LRK_NCCL(h, n->AllReduce(d_cnt, d_cnt, (size_t)I, ncclUint64, ncclSum, (ncclComm_t)h->comm, st));
-    std::vector<int64_t> cnt((size_t)I);
-    LRK_CUDA(h, cudaMemcpyAsync(cnt.data(), d_cnt, sizeof(int64_t) * (size_t)I, cudaMemcpyDeviceToHost, st));
-    LRK_CUDA(h, cudaStreamSynchronize(st));
-    dsgd_item_bounds(cnt.data(), I, world, s->bounds);
-    s->max_blk = 0;
-    for (int b = 0; b < world; ++b) s->max_blk = std::max(s->max_blk, s->bounds[b + 1] - s->bounds[b]);
-    LRK_CUDA(h, cudaMemcpyAsync(s->d_bounds, s->bounds.data(), sizeof(int32_t) * ((size_t)world + 1), cudaMemcpyHostToDevice, st));
-
-    // bucket by item block; inside a block: item-run tiles, then the shuffled rest (staging.cuh, stage_tile_keys)
-    s->seg_off.assign((size_t)world + 1, 0);
-    dsgd_block_counts_kernel<<<ib, 256, 0, st>>>(h->d_item_deg, I, s->d_bounds, world, d_small); LRK_LAUNCH_CHECK(h);
-    h->group.reset();
-    const bool want_group = lrk_use_group_kernel(h) && group_order_supported(U, I, nnz, world);
-    if (nnz > 0 && want_group) {
-        LRK_CUDA(h, cudaMemsetAsync(w.max_deg, 0, sizeof(uint32_t) * 64, st));
-        if ((rc = stage_group_stream(h, h->d_rowptr, h->d_col, row_of, d_val, U, I, nnz, s->d_bounds, world, sgd_group_resident_workers(h),
-                                     h->cfg.seed + 977u * h->rank, sc, w.tmp, tmp_bytes, keys, keys2, idx, perm, h->d_su, h->d_si, h->d_sr, &h->group))) return rc;
-    } else if (nnz > 0) {
-        if ((rc = stage_tile_keys(h, h->d_col, I, nnz, s->d_bounds, world, h->cfg.seed + 977u * h->rank, w, keys, idx))) return rc;
-        size_t tb = tmp_bytes;
-        LRK_CUDA(h, cub::DeviceRadixSort::SortPairs(w.tmp, tb, keys, keys2, idx, perm, (int)nnz, 0, 64, st));
-        dsgd_gather_kernel<<<nb, 256, 0, st>>>(perm, keys2, row_of, h->d_col, d_val, s->d_bounds, nnz, h->d_su, h->d_si, h->d_sr);
-        LRK_LAUNCH_CHECK(h);
-    }
-    unsigned long long small[64];
-    uint32_t md[64] = {0}, last_base = 0, last_runs = 0;
-    if (nnz > 0 && !h->group) {
-        LRK_CUDA(h, cudaMemcpyAsync(&last_base, w.run_base + (I - 1), sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
-        LRK_CUDA(h, cudaMemcpyAsync(&last_runs, w.runs + (I - 1), sizeof(uint32_t), cudaMemcpyDeviceToHost, st));
-    }
-    LRK_CUDA(h, cudaMemcpyAsync(small, d_small, sizeof small, cudaMemcpyDeviceToHost, st));
-    if (nnz > 0) LRK_CUDA(h, cudaMemcpyAsync(md, w.max_deg, sizeof md, cudaMemcpyDeviceToHost, st));
-    LRK_CUDA(h, cudaStreamSynchronize(st));
-    h->run_tiles = (int64_t)last_base + (int64_t)last_runs;
-    h->max_item_deg = 0;
-    for (int b = 0; b < world; ++b) h->max_item_deg = std::max(h->max_item_deg, md[b]);
-    for (int b = 0; b < world; ++b) s->seg_off[(size_t)b + 1] = s->seg_off[(size_t)b] + (int64_t)small[b];
     if (h->cfg.model == LRK_MODEL_BPR) {
         // BPRRecommender.java:48-58 draws numRates samples per iteration, the user uniformly over ALL users: this rank's share is
         // numRates * (its users / all users)
-        double tot[2] = {(double)nnz, (double)U};
-        double* d_tot = reinterpret_cast<double*>(d_cnt);
+        LrkScratch sc;
+        if ((rc = lrk_scratch_begin(h, 256, &sc))) return rc;
+        double tot[2] = {(double)h->nnz, (double)h->U};
+        double* d_tot = sc.take<double>(2);
         LRK_CUDA(h, cudaMemcpyAsync(d_tot, tot, sizeof tot, cudaMemcpyHostToDevice, st));
-        LRK_NCCL(h, n->AllReduce(d_tot, d_tot, 2, ncclFloat64, ncclSum, (ncclComm_t)h->comm, st));
+        LRK_NCCL(h, nccl_api()->AllReduce(d_tot, d_tot, 2, ncclFloat64, ncclSum, (ncclComm_t)h->comm, st));
         LRK_CUDA(h, cudaMemcpyAsync(tot, d_tot, sizeof tot, cudaMemcpyDeviceToHost, st));
         LRK_CUDA(h, cudaStreamSynchronize(st));
-        s->bpr_samples = tot[1] > 0.0 ? (int64_t)(tot[0] * ((double)U / tot[1]) + 0.5) : 0;
+        s->bpr_samples = tot[1] > 0.0 ? (int64_t)(tot[0] * ((double)h->U / tot[1]) + 0.5) : 0;
     }
     s->buf_floats = (size_t)s->max_blk * h->ld + (size_t)s->max_blk;
     s->buf_floats = (s->buf_floats + 3) & ~(size_t)3;                       // float4-copyable
     for (int j = 0; j < 2; ++j) if ((rc = lrk_dev_alloc(h, &s->qbuf[j], s->buf_floats))) return rc;
-    h->has_train = true;
-    topn_tc_invalidate(h);
     return LRK_OK;
 }
 
-// P/bu: the rank's user block; Q/bi: the FULL item factors (identical on every rank)
-static int dsgd_set_factors(lrk_handle_s* h, const double* P, const double* Q, const double* bu, const double* bi, double mu) {
+// the rest of lrk_set_factors on a rank (P/bu: the rank's user block; Q/bi: the FULL item factors, identical on every rank):
+// the rank starts the epoch holding item block `rank`
+static int dsgd_load_ring(lrk_handle_s* h) {
     DsgdState* s = h->dsgd.get();
     cudaStream_t st = h->stream;
-    const int k = h->k, ld = h->ld;
-    const int64_t U = h->U, I = h->I;
-    const bool biased = h->cfg.model == LRK_MODEL_BIASEDMF;
-    int rc;
-    if ((rc = lrk_dev_alloc(h, &h->P64, (size_t)U * k))) return rc;
-    if ((rc = lrk_dev_alloc(h, &h->Q64, (size_t)I * k))) return rc;
-    if ((rc = lrk_dev_alloc(h, &h->P32, (size_t)U * ld))) return rc;
-    if ((rc = lrk_dev_alloc(h, &h->Q32, (size_t)I * ld))) return rc;
-    if ((rc = lrk_dev_alloc(h, &h->bu64, (size_t)U))) return rc;
-    if ((rc = lrk_dev_alloc(h, &h->bi64, (size_t)I))) return rc;
-    if ((rc = lrk_dev_alloc(h, &h->bu32, (size_t)U))) return rc;
-    if ((rc = lrk_dev_alloc(h, &h->bi32, (size_t)I + 4))) return rc;
-    LRK_CUDA(h, cudaMemcpyAsync(h->P64, P, sizeof(double) * (size_t)U * k, cudaMemcpyHostToDevice, st));
-    LRK_CUDA(h, cudaMemcpyAsync(h->Q64, Q, sizeof(double) * (size_t)I * k, cudaMemcpyHostToDevice, st));
-    if (biased) {
-        LRK_CUDA(h, cudaMemcpyAsync(h->bu64, bu, sizeof(double) * (size_t)U, cudaMemcpyHostToDevice, st));
-        LRK_CUDA(h, cudaMemcpyAsync(h->bi64, bi, sizeof(double) * (size_t)I, cudaMemcpyHostToDevice, st));
-    } else {
-        LRK_CUDA(h, cudaMemsetAsync(h->bu64, 0, sizeof(double) * (size_t)U, st));
-        LRK_CUDA(h, cudaMemsetAsync(h->bi64, 0, sizeof(double) * (size_t)I, st));
-    }
-    f64_to_f32_rows_kernel<<<lrk_ceil_div(U * ld, 256), 256, 0, st>>>(h->P64, h->P32, U, k, ld); LRK_LAUNCH_CHECK(h);
-    f64_to_f32_rows_kernel<<<lrk_ceil_div(I * ld, 256), 256, 0, st>>>(h->Q64, h->Q32, I, k, ld); LRK_LAUNCH_CHECK(h);
-    f64_to_f32_rows_kernel<<<lrk_ceil_div(U, 256), 256, 0, st>>>(h->bu64, h->bu32, U, 1, 1); LRK_LAUNCH_CHECK(h);
-    f64_to_f32_rows_kernel<<<lrk_ceil_div(I, 256), 256, 0, st>>>(h->bi64, h->bi32, I, 1, 1); LRK_LAUNCH_CHECK(h);
-    // the rank starts the epoch holding item block `rank`
     const int b = dsgd_block_at(h->rank, h->world, 0);
     const int32_t first = s->bounds[b], rows = s->bounds[b + 1] - first;
     LRK_CUDA(h, cudaMemsetAsync(s->qbuf[0], 0, sizeof(float) * s->buf_floats, st));
     LRK_CUDA(h, cudaMemsetAsync(s->qbuf[1], 0, sizeof(float) * s->buf_floats, st));
     if (rows > 0) {
-        dsgd_pack_block_kernel<<<lrk_ceil_div((int64_t)rows * ld + rows, 256), 256, 0, st>>>(h->Q32, h->bi32, first, rows, ld, s->max_blk, s->qbuf[0]);
+        dsgd_pack_block_kernel<<<lrk_ceil_div((int64_t)rows * h->ld + rows, 256), 256, 0, st>>>(h->Q32, h->bi32, first, rows, h->ld, s->max_blk, s->qbuf[0]);
         LRK_LAUNCH_CHECK(h);
     }
     s->cur = 0; s->cur_block = b;
     s->fused.needs_reset = s->fused.mapped;
-    if (k_lrk_models[h->cfg.model].damped) { int rc_n = refresh_user_norm2(h, false); if (rc_n) return rc_n; }
-    LRK_CUDA(h, cudaStreamSynchronize(st));
-    h->prev_loss = -1.0; h->conc_div = 1; h->good_epochs = 0; h->epochs_done = 0;
-    h->mu = mu; h->has_factors = true; h->f64_valid = false;
-    topn_tc_invalidate(h);
     return LRK_OK;
 }
 

@@ -35,29 +35,20 @@ static int gbpr_stage(lrk_handle_s* h) {
     if ((rc = lrk_dev_alloc(h, &g->d_colptr, (size_t)I + 1))) return rc;
     if ((rc = lrk_dev_alloc(h, &g->d_cusers, (size_t)nnz))) return rc;
     if (nnz == 0) { LRK_CUDA(h, cudaMemsetAsync(g->d_colptr, 0, sizeof(int64_t) * ((size_t)I + 1), st)); return LRK_OK; }
-    size_t tb_sort = 0, tb_scan = 0;
-    int end_bit = 1;
-    while (end_bit < 32 && ((int64_t)1 << end_bit) < (int64_t)I) ++end_bit;
-    LRK_CUDA(h, cub::DeviceRadixSort::SortPairs(nullptr, tb_sort, (uint32_t*)nullptr, (uint32_t*)nullptr, (int32_t*)nullptr, (int32_t*)nullptr, (int)nnz, 0, end_bit, st));
-    LRK_CUDA(h, cub::DeviceScan::ExclusiveSum(nullptr, tb_scan, (uint32_t*)nullptr, (uint32_t*)nullptr, (int)I, st));
-    const size_t tb = std::max(tb_sort, tb_scan) + 256;
+    const size_t tb = by_item_order_tmp_bytes(I, nnz);
     LrkScratch sc;
-    if ((rc = lrk_scratch_begin(h, (size_t)nnz * 16 + (size_t)I * 8 + tb + 16 * 256, &sc))) return rc;
-    uint32_t *k_in = sc.take<uint32_t>((size_t)nnz), *k_out = sc.take<uint32_t>((size_t)nnz);
+    if ((rc = lrk_scratch_begin(h, (size_t)nnz * 20 + (size_t)I * 8 + tb + 16 * 256, &sc))) return rc;
+    uint32_t *keys = sc.take<uint32_t>((size_t)nnz), *keys_out = sc.take<uint32_t>((size_t)nnz), *ids = sc.take<uint32_t>((size_t)nnz);
+    uint32_t* perm = sc.take<uint32_t>((size_t)nnz);
     int32_t* rows = sc.take<int32_t>((size_t)nnz);
     uint32_t *deg = sc.take<uint32_t>((size_t)I), *deg_ex = sc.take<uint32_t>((size_t)I);
     void* tmp = sc.take<char>(tb);
-    if (!k_in || !k_out || !rows || !deg || !deg_ex || !tmp) return lrk_fail(h, LRK_ERR_NOMEM, "gbpr_stage", "scratch arena too small", __FILE__, __LINE__);
+    if (!keys || !keys_out || !ids || !perm || !rows || !deg || !deg_ex || !tmp) return lrk_fail(h, LRK_ERR_NOMEM, "gbpr_stage", "scratch arena too small", __FILE__, __LINE__);
     const int nb = lrk_ceil_div(nnz, 256);
     coo_rows_kernel<<<nb, 256, 0, st>>>(h->d_rowptr, U, nnz, rows); LRK_LAUNCH_CHECK(h);
-    LRK_CUDA(h, cudaMemcpyAsync(k_in, h->d_col, sizeof(uint32_t) * (size_t)nnz, cudaMemcpyDeviceToDevice, st));
-    LRK_CUDA(h, cudaMemsetAsync(deg, 0, sizeof(uint32_t) * (size_t)I, st));
-    item_degree_kernel<<<nb, 256, 0, st>>>(h->d_col, nnz, deg); LRK_LAUNCH_CHECK(h);
-    size_t t1 = tb;
-    LRK_CUDA(h, cub::DeviceScan::ExclusiveSum(tmp, t1, deg, deg_ex, (int)I, st));
-    gbpr_colptr_kernel<<<lrk_ceil_div(I, 256), 256, 0, st>>>(deg_ex, deg, I, g->d_colptr); LRK_LAUNCH_CHECK(h);
-    t1 = tb;
-    LRK_CUDA(h, cub::DeviceRadixSort::SortPairs(tmp, t1, k_in, k_out, rows, g->d_cusers.ptr, (int)nnz, 0, end_bit, st));   // stable: users ascending
+    if ((rc = by_item_order(h, h->d_col, I, nnz, deg, deg_ex, perm, keys, keys_out, ids, tmp, tb))) return rc;
+    csc_colptr_kernel<<<lrk_ceil_div(I, 256), 256, 0, st>>>(deg_ex, deg, I, g->d_colptr); LRK_LAUNCH_CHECK(h);
+    csc_rows_kernel<<<nb, 256, 0, st>>>(perm, rows, nnz, g->d_cusers); LRK_LAUNCH_CHECK(h);   // users ascending inside an item
     LRK_CUDA(h, cudaStreamSynchronize(st));
     return LRK_OK;
 }
@@ -300,25 +291,15 @@ int lrk_set_train_csr(lrk_handle_t h, int32_t U, int32_t I, const int64_t* rowpt
     const int64_t nnz = rowptr[U];
     LRK_REQUIRE(h, nnz >= 0 && nnz < (int64_t)0x7fffffffLL, "nnz out of range (the staging sorts take an int count: at most 2^31 - 1 train entries per handle)");
     LRK_CUDA(h, cudaSetDevice(h->cfg.device));
-    if (h->world > 1) return dsgd_set_train_csr(h, U, I, rowptr, col, val);
     cudaStream_t st = h->stream;
-    h->has_train = false;
-    int rc;
-    if ((rc = lrk_dev_alloc(h, &h->d_rowptr, (size_t)U + 1))) return rc;
-    if ((rc = lrk_dev_alloc(h, &h->d_col, (size_t)nnz))) return rc;
-    if ((rc = lrk_dev_alloc(h, &h->d_su, (size_t)nnz))) return rc;
-    if ((rc = lrk_dev_alloc(h, &h->d_si, (size_t)nnz))) return rc;
-    if ((rc = lrk_dev_alloc(h, &h->d_sr, (size_t)nnz))) return rc;
-    LRK_CUDA(h, cudaMemcpyAsync(h->d_rowptr, rowptr, sizeof(int64_t) * ((size_t)U + 1), cudaMemcpyHostToDevice, st));
-    LRK_CUDA(h, cudaMemcpyAsync(h->d_col, col, sizeof(int32_t) * (size_t)nnz, cudaMemcpyHostToDevice, st));
-    h->U = U; h->I = I; h->nnz = nnz;
     // BiasedMF / PMF in atomic mode with LRK_SGD_GROUP=1 train with the user-group kernel over a unit-ordered stream (sgd_group.cuh);
     // everything else keeps the item-run-tile stream of sgd.cuh
     h->group.reset();
-    const bool want_group = lrk_use_group_kernel(h) && group_order_supported(U, I, nnz, 1);
-    rc = stage_coo_from_csr(h, h->d_rowptr, h->d_col, val, U, I, nnz, h->d_su, h->d_si, h->d_sr, /*validate=*/true,
-                            want_group ? sgd_group_resident_workers(h) : 0, &h->group);
+    const bool want_group = lrk_use_group_kernel(h) && group_order_supported(U, I, nnz, h->world);
+    if (h->world > 1 && !h->dsgd) h->dsgd.reset(new DsgdState());
+    int rc = stage_train_csr(h, U, I, rowptr, col, val, want_group ? sgd_group_resident_workers(h) : 0, h->dsgd.get());
     if (rc) return rc;
+    if (h->world > 1 && (rc = dsgd_set_train_csr(h))) return rc;
     if (h->cfg.model == LRK_MODEL_RANKSGD && nnz > 0) {
         // sampling table of the negatives: inclusive prefix sums of the item degrees (RankSGDRecommender.java:47-57)
         if ((rc = lrk_dev_alloc(h, &h->d_item_cum, (size_t)I))) return rc;
@@ -355,7 +336,6 @@ int lrk_set_factors(lrk_handle_t h, const double* P, const double* Q, const doub
     // bit for bit with b_u = mu = 0, whatever global mean or user biases the caller passes
     if (h->cfg.model == LRK_MODEL_GBPR) { bu = nullptr; mu = 0.0; }
     LRK_CUDA(h, cudaSetDevice(h->cfg.device));
-    if (h->world > 1) return dsgd_set_factors(h, P, Q, bu, bi, mu);
     cudaStream_t st = h->stream;
     const int k = h->k, ld = h->ld;
     const int64_t U = h->U, I = h->I;
@@ -378,10 +358,11 @@ int lrk_set_factors(lrk_handle_t h, const double* P, const double* Q, const doub
     f64_to_f32_rows_kernel<<<lrk_ceil_div(I * ld, 256), 256, 0, st>>>(h->Q64, h->Q32, I, k, ld); LRK_LAUNCH_CHECK(h);
     f64_to_f32_rows_kernel<<<lrk_ceil_div(U, 256), 256, 0, st>>>(h->bu64, h->bu32, U, 1, 1); LRK_LAUNCH_CHECK(h);
     f64_to_f32_rows_kernel<<<lrk_ceil_div(I, 256), 256, 0, st>>>(h->bi64, h->bi32, I, 1, 1); LRK_LAUNCH_CHECK(h);
-    if (m.damped && (rc = refresh_user_norm2(h, true))) return rc;
+    if (m.damped && (rc = refresh_user_norm2(h, false))) return rc;
     if (h->aobpr) h->aobpr->count = 0;                 // a new trainModel(): countIter starts at 0 (AoBPRRecommender.java:88)
-    if (h->h_pnorm2) { h->pnorm2_prev = 0.f; h->pnorm2_host = *h->h_pnorm2; }
+    if (h->world > 1 && (rc = dsgd_load_ring(h))) return rc;
     LRK_CUDA(h, cudaStreamSynchronize(st));   // host buffers may be reused by the caller on return
+    if (h->h_pnorm2) { h->pnorm2_prev = 0.f; h->pnorm2_host = *h->h_pnorm2; }
     h->mu = mu;
     h->has_factors = true;
     h->f64_valid = true;

@@ -208,12 +208,6 @@ __global__ void gbpr_apply_kernel(float* __restrict__ dst, const float* __restri
     if (t < n) dst[t] += acc[t];
 }
 // train CSC from the CSR: (item, user) pairs sorted by item (stable: users ascending inside an item)
-__global__ void gbpr_colptr_kernel(const uint32_t* __restrict__ deg_excl, const uint32_t* __restrict__ deg, int32_t I, int64_t* __restrict__ colptr) {
-    const int32_t i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i < I) colptr[i] = (int64_t)deg_excl[i];
-    if (i == I - 1) colptr[I] = (int64_t)deg_excl[i] + (int64_t)deg[i];
-}
-
 struct GbprState {
     LrkBuf<int64_t> d_colptr;
     LrkBuf<int32_t> d_cusers;

@@ -1,4 +1,5 @@
-"""The DSGD stratum schedule (host logic) -- the same pure functions as librec_b200/csrc/dsgd.cuh.
+"""The DSGD stratum schedule (host logic) -- the same pure functions as librec_b200/csrc/dsgd.cuh and staging.cuh (item blocks,
+stream order).
 
 World of G ranks, one per GPU.  Rank g owns a user shard for the whole run.  Items are cut into G
 contiguous blocks balanced by global rating count.  In sub-epoch s rank g trains on item block
@@ -41,6 +42,50 @@ def item_bounds(item_count, world):
             bounds[j] = bounds[j - 1]
     bounds[world] = I
     return bounds
+
+
+RUN_MIN_DEGREE = 128          # LRK_RUN_MIN_DEGREE: items with at least this many ratings in a block shard get run tiles
+_M64 = (1 << 64) - 1
+
+
+def _hash32(x):
+    """lrk_hash32 (csrc/staging.cuh): the splitmix64 finaliser, high word; x: uint64 array"""
+    with np.errstate(over="ignore"):
+        x = x + np.uint64(0x9E3779B97F4A7C15)
+        x = (x ^ (x >> np.uint64(30))) * np.uint64(0xBF58476D1CE4E5B9)
+        x = (x ^ (x >> np.uint64(27))) * np.uint64(0x94D049BB133111EB)
+        x = x ^ (x >> np.uint64(31))
+    return x >> np.uint64(32)
+
+
+def stream_order(rowptr, col, val, I, seed, bounds=None):
+    """The staged COO stream of the SGD epoch (csrc/staging.cuh, stage_tile_keys) -> (su, si, sr, run_tiles, max_item_deg).
+    Per item block (one block without bounds, otherwise the DSGD item blocks): [item-run tiles] [the rest, shuffled], i.e. one
+    stable sort of entry e on  key = block:6 | is_rest:1 | hash:32 | tile or entry id:25.  An item with deg >= RUN_MIN_DEGREE
+    gives deg // 32 tiles of 32 ratings, in CSR order; its remaining ratings join the rest.  seed: the handle's seed
+    (+ 977 * rank on a DSGD rank).  With bounds the item ids of the stream are local to their block."""
+    rowptr, col = np.asarray(rowptr, np.int64), np.asarray(col, np.int64)
+    n = col.shape[0]
+    row_of = np.repeat(np.arange(rowptr.shape[0] - 1), np.diff(rowptr))
+    deg = np.bincount(col, minlength=I)
+    runs = np.where(deg >= RUN_MIN_DEGREE, deg // 32, 0)
+    run_base = np.cumsum(runs) - runs
+    order = np.argsort(col, kind="stable")                          # the by-item order
+    rank = np.empty(n, np.int64)
+    rank[order] = np.arange(n) - (np.cumsum(deg) - deg)[col[order]]
+    blk = np.searchsorted(np.asarray(bounds[1:-1]), col, side="right") if bounds is not None else np.zeros(n, np.int64)
+    e = np.arange(n, dtype=np.uint64)
+    tile = (run_base[col] + rank // 32).astype(np.uint64)
+    in_run = rank < 32 * runs[col]
+    m_tile, m_rest = np.uint64((seed * 0xA24BAED4963EE407) & _M64), np.uint64((seed * 0xD6E8FEB86659FD93) & _M64)
+    low25 = np.uint64(0x1FFFFFF)
+    key_tile = (_hash32(tile ^ m_tile) << np.uint64(25)) | (tile & low25)
+    key_rest = np.uint64(1 << 57) | (_hash32(e ^ m_rest) << np.uint64(25)) | (e & low25)
+    key = (blk.astype(np.uint64) << np.uint64(58)) | np.where(in_run, key_tile, key_rest)
+    perm = np.argsort(key, kind="stable")
+    si = col[perm] - (np.asarray(bounds, np.int64)[blk[perm]] if bounds is not None else 0)
+    return (row_of[perm].astype(np.int32), si.astype(np.int32), np.asarray(val, np.float64)[perm].astype(np.float32),
+            int(runs.sum()), int(deg.max()) if n else 0)
 
 
 def segments(col, bounds):

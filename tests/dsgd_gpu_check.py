@@ -5,7 +5,8 @@
 (3) BPR across ranks (every rank keeps the full item matrix and samples like the reference over the whole catalogue; the change
     of the item matrix is all-reduced 8 times per epoch, csrc/dsgd.cuh dsgd_bpr_epoch): Precision@10 on the binarised C1 split at
     least 90 % of the single-GPU BPR of the same library (r01's stratified sampler reached 0.225 / 0.142 on 2 / 8 ranks vs 0.325).
-(4) an invalid CSR shard on one rank fails on every rank; (5) BPR on a catalogue as small as the world size does not hang.
+(4) an invalid CSR shard on one rank fails on every rank; (5) BPR on a catalogue as small as the world size does not hang;
+(6) every rank's staged stream and lrk_stage_stats equal the restatement of librec_b200/dsgd_plan.py (stream_order).
 Prints "DSGD-CHECK OK" on rank 0.  `--fused` runs the same checks through the experimental fused epoch kernel.
 """
 import json
@@ -98,7 +99,27 @@ def main():
     ok5 = bool(np.isfinite(l5).all())
     if rank == 0:
         print("invalid shard fails everywhere: %s   width-1 BPR blocks are skipped: %s (losses %s)" % (ok4, ok5, l5))
-    ok2 = ok2 and ok4 and ok5
+    # (6) the rank's C1 shard is staged in the order stream_order restates: item blocks from the GLOBAL item counts, the block in
+    #     the top key bits, block-local item ids, the handle's seed + 977 * rank
+    from librec_b200.dsgd_plan import item_bounds, stream_order
+    h6 = capi.Handle(capi.MODEL_BIASEDMF, 8, device=local, seed=1)
+    uid = [capi.comm_unique_id() if rank == 0 else None]
+    dist.broadcast_object_list(uid, src=0)
+    h6.comm_init(rank, world, uid[0])
+    h6.set_train_csr(mine.U, mine.I, mine.rowptr, mine.col, mine.val)
+    bounds = item_bounds(np.bincount(tr.col, minlength=tr.I), world)
+    su, si, sr, run_tiles, max_deg = stream_order(mine.rowptr, mine.col, mine.val, tr.I, 1 + 977 * rank, bounds)
+    gu, gi, gr, _ = h6.debug_stream(mine.col.shape[0])
+    st6 = h6.stage_stats()
+    h6.close()
+    ok6 = (np.array_equal(gu, su) and np.array_equal(gi, si) and np.array_equal(gr.view(np.int32), sr.view(np.int32))
+           and (st6["ratings"], st6["run_tile_ratings"], st6["max_item_degree"]) == (mine.col.shape[0], 32 * run_tiles, max_deg))
+    all6 = [None] * world
+    dist.all_gather_object(all6, bool(ok6))
+    ok6 = all(all6)
+    if rank == 0:
+        print("staged stream of every rank = stream_order: %s (%s; rank 0: %d run-tile ratings)" % (ok6, all6, 32 * run_tiles))
+    ok2 = ok2 and ok4 and ok5 and ok6
     if rank == 0:
         print("conflict-free:", r1)
         print("C1 DSGD world=%d:" % world, r2)
