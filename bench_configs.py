@@ -1,6 +1,8 @@
 #!/usr/bin/env python
 """Secondary measurements on one B200 for the BASELINE.json configs that bench.py does not headline:
   C3: BPR k=128 SGD epoch (samples/s) on the synthetic ML-20M shape (implicit feedback, device-side sampling)
+  BPR reference order (--only bprref): k=10 and k=128 on the binarised ML-20M shape, bit-identical to the StrictMath epoch of
+  tests/bpr_strict_reference.cpp
   N3 (--only n3): RankSGD k=10 (ranksgd-test.properties) on the ML-20M shape, one update per train entry
   C4: PMF k=128 SGD epoch (updates/s) on the synthetic Netflix shape (480 189 x 17 770, 100 480 507 ratings); under torchrun
       (N ranks) the users are split into N contiguous blocks and the epoch runs as DSGD (strong scaling of the one data set)
@@ -143,6 +145,62 @@ def run_reference_order(name, model_name, shape, k, lr, reg, reg_b):
                       "schedule_build_s": t_stage, "max_item_degree": int(np.bincount(d["col"], minlength=I).max()), "losses": losses}), flush=True)
 
 
+def _chain_length(U, trip):
+    """longest dependency chain of an epoch's samples: a sample follows the previous ones that touched its user or either item"""
+    lv_u, lv_i = [0] * U, {}
+    longest = 0
+    for u, i, j in trip.tolist():
+        lv = max(lv_u[u], lv_i.get(i, 0), lv_i.get(j, 0)) + 1
+        lv_u[u] = lv_i[i] = lv_i[j] = lv
+        longest = max(longest, lv)
+    return longest
+
+
+def run_bpr_reference_order(k):
+    """BPR in reference order (csrc/sgd_bpr_exact.cuh) on the binarised ML-20M shape: one epoch timed after a warm-up epoch, both
+    compared bit for bit with the StrictMath epoch of tests/bpr_strict_reference.cpp run from the same state on one CPU core"""
+    import subprocess
+    import time
+    from librec_b200 import capi, synth
+    sys.path.insert(0, os.path.join(ROOT, "tests"))
+    import bpr_strict
+    L = bpr_strict.lib()
+    card = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit", "--format=csv,noheader"], stdout=subprocess.PIPE,
+                          text=True).stdout.strip().splitlines()[0]
+    d = synth.make_ratings("ml-20m", binary=True)
+    U, I, nnz = d["U"], d["I"], int(d["rowptr"][-1])
+    P, Q, _, _ = synth.init_factors(U, I, k, 11, False)
+    lr, reg = 0.01, 0.01                                                   # bpr-test.properties
+    with capi.Handle(capi.MODEL_BPR, k, seed=1, update_mode=capi.UPDATE_REFERENCE_ORDER) as h:
+        h.set_train_csr(U, I, d["rowptr"], d["col"], d["val"])
+        h.set_factors(P, Q)
+        s0 = int(h.get_matrix("jdk.random.state", (1,))[0])
+        h.sgd_epoch(lr, reg, reg, 0.0, 1)                                 # warm-up
+        warm_ms = h.last_epoch_ms()
+        h.synchronize()
+        t0 = time.perf_counter()
+        trip = h.bpr_peek_samples(2, 0, nnz)                              # the draw stage alone, plus the copy of the triples
+        draw_ms = (time.perf_counter() - t0) * 1e3
+        h.sgd_epoch(lr, reg, reg, 0.0, 2)
+        ms = h.last_epoch_ms()
+        gP, gQ, _, _ = h.get_factors()
+        gs = int(h.get_matrix("jdk.random.state", (1,))[0])
+    L.lro_set_jrandom_state(s0)
+    oP, oQ, oms = P.copy(), Q.copy(), []
+    for _ in range(2):
+        t0 = time.perf_counter()
+        L.lro_bpr_epoch_strict(U, I, d["rowptr"], d["col"], k, oP, oQ, lr, reg, reg, nnz, None, None)
+        oms.append((time.perf_counter() - t0) * 1e3)
+    same = bool(np.array_equal(gP.view(np.int64), oP.view(np.int64)) and np.array_equal(gQ.view(np.int64), oQ.view(np.int64))
+                and gs == L.lro_jrandom_state())
+    print(json.dumps({"config": "BPR-reforder k=%d" % k, "mode": "LRK_UPDATE_REFERENCE_ORDER (BPR: java.util.Random stream, fp64, bit-identical)",
+                      "metric": "BPR samples/s", "value": nnz / (ms * 1e-3), "unit": "samples/s", "n_gpus": 1, "card": card,
+                      "ms_per_epoch": ms, "warmup_epoch_ms": warm_ms, "draw_stage_and_copy_ms": draw_ms, "chain_length": _chain_length(U, trip),
+                      "oracle_one_core_ms_per_epoch": oms, "speedup_vs_oracle": oms[1] / ms, "bit_identical_to_oracle": same,
+                      "workload": "bpr k=%d, synthetic binarised ml-20m shape (%d x %d, %d samples per epoch), lr %g reg %g" % (k, U, I, nnz, lr, reg)}),
+          flush=True)
+
+
 def run_svdpp(steps, warmup, oracle_epochs=2):
     """N3: SVD++ (svdpp-test.properties: k=20, lr 0.002, reg 0.01) on the ML-20M shape; the oracle's sequential loop runs the first
     epochs beside it so that the loss curve at full concurrency is seen next to the reference's"""
@@ -251,6 +309,9 @@ if __name__ == "__main__":
         run_reference_order("C2-reforder", "biasedmf", "ml-20m", 64, 0.002, 0.01, 0.01)
         run_reference_order("C4p-reforder", "pmf", "netflix-10m", 128, 0.01, 0.08, 0.0)
         run_reference_order("C4-reforder", "pmf", "netflix", 128, 0.01, 0.08, 0.0)
+    if a.only == "bprref":
+        run_bpr_reference_order(10)
+        run_bpr_reference_order(128)
     if a.only == "aobpr":
         run("N3-AoBPR", "aobpr", "ml-20m", 10, 0.01, 0.01, a.steps, a.warmup)       # aobpr-test-like: lambda 0.05 * numItems
     if a.only == "svdpp":

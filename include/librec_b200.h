@@ -89,7 +89,12 @@ typedef enum {
     LRK_UPDATE_HOGWILD = 1, /* plain racy read-modify-write stores                                      */
     /* parity mode: the reference's sequential CSR-order walk executed as a dependency wavefront in
      * fp64 with Java's operation order -- learned factors are bit-identical to the reference
-     * arithmetic; throughput is bounded by the longest dependency chain (BiasedMF / PMF only) */
+     * arithmetic; throughput is bounded by the longest dependency chain.  BiasedMF, PMF and BPR.
+     * BPR: each epoch draws numRates samples from the reference's java.util.Random state (Randoms.r, see
+     * "jdk.random.state" under lrk_set_matrix) exactly as BPRRecommender.java:54-67 does, and applies them in
+     * sample order; Maths.logistic is evaluated with StrictMath.exp (fdlibm), so the factors and the generator state
+     * after the epoch equal a JVM's whose Math.exp is StrictMath.exp.  Single GPU, fp64 masters as the working set,
+     * no rollback safeguard; the reported loss may differ from the sequential sum in its last bits. */
     LRK_UPDATE_REFERENCE_ORDER = 2
 } lrk_update_mode;
 
@@ -163,7 +168,12 @@ LRK_API int lrk_set_param(lrk_handle_t h, const char* name, double value);
 
 /* model matrices beyond P / Q / biases, row-major doubles like lrk_set_factors (call after it):
  *   "svdpp.y"  impItemFactors, numItems x numFactors (SVDPlusPlusRecommender.java:55-56)
- *   "eals.confidences"  confidences, numItems doubles (EALSRecommender.java:50,65-83); needs only lrk_set_train_csr before it */
+ *   "eals.confidences"  confidences, numItems doubles (EALSRecommender.java:50,65-83); needs only lrk_set_train_csr before it
+ *   "jdk.random.state"  BPR in LRK_UPDATE_REFERENCE_ORDER only: 1 double, the 48-bit state of Randoms.r (java.util.Random.seed,
+ *                       math/algorithm/Randoms.java:31) as an exact integer in [0, 2^48).  Set it before the first epoch and read it
+ *                       after the last, so that the caller's generator continues where the epochs left it.  Defaults to
+ *                       new Random(cfg.seed)'s scrambled seed; lrk_set_train_csr and lrk_set_factors leave it alone.  Any time,
+ *                       no ordering with the other calls. */
 LRK_API int lrk_set_matrix(lrk_handle_t h, const char* name, const double* values);
 LRK_API int lrk_get_matrix(lrk_handle_t h, const char* name, double* values);
 
@@ -172,7 +182,7 @@ LRK_API int lrk_get_matrix(lrk_handle_t h, const char* name, double* values);
  *   BiasedMFRecommender.java:68-100, PMFSimilarityRecommender.java:59-90, BPRRecommender.java:48-93.
  * lr/reg_u/reg_i are the float fields of MatrixFactorizationRecommender.java:16,54,59; reg_b is the
  * double regBias (BiasedMFRecommender.java:36; ignored unless BIASEDMF).  epoch_idx is the 1-based
- * iteration number (selects the BPR sample stream).  *loss_out receives the epoch loss with the
+ * iteration number (selects the BPR sample stream; reference-order BPR continues its java.util.Random state instead).  *loss_out receives the epoch loss with the
  * reference's definition (0.5 * (sum e^2 + reg terms); BPR: sum -ln sigma(x) + reg terms, no 0.5),
  * so isConverged()/updateLRate() stay on the caller's side.  Returns LRK_ERR_DIVERGED (and still
  * writes *loss_out) when the loss is NaN/Inf. */
@@ -204,7 +214,9 @@ LRK_API int lrk_sgd_safeguard_state(lrk_handle_t h, int32_t* conc_div, int64_t* 
 /* number of kernels this handle has launched since creation */
 LRK_API int lrk_launch_count(lrk_handle_t h, uint64_t* out);
 /* debug / test aid: the (user, positive item, negative item) triples that BPR epoch `epoch_idx`
- * draws for samples [first, first+n) -- out is int32[3*n]; GBPR: int32[11*n] = {u, i, j, the group's users (8 slots, -1 padded)}. */
+ * draws for samples [first, first+n) -- out is int32[3*n]; GBPR: int32[11*n] = {u, i, j, the group's users (8 slots, -1 padded)}.
+ * BPR in LRK_UPDATE_REFERENCE_ORDER: samples [first, first+n) of the NEXT epoch, drawn from the current "jdk.random.state",
+ * which the call does not advance (first + n may exceed numRates: the stream continues); epoch_idx is ignored. */
 LRK_API int lrk_bpr_peek_samples(lrk_handle_t h, int32_t epoch_idx, int64_t first, int64_t n, int32_t* out);
 
 /* ---- prediction --------------------------------------------------------------------- */

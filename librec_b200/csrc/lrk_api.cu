@@ -6,6 +6,7 @@
 #include "staging_group.cuh"
 #include "sgd_group.cuh"
 #include "sgd_exact.cuh"
+#include "sgd_bpr_exact.cuh"
 #include "sgd_gbpr.cuh"
 #include "sgd_svdpp.cuh"
 #include "sgd_aobpr.cuh"
@@ -217,8 +218,8 @@ int lrk_create(const lrk_config_t* cfg, lrk_handle_t* out) {
         return lrk_fail(nullptr, LRK_ERR_INVALID, "lrk_create", "WRMF on the device needs rec.factor.number <= 112 (the Gauss-Jordan step lives in shared memory)", __FILE__, __LINE__);
     if (cfg->update_mode < LRK_UPDATE_ATOMIC || cfg->update_mode > LRK_UPDATE_REFERENCE_ORDER)
         return lrk_fail(nullptr, LRK_ERR_INVALID, "lrk_create", "unknown update_mode", __FILE__, __LINE__);
-    if (cfg->update_mode == LRK_UPDATE_REFERENCE_ORDER && !k_lrk_models[cfg->model].rating)
-        return lrk_fail(nullptr, LRK_ERR_INVALID, "lrk_create", "reference-order mode covers BiasedMF and PMF", __FILE__, __LINE__);
+    if (cfg->update_mode == LRK_UPDATE_REFERENCE_ORDER && !k_lrk_models[cfg->model].rating && cfg->model != LRK_MODEL_BPR)
+        return lrk_fail(nullptr, LRK_ERR_INVALID, "lrk_create", "reference-order mode covers BiasedMF, PMF and BPR", __FILE__, __LINE__);
     int ndev = 0;
     LRK_CUDA(nullptr, cudaGetDeviceCount(&ndev));
     if (cfg->device < 0 || cfg->device >= ndev)
@@ -247,6 +248,11 @@ int lrk_create(const lrk_config_t* cfg, lrk_handle_t* out) {
         if (cudaEventCreate(&h->ev0) != cudaSuccess || cudaEventCreate(&h->ev1) != cudaSuccess) { rc = LRK_ERR_CUDA; break; }
         if (lrk_dev_alloc(h, &h->d_loss, 8) != LRK_OK) { rc = LRK_ERR_NOMEM; break; }
         if (cudaMallocHost((void**)&h->h_loss, 64) != cudaSuccess) { rc = LRK_ERR_NOMEM; break; }
+        if (cfg->model == LRK_MODEL_BPR && cfg->update_mode == LRK_UPDATE_REFERENCE_ORDER) {
+            h->bprref.reset(new (std::nothrow) BprRefState());
+            if (!h->bprref) { rc = LRK_ERR_NOMEM; break; }
+            h->bprref->jstate = (cfg->seed ^ LRK_JR_MULT) & LRK_JR_MASK;              // new Random(seed)
+        }
     } while (0);
     if (rc != LRK_OK) {
         lrk_fail(nullptr, rc, "lrk_create", cudaGetErrorString(cudaGetLastError()), __FILE__, __LINE__);
@@ -311,7 +317,8 @@ int lrk_set_train_csr(lrk_handle_t h, int32_t U, int32_t I, const int64_t* rowpt
         LRK_CUDA(h, cudaStreamSynchronize(st));
         h->launches++;
     }
-    if (h->cfg.update_mode == LRK_UPDATE_REFERENCE_ORDER) {
+    if (h->bprref) bpr_ref_stage(h->bprref.get(), U, I, rowptr);
+    else if (h->cfg.update_mode == LRK_UPDATE_REFERENCE_ORDER) {
         h->exact.reset();
         if ((rc = exact_build_schedule(h, &h->exact, U, I, rowptr, col, val))) return rc;
     }
@@ -421,6 +428,12 @@ int lrk_sgd_epoch(lrk_handle_t h, float lr, float reg_u, float reg_i, double reg
         // fp64 masters are the working set in this mode
         int rc = refresh_masters(h);
         if (rc) return rc;
+        if (h->bprref) {
+            int64_t end = 0;
+            e.enqueue = [&](int) { return bpr_ref_epoch(h, h->bprref.get(), lr, reg_u, reg_i, &end); };
+            e.after_sync = [&] { return bpr_ref_finish(h, h->bprref.get(), end); };
+            return lrk_epoch(h, e, loss_out);
+        }
         e.enqueue = [&](int) { return h->nnz > 0 ? exact_epoch(h, h->exact.get(), lr, reg_u, reg_i, reg_b) : (int)LRK_OK; };
         return lrk_epoch(h, e, loss_out);
     }
@@ -508,6 +521,12 @@ int lrk_set_param(lrk_handle_t h, const char* name, double value) {
 int lrk_set_matrix(lrk_handle_t h, const char* name, const double* values) {
     LRK_REQUIRE(h, h != nullptr && name != nullptr && values != nullptr, "NULL argument");
     LRK_NOT_MULTI(h, "lrk_set_matrix");
+    if (!strcmp(name, "jdk.random.state") && h->bprref) {
+        const double v = values[0];
+        LRK_REQUIRE(h, v >= 0.0 && v < 281474976710656.0 && v == std::floor(v), "jdk.random.state must be an integer in [0, 2^48)");
+        h->bprref->jstate = (uint64_t)v;
+        return LRK_OK;
+    }
     if (!strcmp(name, "eals.confidences") && h->cfg.model == LRK_MODEL_EALS) {
         LRK_REQUIRE(h, h->has_train, "call lrk_set_train_csr first (it fixes numItems)");
         LRK_CUDA(h, cudaSetDevice(h->cfg.device));
@@ -540,6 +559,10 @@ int lrk_set_matrix(lrk_handle_t h, const char* name, const double* values) {
 int lrk_get_matrix(lrk_handle_t h, const char* name, double* values) {
     LRK_REQUIRE(h, h != nullptr && name != nullptr && values != nullptr, "NULL argument");
     LRK_NOT_MULTI(h, "lrk_get_matrix");
+    if (!strcmp(name, "jdk.random.state") && h->bprref) {
+        values[0] = (double)h->bprref->jstate;          // < 2^48: exact
+        return LRK_OK;
+    }
     if (!strcmp(name, "eals.confidences") && h->cfg.model == LRK_MODEL_EALS) {
         AlsState* a = h->als.get();
         LRK_REQUIRE(h, a != nullptr && a->has_conf, "matrix not set");
@@ -638,6 +661,18 @@ int lrk_bpr_peek_samples(lrk_handle_t h, int32_t epoch_idx, int64_t first, int64
     LRK_REQUIRE(h, h->world == 1, "not available in DSGD mode");
     LRK_CUDA(h, cudaSetDevice(h->cfg.device));
     if (n == 0) return LRK_OK;
+    if (h->bprref) {                                    // the next epoch's samples from the current generator state, which stays
+        LrkScratch sc;
+        int rc;
+        if ((rc = lrk_scratch_begin(h, sizeof(int32_t) * 3 * (size_t)n + 256, &sc))) return rc;
+        int32_t* d_out = sc.take<int32_t>(3 * (size_t)n);
+        if (!d_out) return lrk_fail(h, LRK_ERR_NOMEM, "lrk_bpr_peek_samples", "scratch arena too small", __FILE__, __LINE__);
+        int64_t end = 0;
+        if ((rc = bpr_ref_draw(h, h->bprref.get(), first, first + n, d_out, &end))) return rc;
+        LRK_CUDA(h, cudaMemcpyAsync(out, d_out, sizeof(int32_t) * 3 * (size_t)n, cudaMemcpyDeviceToHost, h->stream));
+        LRK_CUDA(h, cudaStreamSynchronize(h->stream));
+        return LRK_OK;
+    }
     SgdParams sp = sgd_params(h, 0.f, 0.f, 0.f, 0.0, epoch_idx);
     if (h->cfg.model == LRK_MODEL_AOBPR) {
         // the draws depend on the factor rankings: those of the current item factors (what the first window of an epoch uses)

@@ -30,6 +30,7 @@ struct LrkBuf {
 
 // model states (one translation unit: lrk_api.cu includes their headers and defines ~lrk_handle_s after them)
 struct GroupUnits; struct TcState; struct GbprState; struct SvdppState; struct AobprState; struct AlsState; struct ExactSchedule; struct DsgdState;
+struct BprRefState;
 struct MultiState;
 
 // owning pointer of a child handle of a multi-device parent (multi.cuh): lrk_destroy selects its device, syncs and deletes it
@@ -111,6 +112,8 @@ struct lrk_handle_s {
 
     // reference-order (wavefront) schedule, see sgd_exact.cuh
     std::unique_ptr<ExactSchedule> exact;
+    // reference-order BPR: the java.util.Random state and the epoch's draw and update buffers, see sgd_bpr_exact.cuh
+    std::unique_ptr<BprRefState> bprref;
 
     // single-process multi-GPU parent (multi.cuh): no device state of its own, forwards to one child per device
     std::unique_ptr<MultiState> multi;

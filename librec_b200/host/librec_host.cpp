@@ -184,6 +184,8 @@ void Randoms::seed(long long s) { g_r.setSeed(s); }
 int Randoms::uniform(int range) { return 0 + g_r.nextInt(range - 0); }
 double Randoms::uniform() { return 0.0 + (1.0 - 0.0) * g_r.nextDouble(); }
 double Randoms::gaussian(double mu, double sigma) { return mu + sigma * g_r.nextGaussian(); }
+uint64_t Randoms::state() { return g_r.seed; }
+void Randoms::setState(uint64_t s) { g_r.seed = s & ((1ULL << 48) - 1); }
 
 void DenseMatrix::init(double mean, double sigma) { for (double& v : values) v = Randoms::gaussian(mean, sigma); }
 void VectorBasedDenseVector::init(double mean, double sigma) { for (double& v : values) v = Randoms::gaussian(mean, sigma); }
@@ -310,6 +312,19 @@ void MatrixFactorizationCudaRecommender::trainModel() {
     }
     check(lrk_get_factors(handle, userFactors.values.data(), itemFactors.values.data(),
                           biased ? userBiases.values.data() : nullptr, biased ? itemBiases.values.data() : nullptr));
+}
+void BPRCudaRecommender::trainModel() {
+    const bool reference = conf.get("rec.cuda.order", "shuffled") == "reference";
+    if (reference) {
+        const double s = (double)Randoms::state();                  // < 2^48: exact
+        check(lrk_set_matrix(handle, "jdk.random.state", &s));
+    }
+    MatrixFactorizationCudaRecommender::trainModel();
+    if (reference) {
+        double s = 0.0;
+        check(lrk_get_matrix(handle, "jdk.random.state", &s));
+        Randoms::setState((uint64_t)s);
+    }
 }
 RecommendedList MatrixFactorizationCudaRecommender::recommendRank() {
     std::vector<int> all((size_t)numUsers);

@@ -55,6 +55,10 @@ public:
     static int uniform(int range);                        // Randoms.java:41-43 -> nextInt(bound)
     static double uniform();                              // Randoms.java:117-119 -> nextDouble
     static double gaussian(double mu, double sigma);      // Randoms.java:158-160 -> mu + sigma * nextGaussian
+    // the generator's 48-bit state (Random.seed of Randoms.r), handed to and taken back from the reference-order BPR epochs on the
+    // device; the cached Gaussian of nextGaussian is not part of it (BPR draws only nextInt)
+    static uint64_t state();
+    static void setState(uint64_t s);
 };
 
 // math/structure/DenseMatrix.java:20 (double[][] in Java; contiguous row-major here)
@@ -190,6 +194,9 @@ public:
     std::string simpleName() const override { return "BPRCudaRecommender"; }
 protected:
     int model() const override { return LRK_MODEL_BPR; }
+    // rec.cuda.order=reference: the device draws the samples from Randoms' own stream, continuing it where setup()'s factor init
+    // left it, and hands the state back after training (the next kcv fold's init continues the same stream)
+    void trainModel() override;
 };
 
 class RankSGDCudaRecommender : public MatrixFactorizationCudaRecommender {      // cf/ranking/RankSGDRecommender.java:37 (SURVEY 8f N3)
